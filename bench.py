@@ -5,6 +5,7 @@ BlueROV2, 64-ray radar, 5 capsules + 3 spheres).
     python bench.py [--gpus N] [--steps K] [--warmup W]                  # our arm (CUDA, through the C ABI)
     python bench.py --impl reference [--gpus N] --steps K --warmup W     # CPU arm: the oracle port on all host cores
     python bench.py --config C2|C3|C4 --scaling weak|strong ...          # the other BASELINE configs / sharding modes
+    python bench.py ... --dump-outputs DIR                               # + the last timed step's outputs as DIR/*.npy
 
 Default = config C4 with 1,048,576 envs PER GPU (weak scaling; at 8 GPUs this is config C5: 8M envs, auto-reset, one
 NCCL all-reduce of the episode statistics per rollout).  `--scaling strong` shards 1,048,576 envs TOTAL over the ranks
@@ -279,6 +280,33 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def last_step_outputs(out, n):
+    """Host copies of what env.step returned in the last timed step (obs, reward, done and the info arrays) for a fixed,
+    seeded sample of envs sized so that every file together stays within DUMP_BYTES (all envs when they fit); integer
+    and flag arrays become float64 / float32.  terminal_observation, episode_return and episode_length are only defined
+    for envs whose episode ended in that step, so their other rows are zeroed: what a layout leaves there is not an output."""
+    import torch
+    obs, reward, done, info = out
+    cols = {"obs": obs, "reward": reward, "done": done, **info}
+    per_env = 8 + sum(t[0].numel() * 8 for t in cols.values())      # bound: every value as float64, plus env_index
+    k = min(n, DUMP_BYTES // per_env)
+    idx = np.arange(n) if k == n else np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+    rows = torch.as_tensor(idx, device=obs.device)
+    arrays = {"env_index": idx.astype(np.float64)}
+    ended = done[rows].bool()
+    for name, t in cols.items():
+        t = t[rows]
+        if name in ("terminal_observation", "episode_return", "episode_length"):
+            t = t * ended.view(-1, *([1] * (t.dim() - 1))).to(t.dtype)
+        if not t.is_floating_point():
+            t = t.to(torch.float32 if name in ("done", "cond_bits") else torch.float64)
+        arrays[name] = t.cpu().numpy()
+    return arrays
+
+
 def timed_steps(env, pool, steps, dev):
     """K steps bracketed by CUDA events on the launching stream; returns (total ms, per-step ms array)."""
     import torch
@@ -367,7 +395,7 @@ def run_ours(args, rank, world, local_rank):
     reduced, n_reduces = None, 0
     evs[0].record()
     for k in range(args.steps):
-        env.step(pool[k % len(pool)])
+        out = env.step(pool[k % len(pool)])
         evs[k + 1].record()
         if world > 1 and (k + 1) % rollout == 0:
             side.wait_stream(torch.cuda.current_stream(dev))
@@ -381,6 +409,9 @@ def run_ours(args, rank, world, local_rank):
     ev_end.record()
     barrier()
     clk_timed_end = sampler.mark()
+    if args.dump_outputs and rank == 0:
+        # the step outputs are views of buffers the passes below overwrite: copied here, written at the end
+        dumped = last_step_outputs(out, N)
     total_ms = evs[0].elapsed_time(ev_end)
     step_ms = np.array([evs[k].elapsed_time(evs[k + 1]) for k in range(args.steps)])
     launches = env.launch_count() - launches0
@@ -598,6 +629,10 @@ def run_ours(args, rank, world, local_rank):
         nb = recorded_numpy_baseline(args.config)
         if nb:
             line["cpu_baseline_numpy"] = nb
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dumped.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -624,7 +659,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-strong-pass", action="store_true")
     ap.add_argument("--no-numa-bind", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (obs, reward, done, info arrays; rank 0's envs, a fixed "
+                         "sample of at most 64 MB) as DIR/<name>.npy, to compare two builds on identical inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
