@@ -195,14 +195,18 @@ __device__ __forceinline__ T cast_sphere(const T rd[3], T ocx, T ocy, T ocz, T c
 // Casts this lane's rays against the obstacles of `mask` (bit k = obstacle k, capsules first; records in shared memory
 // at pre_env + k * kPreStride), clamps (sensor.py:117), writes the 2x2 zero-padded max-pool of the distances straight into
 // the env's observation row (obs[16:], docking3d.py:487) and returns sum(max((d/d_max)^2, eps_c) * beta) on every lane.
-//   R: post-step Rzyx (row-major); poison: 0, or NaN for a non-finite pose (added to every distance so that a blown-up
-//   state poisons the radar outputs like the reference's NaN propagation does).  Must be called by all 32 lanes.
+//   R: post-step Rzyx (row-major); poison: 0, or NaN for a non-finite pose.  Must be called by all 32 lanes.
+// A non-finite pose makes every capsule test return -inf and every sphere test NaN; where no distance is positive the
+// reference takes the value of its FIRST obstacle column (docking3d.py:438-439), which is a capsule whenever the env has
+// one (-inf -> max_dist, sensor.py:117) and the sphere column otherwise (NaN).  So the poison is added to every distance
+// of sphere-only envs and to none of envs with capsules.
 template <typename T, int RPL, bool DBG, typename LANE>
 __device__ __forceinline__ T radar_env(const KParams<T> &p, const LANE &rl, const T R[9], T poison, unsigned mask,
                                        const T *pre_env, T *s_ray, int lane, int64_t ie) {
     using P2 = typename Pair<T>::type;
     const int n_caps = p.n_caps, n_sph = p.n_sph, n_r = p.n_rays;
     const T dmax = rl.dmax, inv_dmax = rl.inv_dmax;
+    if (n_caps > 0 || n_sph == 0) poison = T(0);
     T best[RPL];
 #pragma unroll
     for (int j = 0; j < RPL; j++) best[j] = Mth<T>::inf();

@@ -311,8 +311,8 @@ __device__ __forceinline__ void dynamics_env(const KParams<T> &p, const int64_t 
     w[REC_LPD] = q.r[6];
     w[REC_DD] = q.delta_d;
     w[REC_COND] = (T)q.cond;
-    // 0 for a finite pose, NaN otherwise: added to every ray distance so that a blown-up state poisons the radar
-    // outputs exactly like the reference's NaN propagation does
+    // 0 for a finite pose, NaN otherwise: such envs take the warp-per-env ray path, and radar_env poisons their ray
+    // distances where the reference's NaN propagation reaches them (envs without capsules)
     w[REC_POISON] = (((pos[0] + pos[1]) + (pos[2] + y[0])) + (y[1] + y[2])) * T(0);
 }
 
@@ -397,8 +397,8 @@ __device__ __forceinline__ bool cull_finish_env(const KParams<T> &p, const int64
             }
         }
         const CullLate<T> L = late();
-        // a non-finite pose poisons the rays like the reference's NaN propagation: such envs go through the ray launch
-        // (without obstacles every ray reads max_dist whatever the pose, docking3d.py:441)
+        // a non-finite pose goes through the warp-per-env ray path, which reproduces the reference's treatment of it
+        // (radar_env; without obstacles every ray reads max_dist whatever the pose, docking3d.py:441)
         poison_free = L.poison == T(0);
         listed = (info & 0xffffu) != 0u || (n_obst > 0 && !poison_free);
         // ---- everything that does not depend on the rays is final for EVERY env: done, condition bits, counters.

@@ -96,8 +96,8 @@ __global__ void __launch_bounds__(kWarpEnvs) step_warp_kernel(const __grid_const
         T spsi, cpsi, att[3];
         float obs16[16];
         step_dynamics<T, VEH, NU, DBG>(p, i, cy, spsi, cpsi, obs16, att);
-        // 0 for a finite pose, NaN otherwise: added to every ray distance so that a blown-up state poisons the
-        // radar outputs exactly like the reference's NaN propagation does
+        // 0 for a finite pose, NaN otherwise: radar_env poisons the ray distances with it where the reference's NaN
+        // propagation reaches them (envs without capsules)
         const T poison = (((cy.pos[0] + cy.pos[1]) + (cy.pos[2] + att[0])) + (att[1] + att[2])) * T(0);
         T *ps = s_pose + tid * kPoseStride;
 #pragma unroll

@@ -84,6 +84,8 @@ def lib():
     dp = C.POINTER(c_d)
     L.orc_ssa.restype = c_d
     L.orc_ssa.argtypes = [c_d]
+    L.orc_Rzyx.restype = None
+    L.orc_Rzyx.argtypes = [c_d, c_d, c_d, dp]
     L.orc_ray_capsule.restype = c_d
     L.orc_ray_capsule.argtypes = [dp, dp, dp, dp, c_d]
     L.orc_ray_spheres.restype = c_d
@@ -263,6 +265,29 @@ def set_env(E, state, goal, heading_goal, capsules, spheres, current, u=None, t_
     E.t_steps = int(t_steps)
     E.cum_reward = 0.0
     return E
+
+
+def copy_env(E):
+    """An independent copy of an OrcEnv (step() advances the env it is given)."""
+    out = OrcEnv()
+    C.memmove(C.byref(out), C.byref(E), C.sizeof(OrcEnv))
+    return out
+
+
+def rzyx(phi, theta, psi):
+    """geomutils.py Rzyx as the oracle evaluates it: body -> NED rotation, 3 x 3."""
+    R = np.zeros(9)
+    lib().orc_Rzyx(float(phi), float(theta), float(psi), _dp(R))
+    return R.reshape(3, 3)
+
+
+def ray_directions(P, att):
+    """World-frame unit ray directions [n_rays, 3] at attitude ``att`` (sensor.py:90-102), formed like orc_step forms
+    them (each row R rd_b / |R rd_b|, summed in the same order)."""
+    R = rzyx(*att)
+    rd_b = np.ctypeslib.as_array(P.rd_b)[:3 * P.n_rays].reshape(-1, 3)
+    v = R[:, 0] * rd_b[:, :1] + R[:, 1] * rd_b[:, 1:2] + R[:, 2] * rd_b[:, 2:3]
+    return v / np.sqrt((v * v).sum(axis=1))[:, None]
 
 
 def step(P, E, action, noise_w=0.0):
