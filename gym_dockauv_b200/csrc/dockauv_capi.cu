@@ -243,9 +243,6 @@ static void fill_kparams(const DockauvParams &s, int64_t n_envs, KParams<T> &k) 
     for (int r = 0; r < 3; r++)
         for (int c = 0; c < 3; c++)
             if (r != c && s.I_b[3 * r + c] != 0.0) sparse = false;
-#ifdef DOCKAUV_FORCE_DENSE_MINV      // tuning builds
-    sparse = false;
-#endif
     k.sparse_minv = sparse ? 1 : 0;
     // the cull code works on float records relative to the goal: every coordinate that matters is within
     // max_dist_from_goal + max_dist of it; beyond ~2 km the float rounding would eat the 2 mm slack -> exact culls
@@ -361,12 +358,6 @@ extern "C" int dockauv_create(const DockauvParams *p, int64_t n_envs, int device
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
         h->kd.sm_count = h->kf.sm_count = sms;
         h->kd.tpe_rays = h->kf.tpe_rays = (p->block_reduce == 2 && h->kd.n_rr <= 64) ? 1 : 0;
-#ifdef DOCKAUV_NO_TPE_RAYS      // tuning builds: every listed env through the warp-per-env ray launch
-        h->kd.tpe_rays = h->kf.tpe_rays = 0;
-#endif
-        // one launch group over the whole batch by default: smaller chunks would keep the records in L2 but lose more
-        // to partial waves than they gain (measured, profiles/r01/NOTES.md)
-        h->kd.chunk_envs = h->kf.chunk_envs = p->split_chunk_envs > 0 ? p->split_chunk_envs : 0;
     }
     *out = h;
     return DOCKAUV_OK;
@@ -496,12 +487,7 @@ static int step_range(DockauvHandle *h, const void *actions, int action_dtype, c
     if (e != cudaSuccess) return fail(DOCKAUV_ECUDA, "step kernel launch failed: %s", cudaGetErrorString(e));
     h->last_begins.push_back(begin);
     const bool staged = dbg == nullptr;   // else: the fused kernel
-    if (layout == DOCKAUV_LAYOUT_PIPELINE && staged) {
-        const int64_t chunk = h->kd.chunk_envs > 0 ? h->kd.chunk_envs : (end - begin);
-        h->launches += (int64_t)dockauv::pipe_launches(h->kd) * ((end - begin + chunk - 1) / chunk);
-    } else {
-        h->launches += 1;
-    }
+    h->launches += layout == DOCKAUV_LAYOUT_PIPELINE && staged ? dockauv::pipe_launches(h->kd) : 1;
     return DOCKAUV_OK;
 }
 

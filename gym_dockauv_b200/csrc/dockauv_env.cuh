@@ -324,6 +324,28 @@ __device__ __forceinline__ T reward_sum13(const T r[13]) {
     return s;
 }
 
+// obs[0:16] of env i straight to its HBM row (four 16-byte stores when n_obs allows them)
+template <typename T, typename V>
+__device__ __forceinline__ void store_obs_head(const KParams<T> &p, int64_t i, const V o[16]) {
+    if ((p.n_obs & 3) == 0) {
+        float4 *orow4 = reinterpret_cast<float4 *>(p.obs + i * p.n_obs);
+#pragma unroll
+        for (int c = 0; c < 4; c++)
+            orow4[c] = make_float4((float)o[4 * c], (float)o[4 * c + 1], (float)o[4 * c + 2], (float)o[4 * c + 3]);
+    } else {
+        float *orow = p.obs + i * p.n_obs;
+#pragma unroll
+        for (int c = 0; c < 16; c++) orow[c] = (float)o[c];
+    }
+}
+
+// 0 for a finite pose, NaN otherwise: radar_env poisons the ray distances with it where the reference's NaN propagation
+// reaches them (envs without capsules)
+template <typename T>
+__device__ __forceinline__ T pose_poison(const T pos[3], const T att[3]) {
+    return (((pos[0] + pos[1]) + (pos[2] + att[0])) + (att[1] + att[2])) * T(0);
+}
+
 // Episode statistics of one warp: each lane remembers the outcome of its env; if any episode of the warp ended,
 // a shuffle reduction folds the contributions and lane 0 issues one global atomic per non-zero statistic.
 struct WarpStats {

@@ -70,7 +70,6 @@ struct KParams {
     //   view_list / ended_list / view_count: work lists, two counters per concurrently stepped range: envs with
     //            something in view (local env index | in-view mask << 32 | condition bits << 48) for the ray launch, envs
     //            whose episode ended (local env index) for the episode-end launch
-    int64_t chunk_envs;             // > 0: the launches of a step are issued per chunk of this many envs
     T *rec;
     float4 *obsf;
     int32_t n_obsf, cull_exact;      // cull_exact: coordinates too large for the float cull -> decide everything in T
@@ -78,7 +77,7 @@ struct KParams {
     unsigned long long *view_list;
     uint32_t *ended_list;
     unsigned int *view_count;
-    int32_t counters_zeroed_at_end;  // 1: the last CTA of the episode-end launch saves and zeroes the list counters (the dynamics launch appends to the lists itself); 0: the dynamics launch zeroes them at its start
+    int32_t counters_zeroed_at_end;  // 1: the last CTA of the episode-end launch saves and zeroes the list counters (steps for which pipe_fuses_cull holds); 0: the dynamics launch zeroes them at its start
     int32_t sm_count;
     int32_t sparse_minv;             // M_inv has only the z_G pattern (diagonal + [0,4] [4,0] [1,3] [3,1]) filled in
     T *delta_d_out;

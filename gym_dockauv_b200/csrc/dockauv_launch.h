@@ -17,17 +17,14 @@ cudaError_t launch_step(const KParams<T> &k, int vehicle, int layout, cudaStream
 template <typename T>
 cudaError_t launch_reset(const KParams<T> &k, const uint8_t *mask_dev, cudaStream_t st);
 
-#ifndef DOCKAUV_FUSE_CULL
-#define DOCKAUV_FUSE_CULL 1         // pipeline layout: the cull + finish code runs inside the dynamics launch ...
-#endif
 #ifndef DOCKAUV_FUSE_MAX_OBSF
-#define DOCKAUV_FUSE_MAX_OBSF 20    // ... when an env has at most this many float4 obstacle records: 80 KB of shared memory per 256-thread CTA, two CTAs per SM stay resident
+#define DOCKAUV_FUSE_MAX_OBSF 20    // pipeline layout: the cull + finish code runs inside the dynamics launch when an env has at most this many float4 obstacle records: 80 KB of shared memory per 256-thread CTA, two CTAs per SM stay resident
 #endif
 // whether the dynamics launch of the pipeline layout takes the cull + finish code in, and how many launches one step over
 // one env range is
 template <typename T>
 inline bool pipe_fuses_cull(const KParams<T> &k) {
-    return DOCKAUV_FUSE_CULL && k.n_caps + k.n_sph > 0 && !k.cull_exact && k.n_obsf > 0 && k.n_obsf <= DOCKAUV_FUSE_MAX_OBSF;
+    return k.n_caps + k.n_sph > 0 && !k.cull_exact && k.n_obsf > 0 && k.n_obsf <= DOCKAUV_FUSE_MAX_OBSF;
 }
 template <typename T>
 inline int pipe_launches(const KParams<T> &k) {

@@ -295,4 +295,26 @@ __device__ __forceinline__ T radar_env(const KParams<T> &p, const LANE &rl, cons
     return oa_dot;
 }
 
+// env i with nothing in view: every ray reads max_dist (sensor.py:113-117), so its pooled cells are all ones
+template <typename T>
+__device__ __forceinline__ void store_clear_cells(const KParams<T> &p, int64_t i) {
+    float *cells = p.obs + i * p.n_obs + 16;
+    if ((p.n_obs & 3) == 0 && (p.n_rr & 3) == 0) {
+        float4 *c4 = reinterpret_cast<float4 *>(cells);
+        for (int c = 0; c < (p.n_rr >> 2); c++) c4[c] = make_float4(1.0f, 1.0f, 1.0f, 1.0f);
+    } else {
+        for (int c = 0; c < p.n_rr; c++) cells[c] = 1.0f;
+    }
+}
+
+// obstacle k of env i as stored (capsules first, then sphere k - n_caps), zero-filled to seven words
+template <typename T>
+__device__ __forceinline__ void load_obstacle(const KParams<T> &p, int64_t i, int k, T o7[7]) {
+    const int64_t N = p.n_envs;
+    const bool is_cap = k < p.n_caps;
+    const T *g = is_cap ? p.capsules + (int64_t)(k * 7) * N + i : p.spheres + (int64_t)((k - p.n_caps) * 4) * N + i;
+#pragma unroll
+    for (int c = 0; c < 7; c++) o7[c] = (c < 4 || is_cap) ? g[(int64_t)c * N] : T(0);
+}
+
 }  // namespace dockauv

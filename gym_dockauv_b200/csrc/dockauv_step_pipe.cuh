@@ -4,16 +4,16 @@
 //      + cull        obs[0:16], done conditions 0..2, the reward terms that need no radar -- a 16-word record per env
 //      + finish      (post-step attitude sines / cosines, position relative to the goal, the reward terms already combined
 //                   in numpy's summation order, delta_d, condition bits) that stays in REGISTERS for the second half of the
-//                   thread (FUSE): the walk over the env's obstacles in FLOAT (float4 records relative to the goal, written
-//                   at reset, waiting in shared memory since the start of the thread; cull_pair_rec): body collision
-//                   (re-decided in T when within 2 mm of the threshold) and the range / field-of-view culls.  Envs with
-//                   something in view (24 % on the C4 workload) are appended to a compact list and their record goes to
-//                   KParams::rec.  Done flag, condition bits and counters are final here for EVERY env (coalesced stores);
-//                   an env with nothing in view is finished completely -- all ray cells read max_dist, r_oa = 0: reward,
-//                   running return, statistics -- and goes on a second list if its episode ended.
-//                   (Obstacle-free scenarios: FIN, the env is finished right after the dynamics.  More float records than
-//                   fit in shared memory, or coordinates too large for them: the cull + finish code runs as a launch of its
-//                   own, cull_finish_kernel, on records read back from KParams::rec.)
+//                   thread (FINISH): the walk over the env's obstacles in FLOAT (float4 records relative to the goal,
+//                   written at reset, waiting in shared memory since the start of the thread; cull_pair_rec): body
+//                   collision (re-decided in T when within 2 mm of the threshold) and the range / field-of-view culls.
+//                   Envs with something in view (24 % on the C4 workload) are appended to a compact list and their record
+//                   goes to KParams::rec.  Done flag, condition bits and counters are final here for EVERY env (coalesced
+//                   stores); an env with nothing in view is finished completely -- all ray cells read max_dist, r_oa = 0:
+//                   reward, running return, statistics -- and goes on a second list if its episode ended.
+//                   (Obstacle-free scenarios: the same code with no obstacle to walk over finishes every env.  More float
+//                   records than fit in shared memory, or coordinates too large for them: the cull + finish code runs as a
+//                   launch of its own, cull_finish_kernel, on records read back from KParams::rec.)
 //   2. rays+finish  rays_thread_kernel: persistent grid.  The listed envs with one or two obstacles in view with LANES =
 //                   ENVS (tiles of 128), the others by one warp each (lanes = rays, next entry in flight while the current
 //                   one is cast; radar_env, dockauv_rays.cuh) on the first CTAs of the same launch; then the reward with its
@@ -48,15 +48,6 @@ constexpr int kDynThreads = DOCKAUV_DYN_THREADS;
 #endif
 #ifndef DOCKAUV_TPE_WARP_CTAS_PER_SM
 #define DOCKAUV_TPE_WARP_CTAS_PER_SM 1   // CTAs per SM of that launch that run the warp-per-env loop over class 3
-#endif
-#ifndef DOCKAUV_TPE_SPLIT
-#define DOCKAUV_TPE_SPLIT 1         // lanes per env in the thread-per-env ray launch (each takes a run of pooled cells; 2: +8 %, 4: +11 % time)
-#endif
-#ifndef DOCKAUV_CULL_PREFETCH
-#define DOCKAUV_CULL_PREFETCH 1     // (without staging) L2 prefetch of the records
-#endif
-#ifndef DOCKAUV_TPE_BODY
-#define DOCKAUV_TPE_BODY 1          // thread-per-env ray tiles: obstacle records rotated into the body frame once instead of every ray into NED
 #endif
 #ifndef DOCKAUV_MINB_RAYS
 #define DOCKAUV_MINB_RAYS 6         // ray launch: (128, 6) = 80 registers, 24 warps per SM
@@ -119,19 +110,12 @@ struct RecIO<float> {
     }
 };
 
-#ifndef DOCKAUV_PDL
-#define DOCKAUV_PDL 1               // ray and episode-end launches as programmatic dependents of the launch before them
-#endif
 // Launch as a PROGRAMMATIC DEPENDENT of the previous launch in the stream: the grid is set up while that launch drains and
 // its threads wait in grid_dependency_wait() until everything the previous launch wrote is visible (no launch before it
 // triggers early, so the wait is for its completion; an early trigger at the top of the launch before -- dependents set up
 // during its last wave -- measured no faster).  What it saves is part of the launch-to-launch gap: 22.5 -> 22.3 us per
 // 65,536-env SimpleDocking3d step, 0.391 -> 0.390 ms per 1M-env C4 step.
-__device__ __forceinline__ void grid_dependency_wait() {
-#if DOCKAUV_PDL
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-#endif
-}
+__device__ __forceinline__ void grid_dependency_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 // one word global -> shared without a register in between (completion: cp_async_wait_all); dst = shared-window address
 template <typename T>
 __device__ __forceinline__ void cp_async_word(unsigned dst_shared, const T *src) {
@@ -165,22 +149,18 @@ __device__ __forceinline__ T step_reward(const KParams<T> &p, T A, T B, T r7, T 
 
 // ------------------------------------------------------------------------------------------------------- 1. dynamics
 // CUR: the ocean current is evaluated (scenario with a current, injected current or noise); SPM: sparse M_inv / C / G;
-// FIN: the scenario has no obstacles -- every ray reads max_dist and nothing can collide, so the env is finished right
-// here (reward, done, counters, statistics, all-ones ray cells; no record, no cull / ray launch);
-// FUSE: the cull + finish code (section 2) runs in this launch, on the record while it is still in registers.
+// FINISH: the cull + finish code (section 2) runs in this launch, on the record while it is still in registers (scenarios
+// without obstacles too: every ray reads max_dist and nothing can collide, so every env is finished here).
 
 // shared memory of one dynamics CTA: park[kParkWords][kDynThreads] words of T that are only needed after the integration
-// (position, goal; FIN / FUSE: running return, step counter), filled by cp.async into the thread's own slots -- no register
+// (position, goal; FINISH: running return, step counter), filled by cp.async into the thread's own slots -- no register
 // during the integration and no memory round trip after it
 constexpr int kParkWords = 8;
 
-// one env of the dynamics launch.  FIN: the env is finished here (steps_here: env-steps this call accounts for in the
-// statistics -- the callers pass the CTA's count from one thread, 0 from the others).  Otherwise the env's record is left
-// in w[kRecWords] and its post-step position in pos[3].
+// one env of the dynamics launch: the env's record is left in w[kRecWords] and its post-step position in pos[3].
 //   stage(): the caller's own cp.async copies for this env (issued after the plain loads)
-template <typename T, int VEH, int NU, bool CUR, bool SPM, bool FIN, bool LATE, typename STAGE>
-__device__ __forceinline__ void dynamics_env(const KParams<T> &p, const int64_t i, const int steps_here, T *dyn_park, T w[kRecWords],
-                                             T pos[3], STAGE stage) {
+template <typename T, int VEH, int NU, bool CUR, bool SPM, typename STAGE>
+__device__ __forceinline__ void dynamics_env(const KParams<T> &p, const int64_t i, T *dyn_park, T w[kRecWords], T pos[3], STAGE stage) {
     const int64_t N = p.n_envs;
     // ---- what the integration starts from goes first: plain loads; the asynchronous copies of everything that is needed
     //      later queue up behind them (issued ahead of the loads, the 21 copies of a thread delayed its first use of a loaded
@@ -197,10 +177,6 @@ __device__ __forceinline__ void dynamics_env(const KParams<T> &p, const int64_t 
         for (int c = 0; c < 3; c++) cp_async_word<T>(sa + c * kPlane, p.state + (int64_t)c * N + i);
 #pragma unroll
         for (int c = 0; c < 3; c++) cp_async_word<T>(sa + (3 + c) * kPlane, p.goal + (int64_t)c * N + i);
-        if (LATE) {
-            cp_async_word<T>(sa + 6 * kPlane, p.ep_return + i);
-            cp_async_word<int32_t>(sa + 7 * kPlane, p.t_steps + i);
-        }
     }
     stage();
     T tr0[6];
@@ -237,70 +213,11 @@ __device__ __forceinline__ void dynamics_env(const KParams<T> &p, const int64_t 
 
     DynOut<T> q;
     dyn_outputs<T>(p, pos, y, tr1, goal, nu_c, penalty, q);
-    // obs[0:16] goes straight to its HBM row (four 16-byte stores); a later launch zeroes the row if the env is reset
-    if ((p.n_obs & 3) == 0) {
-        float4 *orow4 = reinterpret_cast<float4 *>(p.obs + i * p.n_obs);
-#pragma unroll
-        for (int c = 0; c < 4; c++)
-            orow4[c] = make_float4((float)q.o[4 * c], (float)q.o[4 * c + 1], (float)q.o[4 * c + 2], (float)q.o[4 * c + 3]);
-    } else {
-        float *orow = p.obs + i * p.n_obs;
-#pragma unroll
-        for (int c = 0; c < 16; c++) orow[c] = (float)q.o[c];
-    }
+    // a later launch zeroes the row if the env is reset
+    store_obs_head<T>(p, i, q.o);
     // np.sum of the 13 reward terms is ((r0+r1)+(r2+r3)) + ((r4+r5)+(r6+r7)) + r8 + .. + r12 (reward_sum13): the two
     // sums that need no radar are formed here, in that order
     const T A = (q.r[0] + q.r[1]) + (q.r[2] + q.r[3]), B = q.r[4] + q.r[5];
-    if (FIN) {
-        // ---- every ray reads max_dist (docking3d.py:441, sensor.py:113-117) -> pooled cells all ones, r_oa = 0
-        float *cells = p.obs + i * p.n_obs + 16;
-        if ((p.n_obs & 3) == 0 && (p.n_rr & 3) == 0) {
-            float4 *c4 = reinterpret_cast<float4 *>(cells);
-            for (int c = 0; c < (p.n_rr >> 2); c++) c4[c] = make_float4(1.0f, 1.0f, 1.0f, 1.0f);
-        } else {
-            for (int c = 0; c < p.n_rr; c++) cells[c] = 1.0f;
-        }
-        const int32_t t_steps = reinterpret_cast<const int32_t *>(dyn_park + 7 * kDynThreads + threadIdx.x)[0];
-        const T ep_before = dyn_park[6 * kDynThreads + threadIdx.x];
-        const uint32_t cond = done_conditions<T>(p, q.cond, t_steps, false);
-        const bool done = cond != 0;
-        const int32_t t_new = t_steps + 1;
-        const T r_oa = p.sum_beta_oa / p.sum_beta_oa - T(1);
-        const T reward = step_reward<T>(p, A, B, q.r[7], q.r[6], r_oa, cond);
-        const T ep_ret = ep_before + reward;
-        p.reward[i] = reward;
-        p.done[i] = done ? 1 : 0;
-        if (p.cond_bits) p.cond_bits[i] = (uint8_t)cond;
-        if (p.delta_d_out) p.delta_d_out[i] = q.delta_d;
-        WarpStats bs;
-        if (done) {
-            if (p.ep_len_out) p.ep_len_out[i] = t_new;
-            if (p.ep_return_out) p.ep_return_out[i] = ep_ret;
-            bs.done = true;
-            bs.cond = cond;
-            bs.length = t_new;
-            bs.ep_return = (double)ep_ret;
-            bs.delta_d = (double)q.delta_d;
-            bs.nan = reward != reward;
-        }
-        if (!(done && p.auto_reset)) {
-            p.ep_return[i] = ep_ret;
-            p.t_steps[i] = t_new;
-        }
-        {   // ended episodes -> the list of the episode-end launch (aggregated over the lanes that are still here)
-            const unsigned am = __activemask();
-            const unsigned em = __ballot_sync(am, done);
-            if (em) {
-                const int lane = threadIdx.x & 31, leader = __ffs(am) - 1;
-                unsigned base = 0;
-                if (lane == leader) base = atomicAdd(&p.view_count[3], (unsigned)__popc(em));
-                base = __shfl_sync(am, base, leader);
-                if (done) p.ended_list[base + __popc(em & ((1u << lane) - 1u))] = (uint32_t)(i - p.env_begin);
-            }
-        }
-        bs.flush_direct(p.stats, steps_here);
-        return;
-    }
 #pragma unroll
     for (int c = 0; c < 6; c++) w[REC_TRIG + c] = tr1[c];
 #pragma unroll
@@ -311,9 +228,8 @@ __device__ __forceinline__ void dynamics_env(const KParams<T> &p, const int64_t 
     w[REC_LPD] = q.r[6];
     w[REC_DD] = q.delta_d;
     w[REC_COND] = (T)q.cond;
-    // 0 for a finite pose, NaN otherwise: such envs take the warp-per-env ray path, and radar_env poisons their ray
-    // distances where the reference's NaN propagation reaches them (envs without capsules)
-    w[REC_POISON] = (((pos[0] + pos[1]) + (pos[2] + y[0])) + (y[1] + y[2])) * T(0);
+    // envs with a non-finite pose take the warp-per-env ray path
+    w[REC_POISON] = pose_poison<T>(pos, y);
 }
 
 // ------------------------------------------------------------------------------------------------------- 2. cull + finish
@@ -368,10 +284,7 @@ __device__ __forceinline__ bool cull_finish_env(const KParams<T> &p, const int64
                 if (hit3 == 2) {      // within 2 mm of the collision threshold (or NaN): decided in T like the other layouts
                     T pos[3], o7[7];
                     pos_of(pos);
-                    const T *g = is_cap ? p.capsules + (int64_t)(k * 7) * N + i : p.spheres + (int64_t)((k - n_caps) * 4) * N + i;
-                    const int n_words = is_cap ? 7 : 4;
-#pragma unroll
-                    for (int c = 0; c < 7; c++) o7[c] = c < n_words ? g[(int64_t)c * N] : T(0);
+                    load_obstacle<T>(p, i, k, o7);
                     hit = obstacle_body_hit<T>(p, pos, o7, is_cap);
                 }
                 info |= view ? (1u << k) : 0u;
@@ -386,10 +299,7 @@ __device__ __forceinline__ bool cull_finish_env(const KParams<T> &p, const int64
             for (int k = 0; k < n_obst; k++) {
                 const bool is_cap = k < n_caps;
                 T o7[7];
-                const T *g = is_cap ? p.capsules + (int64_t)(k * 7) * N + i : p.spheres + (int64_t)((k - n_caps) * 4) * N + i;
-                const int n_words = is_cap ? 7 : 4;
-#pragma unroll
-                for (int c = 0; c < 7; c++) o7[c] = c < n_words ? g[(int64_t)c * N] : T(0);
+                load_obstacle<T>(p, i, k, o7);
                 bool hit, view;
                 obstacle_pair<T, false>(p, pos, Rm, o7, is_cap, nullptr, hit, view);
                 info |= view ? (1u << k) : 0u;
@@ -418,14 +328,8 @@ __device__ __forceinline__ bool cull_finish_env(const KParams<T> &p, const int64
         if (listed) {
             p.t_steps[i] = t_new;        // the ray launch reads it back (and zeroes it if it re-initialises the env)
         } else {
-            // ---- nothing in view: every ray reads max_dist (sensor.py:113-117) -> pooled cells all ones, r_oa = 0
-            float *cells = p.obs + i * p.n_obs + 16;
-            if ((p.n_obs & 3) == 0 && (p.n_rr & 3) == 0) {
-                float4 *c4 = reinterpret_cast<float4 *>(cells);
-                for (int c = 0; c < (p.n_rr >> 2); c++) c4[c] = make_float4(1.0f, 1.0f, 1.0f, 1.0f);
-            } else {
-                for (int c = 0; c < p.n_rr; c++) cells[c] = 1.0f;
-            }
+            // ---- nothing in view: pooled cells all ones, r_oa = 0
+            store_clear_cells<T>(p, i);
             const T ep_ret = L.ep_return + reward;
             if (done) {
                 if (p.ep_return_out) p.ep_return_out[i] = ep_ret;
@@ -472,38 +376,38 @@ __device__ __forceinline__ bool cull_finish_env(const KParams<T> &p, const int64
     return listed;
 }
 
-// ---- the dynamics launch (with the cull + finish code in it when FUSE)
-// FUSE: the env's float obstacle records travel global -> shared by cp.async at the very start ([slot][thread], dynamic
-// shared memory: 16 n_obsf bytes per thread) and wait there through the integration; the record never leaves the registers
-// unless the env ends up on a view list.  Against the separate cull launch this saves the record's round trip through HBM
-// (128 B written for every env, 128 B read back) and every memory wait of the obstacle loop.
-template <typename T, int VEH, int NU, bool CUR, bool SPM, bool FIN, bool FUSE>
-__global__ void
-#ifdef DOCKAUV_DYN_MAXNREG
-__maxnreg__(DOCKAUV_DYN_MAXNREG)
-#else
-__launch_bounds__(kDynThreads, DOCKAUV_MINB_A)
-#endif
-dynamics_kernel(const __grid_constant__ KParams<T> p) {
-    extern __shared__ __align__(16) unsigned char dyn_smem[];      // FUSE: float4 [n_obsf][kDynThreads]
+// ---- the dynamics launch (with the cull + finish code in it when FINISH)
+// FINISH: the env's running return, step counter and float obstacle records travel global -> shared by cp.async at the
+// very start (records: [slot][thread], dynamic shared memory: 16 n_obsf bytes per thread) and wait there through the
+// integration; the record never leaves the registers unless the env ends up on a view list.  Against the separate cull
+// launch this saves the record's round trip through HBM (128 B written for every env, 128 B read back) and every memory
+// wait of the obstacle loop.
+template <typename T, int VEH, int NU, bool CUR, bool SPM, bool FINISH>
+__global__ void __launch_bounds__(kDynThreads, DOCKAUV_MINB_A) dynamics_kernel(const __grid_constant__ KParams<T> p) {
+    extern __shared__ __align__(16) unsigned char dyn_smem[];      // FINISH: float4 [n_obsf][kDynThreads]
     __shared__ __align__(8) T dyn_park[kParkWords * kDynThreads];
     const int64_t i0 = p.env_begin + (int64_t)blockIdx.x * kDynThreads;
     const int64_t i = i0 + threadIdx.x;
     const bool active = i < p.env_end;
     prefetch_dynamics_inputs<T, NU>(p, i, threadIdx.x & 31, true);
     T w[kRecWords], pos[3];
-    if (!FUSE) {
-        // the cull launch appends to the lists: this launch empties them
-        if (blockIdx.x == 0 && threadIdx.x < kListCounters) p.view_count[threadIdx.x] = 0u;
+    // a launch after this one appends to the lists: this launch empties them, unless the episode-end launch does.
+    // Without obstacles this launch appends to them itself: block 0 zeroes the counters long before any other block has
+    // finished its integration, which CUDA does not guarantee to be ordered (DESIGN.md section 8)
+    if (!(FINISH && p.counters_zeroed_at_end) && blockIdx.x == 0 && threadIdx.x < kListCounters) p.view_count[threadIdx.x] = 0u;
+    if (!FINISH) {
         if (!active) return;
-        dynamics_env<T, VEH, NU, CUR, SPM, FIN, FIN>(p, i, threadIdx.x == 0 ? (int)min((int64_t)kDynThreads, p.env_end - i0) : 0, dyn_park, w, pos,
-                                                     []() {});
-        if (!FIN) RecIO<T>::store(p.rec + i * kRecWords, w);
+        dynamics_env<T, VEH, NU, CUR, SPM>(p, i, dyn_park, w, pos, []() {});
+        RecIO<T>::store(p.rec + i * kRecWords, w);
         return;
     }
     const float4 *s_obs = reinterpret_cast<const float4 *>(dyn_smem) + threadIdx.x;
     if (active) {
-        dynamics_env<T, VEH, NU, CUR, SPM, false, true>(p, i, 0, dyn_park, w, pos, [&]() {
+        dynamics_env<T, VEH, NU, CUR, SPM>(p, i, dyn_park, w, pos, [&]() {
+            const unsigned sp = (unsigned)__cvta_generic_to_shared(dyn_park + threadIdx.x);
+            constexpr unsigned kPlane = kDynThreads * (unsigned)sizeof(T);
+            cp_async_word<T>(sp + 6 * kPlane, p.ep_return + i);
+            cp_async_word<int32_t>(sp + 7 * kPlane, p.t_steps + i);
             const unsigned sa = (unsigned)__cvta_generic_to_shared(s_obs);
             for (int sl = 0; sl < p.n_obsf; sl++)
                 asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa + (unsigned)(sl * kDynThreads * 16)),
@@ -543,10 +447,8 @@ __global__ void __launch_bounds__(kCullThreads, DOCKAUV_MINB_CULL) cull_finish_k
 #pragma unroll
     for (int c = 0; c < 10; c++) w[c] = T(0);
     if (active) {
-#if DOCKAUV_CULL_PREFETCH
         if (!p.cull_exact)
             for (int sl = 0; sl < p.n_obsf; sl++) asm volatile("prefetch.global.L2 [%0];" ::"l"(p.obsf + (int64_t)sl * N + i));
-#endif
         RecIO<T>::template load<0, 5>(rec, w);       // trig, prel, A
         const unsigned sa = (unsigned)__cvta_generic_to_shared(cull_park) + (unsigned)threadIdx.x * 16u;
         constexpr unsigned kPlane = kCullThreads * 16u;
@@ -619,6 +521,22 @@ struct RaysSmem {
 #endif
 constexpr int kRayWarps = DOCKAUV_RAY_WARPS;     // warps per CTA of the ray launch
 
+// what the cull code left open for a listed env: the reward with its obstacle-avoidance term (oa_dot: the env's weighted
+// sum, docking3d.py:767-792) and the running return, stored when `store`.  Returns the reward, the new return in ep_ret.
+template <typename T>
+__device__ __forceinline__ T finish_listed(const KParams<T> &p, int64_t ie, uint32_t cond, T oa_dot, T A, T B, T r7, T lp_d,
+                                           T ep_before, bool store, T &ep_ret) {
+    const T r_oa = p.sum_beta_oa / oa_dot - T(1);      // docking3d.py:792 (IEEE division: the other layouts' bits)
+    const T reward = step_reward<T>(p, A, B, r7, lp_d, r_oa, cond);
+    ep_ret = ep_before + reward;
+    if (store) {
+        const bool done = cond != 0;
+        p.reward[ie] = reward;
+        if (done && p.ep_return_out) p.ep_return_out[ie] = ep_ret;
+        if (!(done && p.auto_reset)) p.ep_return[ie] = ep_ret;
+    }
+    return reward;
+}
 
 // the loop of ONE warp over the class-3 list: warp w_global of n_warps (called by all 32 lanes; smem_raw = the CTA's
 // dynamic shared memory, kRayWarps * RaysSmem::warp_words words)
@@ -699,17 +617,11 @@ __device__ __forceinline__ void rays_warp_loop(const KParams<T> &p, unsigned cha
         // ---- cast rays against the in-view obstacles, pooled cells to the observation row
         const T oa_dot = radar_env<T, RPL, false, RayLaneShared<T, RPL>>(p, rl, R, poison, mask, s_pre, s_ray, lane, ie);
 
-        // ---- what the cull code left open: the reward with its obstacle-avoidance term and the running return
-        //      (every lane computes the same values from the staged record, lane 0 stores)
-        const T r_oa = p.sum_beta_oa / oa_dot - T(1);      // docking3d.py:792 (IEEE division: the other layouts' bits)
-        const T reward = step_reward<T>(p, s_ent[REC_A], s_ent[REC_B], s_ent[REC_R7], s_ent[REC_LPD], r_oa, cond);
-        const T ep_ret = s_ent[19] + reward;
+        // ---- reward and running return (every lane computes the same values from the staged record, lane 0 stores)
+        T ep_ret;
+        const T reward = finish_listed<T>(p, ie, cond, oa_dot, s_ent[REC_A], s_ent[REC_B], s_ent[REC_R7], s_ent[REC_LPD], s_ent[19],
+                                          lane == 0, ep_ret);
         const bool done = cond != 0;
-        if (lane == 0) {
-            p.reward[ie] = reward;
-            if (done && p.ep_return_out) p.ep_return_out[ie] = ep_ret;
-            if (!(done && p.auto_reset)) p.ep_return[ie] = ep_ret;
-        }
         if (done) {       // warp-uniform, ~1 % of the listed envs
             const int32_t t_new = reinterpret_cast<const int32_t *>(s_ent + 20)[0];     // already incremented by the cull code
             double mine = 0.0;
@@ -739,24 +651,23 @@ __global__ void __launch_bounds__(kRayWarps * 32, DOCKAUV_MINB_RAYS * 4 / kRayWa
 
 // ------------------------------------------------------------------------------------------------------- 3b. rays, thread per env
 // The envs with exactly one or two obstacles in view -- nine in ten of the listed ones -- with LANES = ENVS: every lane
-// walks over the rays of its own env (SPLIT lanes share one env, each takes a contiguous run of pooled cells), the
-// ray-test records of its obstacles stay in registers.  Against the warp-per-env mapping, everything that is per-env
-// scalar work there (list entry, record fetch, Rzyx, obstacle records, reward: ~450 of its ~600 warp instructions per env,
-// done by 32 lanes redundantly) is amortised over the envs of a warp here.  The ray tests are straight-line code
-// (cast_capsule_bf; spheres take the same path as degenerate capsules, so lanes never diverge on the obstacle type) and
-// the four rays of a pooled cell are independent chains the compiler interleaves.  The body-frame ray table is walked in
-// pooled-cell order (shared memory), so a cell's maximum is complete after four rays and goes straight into the
-// observation row.  One persistent launch covers both classes: tiles of class 2 (the longer ones) first, then class 1.
+// walks over the rays of its own env, the ray-test records of its obstacles stay in registers.  Against the
+// warp-per-env mapping, everything that is per-env scalar work there (list entry, record fetch, Rzyx, obstacle records,
+// reward: ~450 of its ~600 warp instructions per env, done by 32 lanes redundantly) is amortised over the envs of a
+// warp here.  The ray tests are straight-line code (cast_capsule_bf; spheres take the same path as degenerate capsules,
+// so lanes never diverge on the obstacle type) and the four rays of a pooled cell are independent chains the compiler
+// interleaves.  The body-frame ray table is walked in pooled-cell order (shared memory), so a cell's maximum is
+// complete after four rays and goes straight into the observation row.  One persistent launch covers both classes:
+// tiles of class 2 (the longer ones) first, then class 1.
 constexpr int kTpeThreads = kRayWarps * 32;      // one CTA shape for both ray mappings of the launch
 constexpr int kTpeMaxCells = 64;      // pooled cells the shared ray table holds
+constexpr int kTpeTabWords = kTpeMaxCells * 4 * 4;
 
-template <typename T, int NOB, int SPLIT>
+template <typename T, int NOB>
 __device__ __forceinline__ void rays_thread_tile(const KParams<T> &p, const T *s_tab, unsigned tile, unsigned count) {
     const int64_t N = p.n_envs;
     const int n_rr = p.n_rr;
-    const unsigned tg = tile * kTpeThreads + threadIdx.x;
-    const unsigned eidx = tg / SPLIT;
-    const int part = (int)(tg % SPLIT);
+    const unsigned eidx = tile * kTpeThreads + threadIdx.x;
     const bool valid = eidx < count;
     const unsigned long long entry = valid ? p.view_list[(int64_t)(NOB - 1) * N + eidx] : 0ull;
     const int64_t ie = p.env_begin + (int64_t)(uint32_t)entry;
@@ -778,15 +689,12 @@ __device__ __forceinline__ void rays_thread_tile(const KParams<T> &p, const T *s
             mask &= mask - 1;
             const bool is_cap = k < p.n_caps;
             sph[o] = !is_cap;
-            const T *g = is_cap ? p.capsules + (int64_t)(k * 7) * N + ie : p.spheres + (int64_t)((k - p.n_caps) * 4) * N + ie;
             T ob[7];
-#pragma unroll
-            for (int c = 0; c < 7; c++) ob[c] = (c < 4 || is_cap) ? g[(int64_t)c * N] : T(0);
+            load_obstacle<T>(p, ie, k, ob);
 #pragma unroll
             for (int c = 0; c < 11; c++) w[o][c] = T(0);
             obstacle_ray_record<T>(pos, ob, is_cap, w[o]);
             if (!is_cap) sphere_as_capsule<T>(w[o]);
-#if DOCKAUV_TPE_BODY
             // the record's two vectors into the BODY frame (R^T v): a ray direction then is its table entry as it stands,
             // (R b) . v = b . (R^T v) -- 18 products per obstacle instead of 9 per ray
 #pragma unroll
@@ -795,38 +703,25 @@ __device__ __forceinline__ void rays_thread_tile(const KParams<T> &p, const T *s
 #pragma unroll
                 for (int c = 0; c < 3; c++) w[o][3 * v + c] = R[c] * x + R[3 + c] * y + R[6 + c] * z;
             }
-#endif
         }
     }
     T h_min[NOB];      // see cast_capsule_bf
 #pragma unroll
     for (int o = 0; o < NOB; o++) h_min[o] = sph[o] ? -Mth<T>::min_normal() : T(0);
-    // ---- this lane's run of pooled cells: multiples of four, so the row is written in 16-byte pieces
-    const int cpp = (((n_rr + SPLIT - 1) / SPLIT) + 3) & ~3;
-    const int c_begin = part * cpp;
     const T dmax = p.radar_max_dist, inv_dmax = T(1) / dmax;
     float *orow = p.obs + ie * p.n_obs + 16;
-    const bool vec_row = (p.n_obs & 3) == 0 && (n_rr & 3) == 0;
-    T oa_part = T(0);
+    const bool vec_row = (p.n_obs & 3) == 0 && (n_rr & 3) == 0;      // the row is written in 16-byte pieces
+    T oa_dot = T(0);
     float o4[4] = {0.0f, 0.0f, 0.0f, 0.0f};
-    // (every lane runs all cpp trips: cast_capsule_bf contains a warp vote; cells beyond the grid are computed and dropped)
+    // (every lane runs all trips, valid or not: cast_capsule_bf contains a warp vote)
 #pragma unroll 1
-    for (int cc = 0; cc < cpp; cc++) {
-        const bool live = c_begin + cc < n_rr;
-        const int cell = live ? c_begin + cc : 0;
+    for (int cell = 0; cell < n_rr; cell++) {
         T dq[4], bwq[4];
 #pragma unroll
         for (int q = 0; q < 4; q++) {
             const T *tb = s_tab + 4 * (4 * cell + q);
-            const T b0 = tb[0], b1 = tb[1], b2 = tb[2];
+            const T rd[3] = {tb[0], tb[1], tb[2]};
             bwq[q] = tb[3];
-            T rd[3];
-#if DOCKAUV_TPE_BODY
-            rd[0] = b0; rd[1] = b1; rd[2] = b2;
-#else
-#pragma unroll
-            for (int c = 0; c < 3; c++) rd[c] = R[3 * c] * b0 + R[3 * c + 1] * b1 + R[3 * c + 2] * b2;
-#endif
             T best = Mth<T>::inf();
 #pragma unroll
             for (int o = 0; o < NOB; o++) {
@@ -838,40 +733,29 @@ __device__ __forceinline__ void rays_thread_tile(const KParams<T> &p, const T *s
         T mx = T(0);                                  // block_reduce pads with cval = 0 (sensor.py:131-137)
 #pragma unroll
         for (int q = 0; q < 4; q++) {
-            if (bwq[q] < T(0) || !live) continue;     // padding slot of the ray table: no ray
-            // obstacle-avoidance partial sum (docking3d.py:767-792), 2x2 max-pool
+            if (bwq[q] < T(0)) continue;              // padding slot of the ray table: no ray
+            // obstacle-avoidance sum (docking3d.py:767-792), 2x2 max-pool
             const T x = dq[q] * inv_dmax;
             const T qq = x * x;
             const T mq = !(qq <= T(0.001)) ? qq : T(0.001);     // np.maximum, NaN propagates
-            oa_part += mq * bwq[q];
+            oa_dot += mq * bwq[q];
             mx = !(dq[q] <= mx) ? dq[q] : mx;         // np.max, NaN propagates
         }
         T o = mx * inv_dmax;                          // clip(d / max_dist, 0, 1), docking3d.py:487
         o = o > T(1) ? T(1) : o;
         if (vec_row) {
             o4[cell & 3] = (float)o;
-            if ((cell & 3) == 3 && valid && live) reinterpret_cast<float4 *>(orow)[cell >> 2] = make_float4(o4[0], o4[1], o4[2], o4[3]);
-        } else if (valid && live) {
+            if ((cell & 3) == 3 && valid) reinterpret_cast<float4 *>(orow)[cell >> 2] = make_float4(o4[0], o4[1], o4[2], o4[3]);
+        } else if (valid) {
             orow[cell] = (float)o;
         }
     }
-    // ---- the env's obstacle-avoidance sum: add up the SPLIT lanes of the env
-    T oa_dot = oa_part;
-#pragma unroll
-    for (int s = 1; s < SPLIT; s <<= 1) oa_dot += __shfl_xor_sync(0xffffffffu, oa_dot, s);
-    if (valid && part == 0) {
-        // ---- what the cull code left open: the reward with its obstacle-avoidance term and the running return
+    if (valid) {
         T wf[6];
         RecIO<T>::template load<4, 3>(rec, wf);       // prel_z, A, B, r7, lp_d, delta_d
-        const T ep_before = p.ep_return[ie];
-        const T r_oa = p.sum_beta_oa / oa_dot - T(1);      // docking3d.py:792
-        const T reward = step_reward<T>(p, wf[1], wf[2], wf[3], wf[4], r_oa, cond);
-        const T ep_ret = ep_before + reward;
-        const bool done = cond != 0;
-        p.reward[ie] = reward;
-        if (done && p.ep_return_out) p.ep_return_out[ie] = ep_ret;
-        if (!(done && p.auto_reset)) p.ep_return[ie] = ep_ret;
-        if (done) {      // ~1 % of the listed envs
+        T ep_ret;
+        const T reward = finish_listed<T>(p, ie, cond, oa_dot, wf[1], wf[2], wf[3], wf[4], p.ep_return[ie], true, ep_ret);
+        if (cond != 0) {      // ~1 % of the listed envs
             WarpStats bs;
             bs.done = true;
             bs.cond = cond;
@@ -888,10 +772,10 @@ __device__ __forceinline__ void rays_thread_tile(const KParams<T> &p, const T *s
 // One launch for all three classes: the first `warp_ctas` CTAs run the warp-per-env loop over class 3 (few entries, each a
 // long latency chain: started first, they run alongside the tiles instead of as a launch of their own that leaves the GPU
 // 60 % idle for 11 us), the others are the persistent tile loop of classes 2 and 1.
-template <typename T, int SPLIT, int RPL>
+template <typename T, int RPL>
 __global__ void __launch_bounds__(kTpeThreads, DOCKAUV_MINB_TPE) rays_thread_kernel(const __grid_constant__ KParams<T> p, unsigned warp_ctas) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    __shared__ __align__(16) T s_tab[kTpeMaxCells * 4 * 4];      // slot = 4 * cell + q: rb[3], bw; bw < 0 marks zero padding
+    __shared__ __align__(16) T s_tab[kTpeTabWords];      // slot = 4 * cell + q: rb[3], bw; bw < 0 marks zero padding
     static_assert(kTpeThreads == kRayWarps * 32, "the two ray mappings share one CTA shape");
     grid_dependency_wait();
     if (blockIdx.x < warp_ctas) {
@@ -900,8 +784,7 @@ __global__ void __launch_bounds__(kTpeThreads, DOCKAUV_MINB_TPE) rays_thread_ker
     }
     const unsigned bid = blockIdx.x - warp_ctas, n_ctas = gridDim.x - warp_ctas;
     const unsigned c1 = p.view_count[0], c2 = p.view_count[1];
-    constexpr unsigned per_tile = kTpeThreads / SPLIT;
-    const unsigned t2 = (c2 + per_tile - 1) / per_tile, t1 = (c1 + per_tile - 1) / per_tile;
+    const unsigned t2 = (c2 + kTpeThreads - 1) / kTpeThreads, t1 = (c1 + kTpeThreads - 1) / kTpeThreads;
     if (bid >= t1 + t2) return;
     const int n_rr = p.n_rr, n_r = p.n_rays;
     for (int t = threadIdx.x; t < 4 * n_rr; t += kTpeThreads) {
@@ -916,8 +799,8 @@ __global__ void __launch_bounds__(kTpeThreads, DOCKAUV_MINB_TPE) rays_thread_ker
     }
     __syncthreads();
     for (unsigned tile = bid; tile < t1 + t2; tile += n_ctas) {
-        if (tile < t2) rays_thread_tile<T, 2, SPLIT>(p, s_tab, tile, c2);
-        else rays_thread_tile<T, 1, SPLIT>(p, s_tab, tile - t2, c1);
+        if (tile < t2) rays_thread_tile<T, 2>(p, s_tab, tile, c2);
+        else rays_thread_tile<T, 1>(p, s_tab, tile - t2, c1);
     }
 }
 
@@ -983,7 +866,6 @@ __global__ void __launch_bounds__(kResetCta) episode_end_kernel(const __grid_con
 // ------------------------------------------------------------------------------------------------------- launcher
 template <typename... KArgs, typename... Args>
 static cudaError_t launch_dependent(void (*kern)(KArgs...), unsigned blocks, unsigned threads, size_t smem, cudaStream_t st, Args... args) {
-#if DOCKAUV_PDL
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(blocks);
     cfg.blockDim = dim3(threads);
@@ -995,47 +877,54 @@ static cudaError_t launch_dependent(void (*kern)(KArgs...), unsigned blocks, uns
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
-#else
-    kern<<<blocks, threads, smem, st>>>(args...);
-    return cudaGetLastError();
-#endif
 }
 
-template <typename T, int VEH, int NU, bool FIN, bool FUSE>
+template <typename T, int VEH, int NU, bool FINISH>
 static cudaError_t launch_dynamics(const KParams<T> &k, unsigned blocks, cudaStream_t st) {
     const bool cur = k.has_current != 0, spm = k.sparse_minv != 0;
-    const int smem = FUSE ? k.n_obsf * kDynThreads * 16 : 0;
+    const int smem = FINISH ? k.n_obsf * kDynThreads * 16 : 0;
     auto go = [&](auto kern) {
-        if (smem > 32 * 1024) {
-            const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-            if (e != cudaSuccess) return e;
-        }
+        const cudaError_t e = allow_dyn_smem(kern, smem, kParkWords * kDynThreads * (int)sizeof(T));
+        if (e != cudaSuccess) return e;
         kern<<<blocks, kDynThreads, smem, st>>>(k);
         return cudaGetLastError();
     };
-    if (cur && spm) return go(dynamics_kernel<T, VEH, NU, true, true, FIN, FUSE>);
-    if (cur) return go(dynamics_kernel<T, VEH, NU, true, false, FIN, FUSE>);
-    if (spm) return go(dynamics_kernel<T, VEH, NU, false, true, FIN, FUSE>);
-    return go(dynamics_kernel<T, VEH, NU, false, false, FIN, FUSE>);
+    if (cur && spm) return go(dynamics_kernel<T, VEH, NU, true, true, FINISH>);
+    if (cur) return go(dynamics_kernel<T, VEH, NU, true, false, FINISH>);
+    if (spm) return go(dynamics_kernel<T, VEH, NU, false, true, FINISH>);
+    return go(dynamics_kernel<T, VEH, NU, false, false, FINISH>);
+}
+
+// the ray launch over the n envs of kc's range, RPL rays per lane
+template <typename T, int RPL>
+static cudaError_t launch_rays(const KParams<T> &kc, int64_t n, cudaStream_t st) {
+    const int smem = kRayWarps * RaysSmem<T, RPL>(kc.n_rays).warp_words * (int)sizeof(T);
+    const int64_t sms = kc.sm_count > 0 ? kc.sm_count : 148;
+    cudaError_t e;
+    if (kc.tpe_rays) {
+        // ---- one launch; thread per env for the envs with one or two obstacles in view (persistent grid over tiles of
+        //      128 lanes; the counts are only known on the device), warp per env for the rest on its first CTAs
+        int64_t tb = (n + kTpeThreads - 1) / kTpeThreads;      // tiles if every env were listed
+        if (tb > sms * DOCKAUV_TPE_CTAS_PER_SM) tb = sms * DOCKAUV_TPE_CTAS_PER_SM;
+        int64_t wb = (n + kRayWarps - 1) / kRayWarps;
+        if (wb > sms * DOCKAUV_TPE_WARP_CTAS_PER_SM) wb = sms * DOCKAUV_TPE_WARP_CTAS_PER_SM;
+        auto kern = rays_thread_kernel<T, RPL>;
+        if ((e = allow_dyn_smem(kern, smem, kTpeTabWords * (int)sizeof(T))) != cudaSuccess) return e;
+        return launch_dependent(kern, (unsigned)(wb + tb), kTpeThreads, smem, st, kc, (unsigned)wb);
+    }
+    // ---- warp per env for every listed env (persistent grid)
+    int64_t blocks = sms * (DOCKAUV_RAY_CTAS_PER_SM * 4 / kRayWarps);
+    const int64_t most = (n + kRayWarps - 1) / kRayWarps;
+    if (blocks > most) blocks = most;
+    auto kern = rays_finish_kernel<T, RPL>;
+    if ((e = allow_dyn_smem(kern, smem, 0)) != cudaSuccess) return e;
+    kern<<<(unsigned)blocks, kRayWarps * 32, smem, st>>>(kc);
+    return cudaGetLastError();
 }
 
 template <typename T, int VEH, int NU>
 static cudaError_t launch_step_pipe(const KParams<T> &k, cudaStream_t st, cudaEvent_t *marks = nullptr, int *n_marks = nullptr) {
     if (wants_debug(k) || k.rec == nullptr) return launch_step_warp<T, VEH, NU>(k, st);   // debug outputs: fused kernel
-    if (k.chunk_envs > 0 && k.chunk_envs < k.env_end - k.env_begin && marks == nullptr) {
-        // chunked: the launches per chunk of envs (measured slower than the whole batch: partial waves of short launches
-        // cost more than an L2-resident record saves; kept for experiments and as a test handle)
-        const int64_t chunk = ((k.chunk_envs + kWarpEnvs - 1) / kWarpEnvs) * kWarpEnvs;
-        for (int64_t b = k.env_begin; b < k.env_end; b += chunk) {
-            KParams<T> kb = k;
-            kb.env_begin = b;
-            kb.env_end = b + chunk < k.env_end ? b + chunk : k.env_end;
-            kb.chunk_envs = 0;
-            cudaError_t e = launch_step_pipe<T, VEH, NU>(kb, st);
-            if (e != cudaSuccess) return e;
-        }
-        return cudaSuccess;
-    }
     const int64_t n = k.env_end - k.env_begin;
     KParams<T> kc = k;
     kc.view_count = k.view_count + kCounterStride * (k.env_begin / kWarpEnvs);   // counters per concurrently stepped env range
@@ -1048,13 +937,12 @@ static cudaError_t launch_step_pipe(const KParams<T> &k, cudaStream_t st, cudaEv
     mark();
     const bool has_obstacles = k.n_caps + k.n_sph > 0;
     const unsigned dyn_blocks = (unsigned)((n + kDynThreads - 1) / kDynThreads);
-    // scenarios without obstacles are finished by the dynamics launch itself (no cull, no rays); with obstacles the cull +
-    // finish code runs inside it whenever the float records of a CTA fit in shared memory
+    // the cull + finish code runs inside the dynamics launch whenever the float records of a CTA fit in shared memory, and
+    // in scenarios without obstacles, where it finishes every env (no cull, no rays)
     const bool fuse = pipe_fuses_cull(k);
     kc.counters_zeroed_at_end = fuse ? 1 : 0;
-    cudaError_t e = !has_obstacles ? launch_dynamics<T, VEH, NU, true, false>(kc, dyn_blocks, st)
-                    : fuse       ? launch_dynamics<T, VEH, NU, false, true>(kc, dyn_blocks, st)
-                                 : launch_dynamics<T, VEH, NU, false, false>(kc, dyn_blocks, st);
+    cudaError_t e = fuse || !has_obstacles ? launch_dynamics<T, VEH, NU, true>(kc, dyn_blocks, st)
+                                           : launch_dynamics<T, VEH, NU, false>(kc, dyn_blocks, st);
     if (e != cudaSuccess) return e;
     mark();
     if (has_obstacles) {
@@ -1063,40 +951,9 @@ static cudaError_t launch_step_pipe(const KParams<T> &k, cudaStream_t st, cudaEv
             if ((e = cudaGetLastError()) != cudaSuccess) return e;
             mark();
         }
-        const int smem = kRayWarps * (k.n_rays <= 64 ? RaysSmem<T, 2>(k.n_rays).warp_words : RaysSmem<T, 8>(k.n_rays).warp_words) * (int)sizeof(T);
-        const int64_t sms = k.sm_count > 0 ? k.sm_count : 148;
-        if (k.tpe_rays) {
-            // ---- rays: one launch; thread per env for the envs with one or two obstacles in view (persistent grid over tiles
-            //      of 128 lanes; the counts are only known on the device), warp per env for the rest on its first CTAs
-            int64_t tb = (n * DOCKAUV_TPE_SPLIT + kTpeThreads - 1) / kTpeThreads;      // tiles if every env were listed
-            if (tb > sms * DOCKAUV_TPE_CTAS_PER_SM) tb = sms * DOCKAUV_TPE_CTAS_PER_SM;
-            int64_t wb = (n + kRayWarps - 1) / kRayWarps;
-            if (wb > sms * DOCKAUV_TPE_WARP_CTAS_PER_SM) wb = sms * DOCKAUV_TPE_WARP_CTAS_PER_SM;
-            if (k.n_rays <= 64) {
-                auto kern = rays_thread_kernel<T, DOCKAUV_TPE_SPLIT, 2>;
-                if (smem > 40 * 1024 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)) != cudaSuccess) return e;
-                if ((e = launch_dependent(kern, (unsigned)(wb + tb), kTpeThreads, smem, st, kc, (unsigned)wb)) != cudaSuccess) return e;
-            } else {
-                auto kern = rays_thread_kernel<T, DOCKAUV_TPE_SPLIT, 8>;
-                if (smem > 40 * 1024 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)) != cudaSuccess) return e;
-                if ((e = launch_dependent(kern, (unsigned)(wb + tb), kTpeThreads, smem, st, kc, (unsigned)wb)) != cudaSuccess) return e;
-            }
-        } else {
-            // ---- rays: warp per env for every listed env (persistent grid)
-            int64_t blocks = sms * (DOCKAUV_RAY_CTAS_PER_SM * 4 / kRayWarps);
-            const int64_t most = (n + kRayWarps - 1) / kRayWarps;
-            if (blocks > most) blocks = most;
-            if (k.n_rays <= 64) {
-                auto kern = rays_finish_kernel<T, 2>;
-                if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)) != cudaSuccess) return e;
-                kern<<<(unsigned)blocks, kRayWarps * 32, smem, st>>>(kc);
-            } else {
-                auto kern = rays_finish_kernel<T, 8>;
-                if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)) != cudaSuccess) return e;
-                kern<<<(unsigned)blocks, kRayWarps * 32, smem, st>>>(kc);
-            }
-        }
-        if ((e = cudaGetLastError()) != cudaSuccess) return e;
+        // rays per lane: 2 covers the stock 63-ray and the 64-ray radar; 8 covers everything up to DOCKAUV_MAX_RAYS
+        e = k.n_rays <= 64 ? launch_rays<T, 2>(kc, n, st) : launch_rays<T, 8>(kc, n, st);
+        if (e != cudaSuccess) return e;
         mark();
     }
     {

@@ -96,26 +96,14 @@ __global__ void __launch_bounds__(kWarpEnvs) step_warp_kernel(const __grid_const
         T spsi, cpsi, att[3];
         float obs16[16];
         step_dynamics<T, VEH, NU, DBG>(p, i, cy, spsi, cpsi, obs16, att);
-        // 0 for a finite pose, NaN otherwise: radar_env poisons the ray distances with it where the reference's NaN
-        // propagation reaches them (envs without capsules)
-        const T poison = (((cy.pos[0] + cy.pos[1]) + (cy.pos[2] + att[0])) + (att[1] + att[2])) * T(0);
         T *ps = s_pose + tid * kPoseStride;
 #pragma unroll
         for (int c = 0; c < 3; c++) ps[c] = cy.pos[c];
 #pragma unroll
         for (int c = 0; c < 9; c++) ps[3 + c] = cy.R[c];
-        ps[12] = poison;
-        // obs[0:16] goes straight to its HBM row (four 16-byte stores); phase C zeroes the row if the env is reset
-        float4 *orow4 = reinterpret_cast<float4 *>(p.obs + i * p.n_obs);
-        if ((p.n_obs & 3) == 0) {
-#pragma unroll
-            for (int c = 0; c < 4; c++)
-                orow4[c] = make_float4(obs16[4 * c], obs16[4 * c + 1], obs16[4 * c + 2], obs16[4 * c + 3]);
-        } else {
-            float *orow = p.obs + i * p.n_obs;
-#pragma unroll
-            for (int c = 0; c < 16; c++) orow[c] = obs16[c];
-        }
+        ps[12] = pose_poison<T>(cy.pos, att);
+        // obs[0:16] to its HBM row; phase C zeroes the row if the env is reset
+        store_obs_head<T>(p, i, obs16);
     }
     __syncwarp();
 
@@ -208,15 +196,7 @@ __global__ void __launch_bounds__(kWarpEnvs) step_warp_kernel(const __grid_const
     // ------------------------------------------------------------------ phase C
     bool done = false;
     if (active) {
-        if (my_view_empty && no_dbg && s_pose[tid * kPoseStride + 12] == T(0)) {
-            float *cells = p.obs + i * p.n_obs + 16;
-            if ((p.n_obs & 3) == 0 && (p.n_rr & 3) == 0) {
-                float4 *c4 = reinterpret_cast<float4 *>(cells);
-                for (int c = 0; c < (p.n_rr >> 2); c++) c4[c] = make_float4(1.0f, 1.0f, 1.0f, 1.0f);
-            } else {
-                for (int c = 0; c < p.n_rr; c++) cells[c] = 1.0f;
-            }
-        }
+        if (my_view_empty && no_dbg && s_pose[tid * kPoseStride + 12] == T(0)) store_clear_cells<T>(p, i);
         const T r_oa = p.sum_beta_oa / my_oa_dot - T(1);      // docking3d.py:792
         done = step_finish<T, DBG>(p, i, cy, r_oa, my_col, bs);
     }
@@ -240,16 +220,21 @@ __global__ void __launch_bounds__(kWarpEnvs) step_warp_kernel(const __grid_const
     bs.flush(p.stats, warp == 0 ? n_here : 0);
 }
 
+// A kernel gets 48 KB of shared memory in all, its static arrays (static_bytes) included, unless it is allowed more
+template <typename K>
+static cudaError_t allow_dyn_smem(K kern, int smem, int static_bytes) {
+    if (smem + static_bytes <= 48 * 1024) return cudaSuccess;
+    return cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+}
+
 template <typename T, int VEH, int NU, int RPL, bool DBG>
 static cudaError_t launch_step_warp_rpl(const KParams<T> &k, cudaStream_t st) {
     const int64_t n = k.env_end - k.env_begin;
     const WarpSmem<T> L(k.n_rays);
     const int smem = L.total;
     auto kern = step_warp_kernel<T, VEH, NU, RPL, DBG>;
-    if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e != cudaSuccess) return e;
-    }
+    const cudaError_t e = allow_dyn_smem(kern, smem, 0);
+    if (e != cudaSuccess) return e;
     const unsigned blocks = (unsigned)((n + kWarpEnvs - 1) / kWarpEnvs);
     kern<<<blocks, kWarpEnvs, smem, st>>>(k);
     return cudaGetLastError();

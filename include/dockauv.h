@@ -129,8 +129,9 @@ typedef struct DockauvParams {
     int32_t action_factor_is_scalar;   /* config "action_reward_factors" was a python scalar */
     int32_t layout;              /* DOCKAUV_LAYOUT_* */
     int32_t force_current;       /* evaluate the ocean current even if the scenario spawns none (injected currents) */
-    int32_t split_chunk_envs;    /* DOCKAUV_LAYOUT_PIPELINE: envs per launch group (0 = library default: the whole batch, in two
-                                    halves on two streams from 131,072 envs on) */
+    int32_t split_chunk_envs;    /* DOCKAUV_LAYOUT_PIPELINE: 0 = library default: the whole batch, in two halves on two streams
+                                    from 131,072 envs on; any other value: the whole batch as one launch group on the
+                                    caller's stream */
     /* rigid body + hydrodynamics (statespace.py) */
     double m;
     double r_G[3];

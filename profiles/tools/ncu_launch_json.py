@@ -42,7 +42,7 @@ def main():
         if short is None:
             continue
         if short == "dynamics":
-            # dynamics_kernel<T, VEH, NU, CUR, SPM, FIN, FUSE>: the last template argument says whether the cull + finish code runs in it
+            # dynamics_kernel<T, VEH, NU, CUR, SPM, FINISH>: the last template argument says whether the cull + finish code runs in it
             args = kname[kname.index("<") + 1:kname.index(">(")].replace("(bool)", "").split(",")
             if args[-1].strip() in ("1", "true"):
                 short = "dynamics_cull_finish"

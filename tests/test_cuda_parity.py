@@ -370,25 +370,29 @@ def test_layouts_agree_bitwise_on_flags_large_batch():
 
 def test_step_in_parts_equals_one_launch_group():
     """A batch that is stepped in two parts on two streams (>= 131,072 envs, odd size) gives the same bits as the same
-    envs stepped as one launch group (split_chunk_envs = N disables the parts)."""
+    envs stepped as one launch group (split_chunk_envs = N disables the parts; so does any other non-zero value, 4096
+    included)."""
     import torch
     from gym_dockauv_b200 import envs
     from gym_dockauv_b200.config import BASE_CONFIG, RADAR_64
     cfg = dict(BASE_CONFIG)
     cfg["radar"] = dict(RADAR_64)
     n = (1 << 19) + 4097
-    es = [envs.ObstaclesDocking3d(cfg, num_envs=n, seed=21, n_synthetic_spheres=3, split_chunk_envs=c) for c in (0, n)]
+    es = [envs.ObstaclesDocking3d(cfg, num_envs=n, seed=21, n_synthetic_spheres=3, split_chunk_envs=c) for c in (0, n, 4096)]
     for e in es:
         e.reset()
     gen = torch.Generator(device="cuda").manual_seed(2)
     for _ in range(12):
         a = torch.rand(n, 6, device="cuda", generator=gen) * 2 - 1
-        (o0, r0, d0, _), (o1, r1, d1, _) = [e.step(a) for e in es]
+        (o0, r0, d0, _), (o1, r1, d1, _), (o2, r2, d2, _) = [e.step(a) for e in es]
         assert torch.equal(o0, o1) and torch.equal(r0, r1) and torch.equal(d0, d1)
+        assert torch.equal(o0, o2) and torch.equal(r0, r2) and torch.equal(d0, d2)
     assert torch.equal(es[0].state, es[1].state) and torch.equal(es[0].episode, es[1].episode)
-    s0, s1 = es[0].get_stats(), es[1].get_stats()
-    assert s0["env_steps"] == s1["env_steps"] == 12 * n and s0["episodes"] == s1["episodes"]
+    assert torch.equal(es[0].state, es[2].state) and torch.equal(es[0].episode, es[2].episode)
+    s0, s1, s2 = es[0].get_stats(), es[1].get_stats(), es[2].get_stats()
+    assert s0["env_steps"] == s1["env_steps"] == s2["env_steps"] == 12 * n and s0["episodes"] == s1["episodes"] == s2["episodes"]
     assert es[0].launch_count() - es[1].launch_count() == 12 * 3      # 6 launches per step against 3 (dynamics + cull, rays, episode end)
+    assert es[2].launch_count() == es[1].launch_count()
     for e in es:
         e.close()
 
