@@ -2,12 +2,15 @@
 """Minimal on-device PPO loop over the batched docking env -- the counterpart of the reference's
 ``train()`` (gym_dockauv/train.py:21-82: ``MODEL('MlpPolicy', env).learn(...)``) without a host round trip per step:
 
-    python examples/ppo_device_rollout.py [--envs 16384] [--steps 64] [--iters 20]
+    python examples/ppo_device_rollout.py [--envs 16384] [--steps 64] [--iters 20] [--record-envs K --record-dir DIR]
 
 * rollouts: ``DeviceRolloutBuffer.collect`` -- the step kernels write observation / reward / done of step t straight
   into row t of the buffer;
 * advantages: ``dockauv_gae`` (one kernel over the stacked rows);
-* the policy / value networks and the clipped-surrogate update are plain PyTorch (they are not part of the step path).
+* the policy / value networks and the clipped-surrogate update are plain PyTorch (they are not part of the step path);
+* ``--record-envs K``: the episodes of K envs spread over the batch are recorded on the device while the run trains
+  (``TrainingRecorder``) and written to ``--record-dir`` as reference-format ``EpisodeDataStorage`` pickles, drained once
+  per iteration.
 
 Prints, per iteration, the mean return of the episodes that ended inside the rollout and the env-steps/s of collection.
 """
@@ -22,6 +25,7 @@ import torch.nn as nn  # noqa: E402
 
 from gym_dockauv_b200 import envs  # noqa: E402
 from gym_dockauv_b200.config import TRAIN_CONFIG  # noqa: E402
+from gym_dockauv_b200.episode_export import TrainingRecorder  # noqa: E402
 from gym_dockauv_b200.rollout import DeviceRolloutBuffer  # noqa: E402
 
 
@@ -48,10 +52,16 @@ def main():
     ap.add_argument("--steps", type=int, default=64)
     ap.add_argument("--iters", type=int, default=20)
     ap.add_argument("--scenario", default="ObstaclesDocking3d")
+    ap.add_argument("--record-envs", type=int, default=0, help="record the episodes of this many envs (at most 1024)")
+    ap.add_argument("--record-dir", default="episode_storage")
     args = ap.parse_args()
     env = envs.SCENARIOS[args.scenario](TRAIN_CONFIG, num_envs=args.envs, seed=0)
     buf = DeviceRolloutBuffer(env, args.steps, gamma=0.99, gae_lambda=0.95)
     buf.reset_env()
+    rec = None
+    if args.record_envs:
+        ids = torch.linspace(0, args.envs - 1, args.record_envs).long().unique().tolist()
+        rec = TrainingRecorder(env, ids, args.record_dir, title="ppo", capacity=max(args.steps, 64))
     net = ActorCritic(env.n_observations, env.n_actions).to(env.device)
     opt = torch.optim.Adam(net.parameters(), lr=3e-4)
     for it in range(args.iters):
@@ -63,6 +73,10 @@ def main():
         torch.cuda.synchronize()
         t_collect = time.perf_counter() - t0
         info = buf.episode_infos()
+        if rec is not None:
+            n_saved = len(rec.drain())
+            if n_saved:
+                print(f"iter {it:3d}  wrote {n_saved} episode pickles to {args.record_dir}", flush=True)
         for _ in range(4):
             for mb in buf.get(batch_size=1 << 16):
                 adv = (mb.advantages - mb.advantages.mean()) / (mb.advantages.std() + 1e-8)

@@ -4,7 +4,7 @@ import ctypes as C
 import os
 
 from .params import (ABI_VERSION, DockauvBuffers, DockauvDebugOut, DockauvParams, DockauvRolloutOut,
-                     DockauvStepOut)
+                     DockauvStepOut, DockauvTapBuffers)
 
 LIB_PATH = os.environ.get("DOCKAUV_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_lib",
                                                         "libdockauv_b200.so")   # DOCKAUV_LIB: tuning builds only
@@ -27,6 +27,7 @@ SYMBOLS = {
     "dockauv_step_graph_captures": (_i, [_vp, C.POINTER(_i64)]),
     "dockauv_step_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _i, C.POINTER(DockauvStepOut)]),
     "dockauv_rollout": (_i, [_vp, _vp, _i, _i, C.POINTER(DockauvRolloutOut), _i, _i, _vp]),
+    "dockauv_set_taps": (_i, [_vp, C.POINTER(_i64), _i, _i, C.POINTER(DockauvTapBuffers)]),
     "dockauv_gae": (_i, [_vp, _i, _vp, _vp, _vp, _i, _i64, C.c_float, C.c_float, _vp, _vp, _vp]),
     "dockauv_stats_ptr": (_i, [_vp, C.POINTER(_vp)]),
     "dockauv_fold_stats": (_i, [_vp, _vp]),

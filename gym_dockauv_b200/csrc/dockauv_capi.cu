@@ -1,8 +1,9 @@
 // dockauv_capi.cu -- C ABI (include/dockauv.h) over the sm_100a step kernels.
 //
 // No torch types, no global state besides a thread-local error string.  All device memory that crosses the
-// boundary is caller-owned; the handle owns only its small ray table, the statistics vector and (lazily) the
-// device staging buffers + streams of the host-buffer entry point.
+// boundary is caller-owned; the handle owns only its small ray table, the statistics vector, (lazily) the
+// device staging buffers + streams of the host-buffer entry point and, while taps are set, the K-env tap shadows and
+// its side stream.
 #include <cuda_runtime.h>
 
 #include <cmath>
@@ -10,6 +11,7 @@
 #include <cstdio>
 #include <cstdint>
 #include <cstring>
+#include <algorithm>
 #include <new>
 #include <vector>
 
@@ -122,6 +124,34 @@ struct DockauvHandle {
     size_t sg_next = 0;            // slot replaced next once the cache is full
     bool sg_enabled = true;
     int64_t sg_captures = 0;
+    DockauvBuffers bound_bufs = {};
+    // episode taps (dockauv_set_taps): two K-env shadows of the tapped envs, stepped on a side stream
+    struct Taps {
+        int n = 0;
+        int64_t capacity = 0;
+        DockauvTapBuffers ring = {};
+        void *mem = nullptr;           // everything below that is a device pointer lives in this one allocation
+        DockauvBuffers shadow = {};    // stepped by the real step's layout: outputs and post-step state (K-env SoA)
+        DockauvBuffers dshadow = {};   // stepped by the single-launch kernel with debug outputs
+        void *actions = nullptr, *noise = nullptr;
+        DockauvStepOut out = {};       // obs, reward, done, cond_bits of `shadow`
+        DockauvStepOut dout = {};      // the same of `dshadow` (not recorded)
+        DockauvDebugOut dbg = {};      // ray_dist, reward_arr, nu_c, state_dot of `dshadow`
+        // pipeline layout: the shadow's own per-env records, float obstacle records, work lists and counters
+        void *rec = nullptr;
+        float4 *obsf = nullptr;
+        unsigned long long *view_list = nullptr;
+        uint32_t *ended_list = nullptr;
+        unsigned int *view_count = nullptr;
+        int shadow_launches = 0;       // launches of one step of `shadow`
+        double *stats = nullptr;       // DOCKAUV_STAT_COPIES replicas nobody reads: the public statistics stay the real step's
+        int64_t *ids = nullptr;
+        unsigned int *sync = nullptr;
+        TapRow *gather_rows = nullptr, *commit_rows = nullptr;
+        int n_gather = 0, n_commit = 0;
+        cudaStream_t st = nullptr, dst = nullptr;      // output shadow + commit; debug shadow (the two run side by side)
+        cudaEvent_t ev_fork = nullptr, ev_join = nullptr, ev_dbg = nullptr;
+    } tap;
 };
 
 static int pooled_dim(int n, int b) { return (n + b - 1) / b; }
@@ -384,8 +414,85 @@ extern "C" int dockauv_destroy(DockauvHandle *h) {
     if (h->st_reward) cudaFree(h->st_reward);
     if (h->st_done) cudaFree(h->st_done);
     if (h->st_cond) cudaFree(h->st_cond);
+    if (h->tap.mem) cudaFree(h->tap.mem);
+    if (h->tap.st) cudaStreamDestroy(h->tap.st);
+    if (h->tap.ev_fork) cudaEventDestroy(h->tap.ev_fork);
+    if (h->tap.ev_join) cudaEventDestroy(h->tap.ev_join);
+    if (h->tap.dst) cudaStreamDestroy(h->tap.dst);
+    if (h->tap.ev_dbg) cudaEventDestroy(h->tap.ev_dbg);
     drop_graphs(h);
     delete h;
+    return DOCKAUV_OK;
+}
+
+// ------------------------------------------------------------------------------------------- episode taps: row tables
+// The gather copies the pre-step rows of the tapped envs from the bound buffers into both shadows and the ring's pre_*
+// fields; the commit copies the shadows' post-step rows into the ring's post-step fields.  One TapRow per component row.
+static int build_tap_rows(DockauvHandle *h) {
+    auto &tp = h->tap;
+    const DockauvBuffers &b = h->bound_bufs;
+    const DockauvTapBuffers &r = tp.ring;
+    const int64_t N = h->n_envs, K = tp.n;
+    const int esz = h->params.precision == DOCKAUV_F64 ? 8 : 4;
+    const int nu = h->params.n_u, nc = h->params.n_capsules, ns = h->params.n_spheres;
+    const int n_scene = 4 + 7 * nc + 4 * ns, n_obs = h->n_obs, n_rays = h->params.n_rays;
+    std::vector<TapRow> g, c;
+    // one gathered row: component `comp` of a bound buffer (env-indexed) -> the same component of both shadows, and row
+    // `ring_row` of a ring field with `ring_rows` rows per slot
+    auto gather = [&](const void *src, void *shadow, void *dshadow, int comp, int e, void *ring, int ring_row, int ring_rows) {
+        TapRow t;
+        t.src = (const char *)src + (int64_t)comp * N * e;
+        t.dst = (char *)shadow + (int64_t)comp * K * e;
+        t.dst2 = dshadow ? (char *)dshadow + (int64_t)comp * K * e : nullptr;
+        t.ring = ring ? (char *)ring + (int64_t)ring_row * K * e : nullptr;
+        t.ring_slot = (int64_t)ring_rows * K * e;
+        t.esz = e;
+        t.src_step = t.dst_step = e;
+        t.src_by_id = 1;
+        g.push_back(t);
+    };
+    for (int k = 0; k < 12; k++) gather(b.state, tp.shadow.state, tp.dshadow.state, k, esz, r.pre_state, k, 12);
+    for (int k = 0; k < nu; k++) gather(b.u_prev, tp.shadow.u_prev, tp.dshadow.u_prev, k, esz, nullptr, 0, 0);
+    for (int k = 0; k < 3; k++) gather(b.goal, tp.shadow.goal, tp.dshadow.goal, k, esz, r.pre_scene, k, n_scene);
+    gather(b.heading_goal, tp.shadow.heading_goal, tp.dshadow.heading_goal, 0, esz, r.pre_scene, 3, n_scene);
+    for (int k = 0; k < 5; k++) gather(b.current, tp.shadow.current, tp.dshadow.current, k, esz, r.pre_current, k, 5);
+    for (int k = 0; k < 7 * nc; k++) gather(b.capsules, tp.shadow.capsules, tp.dshadow.capsules, k, esz, r.pre_scene, 4 + k, n_scene);
+    for (int k = 0; k < 4 * ns; k++) gather(b.spheres, tp.shadow.spheres, tp.dshadow.spheres, k, esz, r.pre_scene, 4 + 7 * nc + k, n_scene);
+    gather(b.ep_return, tp.shadow.ep_return, tp.dshadow.ep_return, 0, esz, r.pre_ep_return, 0, 1);
+    gather(b.t_steps, tp.shadow.t_steps, tp.dshadow.t_steps, 0, 4, r.pre_t_steps, 0, 1);
+    gather(b.episode, tp.shadow.episode, tp.dshadow.episode, 0, 4, r.pre_episode, 0, 1);
+    // the real step's float obstacle records (pipeline layout): the shadow culls exactly what the real step culls
+    if (tp.obsf)
+        for (int k = 0; k < h->kd.n_obsf; k++) gather(h->kd.obsf, tp.obsf, nullptr, k, 16, nullptr, 0, 0);
+    // one committed row: row `comp` of a shadow field (tap-indexed, `step` bytes apart) -> row `comp` of a ring field
+    auto commit = [&](const void *src, void *ring, int comp, int e, int rows, int step) {
+        TapRow t;
+        t.src = (const char *)src + (int64_t)comp * (step == e ? K * e : e);
+        t.dst = t.dst2 = nullptr;
+        t.ring = (char *)ring + (int64_t)comp * (step == e ? K * e : e);
+        t.ring_slot = (int64_t)rows * K * e;
+        t.esz = e;
+        t.src_step = t.dst_step = step;
+        t.src_by_id = 0;
+        c.push_back(t);
+    };
+    for (int k = 0; k < 12; k++) commit(tp.shadow.state, r.state, k, esz, 12, esz);
+    for (int k = 0; k < nu; k++) commit(tp.shadow.u_prev, r.u, k, esz, nu, esz);
+    for (int k = 0; k < 12; k++) commit(tp.dbg.state_dot, r.state_dot, k, esz, 12, esz);
+    for (int k = 0; k < 3; k++) commit(tp.dbg.nu_c, r.nu_c, k, esz, 3, esz);
+    for (int k = 0; k < n_rays; k++) commit(tp.dbg.ray_dist, r.ray_dist, k, esz, n_rays, esz);
+    for (int k = 0; k < 13; k++) commit(tp.dbg.reward_arr, r.reward_arr, k, esz, 13, esz);
+    commit(tp.out.reward, r.reward, 0, esz, 1, esz);
+    commit(tp.out.done, r.done, 0, 1, 1, 1);
+    commit(tp.out.cond_bits, r.cond_bits, 0, 1, 1, 1);
+    // observation rows are tap-major ([K][n_obs] in the shadow, [S][K][n_obs] in the ring): column k of every row
+    for (int k = 0; k < n_obs; k++) commit(tp.out.obs, r.obs, k, 4, n_obs, 4 * n_obs);
+    if ((int)g.size() != tp.n_gather || (int)c.size() != tp.n_commit)
+        return fail(DOCKAUV_EINVAL, "internal: tap row tables have %zu / %zu rows, %d / %d reserved", g.size(), c.size(),
+                    tp.n_gather, tp.n_commit);
+    DeviceGuard guard(h->device);
+    CUDA_TRY(cudaMemcpy(tp.gather_rows, g.data(), sizeof(TapRow) * g.size(), cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMemcpy(tp.commit_rows, c.data(), sizeof(TapRow) * c.size(), cudaMemcpyHostToDevice));
     return DOCKAUV_OK;
 }
 
@@ -412,7 +519,12 @@ extern "C" int dockauv_bind(DockauvHandle *h, const DockauvBuffers *b) {
         return fail(DOCKAUV_EINVAL, "obstacle buffer is null but the handle has obstacles");
     bind_k<double>(h->kd, *b);
     bind_k<float>(h->kf, *b);
+    h->bound_bufs = *b;
     h->bound = true;
+    if (h->tap.n > 0) {
+        const int rc = build_tap_rows(h);
+        if (rc != DOCKAUV_OK) return rc;
+    }
     {   // float obstacle records of whatever the buffers hold now (later writers: dockauv_reset, dockauv_refresh_obstacles)
         DeviceGuard guard(h->device);
         if (h->params.precision == DOCKAUV_F64) CUDA_TRY(launch_refresh_obstacles<double>(h->kd, (cudaStream_t)0));
@@ -434,6 +546,11 @@ static int resolve_layout(const DockauvHandle *h) {
     // is dynamics + finish only; thread-per-env stays as the independently written cross-check
     if (layout == DOCKAUV_LAYOUT_AUTO) layout = DOCKAUV_LAYOUT_PIPELINE;
     return layout;
+}
+
+// the current is "on" when the scenario spawns one, the caller asked for it, or noise is configured
+static bool current_on(const DockauvHandle *h) {
+    return scenario_has_current(h->params.scenario) || h->params.force_current != 0 || h->params.cur_sigma > 0.0;
 }
 
 template <typename T>
@@ -465,9 +582,7 @@ static int step_range(DockauvHandle *h, const void *actions, int action_dtype, c
                       int64_t end, cudaStream_t st, bool with_marks = false) {
     const bool actf32 = action_dtype == DOCKAUV_ACT_F32;
     const int layout = resolve_layout(h);
-    // the current is "on" when the scenario spawns one, the caller asked for it, or noise is configured
-    const bool has_current = scenario_has_current(h->params.scenario) || h->params.force_current != 0 ||
-                             h->params.cur_sigma > 0.0;
+    const bool has_current = current_on(h);
     cudaError_t e;
     if (h->params.precision == DOCKAUV_F64) {
         KParams<double> k = h->kd;
@@ -488,6 +603,90 @@ static int step_range(DockauvHandle *h, const void *actions, int action_dtype, c
     h->last_begins.push_back(begin);
     const bool staged = dbg == nullptr;   // else: the fused kernel
     h->launches += layout == DOCKAUV_LAYOUT_PIPELINE && staged ? dockauv::pipe_launches(h->kd) : 1;
+    return DOCKAUV_OK;
+}
+
+// ------------------------------------------------------------------------------------------- episode taps: launches
+// With taps set, every step issues, besides its own launches, the gather on the caller's stream before the step's first
+// launch (the only serial addition), then, on two tap streams forked after it, two shadow steps over K-env copies of the
+// tapped envs side by side, and the commit once both are done.  The first shadow is stepped by the handle's own layout with the real step's inputs (state,
+// float obstacle records, actions, noise), so its outputs and post-step state are those of the real step in either
+// precision; the second by the single-launch kernel with debug outputs (the fields only that kernel has).  Neither
+// touches a real env, output or statistic.  tap_end joins the tap stream back, so the next step's gather, which rewrites
+// the shadows, is ordered after this step's commit.
+static TapLaunch tap_launch(const DockauvHandle *h, bool gather, const void *actions, int action_dtype, const void *noise) {
+    const auto &tp = h->tap;
+    TapLaunch t;
+    memset(&t, 0, sizeof(t));
+    t.rows = gather ? tp.gather_rows : tp.commit_rows;
+    t.n_rows = gather ? tp.n_gather : tp.n_commit;
+    t.n_taps = tp.n;
+    t.ids = tp.ids;
+    t.count = tp.ring.count;
+    t.capacity = tp.capacity;
+    t.sync = tp.sync;
+    t.actions = actions;
+    t.act_f32 = action_dtype == DOCKAUV_ACT_F32 ? 1 : 0;
+    t.n_u = h->params.n_u;
+    t.shadow_actions = tp.actions;
+    t.noise = noise;
+    t.shadow_noise = tp.noise;
+    return t;
+}
+
+template <typename T>
+static cudaError_t tap_issue(DockauvHandle *h, const KParams<T> &real, const void *actions, int action_dtype,
+                             const void *noise, cudaStream_t st) {
+    auto &tp = h->tap;
+    cudaError_t e = launch_tap_gather<T>(real, tap_launch(h, true, actions, action_dtype, noise), st);
+    if (e == cudaSuccess) e = cudaEventRecord(tp.ev_fork, st);
+    if (e == cudaSuccess) e = cudaStreamWaitEvent(tp.st, tp.ev_fork, 0);
+    if (e == cudaSuccess) e = cudaStreamWaitEvent(tp.dst, tp.ev_fork, 0);
+    if (e != cudaSuccess) return e;
+    // the shadow: the real step's own layout, so its outputs and post-step state are those of the real step
+    KParams<T> k = real;
+    k.n_envs = tp.n;
+    k.env_begin = 0;
+    k.env_end = tp.n;
+    bind_k<T>(k, tp.shadow);
+    set_io<T>(k, tp.actions, action_dtype == DOCKAUV_ACT_F32, tp.noise, tp.out, nullptr, 0);
+    k.has_current = current_on(h);
+    k.stats = tp.stats;
+    k.rec = (T *)tp.rec;
+    k.obsf = tp.obsf;
+    k.view_list = tp.view_list;
+    k.ended_list = tp.ended_list;
+    k.view_count = tp.view_count;
+    e = launch_step<T>(k, h->params.vehicle, resolve_layout(h), tp.st);
+    if (e != cudaSuccess) return e;
+    // the debug shadow: the single-launch kernel with debug outputs (state_dot, nu_c, ray distances, reward terms)
+    KParams<T> d = k;
+    bind_k<T>(d, tp.dshadow);
+    set_io<T>(d, tp.actions, action_dtype == DOCKAUV_ACT_F32, tp.noise, tp.dout, &tp.dbg, 0);
+    d.rec = nullptr;
+    d.obsf = nullptr;
+    d.view_list = nullptr;
+    d.ended_list = nullptr;
+    d.view_count = nullptr;
+    e = launch_step<T>(d, h->params.vehicle, DOCKAUV_LAYOUT_WARP_RAYS, tp.dst);
+    if (e == cudaSuccess) e = cudaEventRecord(tp.ev_dbg, tp.dst);
+    if (e == cudaSuccess) e = cudaStreamWaitEvent(tp.st, tp.ev_dbg, 0);
+    if (e == cudaSuccess) e = launch_tap_commit<T>(real, tap_launch(h, false, actions, action_dtype, noise), tp.st);
+    if (e == cudaSuccess) e = cudaEventRecord(tp.ev_join, tp.st);
+    return e;
+}
+
+static int tap_begin(DockauvHandle *h, const void *actions, int action_dtype, const void *noise, cudaStream_t st) {
+    if (h->tap.n == 0) return DOCKAUV_OK;
+    const cudaError_t e = h->params.precision == DOCKAUV_F64 ? tap_issue<double>(h, h->kd, actions, action_dtype, noise, st)
+                                                             : tap_issue<float>(h, h->kf, actions, action_dtype, noise, st);
+    if (e != cudaSuccess) return fail(DOCKAUV_ECUDA, "tap launch failed: %s", cudaGetErrorString(e));
+    h->launches += 3 + h->tap.shadow_launches;      // gather, debug shadow, commit + the shadow's step
+    return DOCKAUV_OK;
+}
+
+static int tap_end(DockauvHandle *h, cudaStream_t st) {
+    if (h->tap.n > 0) CUDA_TRY(cudaStreamWaitEvent(st, h->tap.ev_join, 0));
     return DOCKAUV_OK;
 }
 
@@ -579,6 +778,15 @@ static int step_device(DockauvHandle *h, const void *actions, int action_dtype, 
     return step_range(h, actions, action_dtype, noise, out, dbg, auto_reset, 0, h->n_envs, st, timing);
 }
 
+// step_device with the tap branch around it (when taps are set)
+static int step_call(DockauvHandle *h, const void *actions, int action_dtype, const void *noise, const DockauvStepOut *out,
+                     const DockauvDebugOut *dbg, int auto_reset, cudaStream_t st, bool timing) {
+    int rc = tap_begin(h, actions, action_dtype, noise, st);
+    if (rc == DOCKAUV_OK) rc = step_device(h, actions, action_dtype, noise, out, dbg, auto_reset, st, timing);
+    if (rc == DOCKAUV_OK) rc = tap_end(h, st);
+    return rc;
+}
+
 #ifndef DOCKAUV_STEP_GRAPHS
 #define DOCKAUV_STEP_GRAPHS 96     // cached step graphs per handle (a trainer alternates between a few tensors; bench.py's pool: 64)
 #endif
@@ -611,7 +819,7 @@ static int step_graph(DockauvHandle *h, const void *actions, int action_dtype, c
         const int64_t before = h->launches;
         h->last_begins.clear();
         if (e == cudaSuccess) {
-            rc = step_device(h, actions, action_dtype, noise, out, nullptr, auto_reset, cs, false);
+            rc = step_call(h, actions, action_dtype, noise, out, nullptr, auto_reset, cs, false);
             e = cudaStreamEndCapture(cs, &graph);
         }
         const int64_t n_launch = h->launches - before;
@@ -667,7 +875,7 @@ extern "C" int dockauv_step(DockauvHandle *h, const void *actions_dev, int actio
         if (cudaStreamIsCapturing(st, &cap) == cudaSuccess && cap == cudaStreamCaptureStatusNone)
             return step_graph(h, actions_dev, action_dtype, noise_dev, out, auto_reset, st);
     }
-    int rc = step_device(h, actions_dev, action_dtype, noise_dev, out, dbg, auto_reset, st, h->timing);
+    int rc = step_call(h, actions_dev, action_dtype, noise_dev, out, dbg, auto_reset, st, h->timing);
     if (rc != DOCKAUV_OK) return rc;
     if (h->timing) {
         CUDA_TRY(cudaEventRecord(h->ev1, st));
@@ -711,6 +919,9 @@ extern "C" int dockauv_step_host(DockauvHandle *h, const void *actions_host, int
                                  const DockauvStepOut *aux) {
     if (!h || !actions_host || !obs_host || !reward_host || !done_host) return fail(DOCKAUV_EINVAL, "null argument");
     if (!h->bound) return fail(DOCKAUV_ESTATE, "dockauv_bind must be called before dockauv_step_host");
+    if (h->tap.n > 0)
+        return fail(DOCKAUV_ESTATE, "taps are set: they record device-driven steps (dockauv_step, dockauv_rollout); remove "
+                                    "them (dockauv_set_taps with n_taps = 0) before dockauv_step_host");
     if (action_dtype != DOCKAUV_ACT_F32 && action_dtype != DOCKAUV_ACT_F64) return fail(DOCKAUV_EINVAL, "bad action dtype");
     DeviceGuard guard(h->device);
     const int64_t N = h->n_envs;
@@ -799,6 +1010,16 @@ static int rollout_issue(DockauvHandle *h, const void *actions, int action_dtype
         so.delta_d_out = o.delta_d_out ? (char *)o.delta_d_out + esz * (size_t)N * t : nullptr;
         return so;
     };
+    if (h->tap.n > 0) {
+        // the taps need one pre-step snapshot per step, so every step is forked and joined on its own (the halves of a
+        // batch stepped in parts cannot run their T steps as one chain each)
+        for (int t = 0; t < n_steps; t++) {
+            const DockauvStepOut so = out_of_step(t);
+            int rc = step_call(h, (const char *)actions + arow * t, action_dtype, nullptr, &so, nullptr, auto_reset, st, false);
+            if (rc != DOCKAUV_OK) return rc;
+        }
+        return DOCKAUV_OK;
+    }
     if (steps_in_parts(h)) {
         // envs never interact and the actions are all known: each part of the batch runs its T steps as ONE chain on
         // its own stream, forked from / joined to the caller's stream once per rollout instead of once per step
@@ -879,6 +1100,139 @@ extern "C" int dockauv_rollout(DockauvHandle *h, const void *actions_dev, int ac
     }
     CUDA_TRY(cudaGraphLaunch(h->rg_exec, st));
     h->launches += h->rg_launches;
+    return DOCKAUV_OK;
+}
+
+// ------------------------------------------------------------------------------------------- episode taps: setup
+extern "C" int dockauv_set_taps(DockauvHandle *h, const int64_t *env_ids_host, int n_taps, int capacity,
+                                const DockauvTapBuffers *bufs) {
+    if (!h) return fail(DOCKAUV_EINVAL, "null handle");
+    if (!h->bound) return fail(DOCKAUV_ESTATE, "dockauv_bind must be called before dockauv_set_taps");
+    if (n_taps < 0 || n_taps > DOCKAUV_MAX_TAPS)
+        return fail(DOCKAUV_EINVAL, "n_taps must be in 0..%d, got %d", DOCKAUV_MAX_TAPS, n_taps);
+    if (n_taps > 0) {
+        if (capacity < 1) return fail(DOCKAUV_EINVAL, "capacity must be at least 1, got %d", capacity);
+        if (!env_ids_host || !bufs) return fail(DOCKAUV_EINVAL, "null env ids or tap buffers");
+        const DockauvTapBuffers &b = *bufs;
+        const void *need[] = {b.count, b.pre_state, b.pre_current, b.pre_scene, b.pre_t_steps, b.pre_episode,
+                              b.pre_ep_return, b.state, b.u, b.state_dot, b.nu_c, b.ray_dist, b.reward_arr, b.obs,
+                              b.reward, b.done, b.cond_bits};
+        for (const void *q : need)
+            if (!q) return fail(DOCKAUV_EINVAL, "a tap buffer is null");
+        std::vector<int64_t> ids(env_ids_host, env_ids_host + n_taps);
+        for (int64_t i : ids)
+            if (i < 0 || i >= h->n_envs)
+                return fail(DOCKAUV_EINVAL, "tap env id %lld out of range 0..%lld", (long long)i, (long long)h->n_envs - 1);
+        std::sort(ids.begin(), ids.end());
+        for (size_t k = 1; k < ids.size(); k++)
+            if (ids[k] == ids[k - 1]) return fail(DOCKAUV_EINVAL, "tap env id %lld given twice", (long long)ids[k]);
+    }
+    DeviceGuard guard(h->device);
+    auto &tp = h->tap;
+    CUDA_TRY(cudaDeviceSynchronize());      // the side branch of an earlier step may still read the old shadow
+    drop_graphs(h);
+    if (tp.mem) CUDA_TRY(cudaFree(tp.mem));
+    tp.mem = nullptr;
+    tp.n = 0;
+    if (n_taps == 0) return DOCKAUV_OK;
+    if (!tp.st) CUDA_TRY(cudaStreamCreateWithFlags(&tp.st, cudaStreamNonBlocking));
+    if (!tp.ev_fork) CUDA_TRY(cudaEventCreateWithFlags(&tp.ev_fork, cudaEventDisableTiming));
+    if (!tp.ev_join) CUDA_TRY(cudaEventCreateWithFlags(&tp.ev_join, cudaEventDisableTiming));
+    if (!tp.dst) CUDA_TRY(cudaStreamCreateWithFlags(&tp.dst, cudaStreamNonBlocking));
+    if (!tp.ev_dbg) CUDA_TRY(cudaEventCreateWithFlags(&tp.ev_dbg, cudaEventDisableTiming));
+    const size_t K = (size_t)n_taps, esz = h->params.precision == DOCKAUV_F64 ? 8 : 4;
+    const int nu = h->params.n_u, nc = h->params.n_capsules, ns = h->params.n_spheres, n_rays = h->params.n_rays;
+    const bool pipe = h->pipe_buf != nullptr;
+    const int n_obsf = pipe ? h->kd.n_obsf : 0;
+    tp.n_gather = 12 + nu + 3 + 1 + 5 + 7 * nc + 4 * ns + 3 + n_obsf;
+    tp.shadow_launches = resolve_layout(h) == DOCKAUV_LAYOUT_PIPELINE ? pipe_launches(h->kd) : 1;
+    tp.n_commit = 12 + nu + 12 + 3 + n_rays + 13 + 3 + h->n_obs;
+    // one allocation, every piece 256-byte aligned (observation rows are written with 16-byte stores)
+    size_t off = 0;
+    auto take = [&](size_t bytes) {
+        const size_t o = off;
+        off += (bytes + 255) & ~(size_t)255;
+        return o;
+    };
+    // one K-env set of persistent state (both shadows have one)
+    struct Shadow {
+        size_t state, u, goal, hg, cur, caps, sph, epr, ts, ep;
+    };
+    auto take_shadow = [&]() {
+        Shadow o;
+        o.state = take(12 * K * esz); o.u = take(nu * K * esz); o.goal = take(3 * K * esz); o.hg = take(K * esz);
+        o.cur = take(5 * K * esz); o.caps = take((size_t)std::max(7 * nc, 1) * K * esz);
+        o.sph = take((size_t)std::max(4 * ns, 1) * K * esz); o.epr = take(K * esz); o.ts = take(4 * K); o.ep = take(4 * K);
+        return o;
+    };
+    const Shadow os = take_shadow(), od = take_shadow();
+    const size_t o_noise = take(K * esz), o_act = take(8 * nu * K), o_obs = take(4 * K * h->n_obs),
+                 o_rew = take(K * esz), o_done = take(K), o_cond = take(K), o_dobs = take(4 * K * h->n_obs),
+                 o_drew = take(K * esz), o_ddone = take(K), o_dcond = take(K), o_ray = take(n_rays * K * esz),
+                 o_rarr = take(13 * K * esz), o_nuc = take(3 * K * esz), o_sdot = take(12 * K * esz),
+                 o_stats = take(kStatsBytes), o_ids = take(8 * K), o_sync = take(4),
+                 o_grows = take(sizeof(TapRow) * tp.n_gather), o_crows = take(sizeof(TapRow) * tp.n_commit);
+    // the pipeline layout's buffers for K envs, as dockauv_create lays them out for n_envs: records, float obstacle
+    // records, three view lists + the ended list, one counter block per 128 envs
+    size_t o_rec = 0, o_obsf = 0, o_list = 0, o_end = 0, o_cnt = 0;
+    if (pipe) {
+        o_rec = take(16 * esz * K);
+        o_obsf = take(16 * (size_t)std::max(n_obsf, 1) * K);
+        o_list = take(3 * 8 * K);
+        o_end = take(4 * ((K + 1) & ~(size_t)1));
+        o_cnt = take(4 * 16 * (K / 128 + 2));
+    }
+    CUDA_TRY(cudaMalloc(&tp.mem, off));
+    CUDA_TRY(cudaMemset(tp.mem, 0, off));
+    char *m = (char *)tp.mem;
+    auto place = [&](DockauvBuffers &b, const Shadow &o) {
+        b.state = m + o.state; b.u_prev = m + o.u; b.goal = m + o.goal; b.heading_goal = m + o.hg; b.current = m + o.cur;
+        b.capsules = m + o.caps; b.spheres = m + o.sph; b.ep_return = m + o.epr;
+        b.t_steps = (int32_t *)(m + o.ts); b.episode = (int32_t *)(m + o.ep);
+    };
+    place(tp.shadow, os);
+    place(tp.dshadow, od);
+    tp.noise = m + o_noise;
+    tp.actions = m + o_act;
+    memset(&tp.out, 0, sizeof(tp.out));
+    tp.out.obs = (float *)(m + o_obs);
+    tp.out.reward = m + o_rew;
+    tp.out.done = (uint8_t *)(m + o_done);
+    tp.out.cond_bits = (uint8_t *)(m + o_cond);
+    memset(&tp.dout, 0, sizeof(tp.dout));
+    tp.dout.obs = (float *)(m + o_dobs);
+    tp.dout.reward = m + o_drew;
+    tp.dout.done = (uint8_t *)(m + o_ddone);
+    tp.dout.cond_bits = (uint8_t *)(m + o_dcond);
+    tp.rec = pipe ? m + o_rec : nullptr;
+    tp.obsf = pipe && n_obsf > 0 ? (float4 *)(m + o_obsf) : nullptr;
+    tp.view_list = pipe ? (unsigned long long *)(m + o_list) : nullptr;
+    tp.ended_list = pipe ? (uint32_t *)(m + o_end) : nullptr;
+    tp.view_count = pipe ? (unsigned int *)(m + o_cnt) : nullptr;
+    memset(&tp.dbg, 0, sizeof(tp.dbg));
+    tp.dbg.ray_dist = m + o_ray;
+    tp.dbg.reward_arr = m + o_rarr;
+    tp.dbg.nu_c = m + o_nuc;
+    tp.dbg.state_dot = m + o_sdot;
+    tp.stats = (double *)(m + o_stats);
+    tp.ids = (int64_t *)(m + o_ids);
+    tp.sync = (unsigned int *)(m + o_sync);
+    tp.gather_rows = (TapRow *)(m + o_grows);
+    tp.commit_rows = (TapRow *)(m + o_crows);
+    tp.n = n_taps;
+    tp.capacity = capacity;
+    tp.ring = *bufs;
+    int rc = build_tap_rows(h);
+    cudaError_t e = cudaSuccess;
+    if (rc == DOCKAUV_OK) e = cudaMemcpy(tp.ids, env_ids_host, 8 * K, cudaMemcpyHostToDevice);
+    if (rc == DOCKAUV_OK && e == cudaSuccess) e = cudaMemset(bufs->count, 0, sizeof(int64_t));
+    if (rc == DOCKAUV_OK && e == cudaSuccess) e = cudaDeviceSynchronize();
+    if (rc != DOCKAUV_OK || e != cudaSuccess) {
+        cudaFree(tp.mem);
+        tp.mem = nullptr;
+        tp.n = 0;
+        return rc != DOCKAUV_OK ? rc : fail(DOCKAUV_ECUDA, "tap setup failed: %s", cudaGetErrorString(e));
+    }
     return DOCKAUV_OK;
 }
 

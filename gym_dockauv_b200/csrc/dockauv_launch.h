@@ -36,4 +36,35 @@ inline int pipe_launches(const KParams<T> &k) {
 template <typename T>
 cudaError_t launch_refresh_obstacles(const KParams<T> &k, cudaStream_t st);
 
+// Episode taps (dockauv_set_taps).  One TapRow copies one component row of K values: element k of `src` (at byte
+// k * src_step, or env_id * src_step when src_by_id) goes to `dst` and `dst2` (byte k * dst_step, nullable) and to the
+// ring slot `*count % capacity` of `ring` (byte slot * ring_slot + k * dst_step, nullable).  esz: 1, 4, 8 or 16 bytes.
+struct TapRow {
+    const char *src;
+    char *dst, *dst2, *ring;
+    int64_t ring_slot;
+    int32_t esz, src_step, dst_step, src_by_id;
+};
+struct TapLaunch {
+    const TapRow *rows;        // device table
+    int32_t n_rows, n_taps;
+    const int64_t *ids;        // local env ids of the taps (device)
+    int64_t *count;            // caller's record counter
+    int64_t capacity;
+    unsigned int *sync;        // commit: CTAs done so far (the last one bumps *count and zeroes it)
+    // gather only: the step's actions and current noise for the shadow
+    const void *actions;
+    int32_t act_f32, n_u;
+    void *shadow_actions;      // [K][n_u] in the actions' dtype
+    const void *noise;         // real[N] of the caller, nullable
+    void *shadow_noise;        // real[K]
+};
+// pre-step rows of the tapped envs -> shadow + ring, and the shadow's actions and noise (the Philox draw of dyn_current
+// for the real env id when the caller passes no noise)
+template <typename T>
+cudaError_t launch_tap_gather(const KParams<T> &k, const TapLaunch &t, cudaStream_t st);
+// shadow results -> ring slot, then ++*count on the device
+template <typename T>
+cudaError_t launch_tap_commit(const KParams<T> &k, const TapLaunch &t, cudaStream_t st);
+
 }  // namespace dockauv

@@ -22,8 +22,8 @@ import torch
 
 from . import _capi
 from .config import BASE_CONFIG, REGISTRATION_DICT
-from .params import (ACT_F32, ACT_F64, F32, F64, N_STATS, SCENARIO_IDS, STAT_NAMES, DockauvBuffers, DockauvDebugOut,
-                     DockauvRolloutOut, DockauvStepOut, pack_params)
+from .params import (ACT_F32, ACT_F64, F32, F64, MAX_TAPS, N_STATS, SCENARIO_IDS, STAT_NAMES, TAP_FIELDS, DockauvBuffers,
+                     DockauvDebugOut, DockauvRolloutOut, DockauvStepOut, DockauvTapBuffers, pack_params)
 
 DONE_NAMES = ("Done-Goal_reached", "Done-out_pos", "Done-out_att", "Done-max_t", "Done-collision")
 
@@ -140,6 +140,7 @@ class BaseDocking3d:
             self._dbg = DockauvDebugOut(*[_ptr(self.debug[k]) for k in ("ray_dist", "reward_arr", "euler_dot", "nu_c",
                                                                        "nav", "obs_f64", "state_dot")])
         self._host = None
+        self.taps = None
         self.t_total_steps = 0
 
     # ------------------------------------------------------------------ lifecycle
@@ -308,6 +309,40 @@ class BaseDocking3d:
                                                 int(self.auto_reset), C.byref(self._out)))
         self.t_total_steps += 1
         return hb["obs"].numpy(), hb["reward"].numpy(), hb["done"].numpy().view(np.bool_), {"cond_bits": hb["cond"].numpy()}
+
+    # ------------------------------------------------------------------ episode taps (dockauv_set_taps)
+    def set_taps(self, env_ids, capacity):
+        """Record every following ``step`` / ``step_into`` / ``rollout`` of the envs ``env_ids`` (local indices, at most
+        1024) into a device ring of ``capacity`` steps, without changing any env's trajectory or output.  Returns the
+        ring: a dict of device tensors, ``count`` (int64[1], steps recorded so far; step j sits in slot j % capacity)
+        and per slot the pre-step inputs (``pre_state`` [S, 12, K], ``pre_current``, ``pre_scene`` (goal, heading goal,
+        capsules, spheres), ``pre_t_steps``, ``pre_episode``, ``pre_ep_return``) and the post-step values before any
+        auto-reset (``state``, ``u``, ``state_dot``, ``nu_c``, ``ray_dist``, ``reward_arr`` [S, n, K], ``obs``
+        [S, K, n_obs], ``reward``, ``done``, ``cond_bits`` [S, K]).  ``step_host`` refuses to run while taps are set."""
+        ids = [int(i) for i in env_ids]
+        K, S = len(ids), int(capacity)
+        if not 0 < K <= MAX_TAPS:
+            raise ValueError(f"between 1 and {MAX_TAPS} env ids, got {K}")
+        dev, dt = self.device, self.dtype
+        z = lambda *shape, dtype=dt: torch.zeros(*shape, dtype=dtype, device=dev)  # noqa: E731
+        n_scene = 4 + 7 * self.n_capsules + 4 * self.n_spheres
+        ring = dict(count=z(1, dtype=torch.int64), pre_state=z(S, 12, K), pre_current=z(S, 5, K),
+                    pre_scene=z(S, n_scene, K), pre_t_steps=z(S, K, dtype=torch.int32),
+                    pre_episode=z(S, K, dtype=torch.int32), pre_ep_return=z(S, K), state=z(S, 12, K),
+                    u=z(S, self.n_actions, K), state_dot=z(S, 12, K), nu_c=z(S, 3, K), ray_dist=z(S, self.n_rays, K),
+                    reward_arr=z(S, 13, K), obs=z(S, K, self.n_observations, dtype=torch.float32), reward=z(S, K),
+                    done=z(S, K, dtype=torch.uint8), cond_bits=z(S, K, dtype=torch.uint8))
+        bufs = DockauvTapBuffers(*[_ptr(ring[k]) for k in TAP_FIELDS])
+        id_arr = (C.c_int64 * K)(*ids)
+        torch.cuda.current_stream(dev).synchronize()      # the ring tensors are zero-filled on the current stream
+        _capi.check(self._lib.dockauv_set_taps(self._handle, id_arr, K, S, C.byref(bufs)))
+        self.taps = dict(ring, env_ids=ids, capacity=S)
+        return self.taps
+
+    def clear_taps(self):
+        """Remove the taps: the next steps are launched exactly as without them."""
+        _capi.check(self._lib.dockauv_set_taps(self._handle, None, 0, 0, None))
+        self.taps = None
 
     # ------------------------------------------------------------------ exact-state injection (parity tests, resume)
     def set_state(self, state=None, u_prev=None, goal=None, heading_goal=None, current=None, capsules=None,

@@ -12,8 +12,9 @@ import numpy as np
 from . import vehicles as _veh
 from .config import validate
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 MAX_U, MAX_CAPSULES, MAX_SPHERES, MAX_RAYS, N_REWARDS, N_STATS = 8, 8, 8, 256, 13, 16
+MAX_TAPS = 1024
 F64, F32 = 0, 1
 ACT_F64, ACT_F32 = 0, 1
 LAYOUTS = {"auto": 0, "thread_per_env": 1, "warp_rays": 2, "pipeline": 4}
@@ -67,6 +68,14 @@ class DockauvDebugOut(C.Structure):
 class DockauvRolloutOut(C.Structure):
     _fields_ = [(k, C.c_void_p) for k in ("obs", "reward", "done", "cond_bits", "terminal_obs", "ep_return_out",
                                           "ep_len_out", "delta_d_out")]
+
+
+TAP_FIELDS = ("count", "pre_state", "pre_current", "pre_scene", "pre_t_steps", "pre_episode", "pre_ep_return", "state",
+              "u", "state_dot", "nu_c", "ray_dist", "reward_arr", "obs", "reward", "done", "cond_bits")
+
+
+class DockauvTapBuffers(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in TAP_FIELDS]
 
 
 def skew(a):

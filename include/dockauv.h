@@ -23,14 +23,16 @@
  *   dockauv_gae                        RolloutBuffer.compute_returns_and_advantage of the PPO caller
  *                                      (stable-baselines3 1.5.0, requirements.txt; selected at train.py:64)
  *   DockauvDebugOut (state_dot, ...)   EpisodeDataStorage.update          utils/datastorage.py:268-288
+ *   dockauv_set_taps                   the same, during training: every step of a few chosen envs recorded on
+ *                                      the device (interval_datastorage, config.py; datastorage.py:268-288)
  *
  * Conventions
  *   - plain C types only; no torch / C++ types cross this boundary.
  *   - all `*_dev` pointers are device pointers on the handle's device.  The library never allocates, frees
  *     or keeps caller buffers beyond what dockauv_bind() registered; the caller (PyTorch) owns them.  The
  *     handle owns its ray table, the statistics vector, the buffers between the launches of a step
- *     (a 16-word record, the ray list entry and a float copy of the obstacles: ~350 bytes per env) and, lazily, device
- *     staging for dockauv_step_host.
+ *     (a 16-word record, the ray list entry and a float copy of the obstacles: ~350 bytes per env), lazily, device
+ *     staging for dockauv_step_host and, while taps are set (dockauv_set_taps), shadow copies of the tapped envs.
  *   - `stream` is a cudaStream_t passed as void* (0 = legacy default stream).  Calls are asynchronous and
  *     stream-ordered; one handle must not be used from two threads at once.  Large batches (>= 131,072 envs)
  *     are stepped as two halves on two handle-owned streams that are forked from / joined to `stream` by
@@ -52,7 +54,7 @@
 extern "C" {
 #endif
 
-#define DOCKAUV_ABI_VERSION 3
+#define DOCKAUV_ABI_VERSION 4
 
 #if defined(__GNUC__)
 #define DOCKAUV_API __attribute__((visibility("default")))
@@ -220,6 +222,24 @@ typedef struct DockauvRolloutOut {
     void *delta_d_out;     /* real[T][N], nullable */
 } DockauvRolloutOut;
 
+/* Ring of per-step records of the tapped envs (dockauv_set_taps): caller-owned device buffers.  S = capacity,
+ * K = n_taps, real = handle precision; component-major inside a slot, tap index fastest. */
+#define DOCKAUV_MAX_TAPS 1024
+typedef struct DockauvTapBuffers {
+    int64_t *count;        /* int64[1]: steps recorded since dockauv_set_taps; the next record goes to slot count % S */
+    /* pre-step inputs of the tapped envs (what the real step read) */
+    void *pre_state;       /* real[S][12][K] */
+    void *pre_current;     /* real[S][5][K] */
+    void *pre_scene;       /* real[S][4 + 7*n_capsules + 4*n_spheres][K]: goal[3], heading_goal, capsules, spheres */
+    int32_t *pre_t_steps, *pre_episode;   /* int32[S][K] */
+    void *pre_ep_return;   /* real[S][K] */
+    /* post-step values, before any auto-reset */
+    void *state, *u, *state_dot, *nu_c, *ray_dist, *reward_arr;   /* real[S][12|n_u|12|3|n_rays|13][K] */
+    float *obs;            /* f32[S][K][n_obs]: the real observation, also for envs whose episode ended */
+    void *reward;          /* real[S][K] */
+    uint8_t *done, *cond_bits;            /* u8[S][K] */
+} DockauvTapBuffers;
+
 typedef struct DockauvHandle DockauvHandle;
 
 DOCKAUV_API int dockauv_abi_version(void);
@@ -275,6 +295,19 @@ DOCKAUV_API int dockauv_step_host(DockauvHandle *h, const void *actions_host, in
  * Stochastic-current handles draw their noise from the handle's Philox stream. */
 DOCKAUV_API int dockauv_rollout(DockauvHandle *h, const void *actions_dev, int action_dtype, int n_steps,
                     const DockauvRolloutOut *out, int auto_reset, int use_graph, void *stream);
+
+/* Record the envs env_ids_host[0..n_taps) (local indices, distinct, < n_envs, n_taps <= DOCKAUV_MAX_TAPS) on every
+ * following dockauv_step / dockauv_rollout into the ring `bufs` (capacity slots); n_taps = 0 removes the taps (capacity
+ * and bufs are then ignored).  Zeroes *bufs->count and drops the cached step and rollout graphs.
+ * Each step first copies the tapped envs' pre-step state into the ring and into two handle-owned K-env shadows (one
+ * launch on `stream`, before the step).  On a handle-owned side stream that joins `stream` before the call returns, one
+ * shadow is stepped by the handle's own layout with the real step's inputs (so obs, reward, done, cond_bits, state and u
+ * are exactly the real step's, before any auto-reset), the other by the single-launch kernel with debug outputs
+ * (state_dot, nu_c, ray_dist, reward_arr); both without auto-reset.  Their results are copied to the ring slot, after
+ * which *count is incremented on the device.  The real step and its outputs are left exactly as they are without taps.
+ * dockauv_step_host refuses to run while taps are set (DOCKAUV_ESTATE): taps record device-driven steps. */
+DOCKAUV_API int dockauv_set_taps(DockauvHandle *h, const int64_t *env_ids_host, int n_taps, int capacity,
+                                 const DockauvTapBuffers *bufs);
 
 /* Generalised advantage estimation over a stacked rollout, one thread per env walking t = T-1 .. 0
  * (float32 like the caller's RolloutBuffer):
