@@ -137,9 +137,11 @@ struct DockauvHandle {
         DockauvStepOut out = {};       // obs, reward, done, cond_bits of `shadow`
         DockauvStepOut dout = {};      // the same of `dshadow` (not recorded)
         DockauvDebugOut dbg = {};      // ray_dist, reward_arr, nu_c, state_dot of `dshadow`
-        // pipeline layout: the shadow's own per-env records, float obstacle records, work lists and counters
+        // pipeline layout: the shadow's own per-env records, float obstacle records, obstacle rows, work lists and
+        // counters
         void *rec = nullptr;
         float4 *obsf = nullptr;
+        void *obsd = nullptr;
         unsigned long long *view_list = nullptr;
         uint32_t *ended_list = nullptr;
         unsigned int *view_count = nullptr;
@@ -360,11 +362,14 @@ extern "C" int dockauv_create(const DockauvParams *p, int64_t n_envs, int device
     }
     if (p->layout == DOCKAUV_LAYOUT_PIPELINE || p->layout == DOCKAUV_LAYOUT_AUTO) {
         // library-owned buffers of the pipeline layout: per-env record T[16] (128-byte aligned), float obstacle records
-        // float4[2 n_caps + n_sph], the ray list u64 and one list counter per 128 envs
+        // float4[2 n_caps + n_sph], obstacle rows T[n_caps + n_sph][8] (256-byte aligned), the ray list u64 and one list
+        // counter per 128 envs
         const size_t esz = p->precision == DOCKAUV_F64 ? 8 : 4;
         const size_t n = (size_t)n_envs;
-        const int n_obsf = 2 * p->n_capsules + p->n_spheres;
-        const size_t off_rec = 0, off_obsf = off_rec + 16 * esz * n, off_list = off_obsf + 16 * (size_t)n_obsf * n;
+        const int n_obsf = 2 * p->n_capsules + p->n_spheres, n_obst = p->n_capsules + p->n_spheres;
+        const size_t off_rec = 0, off_obsf = off_rec + 16 * esz * n;
+        const size_t off_obsd = (off_obsf + 16 * (size_t)n_obsf * n + 255) & ~(size_t)255;
+        const size_t off_list = off_obsd + 8 * esz * (size_t)n_obst * n;
         const size_t off_end = off_list + 3 * 8 * n, off_cnt = off_end + 4 * ((n + 1) & ~(size_t)1);      // three view lists
         const size_t n_cnt = 16 * (n / 128 + 2);     // counter block (kCounterStride words) per concurrently stepped env range
         cudaError_t e5 = cudaMalloc(&h->pipe_buf, off_cnt + 4 * n_cnt);
@@ -381,6 +386,8 @@ extern "C" int dockauv_create(const DockauvParams *p, int64_t n_envs, int device
         h->kf.rec = (float *)(base + off_rec);
         h->kd.obsf = h->kf.obsf = n_obsf > 0 ? (float4 *)(base + off_obsf) : nullptr;
         h->kd.n_obsf = h->kf.n_obsf = n_obsf;
+        h->kd.obsd = n_obst > 0 ? (double *)(base + off_obsd) : nullptr;
+        h->kf.obsd = n_obst > 0 ? (float *)(base + off_obsd) : nullptr;
         h->kd.view_list = h->kf.view_list = (unsigned long long *)(base + off_list);
         h->kd.ended_list = h->kf.ended_list = (uint32_t *)(base + off_end);
         h->kd.view_count = h->kf.view_count = (unsigned int *)(base + off_cnt);
@@ -464,6 +471,22 @@ static int build_tap_rows(DockauvHandle *h) {
     // the real step's float obstacle records (pipeline layout): the shadow culls exactly what the real step culls
     if (tp.obsf)
         for (int k = 0; k < h->kd.n_obsf; k++) gather(h->kd.obsf, tp.obsf, nullptr, k, 16, nullptr, 0, 0);
+    // and its obstacle rows (env-major: 16-byte piece j of every tapped env's rows, one env's rows apart)
+    if (tp.obsd) {
+        const int row_bytes = 8 * esz * (nc + ns);
+        for (int j = 0; j < row_bytes / 16; j++) {
+            TapRow t;
+            t.src = (const char *)h->kd.obsd + 16 * j;
+            t.dst = (char *)tp.obsd + 16 * j;
+            t.dst2 = nullptr;
+            t.ring = nullptr;
+            t.ring_slot = 0;
+            t.esz = 16;
+            t.src_step = t.dst_step = row_bytes;
+            t.src_by_id = 1;
+            g.push_back(t);
+        }
+    }
     // one committed row: row `comp` of a shadow field (tap-indexed, `step` bytes apart) -> row `comp` of a ring field
     auto commit = [&](const void *src, void *ring, int comp, int e, int rows, int step) {
         TapRow t;
@@ -654,6 +677,7 @@ static cudaError_t tap_issue(DockauvHandle *h, const KParams<T> &real, const voi
     k.stats = tp.stats;
     k.rec = (T *)tp.rec;
     k.obsf = tp.obsf;
+    k.obsd = (T *)tp.obsd;
     k.view_list = tp.view_list;
     k.ended_list = tp.ended_list;
     k.view_count = tp.view_count;
@@ -665,6 +689,7 @@ static cudaError_t tap_issue(DockauvHandle *h, const KParams<T> &real, const voi
     set_io<T>(d, tp.actions, action_dtype == DOCKAUV_ACT_F32, tp.noise, tp.dout, &tp.dbg, 0);
     d.rec = nullptr;
     d.obsf = nullptr;
+    d.obsd = nullptr;
     d.view_list = nullptr;
     d.ended_list = nullptr;
     d.view_count = nullptr;
@@ -1144,7 +1169,8 @@ extern "C" int dockauv_set_taps(DockauvHandle *h, const int64_t *env_ids_host, i
     const int nu = h->params.n_u, nc = h->params.n_capsules, ns = h->params.n_spheres, n_rays = h->params.n_rays;
     const bool pipe = h->pipe_buf != nullptr;
     const int n_obsf = pipe ? h->kd.n_obsf : 0;
-    tp.n_gather = 12 + nu + 3 + 1 + 5 + 7 * nc + 4 * ns + 3 + n_obsf;
+    const size_t row_bytes = 8 * esz * (size_t)(nc + ns);      // one env's obstacle rows
+    tp.n_gather = 12 + nu + 3 + 1 + 5 + 7 * nc + 4 * ns + 3 + n_obsf + (pipe ? (int)(row_bytes / 16) : 0);
     tp.shadow_launches = resolve_layout(h) == DOCKAUV_LAYOUT_PIPELINE ? pipe_launches(h->kd) : 1;
     tp.n_commit = 12 + nu + 12 + 3 + n_rays + 13 + 3 + h->n_obs;
     // one allocation, every piece 256-byte aligned (observation rows are written with 16-byte stores)
@@ -1173,11 +1199,12 @@ extern "C" int dockauv_set_taps(DockauvHandle *h, const int64_t *env_ids_host, i
                  o_stats = take(kStatsBytes), o_ids = take(8 * K), o_sync = take(4),
                  o_grows = take(sizeof(TapRow) * tp.n_gather), o_crows = take(sizeof(TapRow) * tp.n_commit);
     // the pipeline layout's buffers for K envs, as dockauv_create lays them out for n_envs: records, float obstacle
-    // records, three view lists + the ended list, one counter block per 128 envs
-    size_t o_rec = 0, o_obsf = 0, o_list = 0, o_end = 0, o_cnt = 0;
+    // records, obstacle rows, three view lists + the ended list, one counter block per 128 envs
+    size_t o_rec = 0, o_obsf = 0, o_obsd = 0, o_list = 0, o_end = 0, o_cnt = 0;
     if (pipe) {
         o_rec = take(16 * esz * K);
         o_obsf = take(16 * (size_t)std::max(n_obsf, 1) * K);
+        o_obsd = take(std::max(row_bytes, (size_t)16) * K);
         o_list = take(3 * 8 * K);
         o_end = take(4 * ((K + 1) & ~(size_t)1));
         o_cnt = take(4 * 16 * (K / 128 + 2));
@@ -1206,6 +1233,7 @@ extern "C" int dockauv_set_taps(DockauvHandle *h, const int64_t *env_ids_host, i
     tp.dout.cond_bits = (uint8_t *)(m + o_dcond);
     tp.rec = pipe ? m + o_rec : nullptr;
     tp.obsf = pipe && n_obsf > 0 ? (float4 *)(m + o_obsf) : nullptr;
+    tp.obsd = pipe && n_obsf > 0 ? m + o_obsd : nullptr;
     tp.view_list = pipe ? (unsigned long long *)(m + o_list) : nullptr;
     tp.ended_list = pipe ? (uint32_t *)(m + o_end) : nullptr;
     tp.view_count = pipe ? (unsigned int *)(m + o_cnt) : nullptr;

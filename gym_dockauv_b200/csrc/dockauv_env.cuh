@@ -6,11 +6,61 @@
 namespace dockauv {
 
 // ------------------------------------------------------------------------------------------- reset
-// Float obstacle records of env i for the cull code (KParams::obsf, see cull_pair_rec), from the obstacles and the
-// goal as they are stored (T).  Capsule k -> slots 2k, 2k+1; sphere s -> slot 2 n_caps + s.
+// Env-major obstacle rows (KParams::obsd): obstacle k of env i (capsules first, then sphere k - n_caps) as stored,
+// zero-filled to eight words, moved as 16-byte pieces (4 in f64, 2 in f32)
+constexpr int kObstRowWords = 8;
+
+template <typename T>
+__device__ __forceinline__ T *obstacle_row(const KParams<T> &p, int64_t i, int k) {
+    return p.obsd + (i * (p.n_caps + p.n_sph) + k) * kObstRowWords;
+}
+
+template <typename T>
+__device__ __forceinline__ void load_obstacle_row(const T *row, T o[kObstRowWords]) {
+    if constexpr (sizeof(T) == 8) {
+        const double2 *s = reinterpret_cast<const double2 *>(row);
+#pragma unroll
+        for (int c = 0; c < 4; c++) {
+            const double2 v = s[c];
+            o[2 * c] = v.x;
+            o[2 * c + 1] = v.y;
+        }
+    } else {
+        const float4 *s = reinterpret_cast<const float4 *>(row);
+#pragma unroll
+        for (int c = 0; c < 2; c++) {
+            const float4 v = s[c];
+            o[4 * c] = v.x;
+            o[4 * c + 1] = v.y;
+            o[4 * c + 2] = v.z;
+            o[4 * c + 3] = v.w;
+        }
+    }
+}
+
+template <typename T>
+__device__ __forceinline__ void store_obstacle_row(T *row, const T o[kObstRowWords]) {
+    if constexpr (sizeof(T) == 8) {
+        double2 *d = reinterpret_cast<double2 *>(row);
+#pragma unroll
+        for (int c = 0; c < 4; c++) d[c] = make_double2(o[2 * c], o[2 * c + 1]);
+    } else {
+        float4 *d = reinterpret_cast<float4 *>(row);
+#pragma unroll
+        for (int c = 0; c < 2; c++) d[c] = make_float4(o[4 * c], o[4 * c + 1], o[4 * c + 2], o[4 * c + 3]);
+    }
+}
+
+// Obstacle rows (KParams::obsd) and float obstacle records of env i for the cull code (KParams::obsf, see
+// cull_pair_rec), from the obstacles and the goal as they are stored (T).  Float records: capsule k -> slots 2k, 2k+1;
+// sphere s -> slot 2 n_caps + s.  The pipeline layout allocates both or neither.
 template <typename T>
 __device__ __forceinline__ void store_capsule_record(const KParams<T> &p, int64_t i, int k, const T cap[7], const T goal[3]) {
     if (p.obsf == nullptr) return;
+    {
+        const T row[kObstRowWords] = {cap[0], cap[1], cap[2], cap[3], cap[4], cap[5], cap[6], T(0)};
+        store_obstacle_row<T>(obstacle_row<T>(p, i, k), row);
+    }
     const double ob[7] = {(double)cap[0], (double)cap[1], (double)cap[2], (double)cap[3], (double)cap[4], (double)cap[5], (double)cap[6]};
     const double g[3] = {(double)goal[0], (double)goal[1], (double)goal[2]};
     float4 q0, q1;
@@ -22,6 +72,10 @@ __device__ __forceinline__ void store_capsule_record(const KParams<T> &p, int64_
 template <typename T>
 __device__ __forceinline__ void store_sphere_record(const KParams<T> &p, int64_t i, int s, const T sph[4], const T goal[3]) {
     if (p.obsf == nullptr) return;
+    {
+        const T row[kObstRowWords] = {sph[0], sph[1], sph[2], sph[3], T(0), T(0), T(0), T(0)};
+        store_obstacle_row<T>(obstacle_row<T>(p, i, p.n_caps + s), row);
+    }
     const double ob[7] = {(double)sph[0], (double)sph[1], (double)sph[2], (double)sph[3], 0.0, 0.0, 0.0};
     const double g[3] = {(double)goal[0], (double)goal[1], (double)goal[2]};
     float4 q0, q1;
@@ -29,7 +83,7 @@ __device__ __forceinline__ void store_sphere_record(const KParams<T> &p, int64_t
     p.obsf[(int64_t)(2 * p.n_caps + s) * p.n_envs + i] = q0;
 }
 
-// Rebuilds the float obstacle records of env i from the bound buffers (after the caller wrote obstacles or goals itself:
+// Rebuilds the obstacle rows and float obstacle records of env i from the bound buffers (after the caller wrote obstacles or goals itself:
 // dockauv_refresh_obstacles).
 template <typename T>
 __global__ void refresh_obstacles_kernel(const __grid_constant__ KParams<T> p) {

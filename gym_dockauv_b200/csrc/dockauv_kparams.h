@@ -59,19 +59,25 @@ struct KParams {
     // debug outputs
     T *dbg_ray_dist, *dbg_reward_arr, *dbg_euler_dot, *dbg_nu_c, *dbg_nav, *dbg_obs, *dbg_state_dot;
     // pipeline layout (library-owned buffers):
-    //   rec      T[n_envs][16], one 16-word record per env written by the dynamics launch (AoS: the ray launch reads
-    //            it with one request per warp): 0..5 sin/cos of the post-step attitude (sphi cphi sth cth spsi cpsi),
-    //            6..8 post-step position relative to the goal, 9 (r0+r1)+(r2+r3), 10 r4+r5, 11 r7 (reward terms that
-    //            need no radar, already combined in numpy's summation order), 12 log_precision(delta_d), 13 delta_d,
-    //            14 done-condition bits 0..2 as a number, 15 NaN poison word (0 for a finite pose)
+    //   rec      T[n_envs][16], one 16-word record per env written by the dynamics launch (AoS: one 128-byte line in
+    //            f64): 0..5 sin/cos of the post-step attitude (sphi cphi sth cth spsi cpsi), 6..8 post-step position
+    //            relative to the goal, 9 (r0+r1)+(r2+r3), 10 r4+r5, 11 r7 (reward terms that need no radar, already
+    //            combined in numpy's summation order), 12 log_precision(delta_d), 13 delta_d, 14 done-condition bits
+    //            0..2 as a number, 15 NaN poison word (0 for a finite pose).  The record of a LISTED env, as the ray launch
+    //            reads it, holds everything that launch needs besides the obstacle rows: words 6..8 are the post-step
+    //            position itself and word 14 the running return before this step (REC_POS, REC_EPR)
     //   obsf     float4[n_obsf][n_envs]: float copy of the obstacles RELATIVE TO THE GOAL for the cull (written by every
     //            reset and by dockauv_refresh_obstacles): capsule k -> slots 2k (bot - goal, radius), 2k+1 (unit axis
     //            (top - bot) / L, L); sphere s -> slot 2 n_caps + s (centre - goal, radius)
+    //   obsd     T[n_envs][n_caps + n_sph][8]: env-major bit copy of the obstacles as stored, one 8-word row each
+    //            (capsule: bot, top, radius, 0; sphere: centre, radius, 0, 0, 0), written wherever obsf is; the pipeline
+    //            layout reads its obstacles in T from here (a row is one 64-byte piece in f64 instead of 7 planes)
     //   view_list / ended_list / view_count: work lists, two counters per concurrently stepped range: envs with
     //            something in view (local env index | in-view mask << 32 | condition bits << 48) for the ray launch, envs
     //            whose episode ended (local env index) for the episode-end launch
     T *rec;
     float4 *obsf;
+    T *obsd;
     int32_t n_obsf, cull_exact;      // cull_exact: coordinates too large for the float cull -> decide everything in T
     int32_t tpe_rays;                // the thread-per-env ray launch covers this radar (2x2 pooling, <= 64 pooled cells)
     unsigned long long *view_list;

@@ -307,14 +307,4 @@ __device__ __forceinline__ void store_clear_cells(const KParams<T> &p, int64_t i
     }
 }
 
-// obstacle k of env i as stored (capsules first, then sphere k - n_caps), zero-filled to seven words
-template <typename T>
-__device__ __forceinline__ void load_obstacle(const KParams<T> &p, int64_t i, int k, T o7[7]) {
-    const int64_t N = p.n_envs;
-    const bool is_cap = k < p.n_caps;
-    const T *g = is_cap ? p.capsules + (int64_t)(k * 7) * N + i : p.spheres + (int64_t)((k - p.n_caps) * 4) * N + i;
-#pragma unroll
-    for (int c = 0; c < 7; c++) o7[c] = (c < 4 || is_cap) ? g[(int64_t)c * N] : T(0);
-}
-
 }  // namespace dockauv

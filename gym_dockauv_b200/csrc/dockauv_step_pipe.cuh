@@ -61,10 +61,14 @@ constexpr int kDynThreads = DOCKAUV_DYN_THREADS;
 // step (dockauv_last_list_counts), 8 the ticket of the episode-end launch, whose last CTA saves and zeroes the live counters
 constexpr int kListCounters = 4, kCounterStride = 16, kCounterLast = 4, kCounterTicket = 8;
 
-// ---- the per-env record written by the dynamics launch
+// ---- the per-env record written by the dynamics launch (KParams::rec).  A listed env's record goes to the ray launch
+//      with the words the ray launch does not read -- position relative to the goal, condition bits (they travel in the
+//      list entry) -- replaced by the post-step position and the running return: with the obstacle rows, that launch then
+//      reads nothing else of the env (the step counter only for the ~1 % whose episode ended)
 constexpr int kRecWords = 16;
 constexpr int REC_TRIG = 0, REC_PREL = 6, REC_A = 9, REC_B = 10, REC_R7 = 11, REC_LPD = 12, REC_DD = 13, REC_COND = 14,
               REC_POISON = 15;
+constexpr int REC_POS = REC_PREL, REC_EPR = REC_COND;
 
 // 16-byte vector access to a record: double -> 8 x double2, float -> 4 x float4
 template <typename T>
@@ -121,6 +125,10 @@ template <typename T>
 __device__ __forceinline__ void cp_async_word(unsigned dst_shared, const T *src) {
     if (sizeof(T) == 8) asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(dst_shared), "l"(src) : "memory");
     else asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst_shared), "l"(src) : "memory");
+}
+// 16 bytes global -> shared past L1 (both addresses 16-byte aligned)
+__device__ __forceinline__ void cp_async_16(unsigned dst_shared, const void *src) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst_shared), "l"(src) : "memory");
 }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
@@ -240,7 +248,8 @@ __device__ __forceinline__ void dynamics_env(const KParams<T> &p, const int64_t 
 //   late()           CullLate: the record words 9..15, running return and step counter -- asked for AFTER the obstacle loop,
 //                    so that a caller that has them in memory does not hold them in registers through the loop
 //   pos_of(q)        post-step position (only for pairs within 2 mm of the collision threshold)
-// Returns whether the env is on a view list (its record must then be in KParams::rec for the ray launch).
+// Returns whether the env is on a view list (its record must then be in KParams::rec for the ray launch, with REC_POS
+// and REC_EPR filled in).
 template <typename T>
 struct CullLate {
     T A, B, r7, lp_d, delta_d, cond012, poison, ep_return;
@@ -282,10 +291,10 @@ __device__ __forceinline__ bool cull_finish_env(const KParams<T> &p, const int64
                 cull_pair_rec<T>(p, prel, Rf, c0, c1, is_cap, hit3, view);
                 bool hit = hit3 == 1;
                 if (hit3 == 2) {      // within 2 mm of the collision threshold (or NaN): decided in T like the other layouts
-                    T pos[3], o7[7];
+                    T pos[3], ob[kObstRowWords];
                     pos_of(pos);
-                    load_obstacle<T>(p, i, k, o7);
-                    hit = obstacle_body_hit<T>(p, pos, o7, is_cap);
+                    load_obstacle_row<T>(obstacle_row<T>(p, i, k), ob);
+                    hit = obstacle_body_hit<T>(p, pos, ob, is_cap);
                 }
                 info |= view ? (1u << k) : 0u;
                 info |= hit ? (1u << 16) : 0u;
@@ -298,10 +307,10 @@ __device__ __forceinline__ bool cull_finish_env(const KParams<T> &p, const int64
 #pragma unroll 1
             for (int k = 0; k < n_obst; k++) {
                 const bool is_cap = k < n_caps;
-                T o7[7];
-                load_obstacle<T>(p, i, k, o7);
+                T ob[kObstRowWords];
+                load_obstacle_row<T>(obstacle_row<T>(p, i, k), ob);
                 bool hit, view;
-                obstacle_pair<T, false>(p, pos, Rm, o7, is_cap, nullptr, hit, view);
+                obstacle_pair<T, false>(p, pos, Rm, ob, is_cap, nullptr, hit, view);
                 info |= view ? (1u << k) : 0u;
                 info |= hit ? (1u << 16) : 0u;
             }
@@ -425,7 +434,12 @@ __global__ void __launch_bounds__(kDynThreads, DOCKAUV_MINB_A) dynamics_kernel(c
             return L;
         },
         [&](T q[3]) { q[0] = pos[0]; q[1] = pos[1]; q[2] = pos[2]; });
-    if (listed) RecIO<T>::store(p.rec + i * kRecWords, w);      // the ray launch reads it
+    if (listed) {      // the ray launch reads it
+#pragma unroll
+        for (int c = 0; c < 3; c++) w[REC_POS + c] = pos[c];
+        w[REC_EPR] = dyn_park[6 * kDynThreads + threadIdx.x];
+        RecIO<T>::store(p.rec + i * kRecWords, w);
+    }
 }
 
 // ---- the cull + finish launch on its own (records from KParams::rec; used when the dynamics launch cannot take it in)
@@ -466,7 +480,7 @@ __global__ void __launch_bounds__(kCullThreads, DOCKAUV_MINB_CULL) cull_finish_k
     }
     const T A = w[REC_A];
     const float4 *ob = p.obsf + i;
-    cull_finish_env<T, kCullThreads>(
+    const bool listed = cull_finish_env<T, kCullThreads>(
         p, i, i0, active, w + REC_TRIG, w + REC_PREL, [&](int sl) { return ob[(int64_t)sl * N]; },
         [&]() {
             CullLate<T> L;
@@ -491,28 +505,35 @@ __global__ void __launch_bounds__(kCullThreads, DOCKAUV_MINB_CULL) cull_finish_k
 #pragma unroll
             for (int c = 0; c < 3; c++) q[c] = p.state[(int64_t)c * N + i];
         });
+    if (listed) {      // the record in the ray launch's form (the running return is still in this thread's slot)
+        T *r = p.rec + i * kRecWords;
+#pragma unroll
+        for (int c = 0; c < 3; c++) r[REC_POS + c] = p.state[(int64_t)c * N + i];
+        r[REC_EPR] = *reinterpret_cast<const T *>(cull_park + 3 * kCullThreads * 16 + threadIdx.x * 16);
+    }
 }
 
 // ------------------------------------------------------------------------------------------------------- 3. rays + finish
 // Shared memory of one warp of the ray launch (T words):
 //   stage[2][kStageWords]   the data of two list entries (double buffer, filled by cp.async one entry ahead):
-//                           0..15 the env's record, 16..18 post-step position, 19 running return, 20 step counter (int),
-//                           24 + 8 k .. obstacle k as stored (7 or 4 words), k < 16
+//                           0..15 the env's record (ray launch form), 16 + 8 k .. obstacle row k, k < 16
 //   pre[16][kPreStride]     ray-test records of the in-view obstacles
 //   ray[ray_stride]         clamped ray distances (pooling scratch)
 //   lane[RayLaneShared]     per-lane ray constants
 // Nothing of the software pipeline lives in registers (round 1 kept the next entry's 24 words there), and neither do the
-// per-lane ray constants: 118 -> 80 registers, six CTAs of four warps per SM instead of four.
-constexpr int kStageObst = 24, kStageWords = kStageObst + 16 * 8;
+// per-lane ray constants: 118 -> 80 registers, six CTAs of four warps per SM instead of four.  A warp's area is a whole
+// number of 16-byte pieces (the stage is filled in 16-byte copies).
+constexpr int kStageObst = kRecWords, kStageWords = kStageObst + 16 * kObstRowWords;
 template <typename T, int RPL>
 struct RaysSmem {
     int warp_words, ray_stride, pre_off, ray_off, lane_off;
     __host__ __device__ RaysSmem(int n_rays) {
+        constexpr int kPiece = 16 / (int)sizeof(T);
         ray_stride = (n_rays + 2) & ~1;
         pre_off = 2 * kStageWords;
         ray_off = pre_off + 16 * kPreStride;
         lane_off = ray_off + ray_stride;
-        warp_words = (lane_off + RayLaneShared<T, RPL>::words() + 1) & ~1;
+        warp_words = (lane_off + RayLaneShared<T, RPL>::words() + kPiece - 1) & ~(kPiece - 1);
     }
 };
 
@@ -547,7 +568,6 @@ __device__ __forceinline__ void rays_warp_loop(const KParams<T> &p, unsigned cha
     T *s_warp = reinterpret_cast<T *>(smem_raw) + warp * L.warp_words;
     T *s_pre = s_warp + L.pre_off;
     T *s_ray = s_warp + L.ray_off;
-    const int64_t N = p.n_envs;
     const unsigned count = p.view_count[2];
     const unsigned long long *list = p.view_list + 2 * p.n_envs;
     unsigned idx = w_global;
@@ -558,31 +578,23 @@ __device__ __forceinline__ void rays_warp_loop(const KParams<T> &p, unsigned cha
     rl.init(p, lane, s_ray, s_warp + L.lane_off);
 
     // software pipeline over the list: the data of entry n + 1 is on its way into the other stage buffer while entry n is
-    // cast.  What a lane fetches: lane c < 20 one word (record, position, running return) through a per-lane pointer and
-    // stride, lane 20 the step counter, lane k < n_obst with bit k of the mask obstacle k.
+    // cast.  What a lane fetches, in 16-byte pieces: lane c < kRecPieces piece c of the record, lane k < n_obst with bit k
+    // of the mask the row of obstacle k.
     const bool lane_is_cap = lane < n_caps;
-    const T *obst_row = lane_is_cap ? p.capsules + (int64_t)(lane * 7) * N : p.spheres + (int64_t)((lane - n_caps) * 4) * N;
-    const int obst_words = lane_is_cap ? 7 : 4;
-    const T *word_src = p.rec + lane;            // lanes 0..15: record word `lane`, stride 16
-    int64_t word_stride = kRecWords;
-    if (lane >= 16) {
-        word_stride = 1;
-        word_src = lane < 19 ? p.state + (int64_t)(lane - 16) * N : p.ep_return;
-    }
+    constexpr int kPieceWords = 16 / (int)sizeof(T);
+    constexpr int kRecPieces = kRecWords / kPieceWords, kRowPieces = kObstRowWords / kPieceWords;
     // shared-window addresses of this lane's slots in stage buffer 0 (buffer 1: + kStageWords words)
-    const unsigned sa_word = (unsigned)__cvta_generic_to_shared(s_warp + lane);
-    const unsigned sa_obst = (unsigned)__cvta_generic_to_shared(s_warp + kStageObst + 8 * (lane & 15));
+    const unsigned sa_rec = (unsigned)__cvta_generic_to_shared(s_warp + kPieceWords * (lane % kRecPieces));
+    const unsigned sa_obst = (unsigned)__cvta_generic_to_shared(s_warp + kStageObst + kObstRowWords * (lane & 15));
     auto fetch = [&](uint64_t entry, int b) {
         const int64_t e = p.env_begin + (int64_t)(uint32_t)entry;
         const unsigned mask = (unsigned)(entry >> 32) & 0xffffu;
         const unsigned boff = b ? (unsigned)(kStageWords * sizeof(T)) : 0u;
-        if (lane < 20) cp_async_word<T>(sa_word + boff, word_src + e * word_stride);
-        if (lane == 20) cp_async_word<int32_t>(sa_word + boff, p.t_steps + e);
+        if (lane < kRecPieces) cp_async_16(sa_rec + boff, p.rec + e * kRecWords + kPieceWords * lane);
         if (lane < n_obst && ((mask >> lane) & 1u)) {
-            const T *g = obst_row + e;
+            const T *g = obstacle_row<T>(p, e, lane);
 #pragma unroll
-            for (int c = 0; c < 7; c++)
-                if (c < obst_words) cp_async_word<T>(sa_obst + boff + c * (unsigned)sizeof(T), g + (int64_t)c * N);
+            for (int c = 0; c < kRowPieces; c++) cp_async_16(sa_obst + boff + 16u * c, g + kPieceWords * c);
         }
     };
     uint64_t cur = list[idx];
@@ -602,13 +614,9 @@ __device__ __forceinline__ void rays_warp_loop(const KParams<T> &p, unsigned cha
         __syncwarp();
         const uint64_t nn = (idx + 2 * n_warps < count) ? list[idx + 2 * n_warps] : 0;
         if (idx + n_warps < count) fetch(nxt, buf ^ 1);
-        const T pos[3] = {s_ent[16], s_ent[17], s_ent[18]};
-        if (lane < n_obst && ((mask >> lane) & 1u)) {
-            T ob[7];
-#pragma unroll
-            for (int c = 0; c < 7; c++) ob[c] = c < obst_words ? s_ent[kStageObst + 8 * lane + c] : T(0);
-            obstacle_ray_record<T>(pos, ob, lane_is_cap, s_pre + lane * kPreStride);
-        }
+        const T pos[3] = {s_ent[REC_POS], s_ent[REC_POS + 1], s_ent[REC_POS + 2]};
+        if (lane < n_obst && ((mask >> lane) & 1u))
+            obstacle_ray_record<T>(pos, s_ent + kStageObst + kObstRowWords * lane, lane_is_cap, s_pre + lane * kPreStride);
         T R[9];
         rzyx<T>(s_ent[0], s_ent[1], s_ent[2], s_ent[3], s_ent[4], s_ent[5], R);
         const T poison = s_ent[REC_POISON];
@@ -619,15 +627,14 @@ __device__ __forceinline__ void rays_warp_loop(const KParams<T> &p, unsigned cha
 
         // ---- reward and running return (every lane computes the same values from the staged record, lane 0 stores)
         T ep_ret;
-        const T reward = finish_listed<T>(p, ie, cond, oa_dot, s_ent[REC_A], s_ent[REC_B], s_ent[REC_R7], s_ent[REC_LPD], s_ent[19],
-                                          lane == 0, ep_ret);
+        const T reward = finish_listed<T>(p, ie, cond, oa_dot, s_ent[REC_A], s_ent[REC_B], s_ent[REC_R7], s_ent[REC_LPD],
+                                          s_ent[REC_EPR], lane == 0, ep_ret);
         const bool done = cond != 0;
         if (done) {       // warp-uniform, ~1 % of the listed envs
-            const int32_t t_new = reinterpret_cast<const int32_t *>(s_ent + 20)[0];     // already incremented by the cull code
             double mine = 0.0;
             if (lane == DOCKAUV_STAT_EPISODES) mine = 1.0;
             else if (lane == DOCKAUV_STAT_SUM_RETURN) mine = (double)ep_ret;
-            else if (lane == DOCKAUV_STAT_SUM_LENGTH) mine = (double)t_new;
+            else if (lane == DOCKAUV_STAT_SUM_LENGTH) mine = (double)p.t_steps[ie];     // already incremented by the cull code
             else if (lane >= DOCKAUV_STAT_COND0 && lane < DOCKAUV_STAT_COND0 + 5) mine = ((cond >> (lane - DOCKAUV_STAT_COND0)) & 1u) ? 1.0 : 0.0;
             else if (lane == DOCKAUV_STAT_SUM_FINAL_DELTA_D) mine = (double)s_ent[REC_DD];
             else if (lane == DOCKAUV_STAT_NAN_ENVS) mine = (reward != reward) ? 1.0 : 0.0;
@@ -678,19 +685,18 @@ __device__ __forceinline__ void rays_thread_tile(const KParams<T> &p, const T *s
     T R[9], w[NOB][11];
     bool sph[NOB];
     {
-        T trig[6], pos[3];
-        RecIO<T>::template load<0, 3>(rec, trig);
-#pragma unroll
-        for (int c = 0; c < 3; c++) pos[c] = p.state[(int64_t)c * N + ie];
-        rzyx<T>(trig[0], trig[1], trig[2], trig[3], trig[4], trig[5], R);
+        T w8[8];      // sin / cos of the attitude, position x, y
+        RecIO<T>::template load<0, 4>(rec, w8);
+        const T pos[3] = {w8[REC_POS], w8[REC_POS + 1], rec[REC_POS + 2]};
+        rzyx<T>(w8[0], w8[1], w8[2], w8[3], w8[4], w8[5], R);
 #pragma unroll
         for (int o = 0; o < NOB; o++) {
             const int k = mask ? __ffs(mask) - 1 : 0;
             mask &= mask - 1;
             const bool is_cap = k < p.n_caps;
             sph[o] = !is_cap;
-            T ob[7];
-            load_obstacle<T>(p, ie, k, ob);
+            T ob[kObstRowWords];
+            load_obstacle_row<T>(obstacle_row<T>(p, ie, k), ob);
 #pragma unroll
             for (int c = 0; c < 11; c++) w[o][c] = T(0);
             obstacle_ray_record<T>(pos, ob, is_cap, w[o]);
@@ -751,10 +757,10 @@ __device__ __forceinline__ void rays_thread_tile(const KParams<T> &p, const T *s
         }
     }
     if (valid) {
-        T wf[6];
-        RecIO<T>::template load<4, 3>(rec, wf);       // prel_z, A, B, r7, lp_d, delta_d
+        T wf[8];
+        RecIO<T>::template load<4, 4>(rec, wf);       // position z, A, B, r7, lp_d, delta_d, running return, poison
         T ep_ret;
-        const T reward = finish_listed<T>(p, ie, cond, oa_dot, wf[1], wf[2], wf[3], wf[4], p.ep_return[ie], true, ep_ret);
+        const T reward = finish_listed<T>(p, ie, cond, oa_dot, wf[1], wf[2], wf[3], wf[4], wf[6], true, ep_ret);
         if (cond != 0) {      // ~1 % of the listed envs
             WarpStats bs;
             bs.done = true;
