@@ -15,6 +15,7 @@
 #include <new>
 #include <vector>
 
+#include "dockauv_device.cuh"
 #include "dockauv_launch.h"
 
 using namespace dockauv;
@@ -1303,6 +1304,106 @@ extern "C" int dockauv_gae(const void *rewards_dev, int reward_precision, const 
     else
         gae_kernel<float><<<blocks, threads, 0, st>>>((const float *)rewards_dev, values_dev, last_values_dev, dones_dev,
                                                       n_steps, n_envs, gamma, gae_lambda, advantages_dev, returns_dev);
+    CUDA_TRY(cudaGetLastError());
+    return DOCKAUV_OK;
+}
+
+// ------------------------------------------------------------------------------------------- replay sampling
+// The warp's 32 rows are copied together: element e of the warp's output block is element e % n of row e / n, so
+// every store instruction writes 32 consecutive elements, and each lane's source row pointer is fetched with a shuffle.
+// Every lane runs the same n iterations (the shuffle needs the whole warp); lanes past the batch store nothing.
+template <typename V>
+__device__ __forceinline__ void copy_warp_rows(const float *src, float *__restrict__ dst, int n, int rows, int lane) {
+#pragma unroll 4
+    for (int e = lane; e < 32 * n; e += 32) {
+        const int r = e / n;
+        const V *s = (const V *)__shfl_sync(0xffffffffu, (unsigned long long)src, r);
+        if (r < rows) ((V *)dst)[e] = __ldg(s + (e - r * n));
+    }
+}
+
+// One thread draws one row from Philox4x32-10 at counter (row, draw): 64 bits scaled onto the n_valid transitions and 64
+// onto the N envs, each by a 64 x 64 -> high-64 multiply (relative bias below n / 2^64, no division); then the warp
+// copies observation, next observation and action rows.  V = float4 when n_obs % 4 == 0, else float.
+template <typename R, typename V>
+__global__ void replay_sample_kernel(DockauvReplayRing ring, int S, int64_t N, int n_obs, int n_u, int slot0, int n_valid,
+                                     int64_t B, uint64_t seed, uint64_t draw, DockauvReplaySample out) {
+    const int lane = threadIdx.x & 31;
+    const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, row0 = row - lane;
+    if (row0 >= B) return;      // whole warps only
+    const int rows = (int)min((int64_t)32, B - row0);
+    const float *o = ring.obs, *nx = ring.obs, *a = ring.actions;
+    if (row < B) {
+        uint32_t c[4] = {(uint32_t)row, (uint32_t)(row >> 32), (uint32_t)draw, (uint32_t)(draw >> 32)};
+        philox4x32_10(c, (uint32_t)seed, (uint32_t)(seed >> 32));
+        // (transition, env) uniform over n_valid * N pairs = transition and env independent and uniform
+        const int k = (int)__umul64hi(((uint64_t)c[2] << 32) | c[3], (uint64_t)n_valid);   // transition t_first + k
+        const int64_t env = (int64_t)__umul64hi(((uint64_t)c[0] << 32) | c[1], (uint64_t)N);
+        const int slot = slot0 + k < S ? slot0 + k : slot0 + k - S, next = slot + 1 == S ? 0 : slot + 1;
+        const int64_t at = (int64_t)slot * N + env;
+        const bool d = ring.done[at] != 0;
+        o = ring.obs + at * n_obs;
+        nx = d ? ring.terminal_obs + at * n_obs : ring.obs + ((int64_t)next * N + env) * n_obs;
+        a = ring.actions + at * n_u;
+        out.reward[row] = (float)((const R *)ring.reward)[at];
+        out.done[row] = d ? 1.0f : 0.0f;
+        if (out.index) out.index[row] = at;
+    }
+    const int vw = (int)(sizeof(V) / sizeof(float));
+    copy_warp_rows<V>(o, out.obs + row0 * n_obs, n_obs / vw, rows, lane);
+    copy_warp_rows<V>(nx, out.next_obs + row0 * n_obs, n_obs / vw, rows, lane);
+    copy_warp_rows<float>(a, out.actions + row0 * n_u, n_u, rows, lane);
+}
+
+template <typename R>
+static void launch_replay_sample(bool vec4, unsigned blocks, cudaStream_t st, const DockauvReplayRing &ring, int S,
+                                 int64_t N, int n_obs, int n_u, int slot0, int n_valid, int64_t B, uint64_t seed,
+                                 uint64_t draw, const DockauvReplaySample &out) {
+    if (vec4)
+        replay_sample_kernel<R, float4><<<blocks, 256, 0, st>>>(ring, S, N, n_obs, n_u, slot0, n_valid, B, seed, draw, out);
+    else
+        replay_sample_kernel<R, float><<<blocks, 256, 0, st>>>(ring, S, N, n_obs, n_u, slot0, n_valid, B, seed, draw, out);
+}
+
+static bool misaligned16(const void *p) { return (((uintptr_t)p) & 15u) != 0; }
+
+extern "C" int dockauv_replay_sample(const DockauvReplayRing *ring, int reward_precision, int n_slots, int64_t n_envs,
+                                     int n_obs, int n_u, int64_t t_first, int64_t n_valid, int64_t batch, uint64_t seed,
+                                     uint64_t draw, const DockauvReplaySample *out, void *stream) {
+    if (!ring) return fail(DOCKAUV_EINVAL, "null ring");
+    if (!out) return fail(DOCKAUV_EINVAL, "null out");
+    if (!ring->obs || !ring->terminal_obs || !ring->actions || !ring->reward || !ring->done)
+        return fail(DOCKAUV_EINVAL, "a ring buffer is null (ring obs, terminal_obs, actions, reward, done are required)");
+    if (!out->obs || !out->actions || !out->next_obs || !out->done || !out->reward)
+        return fail(DOCKAUV_EINVAL, "an out buffer is null (out obs, actions, next_obs, done, reward are required)");
+    if (reward_precision != DOCKAUV_F64 && reward_precision != DOCKAUV_F32)
+        return fail(DOCKAUV_EINVAL, "bad reward_precision %d", reward_precision);
+    if (n_slots < 2 || n_slots > (1 << 30)) return fail(DOCKAUV_EINVAL, "n_slots must be in 2..2^30, got %d", n_slots);
+    if (n_envs <= 0 || n_envs > ((int64_t)1 << 32))
+        return fail(DOCKAUV_EINVAL, "n_envs must be in 1..2^32, got %lld", (long long)n_envs);
+    if (n_obs < 1 || n_obs > 16 + DOCKAUV_MAX_RAYS)
+        return fail(DOCKAUV_EINVAL, "n_obs must be in 1..%d, got %d", 16 + DOCKAUV_MAX_RAYS, n_obs);
+    if (n_u < 1 || n_u > DOCKAUV_MAX_U) return fail(DOCKAUV_EINVAL, "n_u must be in 1..%d, got %d", DOCKAUV_MAX_U, n_u);
+    if (t_first < 0) return fail(DOCKAUV_EINVAL, "t_first must not be negative, got %lld", (long long)t_first);
+    if (n_valid < 1 || n_valid > n_slots - 1)
+        return fail(DOCKAUV_EINVAL, "n_valid must be in 1..n_slots - 1 = %d (the slot the next step overwrites is never valid), "
+                                    "got %lld", n_slots - 1, (long long)n_valid);
+    if (batch <= 0 || batch > (int64_t)INT32_MAX)
+        return fail(DOCKAUV_EINVAL, "batch must be in 1..2^31 - 1, got %lld", (long long)batch);
+    const bool vec4 = (n_obs & 3) == 0;
+    if (vec4 && (misaligned16(ring->obs) || misaligned16(ring->terminal_obs) || misaligned16(out->obs) ||
+                 misaligned16(out->next_obs)))
+        return fail(DOCKAUV_EINVAL, "ring obs / terminal_obs and out obs / next_obs must be 16-byte aligned (n_obs = %d is a "
+                                    "multiple of 4: rows move as 128-bit loads and stores)", n_obs);
+    cudaStream_t st = (cudaStream_t)stream;
+    const unsigned blocks = (unsigned)((batch + 255) / 256);
+    const int slot0 = (int)(t_first % n_slots);
+    if (reward_precision == DOCKAUV_F64)
+        launch_replay_sample<double>(vec4, blocks, st, *ring, n_slots, n_envs, n_obs, n_u, slot0, (int)n_valid, batch, seed,
+                                     draw, *out);
+    else
+        launch_replay_sample<float>(vec4, blocks, st, *ring, n_slots, n_envs, n_obs, n_u, slot0, (int)n_valid, batch, seed,
+                                    draw, *out);
     CUDA_TRY(cudaGetLastError());
     return DOCKAUV_OK;
 }

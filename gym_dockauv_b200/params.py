@@ -78,6 +78,14 @@ class DockauvTapBuffers(C.Structure):
     _fields_ = [(k, C.c_void_p) for k in TAP_FIELDS]
 
 
+class DockauvReplayRing(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in ("obs", "terminal_obs", "actions", "reward", "done")]
+
+
+class DockauvReplaySample(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in ("obs", "actions", "next_obs", "done", "reward", "index")]
+
+
 def skew(a):
     """S(a) b = a x b (utils/geomutils.py:106-128)."""
     return np.array([[0.0, -a[2], a[1]], [a[2], 0.0, -a[0]], [-a[1], a[0], 0.0]])

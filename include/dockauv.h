@@ -22,6 +22,7 @@
  *                                      (train.py:107-118), for action sequences that are known up front
  *   dockauv_gae                        RolloutBuffer.compute_returns_and_advantage of the PPO caller
  *                                      (stable-baselines3 1.5.0, requirements.txt; selected at train.py:64)
+ *   dockauv_replay_sample              ReplayBuffer.sample of the SAC caller (MODEL = SAC at train.py:64)
  *   DockauvDebugOut (state_dot, ...)   EpisodeDataStorage.update          utils/datastorage.py:268-288
  *   dockauv_set_taps                   the same, during training: every step of a few chosen envs recorded on
  *                                      the device (interval_datastorage, config.py; datastorage.py:268-288)
@@ -318,6 +319,32 @@ DOCKAUV_API int dockauv_set_taps(DockauvHandle *h, const int64_t *env_ids_host, 
 DOCKAUV_API int dockauv_gae(const void *rewards_dev, int reward_precision, const float *values_dev,
                 const float *last_values_dev, const uint8_t *dones_dev, int n_steps, int64_t n_envs, float gamma,
                 float gae_lambda, float *advantages_dev, float *returns_dev, void *stream);
+
+/* Replay ring of an off-policy caller: S slots of the whole batch, written by dockauv_step (slot t % S holds the
+ * observation acted on at step t, the action, the reward and done flag of step t, and the last real observation of the
+ * envs whose episode ended at step t). */
+typedef struct DockauvReplayRing {      /* caller-owned device buffers, S slots of N envs, env index fastest in a slot */
+    const float *obs;                   /* f32[S][N][n_obs] */
+    const float *terminal_obs;          /* f32[S][N][n_obs] (read only for rows whose done flag is set) */
+    const float *actions;               /* f32[S][N][n_u] */
+    const void *reward;                 /* real[S][N], precision per reward_precision */
+    const uint8_t *done;                /* u8[S][N] */
+} DockauvReplayRing;
+typedef struct DockauvReplaySample {    /* f32 outputs, B rows, contiguous */
+    float *obs, *actions, *next_obs, *done, *reward;
+    int64_t *index;                     /* nullable: slot * N + env of each row (tests, prioritised callers) */
+} DockauvReplaySample;
+
+/* `batch` transitions drawn uniformly from the n_valid * n_envs (transition, env) pairs t_first .. t_first + n_valid - 1
+ * (n_valid <= n_slots - 1: the slot the next step overwrites is never drawn).  Transition t lives in slot t % n_slots;
+ * its next observation is terminal_obs of that slot where the done flag is set, else obs of slot (t + 1) % n_slots.
+ * Row k is drawn from the Philox stream keyed by `seed` at counter (draw, k), so equal arguments give bit-identical
+ * output.  Rewards are rounded to f32 once, done is written as 0.0 / 1.0.  One launch on `stream`, no host
+ * synchronisation.  When n_obs is a multiple of 4 observation rows move in 16-byte pieces: ring and output
+ * observation arrays must then be 16-byte aligned (DOCKAUV_EINVAL otherwise).  Needs no handle. */
+DOCKAUV_API int dockauv_replay_sample(const DockauvReplayRing *ring, int reward_precision, int n_slots, int64_t n_envs,
+                                      int n_obs, int n_u, int64_t t_first, int64_t n_valid, int64_t batch,
+                                      uint64_t seed, uint64_t draw, const DockauvReplaySample *out, void *stream);
 
 /* Episode statistics accumulated on the device since the last clear (DOCKAUV_STAT_*).  stats_dev points at
  * double[DOCKAUV_N_STATS] on the device: it is the send buffer of the per-rollout NCCL all-reduce.  The kernels
