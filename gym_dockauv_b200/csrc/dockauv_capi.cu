@@ -13,6 +13,8 @@
 #include <cstring>
 #include <algorithm>
 #include <new>
+#include <type_traits>
+#include <utility>
 #include <vector>
 
 #include "dockauv_device.cuh"
@@ -56,16 +58,77 @@ struct DeviceGuard {
 static const int kHostStreams = 3;
 static const size_t kStatsBytes = sizeof(double) * DOCKAUV_N_STATS * DOCKAUV_STAT_COPIES;   // replica 0 = the public vector
 
+// Captured launch sequences keyed by everything they bake in (pointers, switches, seed), up to `capacity` of them; once
+// full, the oldest capture is replaced.  Keys are zero-filled and compared byte for byte, so a field added to a key
+// struct takes part without further code.
+template <typename Key>
+struct GraphCache {
+    static_assert(std::is_trivially_copyable<Key>::value && std::has_unique_object_representations<Key>::value &&
+                      sizeof(Key) % 8 == 0,
+                  "graph keys are compared byte for byte: plain data without padding, whole 64-bit words");
+    struct Graph {
+        Key key;
+        cudaGraphExec_t exec = nullptr;
+        int64_t launches = 0;              // kernels in the captured sequence
+        std::vector<int64_t> begins;       // first env of every range its last step stepped (dockauv_last_list_counts)
+    };
+    size_t capacity;
+    std::vector<Graph> graphs;
+    size_t next = 0;                       // slot replaced next once the cache is full
+    int64_t captures = 0;                  // how many sequences were captured (tests: replays must not re-capture)
+    explicit GraphCache(size_t cap) : capacity(cap) {}
+    // word by word, out at the first difference (an out-of-line memcmp per entry made a lookup in a 64-graph cache ~4x
+    // slower on the host)
+    static bool same(const Key &a, const Key &b) {
+        const char *p = (const char *)&a, *q = (const char *)&b;
+        for (size_t i = 0; i < sizeof(Key); i += 8) {
+            uint64_t x, y;
+            memcpy(&x, p + i, 8);
+            memcpy(&y, q + i, 8);
+            if (x != y) return false;
+        }
+        return true;
+    }
+    Graph *find(const Key &key) {
+        for (auto &g : graphs)
+            if (same(g.key, key)) return &g;
+        return nullptr;
+    }
+    Graph *add(Graph &&fresh) {
+        captures += 1;
+        if (graphs.size() < capacity) {
+            graphs.push_back(std::move(fresh));
+            return &graphs.back();
+        }
+        Graph &victim = graphs[next];
+        next = (next + 1) % graphs.size();
+        cudaGraphExecDestroy(victim.exec);
+        victim = std::move(fresh);
+        return &victim;
+    }
+    void clear() {
+        for (auto &g : graphs) cudaGraphExecDestroy(g.exec);
+        graphs.clear();
+        next = 0;
+    }
+};
+
+#ifndef DOCKAUV_STEP_GRAPHS
+#define DOCKAUV_STEP_GRAPHS 96     // cached step graphs per handle (a trainer alternates between a few tensors; bench.py's pool: 64)
+#endif
+
 struct DockauvHandle {
     DockauvParams params;
     int64_t n_envs = 0;
     int device = 0;
     int n_obs = 0;
+    size_t esz = 0;                // bytes of one real: 8 (f64 handle) or 4 (f32)
     bool bound = false;
-    KParams<double> kd;
+    KParams<double> kd;            // only the one of the handle's precision is filled and read (with_k)
     KParams<float> kf;
     void *ray_tab = nullptr;
-    void *pipe_buf = nullptr;      // pipeline layout: per-env records, float obstacle records, ray list + counters
+    PipeBuffers pipe;              // pipeline layout: per-env records, float obstacle records and rows, work lists + counters
+    void *pipe_buf = nullptr;
     double *stats = nullptr;
     int64_t launches = 0;
     bool timing = false;
@@ -83,48 +146,24 @@ struct DockauvHandle {
     void *st_reward = nullptr;
     uint8_t *st_done = nullptr, *st_cond = nullptr;
     // rollout graph cache: one captured launch sequence, re-captured when the key changes
-    cudaGraphExec_t rg_exec = nullptr;
-    int64_t rg_launches = 0;       // kernel nodes in the captured sequence
     struct RolloutKey {
-        const void *actions = nullptr;
-        DockauvRolloutOut out = {};
-        int64_t n_steps = 0, action_dtype = 0, auto_reset = 0;      // 64-bit fields: no padding bytes in the key
-        uint64_t seed = 0;
-        bool operator==(const RolloutKey &o) const {
-            return actions == o.actions && out.obs == o.out.obs && out.reward == o.out.reward && out.done == o.out.done &&
-                   out.cond_bits == o.out.cond_bits && out.terminal_obs == o.out.terminal_obs &&
-                   out.ep_return_out == o.out.ep_return_out && out.ep_len_out == o.out.ep_len_out &&
-                   out.delta_d_out == o.out.delta_d_out && n_steps == o.n_steps && action_dtype == o.action_dtype &&
-                   auto_reset == o.auto_reset && seed == o.seed;
-        }
-    } rg_key;
-    int64_t rg_captures = 0;       // how many times a rollout graph was captured (tests: replays must not re-capture)
+        const void *actions;
+        DockauvRolloutOut out;
+        int64_t n_steps, action_dtype, auto_reset;
+        uint64_t seed;
+    };
+    GraphCache<RolloutKey> rg{1};
     // step graph cache: the launch sequence of ONE dockauv_step (launches of both halves, fork / join events) captured per
     // set of pointers and replayed; trainers alternate between a handful of action / output tensors
     struct StepKey {
-        const void *actions = nullptr, *noise = nullptr;
-        DockauvStepOut out = {};
-        int64_t action_dtype = 0, auto_reset = 0;
-        uint64_t seed = 0;
-        bool operator==(const StepKey &o) const {
-            return actions == o.actions && noise == o.noise && out.obs == o.out.obs && out.reward == o.out.reward &&
-                   out.done == o.out.done && out.cond_bits == o.out.cond_bits && out.terminal_obs == o.out.terminal_obs &&
-                   out.ep_return_out == o.out.ep_return_out && out.ep_len_out == o.out.ep_len_out &&
-                   out.delta_d_out == o.out.delta_d_out && action_dtype == o.action_dtype && auto_reset == o.auto_reset &&
-                   seed == o.seed;
-        }
+        const void *actions, *noise;
+        DockauvStepOut out;
+        int64_t action_dtype, auto_reset;
+        uint64_t seed;
     };
-    struct StepGraph {
-        StepKey key;
-        cudaGraphExec_t exec = nullptr;
-        int64_t launches = 0;
-        std::vector<int64_t> begins;
-    };
-    std::vector<int64_t> last_begins;     // first env of every range the most recent step call stepped (their list counters)
-    std::vector<StepGraph> sg;
-    size_t sg_next = 0;            // slot replaced next once the cache is full
+    GraphCache<StepKey> sg{DOCKAUV_STEP_GRAPHS};
     bool sg_enabled = true;
-    int64_t sg_captures = 0;
+    std::vector<int64_t> last_begins;     // first env of every range the most recent device step stepped (their list counters)
     DockauvBuffers bound_bufs = {};
     // episode taps (dockauv_set_taps): two K-env shadows of the tapped envs, stepped on a side stream
     struct Taps {
@@ -138,15 +177,9 @@ struct DockauvHandle {
         DockauvStepOut out = {};       // obs, reward, done, cond_bits of `shadow`
         DockauvStepOut dout = {};      // the same of `dshadow` (not recorded)
         DockauvDebugOut dbg = {};      // ray_dist, reward_arr, nu_c, state_dot of `dshadow`
-        // pipeline layout: the shadow's own per-env records, float obstacle records, obstacle rows, work lists and
-        // counters
-        void *rec = nullptr;
-        float4 *obsf = nullptr;
-        void *obsd = nullptr;
-        unsigned long long *view_list = nullptr;
-        uint32_t *ended_list = nullptr;
-        unsigned int *view_count = nullptr;
-        int shadow_launches = 0;       // launches of one step of `shadow`
+        // pipeline layout: the shadow's own pipeline buffers for K envs (pipe_buf null for the other layouts)
+        PipeBuffers pipe;
+        void *pipe_buf = nullptr;
         double *stats = nullptr;       // DOCKAUV_STAT_COPIES replicas nobody reads: the public statistics stay the real step's
         int64_t *ids = nullptr;
         unsigned int *sync = nullptr;
@@ -160,14 +193,14 @@ struct DockauvHandle {
 static int pooled_dim(int n, int b) { return (n + b - 1) / b; }
 
 static void drop_graphs(DockauvHandle *h) {      // captured launch sequences hold the old pointers / seed
-    if (h->rg_exec) {
-        cudaGraphExecDestroy(h->rg_exec);
-        h->rg_exec = nullptr;
-    }
-    for (auto &g : h->sg)
-        if (g.exec) cudaGraphExecDestroy(g.exec);
+    h->rg.clear();
     h->sg.clear();
-    h->sg_next = 0;
+}
+
+// f(k) with the handle's KParams in its precision: the one place that chooses between kd and kf
+template <typename F>
+static auto with_k(DockauvHandle *h, F &&f) {
+    return h->params.precision == DOCKAUV_F64 ? f(h->kd) : f(h->kf);
 }
 
 extern "C" int dockauv_abi_version(void) { return DOCKAUV_ABI_VERSION; }
@@ -333,69 +366,43 @@ extern "C" int dockauv_create(const DockauvParams *p, int64_t n_envs, int device
     h->n_envs = n_envs;
     h->device = device;
     h->n_obs = dockauv_n_obs(p);
-    fill_kparams<double>(*p, n_envs, h->kd);
-    fill_kparams<float>(*p, n_envs, h->kf);
+    h->esz = with_k(h, [](auto &k) { return sizeof(k.m); });
     // ray table in global memory: rd_b[3][n_rays] then beta_oa[n_rays], in the handle's precision
-    {
-        const int n = p->n_rays;
-        const size_t esz = p->precision == DOCKAUV_F64 ? 8 : 4;
-        std::vector<char> host(esz * 4 * n);
+    const int n = p->n_rays;
+    std::vector<char> tab(h->esz * 4 * n);
+    with_k(h, [&](auto &k) {
+        fill_kparams(*p, n_envs, k);
         for (int i = 0; i < n; i++)
-            for (int c = 0; c < 4; c++) {
-                double v = c < 3 ? p->rd_b[3 * i + c] : p->beta_oa[i];
-                if (esz == 8) ((double *)host.data())[c * n + i] = v;
-                else ((float *)host.data())[c * n + i] = (float)v;
-            }
-        cudaError_t e1 = cudaMalloc(&h->ray_tab, host.size());
-        cudaError_t e2 = e1 == cudaSuccess ? cudaMemcpy(h->ray_tab, host.data(), host.size(), cudaMemcpyHostToDevice) : e1;
-        cudaError_t e3 = e2 == cudaSuccess ? cudaMalloc((void **)&h->stats, kStatsBytes) : e2;
-        cudaError_t e4 = e3 == cudaSuccess ? cudaMemset(h->stats, 0, kStatsBytes) : e3;
-        if (e4 != cudaSuccess) {
-            if (h->ray_tab) cudaFree(h->ray_tab);
-            if (h->stats) cudaFree(h->stats);
-            delete h;
-            return fail(DOCKAUV_ECUDA, "device allocation failed: %s", cudaGetErrorString(e4));
-        }
-        h->kd.ray_tab = (const double *)h->ray_tab;
-        h->kf.ray_tab = (const float *)h->ray_tab;
-        h->kd.stats = h->stats;
-        h->kf.stats = h->stats;
+            for (int c = 0; c < 4; c++)
+                ((decltype(k.m) *)tab.data())[c * n + i] = (decltype(k.m))(c < 3 ? p->rd_b[3 * i + c] : p->beta_oa[i]);
+    });
+    cudaError_t e1 = cudaMalloc(&h->ray_tab, tab.size());
+    if (e1 == cudaSuccess) e1 = cudaMemcpy(h->ray_tab, tab.data(), tab.size(), cudaMemcpyHostToDevice);
+    if (e1 == cudaSuccess) e1 = cudaMalloc((void **)&h->stats, kStatsBytes);
+    if (e1 == cudaSuccess) e1 = cudaMemset(h->stats, 0, kStatsBytes);
+    if (e1 != cudaSuccess) {
+        dockauv_destroy(h);
+        return fail(DOCKAUV_ECUDA, "device allocation failed: %s", cudaGetErrorString(e1));
     }
+    with_k(h, [&](auto &k) {
+        k.ray_tab = (decltype(k.ray_tab))h->ray_tab;
+        k.stats = h->stats;
+    });
     if (p->layout == DOCKAUV_LAYOUT_PIPELINE || p->layout == DOCKAUV_LAYOUT_AUTO) {
-        // library-owned buffers of the pipeline layout: per-env record T[16] (128-byte aligned), float obstacle records
-        // float4[2 n_caps + n_sph], obstacle rows T[n_caps + n_sph][8] (256-byte aligned), the ray list u64 and one list
-        // counter per 128 envs
-        const size_t esz = p->precision == DOCKAUV_F64 ? 8 : 4;
-        const size_t n = (size_t)n_envs;
-        const int n_obsf = 2 * p->n_capsules + p->n_spheres, n_obst = p->n_capsules + p->n_spheres;
-        const size_t off_rec = 0, off_obsf = off_rec + 16 * esz * n;
-        const size_t off_obsd = (off_obsf + 16 * (size_t)n_obsf * n + 255) & ~(size_t)255;
-        const size_t off_list = off_obsd + 8 * esz * (size_t)n_obst * n;
-        const size_t off_end = off_list + 3 * 8 * n, off_cnt = off_end + 4 * ((n + 1) & ~(size_t)1);      // three view lists
-        const size_t n_cnt = 16 * (n / 128 + 2);     // counter block (kCounterStride words) per concurrently stepped env range
-        cudaError_t e5 = cudaMalloc(&h->pipe_buf, off_cnt + 4 * n_cnt);
-        if (e5 == cudaSuccess) e5 = cudaMemset(h->pipe_buf, 0, off_cnt + 4 * n_cnt);
-        if (e5 != cudaSuccess) {
-            cudaFree(h->ray_tab);
-            cudaFree(h->stats);
-            if (h->pipe_buf) cudaFree(h->pipe_buf);
-            delete h;
-            return fail(DOCKAUV_ECUDA, "device allocation of the pipeline buffers failed: %s", cudaGetErrorString(e5));
+        h->pipe = pipe_buffers(n_envs, h->esz, p->n_capsules, p->n_spheres);
+        cudaError_t e2 = cudaMalloc(&h->pipe_buf, h->pipe.bytes);
+        if (e2 == cudaSuccess) e2 = cudaMemset(h->pipe_buf, 0, h->pipe.bytes);
+        if (e2 != cudaSuccess) {
+            dockauv_destroy(h);
+            return fail(DOCKAUV_ECUDA, "device allocation of the pipeline buffers failed: %s", cudaGetErrorString(e2));
         }
-        char *base = (char *)h->pipe_buf;
-        h->kd.rec = (double *)(base + off_rec);
-        h->kf.rec = (float *)(base + off_rec);
-        h->kd.obsf = h->kf.obsf = n_obsf > 0 ? (float4 *)(base + off_obsf) : nullptr;
-        h->kd.n_obsf = h->kf.n_obsf = n_obsf;
-        h->kd.obsd = n_obst > 0 ? (double *)(base + off_obsd) : nullptr;
-        h->kf.obsd = n_obst > 0 ? (float *)(base + off_obsd) : nullptr;
-        h->kd.view_list = h->kf.view_list = (unsigned long long *)(base + off_list);
-        h->kd.ended_list = h->kf.ended_list = (uint32_t *)(base + off_end);
-        h->kd.view_count = h->kf.view_count = (unsigned int *)(base + off_cnt);
         int sms = 0;
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-        h->kd.sm_count = h->kf.sm_count = sms;
-        h->kd.tpe_rays = h->kf.tpe_rays = (p->block_reduce == 2 && h->kd.n_rr <= 64) ? 1 : 0;
+        with_k(h, [&](auto &k) {
+            point_pipe(k, h->pipe, h->pipe_buf);
+            k.sm_count = sms;
+            k.tpe_rays = (p->block_reduce == 2 && k.n_rr <= 64) ? 1 : 0;
+        });
     }
     *out = h;
     return DOCKAUV_OK;
@@ -441,7 +448,7 @@ static int build_tap_rows(DockauvHandle *h) {
     const DockauvBuffers &b = h->bound_bufs;
     const DockauvTapBuffers &r = tp.ring;
     const int64_t N = h->n_envs, K = tp.n;
-    const int esz = h->params.precision == DOCKAUV_F64 ? 8 : 4;
+    const int esz = (int)h->esz;
     const int nu = h->params.n_u, nc = h->params.n_capsules, ns = h->params.n_spheres;
     const int n_scene = 4 + 7 * nc + 4 * ns, n_obs = h->n_obs, n_rays = h->params.n_rays;
     std::vector<TapRow> g, c;
@@ -469,25 +476,29 @@ static int build_tap_rows(DockauvHandle *h) {
     gather(b.ep_return, tp.shadow.ep_return, tp.dshadow.ep_return, 0, esz, r.pre_ep_return, 0, 1);
     gather(b.t_steps, tp.shadow.t_steps, tp.dshadow.t_steps, 0, 4, r.pre_t_steps, 0, 1);
     gather(b.episode, tp.shadow.episode, tp.dshadow.episode, 0, 4, r.pre_episode, 0, 1);
-    // the real step's float obstacle records (pipeline layout): the shadow culls exactly what the real step culls
-    if (tp.obsf)
-        for (int k = 0; k < h->kd.n_obsf; k++) gather(h->kd.obsf, tp.obsf, nullptr, k, 16, nullptr, 0, 0);
-    // and its obstacle rows (env-major: 16-byte piece j of every tapped env's rows, one env's rows apart)
-    if (tp.obsd) {
-        const int row_bytes = 8 * esz * (nc + ns);
-        for (int j = 0; j < row_bytes / 16; j++) {
-            TapRow t;
-            t.src = (const char *)h->kd.obsd + 16 * j;
-            t.dst = (char *)tp.obsd + 16 * j;
-            t.dst2 = nullptr;
-            t.ring = nullptr;
-            t.ring_slot = 0;
-            t.esz = 16;
-            t.src_step = t.dst_step = row_bytes;
-            t.src_by_id = 1;
-            g.push_back(t);
+    with_k(h, [&](auto &real) {
+        auto shadow = real;
+        point_pipe(shadow, tp.pipe, tp.pipe_buf);
+        // the real step's float obstacle records (pipeline layout): the shadow culls exactly what the real step culls
+        if (shadow.obsf)
+            for (int k = 0; k < real.n_obsf; k++) gather(real.obsf, shadow.obsf, nullptr, k, 16, nullptr, 0, 0);
+        // and its obstacle rows (env-major: 16-byte piece j of every tapped env's rows, one env's rows apart)
+        if (shadow.obsd) {
+            const int row_bytes = 8 * esz * (nc + ns);
+            for (int j = 0; j < row_bytes / 16; j++) {
+                TapRow t;
+                t.src = (const char *)real.obsd + 16 * j;
+                t.dst = (char *)shadow.obsd + 16 * j;
+                t.dst2 = nullptr;
+                t.ring = nullptr;
+                t.ring_slot = 0;
+                t.esz = 16;
+                t.src_step = t.dst_step = row_bytes;
+                t.src_by_id = 1;
+                g.push_back(t);
+            }
         }
-    }
+    });
     // one committed row: row `comp` of a shadow field (tap-indexed, `step` bytes apart) -> row `comp` of a ring field
     auto commit = [&](const void *src, void *ring, int comp, int e, int rows, int step) {
         TapRow t;
@@ -541,8 +552,7 @@ extern "C" int dockauv_bind(DockauvHandle *h, const DockauvBuffers *b) {
         return fail(DOCKAUV_EINVAL, "a required state buffer is null");
     if ((h->params.n_capsules > 0 && !b->capsules) || (h->params.n_spheres > 0 && !b->spheres))
         return fail(DOCKAUV_EINVAL, "obstacle buffer is null but the handle has obstacles");
-    bind_k<double>(h->kd, *b);
-    bind_k<float>(h->kf, *b);
+    with_k(h, [&](auto &k) { bind_k(k, *b); });
     h->bound_bufs = *b;
     h->bound = true;
     if (h->tap.n > 0) {
@@ -551,8 +561,7 @@ extern "C" int dockauv_bind(DockauvHandle *h, const DockauvBuffers *b) {
     }
     {   // float obstacle records of whatever the buffers hold now (later writers: dockauv_reset, dockauv_refresh_obstacles)
         DeviceGuard guard(h->device);
-        if (h->params.precision == DOCKAUV_F64) CUDA_TRY(launch_refresh_obstacles<double>(h->kd, (cudaStream_t)0));
-        else CUDA_TRY(launch_refresh_obstacles<float>(h->kf, (cudaStream_t)0));
+        CUDA_TRY(with_k(h, [](auto &k) { return launch_refresh_obstacles(k, (cudaStream_t)0); }));
         CUDA_TRY(cudaStreamSynchronize((cudaStream_t)0));
     }
     drop_graphs(h);
@@ -604,29 +613,18 @@ static void set_io(KParams<T> &k, const void *actions, bool act_f32, const void 
 static int step_range(DockauvHandle *h, const void *actions, int action_dtype, const void *noise,
                       const DockauvStepOut *out, const DockauvDebugOut *dbg, int auto_reset, int64_t begin,
                       int64_t end, cudaStream_t st, bool with_marks = false) {
-    const bool actf32 = action_dtype == DOCKAUV_ACT_F32;
-    const int layout = resolve_layout(h);
-    const bool has_current = current_on(h);
-    cudaError_t e;
-    if (h->params.precision == DOCKAUV_F64) {
-        KParams<double> k = h->kd;
-        set_io<double>(k, actions, actf32, noise, *out, dbg, auto_reset);
+    int n = 0;
+    const cudaError_t e = with_k(h, [&](auto &kh) {
+        auto k = kh;
+        set_io(k, actions, action_dtype == DOCKAUV_ACT_F32, noise, *out, dbg, auto_reset);
         k.env_begin = begin;
         k.env_end = end;
-        k.has_current = has_current;
-        e = launch_step<double>(k, h->params.vehicle, layout, st, with_marks ? h->marks : nullptr, with_marks ? &h->n_marks : nullptr);
-    } else {
-        KParams<float> k = h->kf;
-        set_io<float>(k, actions, actf32, noise, *out, dbg, auto_reset);
-        k.env_begin = begin;
-        k.env_end = end;
-        k.has_current = has_current;
-        e = launch_step<float>(k, h->params.vehicle, layout, st, with_marks ? h->marks : nullptr, with_marks ? &h->n_marks : nullptr);
-    }
+        k.has_current = current_on(h);
+        return launch_step(k, h->params.vehicle, resolve_layout(h), st, &n, with_marks ? h->marks : nullptr,
+                           with_marks ? &h->n_marks : nullptr);
+    });
     if (e != cudaSuccess) return fail(DOCKAUV_ECUDA, "step kernel launch failed: %s", cudaGetErrorString(e));
-    h->last_begins.push_back(begin);
-    const bool staged = dbg == nullptr;   // else: the fused kernel
-    h->launches += layout == DOCKAUV_LAYOUT_PIPELINE && staged ? dockauv::pipe_launches(h->kd) : 1;
+    h->launches += n;
     return DOCKAUV_OK;
 }
 
@@ -658,9 +656,10 @@ static TapLaunch tap_launch(const DockauvHandle *h, bool gather, const void *act
     return t;
 }
 
+// *n_launches receives the launches enqueued: gather, the shadow's step, the debug shadow's step, commit
 template <typename T>
 static cudaError_t tap_issue(DockauvHandle *h, const KParams<T> &real, const void *actions, int action_dtype,
-                             const void *noise, cudaStream_t st) {
+                             const void *noise, cudaStream_t st, int *n_launches) {
     auto &tp = h->tap;
     cudaError_t e = launch_tap_gather<T>(real, tap_launch(h, true, actions, action_dtype, noise), st);
     if (e == cudaSuccess) e = cudaEventRecord(tp.ev_fork, st);
@@ -676,38 +675,30 @@ static cudaError_t tap_issue(DockauvHandle *h, const KParams<T> &real, const voi
     set_io<T>(k, tp.actions, action_dtype == DOCKAUV_ACT_F32, tp.noise, tp.out, nullptr, 0);
     k.has_current = current_on(h);
     k.stats = tp.stats;
-    k.rec = (T *)tp.rec;
-    k.obsf = tp.obsf;
-    k.obsd = (T *)tp.obsd;
-    k.view_list = tp.view_list;
-    k.ended_list = tp.ended_list;
-    k.view_count = tp.view_count;
-    e = launch_step<T>(k, h->params.vehicle, resolve_layout(h), tp.st);
+    point_pipe(k, tp.pipe, tp.pipe_buf);
+    int n_shadow = 0, n_dbg = 0;
+    e = launch_step<T>(k, h->params.vehicle, resolve_layout(h), tp.st, &n_shadow);
     if (e != cudaSuccess) return e;
     // the debug shadow: the single-launch kernel with debug outputs (state_dot, nu_c, ray distances, reward terms)
     KParams<T> d = k;
     bind_k<T>(d, tp.dshadow);
     set_io<T>(d, tp.actions, action_dtype == DOCKAUV_ACT_F32, tp.noise, tp.dout, &tp.dbg, 0);
-    d.rec = nullptr;
-    d.obsf = nullptr;
-    d.obsd = nullptr;
-    d.view_list = nullptr;
-    d.ended_list = nullptr;
-    d.view_count = nullptr;
-    e = launch_step<T>(d, h->params.vehicle, DOCKAUV_LAYOUT_WARP_RAYS, tp.dst);
+    point_pipe(d, tp.pipe, nullptr);
+    e = launch_step<T>(d, h->params.vehicle, DOCKAUV_LAYOUT_WARP_RAYS, tp.dst, &n_dbg);
     if (e == cudaSuccess) e = cudaEventRecord(tp.ev_dbg, tp.dst);
     if (e == cudaSuccess) e = cudaStreamWaitEvent(tp.st, tp.ev_dbg, 0);
     if (e == cudaSuccess) e = launch_tap_commit<T>(real, tap_launch(h, false, actions, action_dtype, noise), tp.st);
     if (e == cudaSuccess) e = cudaEventRecord(tp.ev_join, tp.st);
+    *n_launches = 2 + n_shadow + n_dbg;
     return e;
 }
 
 static int tap_begin(DockauvHandle *h, const void *actions, int action_dtype, const void *noise, cudaStream_t st) {
     if (h->tap.n == 0) return DOCKAUV_OK;
-    const cudaError_t e = h->params.precision == DOCKAUV_F64 ? tap_issue<double>(h, h->kd, actions, action_dtype, noise, st)
-                                                             : tap_issue<float>(h, h->kf, actions, action_dtype, noise, st);
+    int n = 0;
+    const cudaError_t e = with_k(h, [&](auto &k) { return tap_issue(h, k, actions, action_dtype, noise, st, &n); });
     if (e != cudaSuccess) return fail(DOCKAUV_ECUDA, "tap launch failed: %s", cudaGetErrorString(e));
-    h->launches += 3 + h->tap.shadow_launches;      // gather, debug shadow, commit + the shadow's step
+    h->launches += n;
     return DOCKAUV_OK;
 }
 
@@ -719,8 +710,7 @@ static int tap_end(DockauvHandle *h, cudaStream_t st) {
 extern "C" int dockauv_set_seed(DockauvHandle *h, uint64_t seed) {
     if (!h) return fail(DOCKAUV_EINVAL, "null handle");
     h->params.seed = seed;
-    h->kd.seed = seed;
-    h->kf.seed = seed;
+    with_k(h, [&](auto &k) { k.seed = seed; });
     return DOCKAUV_OK;
 }
 
@@ -728,9 +718,7 @@ extern "C" int dockauv_reset(DockauvHandle *h, const uint8_t *mask_dev, void *st
     if (!h) return fail(DOCKAUV_EINVAL, "null handle");
     if (!h->bound) return fail(DOCKAUV_ESTATE, "dockauv_bind must be called before dockauv_reset");
     DeviceGuard guard(h->device);
-    cudaStream_t st = (cudaStream_t)stream;
-    if (h->params.precision == DOCKAUV_F64) CUDA_TRY(launch_reset<double>(h->kd, mask_dev, st));
-    else CUDA_TRY(launch_reset<float>(h->kf, mask_dev, st));
+    CUDA_TRY(with_k(h, [&](auto &k) { return launch_reset(k, mask_dev, (cudaStream_t)stream); }));
     h->launches += 1;
     return DOCKAUV_OK;
 }
@@ -739,12 +727,12 @@ extern "C" int dockauv_refresh_obstacles(DockauvHandle *h, void *stream) {
     if (!h) return fail(DOCKAUV_EINVAL, "null handle");
     if (!h->bound) return fail(DOCKAUV_ESTATE, "dockauv_bind must be called before dockauv_refresh_obstacles");
     DeviceGuard guard(h->device);
-    cudaStream_t st = (cudaStream_t)stream;
-    if (h->kd.obsf == nullptr) return DOCKAUV_OK;
-    if (h->params.precision == DOCKAUV_F64) CUDA_TRY(launch_refresh_obstacles<double>(h->kd, st));
-    else CUDA_TRY(launch_refresh_obstacles<float>(h->kf, st));
-    h->launches += 1;
-    return DOCKAUV_OK;
+    return with_k(h, [&](auto &k) {
+        if (k.obsf == nullptr) return DOCKAUV_OK;
+        CUDA_TRY(launch_refresh_obstacles(k, (cudaStream_t)stream));
+        h->launches += 1;
+        return DOCKAUV_OK;
+    });
 }
 
 static int ensure_streams(DockauvHandle *h) {
@@ -779,17 +767,27 @@ static int check_rows(const DockauvHandle *h, const float *obs, const float *ter
     return DOCKAUV_OK;
 }
 
-static int step_parts(DockauvHandle *h, const void *actions, int action_dtype, const void *noise,
-                      const DockauvStepOut *out, int auto_reset, cudaStream_t st) {
+// Issues issue(begin, end, stream) for every env range of a device step and records the ranges as those of the most
+// recent step (their list counters).  The range is the whole batch on the caller's stream, or, for large batches of the
+// pipeline layout (unless `whole`), DOCKAUV_STEP_PARTS ranges of a multiple of 4096 envs, each on an internal stream
+// forked from / joined to the caller's stream by events.
+template <typename F>
+static int over_ranges(DockauvHandle *h, bool whole, cudaStream_t st, F &&issue) {
+    const int64_t N = h->n_envs;
+    h->last_begins.clear();
+    if (whole || !steps_in_parts(h)) {
+        h->last_begins.push_back(0);
+        return issue((int64_t)0, N, st);
+    }
     int rc = ensure_streams(h);
     if (rc != DOCKAUV_OK) return rc;
-    const int64_t N = h->n_envs;
     const int64_t part = (((N + DOCKAUV_STEP_PARTS - 1) / DOCKAUV_STEP_PARTS + 4095) / 4096) * 4096;   // at most PARTS ranges
     CUDA_TRY(cudaEventRecord(h->ev_fork, st));
     int s = 0;
     for (int64_t b = 0; b < N; b += part, s++) {
+        h->last_begins.push_back(b);
         CUDA_TRY(cudaStreamWaitEvent(h->hs[s], h->ev_fork, 0));
-        rc = step_range(h, actions, action_dtype, noise, out, nullptr, auto_reset, b, b + part < N ? b + part : N, h->hs[s]);
+        rc = issue(b, b + part < N ? b + part : N, h->hs[s]);
         if (rc != DOCKAUV_OK) return rc;
         CUDA_TRY(cudaEventRecord(h->hev[s], h->hs[s]));
         CUDA_TRY(cudaStreamWaitEvent(st, h->hev[s], 0));
@@ -800,8 +798,9 @@ static int step_parts(DockauvHandle *h, const void *actions, int action_dtype, c
 // one batched step on the device: in parts for large batches of the pipeline layout, else one launch group
 static int step_device(DockauvHandle *h, const void *actions, int action_dtype, const void *noise,
                        const DockauvStepOut *out, const DockauvDebugOut *dbg, int auto_reset, cudaStream_t st, bool timing) {
-    if (!timing && dbg == nullptr && steps_in_parts(h)) return step_parts(h, actions, action_dtype, noise, out, auto_reset, st);
-    return step_range(h, actions, action_dtype, noise, out, dbg, auto_reset, 0, h->n_envs, st, timing);
+    return over_ranges(h, timing || dbg != nullptr, st, [&](int64_t b, int64_t e, cudaStream_t s) {
+        return step_range(h, actions, action_dtype, noise, out, dbg, auto_reset, b, e, s, timing);
+    });
 }
 
 // step_device with the tap branch around it (when taps are set)
@@ -813,64 +812,35 @@ static int step_call(DockauvHandle *h, const void *actions, int action_dtype, co
     return rc;
 }
 
-#ifndef DOCKAUV_STEP_GRAPHS
-#define DOCKAUV_STEP_GRAPHS 96     // cached step graphs per handle (a trainer alternates between a few tensors; bench.py's pool: 64)
-#endif
-// One dockauv_step as a CUDA graph: the launch sequence (both halves, their fork / join events) is captured once per set
-// of pointers and replayed -- one graph launch instead of six kernel launches and four event operations, and no
-// launch-to-launch gaps on the device (what makes a 65,536-env step 24 us instead of 29).
-static int step_graph(DockauvHandle *h, const void *actions, int action_dtype, const void *noise, const DockauvStepOut *out,
-                      int auto_reset, cudaStream_t st) {
-    DockauvHandle::StepKey key;
-    key.actions = actions;
-    key.noise = noise;
-    key.out = *out;
-    key.action_dtype = action_dtype;
-    key.auto_reset = auto_reset;
-    key.seed = h->params.seed;
-    DockauvHandle::StepGraph *g = nullptr;
-    for (auto &c : h->sg)
-        if (c.key == key) {
-            g = &c;
-            break;
-        }
+// Replays the graph cached under `key`, first capturing what issue(stream) enqueues when there is none: on a private
+// stream (the caller's may be the legacy default stream, which cannot be captured).  The captured launches count once
+// per replay, and a replay restores the step ranges recorded during the capture.
+template <typename Key, typename F>
+static int graph_call(DockauvHandle *h, GraphCache<Key> &cache, const Key &key, const char *what, cudaStream_t st,
+                      F &&issue) {
+    auto *g = cache.find(key);
     if (g == nullptr) {
-        // capture on a private stream (the caller's may be the legacy default stream, which cannot be captured)
+        typename GraphCache<Key>::Graph fresh;
+        fresh.key = key;
         cudaStream_t cs = nullptr;
         CUDA_TRY(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
         cudaGraph_t graph = nullptr;
-        cudaGraphExec_t exec = nullptr;
         cudaError_t e = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
         int rc = DOCKAUV_OK;
         const int64_t before = h->launches;
-        h->last_begins.clear();
         if (e == cudaSuccess) {
-            rc = step_call(h, actions, action_dtype, noise, out, nullptr, auto_reset, cs, false);
+            rc = issue(cs);
             e = cudaStreamEndCapture(cs, &graph);
         }
-        const int64_t n_launch = h->launches - before;
-        h->launches = before;       // captured, not launched; every replay counts them
-        if (e == cudaSuccess && rc == DOCKAUV_OK) e = cudaGraphInstantiate(&exec, graph, 0);
+        fresh.launches = h->launches - before;
+        h->launches = before;       // captured, not launched
+        fresh.begins = h->last_begins;
+        if (e == cudaSuccess && rc == DOCKAUV_OK) e = cudaGraphInstantiate(&fresh.exec, graph, 0);
         if (graph) cudaGraphDestroy(graph);
         cudaStreamDestroy(cs);
         if (rc != DOCKAUV_OK) return rc;
-        if (e != cudaSuccess) return fail(DOCKAUV_ECUDA, "step graph capture failed: %s", cudaGetErrorString(e));
-        DockauvHandle::StepGraph fresh;
-        fresh.key = key;
-        fresh.exec = exec;
-        fresh.launches = n_launch;
-        fresh.begins = h->last_begins;
-        if (h->sg.size() < (size_t)DOCKAUV_STEP_GRAPHS) {
-            h->sg.push_back(fresh);
-            g = &h->sg.back();
-        } else {
-            DockauvHandle::StepGraph &victim = h->sg[h->sg_next];
-            h->sg_next = (h->sg_next + 1) % h->sg.size();
-            cudaGraphExecDestroy(victim.exec);
-            victim = fresh;
-            g = &victim;
-        }
-        h->sg_captures += 1;
+        if (e != cudaSuccess) return fail(DOCKAUV_ECUDA, "%s graph capture failed: %s", what, cudaGetErrorString(e));
+        g = cache.add(std::move(fresh));
     }
     CUDA_TRY(cudaGraphLaunch(g->exec, st));
     h->launches += g->launches;
@@ -895,11 +865,24 @@ extern "C" int dockauv_step(DockauvHandle *h, const void *actions_dev, int actio
         }
         CUDA_TRY(cudaEventRecord(h->ev0, st));
     }
-    h->last_begins.clear();
+    // One dockauv_step as a CUDA graph: the launch sequence (both halves, their fork / join events) is captured once per
+    // set of pointers and replayed -- one graph launch instead of six kernel launches and four event operations, and no
+    // launch-to-launch gaps on the device (what makes a 65,536-env step 24 us instead of 29).
     if (!h->timing && dbg == nullptr && h->sg_enabled) {
         cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-        if (cudaStreamIsCapturing(st, &cap) == cudaSuccess && cap == cudaStreamCaptureStatusNone)
-            return step_graph(h, actions_dev, action_dtype, noise_dev, out, auto_reset, st);
+        if (cudaStreamIsCapturing(st, &cap) == cudaSuccess && cap == cudaStreamCaptureStatusNone) {
+            DockauvHandle::StepKey key;
+            memset(&key, 0, sizeof(key));
+            key.actions = actions_dev;
+            key.noise = noise_dev;
+            key.out = *out;
+            key.action_dtype = action_dtype;
+            key.auto_reset = auto_reset;
+            key.seed = h->params.seed;
+            return graph_call(h, h->sg, key, "step", st, [&](cudaStream_t cs) {
+                return step_call(h, actions_dev, action_dtype, noise_dev, out, nullptr, auto_reset, cs, false);
+            });
+        }
     }
     int rc = step_call(h, actions_dev, action_dtype, noise_dev, out, dbg, auto_reset, st, h->timing);
     if (rc != DOCKAUV_OK) return rc;
@@ -918,7 +901,7 @@ extern "C" int dockauv_enable_step_graph(DockauvHandle *h, int enabled) {
 
 extern "C" int dockauv_step_graph_captures(DockauvHandle *h, int64_t *n) {
     if (!h || !n) return fail(DOCKAUV_EINVAL, "null argument");
-    *n = h->sg_captures;
+    *n = h->sg.captures;
     return DOCKAUV_OK;
 }
 
@@ -926,7 +909,6 @@ extern "C" int dockauv_step_graph_captures(DockauvHandle *h, int64_t *n) {
 static int ensure_host_pipeline(DockauvHandle *h, size_t action_bytes) {
     int rc0 = ensure_streams(h);
     if (rc0 != DOCKAUV_OK) return rc0;
-    const size_t esz = h->params.precision == DOCKAUV_F64 ? 8 : 4;
     if (h->st_actions_bytes < action_bytes) {
         if (h->st_actions) CUDA_TRY(cudaFree(h->st_actions));
         h->st_actions = nullptr;
@@ -934,7 +916,7 @@ static int ensure_host_pipeline(DockauvHandle *h, size_t action_bytes) {
         h->st_actions_bytes = action_bytes;
     }
     if (!h->st_obs) CUDA_TRY(cudaMalloc((void **)&h->st_obs, sizeof(float) * h->n_obs * (size_t)h->n_envs));
-    if (!h->st_reward) CUDA_TRY(cudaMalloc(&h->st_reward, esz * (size_t)h->n_envs));
+    if (!h->st_reward) CUDA_TRY(cudaMalloc(&h->st_reward, h->esz * (size_t)h->n_envs));
     if (!h->st_done) CUDA_TRY(cudaMalloc((void **)&h->st_done, (size_t)h->n_envs));
     if (!h->st_cond) CUDA_TRY(cudaMalloc((void **)&h->st_cond, (size_t)h->n_envs));
     return DOCKAUV_OK;
@@ -952,7 +934,7 @@ extern "C" int dockauv_step_host(DockauvHandle *h, const void *actions_host, int
     DeviceGuard guard(h->device);
     const int64_t N = h->n_envs;
     const size_t asz = (action_dtype == DOCKAUV_ACT_F32 ? 4 : 8) * (size_t)h->params.n_u;
-    const size_t esz = h->params.precision == DOCKAUV_F64 ? 8 : 4;
+    const size_t esz = h->esz;
     int rc = ensure_host_pipeline(h, asz * (size_t)N);
     if (rc != DOCKAUV_OK) return rc;
     h->last_begins.clear();
@@ -1005,6 +987,7 @@ extern "C" int dockauv_step_host(DockauvHandle *h, const void *actions_host, int
                                  cudaMemcpyHostToDevice, st));
         rc = step_range(h, h->st_actions, action_dtype, nullptr, &out, nullptr, auto_reset, b, e, st);
         if (rc != DOCKAUV_OK) return rc;
+        h->last_begins.push_back(b);
         CUDA_TRY(cudaMemcpyAsync(obs_host + (size_t)h->n_obs * b, h->st_obs + (size_t)h->n_obs * b,
                                  sizeof(float) * h->n_obs * (e - b), cudaMemcpyDeviceToHost, st));
         if ((c + 1) % (2 * kHostStreams) == 0 || e == N) {
@@ -1021,7 +1004,7 @@ extern "C" int dockauv_step_host(DockauvHandle *h, const void *actions_host, int
 static int rollout_issue(DockauvHandle *h, const void *actions, int action_dtype, int n_steps,
                          const DockauvRolloutOut &o, int auto_reset, cudaStream_t st) {
     const int64_t N = h->n_envs;
-    const size_t esz = h->params.precision == DOCKAUV_F64 ? 8 : 4;
+    const size_t esz = h->esz;
     const size_t arow = (action_dtype == DOCKAUV_ACT_F32 ? 4 : 8) * (size_t)h->params.n_u * (size_t)N;
     const size_t orow = (size_t)h->n_obs * (size_t)N;
     auto out_of_step = [&](int t) {
@@ -1046,33 +1029,17 @@ static int rollout_issue(DockauvHandle *h, const void *actions, int action_dtype
         }
         return DOCKAUV_OK;
     }
-    if (steps_in_parts(h)) {
-        // envs never interact and the actions are all known: each part of the batch runs its T steps as ONE chain on
-        // its own stream, forked from / joined to the caller's stream once per rollout instead of once per step
-        int rc = ensure_streams(h);
-        if (rc != DOCKAUV_OK) return rc;
-        const int64_t part = (((N + DOCKAUV_STEP_PARTS - 1) / DOCKAUV_STEP_PARTS + 4095) / 4096) * 4096;   // at most PARTS ranges
-        CUDA_TRY(cudaEventRecord(h->ev_fork, st));
-        int s = 0;
-        for (int64_t b = 0; b < N; b += part, s++) {
-            const int64_t e = b + part < N ? b + part : N;
-            CUDA_TRY(cudaStreamWaitEvent(h->hs[s], h->ev_fork, 0));
-            for (int t = 0; t < n_steps; t++) {
-                const DockauvStepOut so = out_of_step(t);
-                rc = step_range(h, (const char *)actions + arow * t, action_dtype, nullptr, &so, nullptr, auto_reset, b, e, h->hs[s]);
-                if (rc != DOCKAUV_OK) return rc;
-            }
-            CUDA_TRY(cudaEventRecord(h->hev[s], h->hs[s]));
-            CUDA_TRY(cudaStreamWaitEvent(st, h->hev[s], 0));
+    // without taps, envs never interact and the actions are all known: each part of a batch stepped in parts runs its T
+    // steps as ONE chain on its own stream, forked from / joined to the caller's stream once per rollout instead of once
+    // per step
+    return over_ranges(h, false, st, [&](int64_t b, int64_t e, cudaStream_t s) {
+        for (int t = 0; t < n_steps; t++) {
+            const DockauvStepOut so = out_of_step(t);
+            const int rc = step_range(h, (const char *)actions + arow * t, action_dtype, nullptr, &so, nullptr, auto_reset, b, e, s);
+            if (rc != DOCKAUV_OK) return rc;
         }
         return DOCKAUV_OK;
-    }
-    for (int t = 0; t < n_steps; t++) {
-        const DockauvStepOut so = out_of_step(t);
-        int rc = step_range(h, (const char *)actions + arow * t, action_dtype, nullptr, &so, nullptr, auto_reset, 0, N, st);
-        if (rc != DOCKAUV_OK) return rc;
-    }
-    return DOCKAUV_OK;
+    });
 }
 
 extern "C" int dockauv_rollout(DockauvHandle *h, const void *actions_dev, int action_dtype, int n_steps,
@@ -1089,44 +1056,16 @@ extern "C" int dockauv_rollout(DockauvHandle *h, const void *actions_dev, int ac
         CUDA_TRY(cudaMemsetAsync(out->ep_len_out, 0, sizeof(int32_t) * (size_t)h->n_envs * (size_t)n_steps, st));
     if (!use_graph) return rollout_issue(h, actions_dev, action_dtype, n_steps, *out, auto_reset, st);
     DockauvHandle::RolloutKey key;
+    memset(&key, 0, sizeof(key));
     key.actions = actions_dev;
     key.out = *out;
     key.n_steps = n_steps;
     key.action_dtype = action_dtype;
     key.auto_reset = auto_reset;
     key.seed = h->params.seed;
-    if (!h->rg_exec || !(key == h->rg_key)) {
-        if (h->rg_exec) {
-            cudaGraphExecDestroy(h->rg_exec);
-            h->rg_exec = nullptr;
-        }
-        // capture on a private stream (the caller's may be the legacy default stream, which cannot be captured)
-        cudaStream_t cs = nullptr;
-        CUDA_TRY(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
-        cudaGraph_t g = nullptr;
-        cudaError_t e = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
-        int rc = DOCKAUV_OK;
-        const int64_t launches_before = h->launches;
-        if (e == cudaSuccess) {
-            rc = rollout_issue(h, actions_dev, action_dtype, n_steps, *out, auto_reset, cs);
-            e = cudaStreamEndCapture(cs, &g);
-        }
-        h->rg_launches = h->launches - launches_before;
-        h->launches = launches_before;      // captured, not launched; every replay below counts them
-        if (e == cudaSuccess && rc == DOCKAUV_OK) e = cudaGraphInstantiate(&h->rg_exec, g, 0);
-        if (g) cudaGraphDestroy(g);
-        cudaStreamDestroy(cs);
-        if (rc != DOCKAUV_OK) return rc;
-        if (e != cudaSuccess) {
-            h->rg_exec = nullptr;
-            return fail(DOCKAUV_ECUDA, "rollout graph capture failed: %s", cudaGetErrorString(e));
-        }
-        h->rg_key = key;
-        h->rg_captures += 1;
-    }
-    CUDA_TRY(cudaGraphLaunch(h->rg_exec, st));
-    h->launches += h->rg_launches;
-    return DOCKAUV_OK;
+    return graph_call(h, h->rg, key, "rollout", st, [&](cudaStream_t cs) {
+        return rollout_issue(h, actions_dev, action_dtype, n_steps, *out, auto_reset, cs);
+    });
 }
 
 // ------------------------------------------------------------------------------------------- episode taps: setup
@@ -1166,13 +1105,13 @@ extern "C" int dockauv_set_taps(DockauvHandle *h, const int64_t *env_ids_host, i
     if (!tp.ev_join) CUDA_TRY(cudaEventCreateWithFlags(&tp.ev_join, cudaEventDisableTiming));
     if (!tp.dst) CUDA_TRY(cudaStreamCreateWithFlags(&tp.dst, cudaStreamNonBlocking));
     if (!tp.ev_dbg) CUDA_TRY(cudaEventCreateWithFlags(&tp.ev_dbg, cudaEventDisableTiming));
-    const size_t K = (size_t)n_taps, esz = h->params.precision == DOCKAUV_F64 ? 8 : 4;
+    const size_t K = (size_t)n_taps, esz = h->esz;
     const int nu = h->params.n_u, nc = h->params.n_capsules, ns = h->params.n_spheres, n_rays = h->params.n_rays;
     const bool pipe = h->pipe_buf != nullptr;
-    const int n_obsf = pipe ? h->kd.n_obsf : 0;
-    const size_t row_bytes = 8 * esz * (size_t)(nc + ns);      // one env's obstacle rows
-    tp.n_gather = 12 + nu + 3 + 1 + 5 + 7 * nc + 4 * ns + 3 + n_obsf + (pipe ? (int)(row_bytes / 16) : 0);
-    tp.shadow_launches = resolve_layout(h) == DOCKAUV_LAYOUT_PIPELINE ? pipe_launches(h->kd) : 1;
+    // the pipeline layout's buffers for K envs, laid out as dockauv_create lays them out for n_envs
+    tp.pipe = pipe ? pipe_buffers((int64_t)K, esz, nc, ns) : PipeBuffers();
+    const int row_pieces = pipe ? (int)(8 * esz * (size_t)(nc + ns) / 16) : 0;      // 16-byte pieces of one env's obstacle rows
+    tp.n_gather = 12 + nu + 3 + 1 + 5 + 7 * nc + 4 * ns + 3 + tp.pipe.n_obsf + row_pieces;
     tp.n_commit = 12 + nu + 12 + 3 + n_rays + 13 + 3 + h->n_obs;
     // one allocation, every piece 256-byte aligned (observation rows are written with 16-byte stores)
     size_t off = 0;
@@ -1199,17 +1138,7 @@ extern "C" int dockauv_set_taps(DockauvHandle *h, const int64_t *env_ids_host, i
                  o_rarr = take(13 * K * esz), o_nuc = take(3 * K * esz), o_sdot = take(12 * K * esz),
                  o_stats = take(kStatsBytes), o_ids = take(8 * K), o_sync = take(4),
                  o_grows = take(sizeof(TapRow) * tp.n_gather), o_crows = take(sizeof(TapRow) * tp.n_commit);
-    // the pipeline layout's buffers for K envs, as dockauv_create lays them out for n_envs: records, float obstacle
-    // records, obstacle rows, three view lists + the ended list, one counter block per 128 envs
-    size_t o_rec = 0, o_obsf = 0, o_obsd = 0, o_list = 0, o_end = 0, o_cnt = 0;
-    if (pipe) {
-        o_rec = take(16 * esz * K);
-        o_obsf = take(16 * (size_t)std::max(n_obsf, 1) * K);
-        o_obsd = take(std::max(row_bytes, (size_t)16) * K);
-        o_list = take(3 * 8 * K);
-        o_end = take(4 * ((K + 1) & ~(size_t)1));
-        o_cnt = take(4 * 16 * (K / 128 + 2));
-    }
+    const size_t o_pipe = take(tp.pipe.bytes);
     CUDA_TRY(cudaMalloc(&tp.mem, off));
     CUDA_TRY(cudaMemset(tp.mem, 0, off));
     char *m = (char *)tp.mem;
@@ -1232,12 +1161,7 @@ extern "C" int dockauv_set_taps(DockauvHandle *h, const int64_t *env_ids_host, i
     tp.dout.reward = m + o_drew;
     tp.dout.done = (uint8_t *)(m + o_ddone);
     tp.dout.cond_bits = (uint8_t *)(m + o_dcond);
-    tp.rec = pipe ? m + o_rec : nullptr;
-    tp.obsf = pipe && n_obsf > 0 ? (float4 *)(m + o_obsf) : nullptr;
-    tp.obsd = pipe && n_obsf > 0 ? m + o_obsd : nullptr;
-    tp.view_list = pipe ? (unsigned long long *)(m + o_list) : nullptr;
-    tp.ended_list = pipe ? (uint32_t *)(m + o_end) : nullptr;
-    tp.view_count = pipe ? (unsigned int *)(m + o_cnt) : nullptr;
+    tp.pipe_buf = pipe ? m + o_pipe : nullptr;
     memset(&tp.dbg, 0, sizeof(tp.dbg));
     tp.dbg.ray_dist = m + o_ray;
     tp.dbg.reward_arr = m + o_rarr;
@@ -1463,25 +1387,27 @@ extern "C" int dockauv_last_list_counts(DockauvHandle *h, int64_t *n_listed, int
     if (!h->pipe_buf) return DOCKAUV_OK;
     DeviceGuard guard(h->device);
     cudaStream_t st = (cudaStream_t)stream;
-    // one counter pair per env range the most recent step call stepped (halves of the batch, chunks of step_host)
-    const size_t n_cnt = 16 * ((size_t)h->n_envs / 128 + 2);
+    // one counter block per env range the most recent step call stepped (parts of the batch, chunks of step_host)
+    const size_t n_cnt = h->pipe.n_counters;
     std::vector<unsigned int> host(n_cnt);
-    CUDA_TRY(cudaMemcpyAsync(host.data(), h->kd.view_count, n_cnt * sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaStreamSynchronize(st));
-    for (int64_t b : h->last_begins) {
-        // fused cull: words 4..7 of a counter block hold the values at the end of the step (0..3 are zero again); else 0..3
-        const size_t k = 16 * (size_t)(b / 128) + (pipe_fuses_cull(h->kd) ? 4 : 0);
-        if (k + 3 < n_cnt) {
-            *n_listed += (int64_t)host[k] + host[k + 1] + host[k + 2];
-            *n_ended += host[k + 3];
+    return with_k(h, [&](auto &k) {
+        CUDA_TRY(cudaMemcpyAsync(host.data(), k.view_count, n_cnt * sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        for (int64_t b : h->last_begins) {
+            // fused cull: the live counters are zero again at the end of the step, and the copies hold its values
+            const size_t w = (size_t)counter_block(b) + (pipe_fuses_cull(k) ? kCounterLast : 0);
+            if (w + kListCounters <= n_cnt) {
+                *n_listed += (int64_t)host[w] + host[w + 1] + host[w + 2];
+                *n_ended += host[w + 3];
+            }
         }
-    }
-    return DOCKAUV_OK;
+        return DOCKAUV_OK;
+    });
 }
 
 extern "C" int dockauv_rollout_captures(DockauvHandle *h, int64_t *n) {
     if (!h || !n) return fail(DOCKAUV_EINVAL, "null argument");
-    *n = h->rg_captures;
+    *n = h->rg.captures;
     return DOCKAUV_OK;
 }
 

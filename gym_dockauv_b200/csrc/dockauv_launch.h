@@ -7,12 +7,13 @@
 
 namespace dockauv {
 
+// One step of k's env range.  *n_launches receives how many kernels it enqueued (valid when it returns cudaSuccess).
 // marks (nullable): kMaxStepLaunches + 1 events; when given, the multi-launch layouts record one before their first
 // launch and one after each launch, *n_marks receives how many were recorded (0 for single-launch layouts)
 constexpr int kMaxStepLaunches = 6;
 template <typename T>
-cudaError_t launch_step(const KParams<T> &k, int vehicle, int layout, cudaStream_t st, cudaEvent_t *marks = nullptr,
-                        int *n_marks = nullptr);
+cudaError_t launch_step(const KParams<T> &k, int vehicle, int layout, cudaStream_t st, int *n_launches,
+                        cudaEvent_t *marks = nullptr, int *n_marks = nullptr);
 
 template <typename T>
 cudaError_t launch_reset(const KParams<T> &k, const uint8_t *mask_dev, cudaStream_t st);
@@ -20,16 +21,59 @@ cudaError_t launch_reset(const KParams<T> &k, const uint8_t *mask_dev, cudaStrea
 #ifndef DOCKAUV_FUSE_MAX_OBSF
 #define DOCKAUV_FUSE_MAX_OBSF 20    // pipeline layout: the cull + finish code runs inside the dynamics launch when an env has at most this many float4 obstacle records: 80 KB of shared memory per 256-thread CTA, two CTAs per SM stay resident
 #endif
-// whether the dynamics launch of the pipeline layout takes the cull + finish code in, and how many launches one step over
-// one env range is
+// whether the dynamics launch of the pipeline layout takes the cull + finish code in
 template <typename T>
 inline bool pipe_fuses_cull(const KParams<T> &k) {
     return k.n_caps + k.n_sph > 0 && !k.cull_exact && k.n_obsf > 0 && k.n_obsf <= DOCKAUV_FUSE_MAX_OBSF;
 }
+
+// Work-list counters (KParams::view_count): one block of kCounterWords words per concurrently stepped env range; the
+// range that starts at env b uses block b / kCounterEnvs.  Words 0..kListCounters-1 are the live counters (view lists of
+// class 1, 2, 3, ended list); steps with the cull code fused into the dynamics launch keep their values at the end of
+// the most recent step in kCounterLast.. (dockauv_last_list_counts), and kCounterTicket is the ticket of the episode-end
+// launch, whose last CTA saves and zeroes the live counters.
+constexpr int kCounterWords = 16, kCounterEnvs = 128;
+constexpr int kListCounters = 4, kCounterLast = 4, kCounterTicket = 8;
+inline int64_t counter_block(int64_t env_begin) { return kCounterWords * (env_begin / kCounterEnvs); }
+
+// The library-owned buffers of the pipeline layout for n envs, as byte offsets into one allocation (every piece 256-byte
+// aligned): per-env records T[n][16], float obstacle records float4[n_obsf][n], obstacle rows T[n][n_obst][8], three view
+// lists u64[n] and the ended list u32[n], and the counter blocks.
+struct PipeBuffers {
+    int n_obsf = 0, n_obst = 0;
+    size_t rec = 0, obsf = 0, obsd = 0, view_list = 0, ended_list = 0, counters = 0;
+    size_t n_counters = 0, bytes = 0;
+};
+inline PipeBuffers pipe_buffers(int64_t n_envs, size_t esz, int n_caps, int n_sph) {
+    PipeBuffers b;
+    const size_t n = (size_t)n_envs;
+    b.n_obsf = 2 * n_caps + n_sph;
+    b.n_obst = n_caps + n_sph;
+    auto take = [&](size_t bytes) {
+        const size_t o = b.bytes;
+        b.bytes += (bytes + 255) & ~(size_t)255;
+        return o;
+    };
+    b.rec = take(16 * esz * n);
+    b.obsf = take(16 * (size_t)b.n_obsf * n);
+    b.obsd = take(8 * esz * (size_t)b.n_obst * n);
+    b.view_list = take(3 * 8 * n);
+    b.ended_list = take(4 * n);
+    b.n_counters = kCounterWords * (n / kCounterEnvs + 2);      // slack: a range may start at any multiple of 4096
+    b.counters = take(4 * b.n_counters);
+    return b;
+}
+// points k at such buffers at `base`, or at none (base == nullptr: the single-launch layouts)
 template <typename T>
-inline int pipe_launches(const KParams<T> &k) {
-    if (k.n_caps + k.n_sph == 0) return 2;      // dynamics (+ finish), episode end
-    return pipe_fuses_cull(k) ? 3 : 4;          // dynamics (+ cull + finish) [, cull + finish], rays, episode end
+inline void point_pipe(KParams<T> &k, const PipeBuffers &b, void *base) {
+    char *m = (char *)base;
+    k.n_obsf = b.n_obsf;
+    k.rec = m ? (T *)(m + b.rec) : nullptr;
+    k.obsf = m && b.n_obsf > 0 ? (float4 *)(m + b.obsf) : nullptr;
+    k.obsd = m && b.n_obst > 0 ? (T *)(m + b.obsd) : nullptr;
+    k.view_list = m ? (unsigned long long *)(m + b.view_list) : nullptr;
+    k.ended_list = m ? (uint32_t *)(m + b.ended_list) : nullptr;
+    k.view_count = m ? (unsigned int *)(m + b.counters) : nullptr;
 }
 
 // float obstacle records of the cull code from the bound obstacle / goal buffers (no-op for handles without them)

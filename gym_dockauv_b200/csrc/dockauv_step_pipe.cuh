@@ -56,11 +56,6 @@ constexpr int kDynThreads = DOCKAUV_DYN_THREADS;
 #define DOCKAUV_RAY_CTAS_PER_SM DOCKAUV_MINB_RAYS   // persistent grid of the ray launch, in 4-warp CTAs per SM (= what is resident)
 #endif
 
-// work-list counters per stepped env range (KParams::view_count): words 0..3 the live counters (view lists of class 1, 2, 3,
-// ended list); steps with the cull code fused into the dynamics launch: 4..7 their values at the end of the most recent
-// step (dockauv_last_list_counts), 8 the ticket of the episode-end launch, whose last CTA saves and zeroes the live counters
-constexpr int kListCounters = 4, kCounterStride = 16, kCounterLast = 4, kCounterTicket = 8;
-
 // ---- the per-env record written by the dynamics launch (KParams::rec).  A listed env's record goes to the ray launch
 //      with the words the ray launch does not read -- position relative to the goal, condition bits (they travel in the
 //      list entry) -- replaced by the post-step position and the running return: with the obstacle rows, that launch then
@@ -929,16 +924,20 @@ static cudaError_t launch_rays(const KParams<T> &kc, int64_t n, cudaStream_t st)
 }
 
 template <typename T, int VEH, int NU>
-static cudaError_t launch_step_pipe(const KParams<T> &k, cudaStream_t st, cudaEvent_t *marks = nullptr, int *n_marks = nullptr) {
-    if (wants_debug(k) || k.rec == nullptr) return launch_step_warp<T, VEH, NU>(k, st);   // debug outputs: fused kernel
+static cudaError_t launch_step_pipe(const KParams<T> &k, cudaStream_t st, int *n_launches, cudaEvent_t *marks, int *n_marks) {
+    if (wants_debug(k) || k.rec == nullptr) {       // debug outputs: fused kernel
+        *n_launches = 1;
+        return launch_step_warp<T, VEH, NU>(k, st);
+    }
     const int64_t n = k.env_end - k.env_begin;
     KParams<T> kc = k;
-    kc.view_count = k.view_count + kCounterStride * (k.env_begin / kWarpEnvs);   // counters per concurrently stepped env range
+    kc.view_count = k.view_count + counter_block(k.env_begin);
     kc.view_list = k.view_list + k.env_begin;
     kc.ended_list = k.ended_list + k.env_begin;
-    int n_mark = 0;
+    int n_mark = 0;      // one mark before the first launch and one after each
     auto mark = [&]() {
-        if (marks) cudaEventRecord(marks[n_mark++], st);
+        if (marks) cudaEventRecord(marks[n_mark], st);
+        n_mark++;
     };
     mark();
     const bool has_obstacles = k.n_caps + k.n_sph > 0;
@@ -970,7 +969,8 @@ static cudaError_t launch_step_pipe(const KParams<T> &k, cudaStream_t st, cudaEv
         if ((e = launch_dependent(episode_end_kernel<T>, (unsigned)blocks, kResetCta, 0, st, kc)) != cudaSuccess) return e;
         mark();
     }
-    if (n_marks) *n_marks = n_mark;
+    *n_launches = n_mark - 1;
+    if (n_marks) *n_marks = marks ? n_mark : 0;
     return cudaGetLastError();
 }
 

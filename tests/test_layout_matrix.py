@@ -95,13 +95,23 @@ def test_exact_cull_matches_float_cull():
 def test_list_counts_match_the_step_outputs(kw):
     """dockauv_last_list_counts after a step: the ended count is the number of done flags, the listed count the number of
     envs with a pooled ray cell below 1 or more (listed = something in view, a superset of real hits) -- with the cull code
-    inside the dynamics launch (counters saved and zeroed by the episode-end launch) and as a launch of its own."""
+    inside the dynamics launch (counters saved and zeroed by the episode-end launch) and as a launch of its own.  After a
+    rollout the counts are those of its last step: without a graph, at the capture and at a replay."""
     import torch
     from gym_dockauv_b200 import envs
     from gym_dockauv_b200.config import BASE_CONFIG, RADAR_64
     cfg = dict(BASE_CONFIG)
     cfg["radar"] = dict(RADAR_64)
     N = 40000                      # one launch group; also stepped in two parts below
+    T = 4
+
+    def check(n, obs, done, where):
+        n_listed, n_ended = env.last_list_counts()
+        assert n_ended == int(done.sum()), where
+        # observation rows of finished envs are zeroed; among the others a cell below 1 needs an obstacle in view
+        hit = int(((obs[:, 16:] < 1.0).any(1) & ~done.bool()).sum())
+        assert hit <= n_listed <= n, (where, hit, n_listed)
+
     for n in (N, 1 << 18):
         env = envs.ObstaclesDocking3d(cfg, num_envs=n, seed=2, **kw)
         env.reset()
@@ -109,10 +119,19 @@ def test_list_counts_match_the_step_outputs(kw):
         gen = torch.Generator(device="cuda").manual_seed(1)
         for t in range(14):
             obs, _, done, info = env.step(torch.rand(n, 6, device="cuda", generator=gen) * 2 - 1)
-            n_listed, n_ended = env.last_list_counts()
-            assert n_ended == int(done.sum()), (n, t)
-            # observation rows of finished envs are zeroed; among the others a cell below 1 needs an obstacle in view
-            hit = int(((obs[:, 16:] < 1.0).any(1) & ~done.bool()).sum())
-            assert hit <= n_listed <= n, (n, t, hit, n_listed)
+            check(n, obs, done, (n, t))
         assert env.get_stats()["episodes"] > 0
+        acts = torch.empty(T, n, 6, device="cuda")
+        obs = torch.zeros(T, n, env.n_observations, device="cuda")
+        rew = torch.zeros(T, n, dtype=env.dtype, device="cuda")
+        done = torch.zeros(T, n, dtype=torch.uint8, device="cuda")
+        for use_graph in (False, True, True):
+            # step counters in the last T steps of an episode: at every step of the rollout some episodes reach max_t
+            env.t_steps.copy_(torch.randint(env.max_timesteps - T + 1, env.max_timesteps + 1, (n,), device="cuda",
+                                            dtype=torch.int32, generator=gen))
+            acts.uniform_(-1, 1, generator=gen)
+            env.rollout(acts, obs, rew, done, use_graph=use_graph)
+            assert int(done[T - 1].sum()) > 0
+            check(n, obs[T - 1], done[T - 1], (n, "rollout", use_graph))
+        assert env.rollout_captures() == 1
         env.close()
