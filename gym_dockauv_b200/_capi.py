@@ -4,7 +4,7 @@ import ctypes as C
 import os
 
 from .params import (ABI_VERSION, DockauvBuffers, DockauvDebugOut, DockauvParams, DockauvReplayRing,
-                     DockauvReplaySample, DockauvRolloutOut, DockauvStepOut, DockauvTapBuffers)
+                     DockauvReplaySample, DockauvRolloutOut, DockauvScenarioBank, DockauvStepOut, DockauvTapBuffers)
 
 LIB_PATH = os.environ.get("DOCKAUV_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_lib",
                                                         "libdockauv_b200.so")   # DOCKAUV_LIB: tuning builds only
@@ -28,6 +28,7 @@ SYMBOLS = {
     "dockauv_step_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _i, C.POINTER(DockauvStepOut)]),
     "dockauv_rollout": (_i, [_vp, _vp, _i, _i, C.POINTER(DockauvRolloutOut), _i, _i, _vp]),
     "dockauv_set_taps": (_i, [_vp, C.POINTER(_i64), _i, _i, C.POINTER(DockauvTapBuffers)]),
+    "dockauv_set_scenario_bank": (_i, [_vp, C.POINTER(DockauvScenarioBank), _vp]),
     "dockauv_gae": (_i, [_vp, _i, _vp, _vp, _vp, _i, _i64, C.c_float, C.c_float, _vp, _vp, _vp]),
     "dockauv_replay_sample": (_i, [C.POINTER(DockauvReplayRing), _i, _i, _i64, _i, _i, _i64, _i64, _i64, C.c_uint64,
                                    C.c_uint64, C.POINTER(DockauvReplaySample), _vp]),

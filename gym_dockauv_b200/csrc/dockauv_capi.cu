@@ -188,6 +188,10 @@ struct DockauvHandle {
         cudaStream_t st = nullptr, dst = nullptr;      // output shadow + commit; debug shadow (the two run side by side)
         cudaEvent_t ev_fork = nullptr, ev_join = nullptr, ev_dbg = nullptr;
     } tap;
+    // scenario bank (dockauv_set_scenario_bank): the caller's table as last accepted (rows == nullptr: none), and the
+    // validation kernel's result word
+    DockauvScenarioBank bank = {};
+    unsigned long long *bank_check = nullptr;
 };
 
 static int pooled_dim(int n, int b) { return (n + b - 1) / b; }
@@ -435,6 +439,7 @@ extern "C" int dockauv_destroy(DockauvHandle *h) {
     if (h->tap.ev_join) cudaEventDestroy(h->tap.ev_join);
     if (h->tap.dst) cudaStreamDestroy(h->tap.dst);
     if (h->tap.ev_dbg) cudaEventDestroy(h->tap.ev_dbg);
+    if (h->bank_check) cudaFree(h->bank_check);
     drop_graphs(h);
     delete h;
     return DOCKAUV_OK;
@@ -675,6 +680,9 @@ static cudaError_t tap_issue(DockauvHandle *h, const KParams<T> &real, const voi
     set_io<T>(k, tp.actions, action_dtype == DOCKAUV_ACT_F32, tp.noise, tp.out, nullptr, 0);
     k.has_current = current_on(h);
     k.stats = tp.stats;
+    k.bank_rows = nullptr;          // the shadows never reset (no auto-reset), and their env count is not the bank's N
+    k.bank_cdf = nullptr;
+    k.bank_row_of_env = nullptr;
     point_pipe(k, tp.pipe, tp.pipe_buf);
     int n_shadow = 0, n_dbg = 0;
     e = launch_step<T>(k, h->params.vehicle, resolve_layout(h), tp.st, &n_shadow);
@@ -758,6 +766,8 @@ static bool steps_in_parts(const DockauvHandle *h) {
     return DOCKAUV_STEP_PARTS > 1 && h->n_envs >= (int64_t)DOCKAUV_PARTS_MIN_ENVS && resolve_layout(h) == DOCKAUV_LAYOUT_PIPELINE &&
            h->params.split_chunk_envs == 0;
 }
+
+static bool misaligned16(const void *p) { return (((uintptr_t)p) & 15u) != 0; }
 
 // obs / terminal_obs rows are written in 16-byte pieces when n_obs is a multiple of 4
 static int check_rows(const DockauvHandle *h, const float *obs, const float *terminal_obs) {
@@ -1189,6 +1199,148 @@ extern "C" int dockauv_set_taps(DockauvHandle *h, const int64_t *env_ids_host, i
     return DOCKAUV_OK;
 }
 
+// ------------------------------------------------------------------------------------------- scenario bank
+// Reasons a bank row is refused, in the order they are checked per field
+enum BankReason { kBankNonFinite = 1, kBankNegRadius, kBankFar, kBankCurrent, kBankCdf };
+static const char *const kBankReasonText[] = {
+    "", "value is not finite", "radius is negative",
+    "obstacle is neither within 2 km of the row's goal at every defining point nor an unused slot (radius 0, every point "
+    "at least 1e5 m from the goal)",
+    "non-zero current on a handle that does not evaluate the current (set force_current)",
+    "cdf must be finite and non-decreasing from >= 0, with cdf[K-1] > 0"};
+
+// Thread per row: the first offending field of the row (field W = the cdf entry) goes into *first_bad as
+// row << 24 | field << 8 | reason, the lowest value winning.
+template <typename T>
+__global__ void bank_validate_kernel(const T *rows, int64_t K, int64_t stride, int nc, int ns, int check_far,
+                                     int current_on, const double *cdf, unsigned long long *first_bad) {
+    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= K) return;
+    const T *row = rows + r * stride;
+    const int W = 15 + 7 * nc + 4 * ns;
+    int field = -1, reason = 0;
+    auto flag = [&](int f, int why) {
+        if (field < 0) {
+            field = f;
+            reason = why;
+        }
+    };
+    for (int f = 0; f < W && field < 0; f++)
+        if (!isfinite((double)row[f])) flag(f, kBankNonFinite);
+    if (field < 0 && !current_on)
+        for (int c = 0; c < 5; c++)
+            if (row[10 + c] != T(0)) flag(10 + c, kBankCurrent);
+    const double g[3] = {(double)row[6], (double)row[7], (double)row[8]};
+    auto dist = [&](const T *q) {
+        const double dx = (double)q[0] - g[0], dy = (double)q[1] - g[1], dz = (double)q[2] - g[2];
+        return sqrt(dx * dx + dy * dy + dz * dz);
+    };
+    for (int s = 0; s < nc + ns && field < 0; s++) {
+        const bool cap = s < nc;
+        const int o = cap ? 15 + 7 * s : 15 + 7 * nc + 4 * (s - nc);
+        const int ri = o + (cap ? 6 : 3);
+        const T *q = row + o;
+        if (row[ri] < T(0)) {
+            flag(ri, kBankNegRadius);
+            break;
+        }
+        if (!check_far) continue;
+        const double d0 = dist(q), d1 = cap ? dist(q + 3) : d0;
+        const bool near = d0 <= 2000.0 && d1 <= 2000.0;
+        const bool unused = row[ri] == T(0) && d0 >= 1e5 && d1 >= 1e5;
+        if (!near && !unused) flag(o, kBankFar);
+    }
+    if (field < 0 && cdf != nullptr) {
+        const double c = cdf[r], prev = r > 0 ? cdf[r - 1] : 0.0;
+        if (!isfinite(c) || !(c >= prev) || (r == K - 1 && !(c > 0.0))) flag(W, kBankCdf);
+    }
+    if (field >= 0) atomicMin(first_bad, ((unsigned long long)r << 24) | ((unsigned long long)field << 8) | (unsigned)reason);
+}
+
+// name of field f of a row (f == W: the cdf entry)
+static void bank_field_name(const DockauvParams &p, int f, char *out, size_t n) {
+    static const char *const head[] = {"pose x", "pose y", "pose z", "pose phi", "pose theta", "pose psi", "goal x",
+                                       "goal y", "goal z", "heading goal", "current V_c", "current alpha",
+                                       "current beta", "current V_min", "current V_max"};
+    static const char *const cap[] = {"bot x", "bot y", "bot z", "top x", "top y", "top z", "r"};
+    static const char *const sph[] = {"centre x", "centre y", "centre z", "r"};
+    const int nc = p.n_capsules, ns = p.n_spheres;
+    if (f < 15) snprintf(out, n, "%s", head[f]);
+    else if (f < 15 + 7 * nc) snprintf(out, n, "capsule %d %s", (f - 15) / 7, cap[(f - 15) % 7]);
+    else if (f < 15 + 7 * nc + 4 * ns) snprintf(out, n, "sphere %d %s", (f - 15 - 7 * nc) / 4, sph[(f - 15 - 7 * nc) % 4]);
+    else snprintf(out, n, "cdf");
+}
+
+extern "C" int dockauv_set_scenario_bank(DockauvHandle *h, const DockauvScenarioBank *b, void *stream) {
+    // what needs no handle first (W >= 15 for every handle: the row without obstacles)
+    if (b) {
+        if (!b->rows) return fail(DOCKAUV_EINVAL, "scenario bank: rows is null (pass a null bank to clear it)");
+        if (b->n_rows < 1 || b->n_rows > (int64_t)INT32_MAX)
+            return fail(DOCKAUV_EINVAL, "scenario bank: n_rows (K) must be in 1..2^31 - 1, got %lld", (long long)b->n_rows);
+        if (misaligned16(b->rows)) return fail(DOCKAUV_EINVAL, "scenario bank: rows must be 16-byte aligned");
+        if (b->row_stride < 15)
+            return fail(DOCKAUV_EINVAL, "scenario bank: row_stride %lld is below the row width W (at least 15 reals)",
+                        (long long)b->row_stride);
+        if ((((uintptr_t)b->cdf) & 7u) != 0 || (((uintptr_t)b->row_of_env) & 3u) != 0)
+            return fail(DOCKAUV_EINVAL, "scenario bank: cdf must be 8-byte and row_of_env 4-byte aligned");
+    }
+    if (!h) return fail(DOCKAUV_EINVAL, "null handle");
+    if (!b) {
+        if (h->bank.rows) drop_graphs(h);
+        h->bank = DockauvScenarioBank{};
+        with_k(h, [](auto &k) {
+            k.bank_rows = nullptr;
+            k.bank_cdf = nullptr;
+            k.bank_row_of_env = nullptr;
+            k.bank_n = k.bank_stride = 0;
+        });
+        return DOCKAUV_OK;
+    }
+    const int nc = h->params.n_capsules, ns = h->params.n_spheres, W = 15 + 7 * nc + 4 * ns;
+    if (b->row_stride < W)
+        return fail(DOCKAUV_EINVAL, "scenario bank: row_stride %lld is below the row width W = 15 + 7 n_capsules + 4 n_spheres "
+                                    "= %d", (long long)b->row_stride, W);
+    if ((b->row_stride * (int64_t)h->esz) % 16 != 0)
+        return fail(DOCKAUV_EINVAL, "scenario bank: row_stride * sizeof(real) = %lld bytes must be a multiple of 16",
+                    (long long)(b->row_stride * (int64_t)h->esz));
+    DeviceGuard guard(h->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!h->bank_check) CUDA_TRY(cudaMalloc((void **)&h->bank_check, sizeof(unsigned long long)));
+    CUDA_TRY(cudaMemsetAsync(h->bank_check, 0xff, sizeof(unsigned long long), st));
+    const int check_far = with_k(h, [](auto &k) { return k.cull_exact ? 0 : 1; });
+    const unsigned blocks = (unsigned)((b->n_rows + 255) / 256);
+    if (h->params.precision == DOCKAUV_F64)
+        bank_validate_kernel<double><<<blocks, 256, 0, st>>>((const double *)b->rows, b->n_rows, b->row_stride, nc, ns,
+                                                             check_far, current_on(h) ? 1 : 0, b->cdf, h->bank_check);
+    else
+        bank_validate_kernel<float><<<blocks, 256, 0, st>>>((const float *)b->rows, b->n_rows, b->row_stride, nc, ns,
+                                                            check_far, current_on(h) ? 1 : 0, b->cdf, h->bank_check);
+    CUDA_TRY(cudaGetLastError());
+    unsigned long long bad = 0;
+    CUDA_TRY(cudaMemcpyAsync(&bad, h->bank_check, sizeof(bad), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    if (bad != ~0ull) {
+        char name[64];
+        const int field = (int)((bad >> 8) & 0xffff), reason = (int)(bad & 0xff);
+        bank_field_name(h->params, field, name, sizeof(name));
+        return fail(DOCKAUV_EINVAL, "scenario bank refused: row %lld, %s: %s", (long long)(bad >> 24), name,
+                    kBankReasonText[reason]);
+    }
+    const DockauvScenarioBank &o = h->bank;
+    if (o.rows != b->rows || o.cdf != b->cdf || o.row_of_env != b->row_of_env || o.n_rows != b->n_rows ||
+        o.row_stride != b->row_stride)
+        drop_graphs(h);          // captured sequences hold the old pointers; the same pointers keep every graph
+    h->bank = *b;
+    with_k(h, [&](auto &k) {
+        k.bank_rows = (decltype(k.bank_rows))b->rows;
+        k.bank_cdf = b->cdf;
+        k.bank_row_of_env = b->row_of_env;
+        k.bank_n = b->n_rows;
+        k.bank_stride = b->row_stride;
+    });
+    return DOCKAUV_OK;
+}
+
 // ------------------------------------------------------------------------------------------- GAE
 template <typename R>
 __global__ void gae_kernel(const R *__restrict__ rewards, const float *__restrict__ values,
@@ -1288,8 +1440,6 @@ static void launch_replay_sample(bool vec4, unsigned blocks, cudaStream_t st, co
     else
         replay_sample_kernel<R, float><<<blocks, 256, 0, st>>>(ring, S, N, n_obs, n_u, slot0, n_valid, B, seed, draw, out);
 }
-
-static bool misaligned16(const void *p) { return (((uintptr_t)p) & 15u) != 0; }
 
 extern "C" int dockauv_replay_sample(const DockauvReplayRing *ring, int reward_precision, int n_slots, int64_t n_envs,
                                      int n_obs, int n_u, int64_t t_first, int64_t n_valid, int64_t batch, uint64_t seed,

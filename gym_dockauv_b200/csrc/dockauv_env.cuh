@@ -246,12 +246,136 @@ __device__ __forceinline__ void reset_env_role(const KParams<T> &p, int64_t i, i
     }
 }
 
+// ------------------------------------------------------------------------------------------- scenario bank reset
+// Row layout (dockauv_set_scenario_bank): pose [0:6], goal [6:9], heading goal [9], current [10:15], then capsule slots
+// (bot, top, r) and sphere slots (centre, r).  The row is drawn from Philox block (gid, episode, kBankCounter): the
+// built-in reset uses blocks below 32 and the current noise 0x80000000 | t, so the three never share a block.
+constexpr uint32_t kBankCounter = 0x40000000u;
+constexpr int kBankPose = 0, kBankGoal = 6, kBankHeading = 9, kBankCurrent = 10, kBankObst = 15;
+
+// the row of env gid's reset that starts episode ep + 1: uniform = high 64 bits of (64-bit word x K); weighted = the
+// first r with cdf[r] > u cdf[K-1] (u the block's 53-bit uniform, so zero-weight rows are never drawn)
+template <typename T>
+__device__ __forceinline__ int64_t bank_draw(const KParams<T> &p, uint64_t gid, uint32_t ep) {
+    uint32_t c[4] = {(uint32_t)gid, (uint32_t)(gid >> 32), ep, kBankCounter};
+    philox4x32_10(c, (uint32_t)p.seed, (uint32_t)(p.seed >> 32));
+    const double *cdf = p.bank_cdf;
+    if (cdf == nullptr) return (int64_t)__umul64hi(((uint64_t)c[0] << 32) | c[1], (uint64_t)p.bank_n);
+    const double x = ((double)(c[0] >> 5) * 67108864.0 + (double)(c[1] >> 6)) * (1.0 / 9007199254740992.0) * cdf[p.bank_n - 1];
+    int64_t lo = 0, hi = p.bank_n - 1;         // x < cdf[K-1]: the answer lies in [lo, hi]
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (cdf[mid] > x) hi = mid;
+        else lo = mid + 1;
+    }
+    return lo;
+}
+
+// N reals of a row from offset o, read as the 16-byte pieces that cover them (rows and their stride are 16-byte
+// multiples, so the pieces stay inside the row)
+template <typename T, int N>
+__device__ __forceinline__ void load_bank_span(const T *row, int o, T out[N]) {
+    constexpr int V = 16 / (int)sizeof(T);
+    constexpr int NP = (N + V - 1) / V + 1;           // pieces for N reals at any offset within a piece
+    const int base = o & ~(V - 1), sh = o - base;
+    T buf[NP * V];
+#pragma unroll
+    for (int c = 0; c < NP; c++) {
+        if (base + c * V >= o + N) break;
+        if constexpr (sizeof(T) == 8) {
+            const double2 v = reinterpret_cast<const double2 *>(row + base)[c];
+            buf[2 * c] = v.x;
+            buf[2 * c + 1] = v.y;
+        } else {
+            const float4 v = reinterpret_cast<const float4 *>(row + base)[c];
+            buf[4 * c] = v.x;
+            buf[4 * c + 1] = v.y;
+            buf[4 * c + 2] = v.z;
+            buf[4 * c + 3] = v.w;
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < N; j++) {
+        T v = buf[j];
+#pragma unroll
+        for (int s = 1; s < V; s++)
+            if (sh == s) v = buf[s + j];
+        out[j] = v;
+    }
+}
+
+// One role of a reset from the bank: the same eight-role split as reset_env_role and the same rule (every role draws the
+// row itself, roles never exchange values).  0 pose, zero nu_r, goal, heading goal, counters, row_of_env; 1 current and
+// u_prev; 2..7 obstacle slots role - 2, role + 4, .. (capsules first, then spheres).
+//   ep: the env's episode counter BEFORE this reset
+template <typename T>
+__device__ __forceinline__ void bank_reset_role(const KParams<T> &p, int64_t i, int role, uint32_t ep) {
+    const int64_t N = p.n_envs;
+    const int n_slots = p.n_caps + p.n_sph;
+    if (role >= 2 && role - 2 >= n_slots) return;
+    const int64_t r = bank_draw<T>(p, p.env_id0 + (uint64_t)i, ep);
+    const T *row = p.bank_rows + r * p.bank_stride;
+    if (role == 0) {
+        T a[10];
+        load_bank_span<T, 10>(row, kBankPose, a);
+#pragma unroll
+        for (int c = 0; c < 6; c++) p.state[(int64_t)c * N + i] = a[c];
+#pragma unroll
+        for (int c = 6; c < 12; c++) p.state[(int64_t)c * N + i] = T(0);     // auvsim.py:55-65
+#pragma unroll
+        for (int c = 0; c < 3; c++) p.goal[(int64_t)c * N + i] = a[kBankGoal + c];
+        p.heading_goal[i] = a[kBankHeading];
+        p.t_steps[i] = 0;
+        p.ep_return[i] = T(0);
+        if (p.bank_row_of_env) {
+            p.bank_row_of_env[N + i] = p.bank_row_of_env[i];
+            p.bank_row_of_env[i] = (int32_t)r;
+        }
+    } else if (role == 1) {
+        T cur[5];
+        load_bank_span<T, 5>(row, kBankCurrent, cur);
+#pragma unroll
+        for (int c = 0; c < 5; c++) p.current[(int64_t)c * N + i] = cur[c];
+        for (int k = 0; k < p.n_u; k++) p.u_prev[(int64_t)k * N + i] = T(0);
+    } else {
+        T goal[3];
+        load_bank_span<T, 3>(row, kBankGoal, goal);
+        for (int s = role - 2; s < n_slots; s += kResetRoles - 2) {
+            if (s < p.n_caps) {
+                T cap[7];
+                load_bank_span<T, 7>(row, kBankObst + 7 * s, cap);
+#pragma unroll
+                for (int j = 0; j < 7; j++) p.capsules[(int64_t)(s * 7 + j) * N + i] = cap[j];
+                store_capsule_record<T>(p, i, s, cap, goal);
+            } else {
+                const int k = s - p.n_caps;
+                T sph[4];
+                load_bank_span<T, 4>(row, kBankObst + 7 * p.n_caps + 4 * k, sph);
+#pragma unroll
+                for (int j = 0; j < 4; j++) p.spheres[(int64_t)(k * 4 + j) * N + i] = sph[j];
+                store_sphere_record<T>(p, i, k, sph, goal);
+            }
+        }
+    }
+}
+
+// the whole bank reset by one thread, kept out of line: the single-launch step kernels reach it through one uniform branch
+template <typename T>
+static __device__ __noinline__ void bank_reset_env(const KParams<T> &p, int64_t i, uint32_t ep) {
+#pragma unroll 1
+    for (int role = 0; role < kResetRoles; role++) bank_reset_role<T>(p, i, role, ep);
+}
+
 // the whole reset by one thread (single-launch layouts: the env's own thread re-initialises it inside the step)
 template <typename T>
 static __device__ __noinline__ void reset_env(const KParams<T> &p, int64_t i) {
     const uint32_t ep = (uint32_t)p.episode[i];
+    if (p.bank_rows != nullptr) {
+        bank_reset_env<T>(p, i, ep);
+    } else {
 #pragma unroll 1
-    for (int role = 0; role < kResetRoles; role++) reset_env_role<T>(p, i, role, ep);
+        for (int role = 0; role < kResetRoles; role++) reset_env_role<T>(p, i, role, ep);
+    }
     p.episode[i] = (int32_t)(ep + 1);
 }
 
@@ -259,26 +383,28 @@ static __device__ __noinline__ void reset_env(const KParams<T> &p, int64_t i) {
 // so they must not share a warp (eight roles on eight lanes of one warp run one after the other: measured, no faster than
 // one thread per reset); as warps they run side by side and every lane of a warp does the same thing for another env.
 //   valid: this lane has an env.  Must be called by all threads of the CTA.
+//   BANK: reset from the scenario bank (KParams::bank_rows) instead of the built-in distributions
 constexpr int kResetCta = 32 * kResetRoles;
 
-template <typename T>
+template <typename T, bool BANK>
 __device__ __forceinline__ void reset_envs_cta(const KParams<T> &p, int64_t i, bool valid) {
     const int role = threadIdx.x >> 5;
     uint32_t ep = 0;
     if (valid) ep = (uint32_t)p.episode[i];
     __syncthreads();                                 // every role has read the episode counter before role 0 bumps it
     if (valid) {
-        reset_env_role<T>(p, i, role, ep);
+        if (BANK) bank_reset_role<T>(p, i, role, ep);
+        else reset_env_role<T>(p, i, role, ep);
         if (role == 0) p.episode[i] = (int32_t)(ep + 1);
     }
 }
 
 // dockauv_reset: one CTA of kResetRoles warps per 32 envs
-template <typename T>
+template <typename T, bool BANK>
 __global__ void __launch_bounds__(kResetCta) reset_kernel(const __grid_constant__ KParams<T> p, const uint8_t *mask) {
     const int64_t i = p.env_begin + (int64_t)blockIdx.x * 32 + (threadIdx.x & 31);
     const bool valid = i < p.env_end && (mask == nullptr || mask[i] != 0);
-    reset_envs_cta<T>(p, i, valid);
+    reset_envs_cta<T, BANK>(p, i, valid);
 }
 
 // ------------------------------------------------------------------------------------------- step pieces

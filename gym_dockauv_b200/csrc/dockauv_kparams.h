@@ -92,6 +92,12 @@ struct KParams {
     // ray table in global memory (handle-owned): rd_b[3][n_rays] then beta_oa[n_rays].  It is not part of this block:
     // the block travels with every launch, and 8 KB of ray table made it 11 KB
     const T *ray_tab;
+    // scenario bank (dockauv_set_scenario_bank), caller-owned; bank_rows == nullptr: the built-in reset.  Last in the
+    // block so that every field above keeps its offset in the constant bank
+    const T *bank_rows;              // real[bank_n][bank_stride], 16-byte aligned rows
+    const double *bank_cdf;          // nullable: running sum of the row weights (weighted draw)
+    int32_t *bank_row_of_env;        // nullable: int32[2][n_envs], row of the running / of the last ended episode
+    int64_t bank_n, bank_stride;
 };
 
 }  // namespace dockauv

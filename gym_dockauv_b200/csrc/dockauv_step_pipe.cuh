@@ -813,7 +813,8 @@ __global__ void __launch_bounds__(kTpeThreads, DOCKAUV_MINB_TPE) rays_thread_ker
 // ray launch): ~4000 warp instructions per reset at 1..8 active lanes, 28 M per half batch, a third of the ray launch; one
 // THREAD per ended env: 40x leaner but a 5500-instruction dependent chain, 70 us for a launch that occupies 5 % of the GPU;
 // eight LANES per env: the roles serialise inside the warp, same 70 us.
-template <typename T>
+//   BANK: finished envs are re-initialised from the scenario bank (KParams::bank_rows)
+template <typename T, bool BANK>
 __global__ void __launch_bounds__(kResetCta) episode_end_kernel(const __grid_constant__ KParams<T> p) {
     grid_dependency_wait();
     const unsigned n_ended = p.view_count[3];
@@ -842,7 +843,7 @@ __global__ void __launch_bounds__(kResetCta) episode_end_kernel(const __grid_con
                 }
             }
         }
-        if (p.auto_reset) reset_envs_cta<T>(p, ie, valid);
+        if (p.auto_reset) reset_envs_cta<T, BANK>(p, ie, valid);
     }
     // ---- steps whose dynamics launch appends to the lists itself (cull code fused in) cannot have that launch empty
     //      them: the last CTA to get here saves the list counters of this step and zeroes them for the next one (every CTA
@@ -966,7 +967,8 @@ static cudaError_t launch_step_pipe(const KParams<T> &k, cudaStream_t st, int *n
         int64_t blocks = n / 1024 + 1;
         const int64_t cap = (int64_t)(k.sm_count > 0 ? k.sm_count : 148) * 4;
         if (blocks > cap) blocks = cap;
-        if ((e = launch_dependent(episode_end_kernel<T>, (unsigned)blocks, kResetCta, 0, st, kc)) != cudaSuccess) return e;
+        auto kern = k.bank_rows != nullptr ? episode_end_kernel<T, true> : episode_end_kernel<T, false>;
+        if ((e = launch_dependent(kern, (unsigned)blocks, kResetCta, 0, st, kc)) != cudaSuccess) return e;
         mark();
     }
     *n_launches = n_mark - 1;

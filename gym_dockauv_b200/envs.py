@@ -23,7 +23,8 @@ import torch
 from . import _capi
 from .config import BASE_CONFIG, REGISTRATION_DICT
 from .params import (ACT_F32, ACT_F64, F32, F64, MAX_TAPS, N_STATS, SCENARIO_IDS, STAT_NAMES, TAP_FIELDS, DockauvBuffers,
-                     DockauvDebugOut, DockauvRolloutOut, DockauvStepOut, DockauvTapBuffers, pack_params)
+                     DockauvDebugOut, DockauvRolloutOut, DockauvScenarioBank, DockauvStepOut, DockauvTapBuffers,
+                     pack_params)
 
 DONE_NAMES = ("Done-Goal_reached", "Done-out_pos", "Done-out_att", "Done-max_t", "Done-collision")
 
@@ -65,6 +66,11 @@ class BaseDocking3d:
             raise TypeError("instantiate one of the scenario classes (SimpleDocking3d, ObstaclesDocking3d, ...)")
         self._lib = _capi.load()
         self.config = env_config
+        self._init_kwargs = dict(device=device, precision=precision, seed=seed, env_id0=env_id0, layout=layout,
+                                 n_spheres=n_spheres, n_synthetic_spheres=n_synthetic_spheres, n_capsules=n_capsules,
+                                 vehicle_xml=vehicle_xml, control_mode=control_mode, cur_mu=cur_mu, cur_sigma=cur_sigma,
+                                 force_current=force_current, auto_reset=auto_reset, debug_outputs=debug_outputs,
+                                 split_chunk_envs=split_chunk_envs)
         self.num_envs = int(num_envs)
         self.device = torch.device(device)
         if self.device.type != "cuda":
@@ -141,6 +147,9 @@ class BaseDocking3d:
                                                                        "nav", "obs_f64", "state_dot")])
         self._host = None
         self.taps = None
+        self._bank = None
+        self.bank_row = None           # scenario bank: row of each env's running episode (-1 = not from the bank)
+        self.ended_bank_row = None     # ... and of the episode its most recent reset ended
         self.t_total_steps = 0
 
     # ------------------------------------------------------------------ lifecycle
@@ -343,6 +352,71 @@ class BaseDocking3d:
         """Remove the taps: the next steps are launched exactly as without them."""
         _capi.check(self._lib.dockauv_set_taps(self._handle, None, 0, 0, None))
         self.taps = None
+
+    # ------------------------------------------------------------------ scenario bank (dockauv_set_scenario_bank)
+    def set_scenario_bank(self, bank, weights=None):
+        """Draw every following reset (``reset`` and the in-step auto-reset) from ``bank``: a ``ScenarioBank`` or a
+        row table [K, stride] in the env dtype on its device (layout in gym_dockauv_b200/scenario_bank.py).  Rows are
+        drawn uniformly, or in proportion to ``weights`` [K] (non-negative).  The library validates the rows on the
+        device and refuses the bank (DockauvError naming the row and field) without changing the previous setting.
+        Passing the bank that is already set again publishes rows rewritten in place (with ``weights``: new weights,
+        as ``set_scenario_weights``); the pointers stay the same, so no step or rollout graph is re-captured.
+        ``bank_row`` / ``ended_bank_row`` then hold the row of each env's running episode and of the episode its
+        most recent reset ended: at a step whose ``done`` is set, ``ended_bank_row[i]`` is the row of the episode that
+        just ended.  The env keeps references to the tensors it hands to the library."""
+        rows = getattr(bank, "rows", bank)
+        if not torch.is_tensor(rows) or rows.dim() != 2 or rows.dtype != self.dtype or rows.device != self.device \
+                or rows.stride(1) != 1:
+            raise ValueError(f"bank rows must be a 2-D {self.dtype} tensor on {self.device} with contiguous rows")
+        if self._bank is not None and self._bank[0] is rows:
+            if weights is None:
+                self._set_bank(*self._bank)
+            else:
+                self.set_scenario_weights(weights)
+            return
+        cdf = None if weights is None else self._cdf(weights, rows.shape[0])
+        row_of_env = torch.full((2, self.num_envs), -1, dtype=torch.int32, device=self.device)
+        self._set_bank(rows, cdf, row_of_env)
+
+    def set_scenario_weights(self, weights):
+        """New draw weights [K] for the bank that is set.  The running sums are rewritten in place (float64
+        ``torch.cumsum``) and re-validated: cached step and rollout graphs stay valid, nothing is re-captured.  On a
+        bank set without weights the first call allocates the sums (one re-capture)."""
+        if self._bank is None:
+            raise RuntimeError("no scenario bank is set")
+        rows, cdf, row_of_env = self._bank
+        K = rows.shape[0]
+        if cdf is None:
+            self._set_bank(rows, self._cdf(weights, K), row_of_env)
+            return
+        old = cdf.clone()
+        torch.cumsum(self._weights(weights, K), 0, out=cdf)
+        try:
+            self._set_bank(rows, cdf, row_of_env)
+        except _capi.DockauvError:
+            cdf.copy_(old)            # the previous weights stay in effect
+            raise
+
+    def clear_scenario_bank(self):
+        """Back to the scenario's built-in reset distributions."""
+        _capi.check(self._lib.dockauv_set_scenario_bank(self._handle, None, self._stream()))
+        self._bank = None
+        self.bank_row = self.ended_bank_row = None
+
+    def _weights(self, weights, K):
+        w = torch.as_tensor(weights).to(device=self.device, dtype=torch.float64).reshape(-1)
+        if w.shape[0] != K:
+            raise ValueError(f"{K} weights expected, got {w.shape[0]}")
+        return w
+
+    def _cdf(self, weights, K):
+        return torch.cumsum(self._weights(weights, K), 0).contiguous()
+
+    def _set_bank(self, rows, cdf, row_of_env):
+        b = DockauvScenarioBank(_ptr(rows), _ptr(cdf), _ptr(row_of_env), rows.shape[0], rows.stride(0))
+        _capi.check(self._lib.dockauv_set_scenario_bank(self._handle, C.byref(b), self._stream()))
+        self._bank = (rows, cdf, row_of_env)
+        self.bank_row, self.ended_bank_row = row_of_env[0], row_of_env[1]
 
     # ------------------------------------------------------------------ exact-state injection (parity tests, resume)
     def set_state(self, state=None, u_prev=None, goal=None, heading_goal=None, current=None, capsules=None,

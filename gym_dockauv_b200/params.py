@@ -86,6 +86,14 @@ class DockauvReplaySample(C.Structure):
     _fields_ = [(k, C.c_void_p) for k in ("obs", "actions", "next_obs", "done", "reward", "index")]
 
 
+SCENARIO_BANK_FIELDS = ("rows", "cdf", "row_of_env", "n_rows", "row_stride")
+
+
+class DockauvScenarioBank(C.Structure):
+    _fields_ = [("rows", C.c_void_p), ("cdf", C.c_void_p), ("row_of_env", C.c_void_p), ("n_rows", C.c_int64),
+                ("row_stride", C.c_int64)]
+
+
 def skew(a):
     """S(a) b = a x b (utils/geomutils.py:106-128)."""
     return np.array([[0.0, -a[2], a[1]], [a[2], 0.0, -a[0]], [-a[1], a[0], 0.0]])

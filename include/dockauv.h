@@ -26,6 +26,8 @@
  *   DockauvDebugOut (state_dot, ...)   EpisodeDataStorage.update          utils/datastorage.py:268-288
  *   dockauv_set_taps                   the same, during training: every step of a few chosen envs recorded on
  *                                      the device (interval_datastorage, config.py; datastorage.py:268-288)
+ *   dockauv_set_scenario_bank          a subclass's own generate_environment override (docking3d.py:795-988):
+ *                                      resets draw caller-supplied initial conditions, uniformly or by weight
  *
  * Conventions
  *   - plain C types only; no torch / C++ types cross this boundary.
@@ -309,6 +311,47 @@ DOCKAUV_API int dockauv_rollout(DockauvHandle *h, const void *actions_dev, int a
  * dockauv_step_host refuses to run while taps are set (DOCKAUV_ESTATE): taps record device-driven steps. */
 DOCKAUV_API int dockauv_set_taps(DockauvHandle *h, const int64_t *env_ids_host, int n_taps, int capacity,
                                  const DockauvTapBuffers *bufs);
+
+/* Scenario bank: a caller-owned device table of K initial conditions that every reset draws from while it is set (the
+ * in-step auto-reset of every layout and dockauv_reset), in place of the scenario's built-in distributions.  It stands
+ * in for a subclass's own generate_environment (docking3d.py:795-988).
+ *
+ * A row holds W = 15 + 7 n_capsules + 4 n_spheres reals in the handle's precision:
+ *   [0:6] pose x y z phi theta psi | [6:9] goal | [9] heading goal | [10:15] current V_c alpha beta V_min V_max |
+ *   capsule slots (bot[3], top[3], r) | sphere slots (centre[3], r)
+ * A reset from row r writes the pose and zeroes nu_r (auvsim.py:55-65), copies goal, heading goal, current and
+ * obstacles (and the library's obstacle copies for the cull), zeroes u_prev, t_steps and ep_return, increments episode
+ * and, when row_of_env is set, moves plane 0 to plane 1 and writes r to plane 0.  Unused obstacle slots take the form the
+ * built-in reset gives them: radius 0 and every point at least 1e5 m from the goal.
+ *
+ * The row is drawn from Philox4x32-10 block (global id lo, global id hi, episode before the reset, 0x40000000): uniform
+ * over K rows (high 64 bits of a 64-bit word times K), or, with cdf, the first r with cdf[r] > u cdf[K-1] for the block's
+ * 53-bit uniform u (zero-weight rows are never drawn).  The draw depends on (seed, global id, episode) only: the same rows
+ * whatever the sharding, and reset(seed=...) reproduces them. */
+typedef struct DockauvScenarioBank {
+    const void   *rows;        /* real[K][row_stride], caller-owned, 16-byte aligned */
+    const double *cdf;         /* nullable: f64[K] running sum of non-negative row weights; NULL = uniform */
+    int32_t      *row_of_env;  /* nullable: int32[2][N]; plane 0 = row of the running episode,
+                                  plane 1 = row of the episode the env's most recent reset ended;
+                                  -1 = none, the caller fills it before the first set */
+    int64_t       n_rows;      /* K, 1 .. 2^31 - 1 */
+    int64_t       row_stride;  /* in reals, >= W, row_stride * sizeof(real) a multiple of 16 */
+} DockauvScenarioBank;
+
+/* Set (bank_or_null non-NULL) or clear (NULL) the scenario bank.  The arguments are checked on the host first (rows,
+ * K, alignment and stride: these checks need no handle and come before the null-handle check), then one validation
+ * kernel reads the K rows and the cdf on `stream`, and the call synchronises `stream`.  A bank is refused
+ * (DOCKAUV_EINVAL, the message names the first offending row and field) when a value is not finite, a radius is
+ * negative, an obstacle is neither within 2 km of its row's goal at every defining point nor in the unused-slot form
+ * (not checked on handles whose float cull is off anyway), a row has a non-zero current on a handle that does not
+ * evaluate the current (force_current), or the cdf is not finite and non-decreasing from >= 0 with cdf[K-1] > 0.  A
+ * refused bank leaves the previous setting in effect.
+ * Graphs: the bank's pointers and K are baked into the captured step and rollout graphs.  A call with other pointers, K
+ * or stride, and clearing, drops the cached graphs; a call with the SAME values only re-validates the contents and keeps
+ * every graph.  That is how rows or weights rewritten in place are published (a curriculum update once per rollout).
+ * Contents rewritten in place without this call are used unvalidated, like buffers written without
+ * dockauv_refresh_obstacles. */
+DOCKAUV_API int dockauv_set_scenario_bank(DockauvHandle *h, const DockauvScenarioBank *bank_or_null, void *stream);
 
 /* Generalised advantage estimation over a stacked rollout, one thread per env walking t = T-1 .. 0
  * (float32 like the caller's RolloutBuffer):
