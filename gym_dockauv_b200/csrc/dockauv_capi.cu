@@ -1544,8 +1544,8 @@ extern "C" int dockauv_last_list_counts(DockauvHandle *h, int64_t *n_listed, int
         CUDA_TRY(cudaMemcpyAsync(host.data(), k.view_count, n_cnt * sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaStreamSynchronize(st));
         for (int64_t b : h->last_begins) {
-            // fused cull: the live counters are zero again at the end of the step, and the copies hold its values
-            const size_t w = (size_t)counter_block(b) + (pipe_fuses_cull(k) ? kCounterLast : 0);
+            // with obstacles the live counters are zero again at the end of the step, and the copies hold its values
+            const size_t w = (size_t)counter_block(b) + (pipe_has_obstacles(k) ? kCounterLast : 0);
             if (w + kListCounters <= n_cnt) {
                 *n_listed += (int64_t)host[w] + host[w + 1] + host[w + 2];
                 *n_ended += host[w + 3];

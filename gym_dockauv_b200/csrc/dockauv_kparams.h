@@ -59,13 +59,14 @@ struct KParams {
     // debug outputs
     T *dbg_ray_dist, *dbg_reward_arr, *dbg_euler_dot, *dbg_nu_c, *dbg_nav, *dbg_obs, *dbg_state_dot;
     // pipeline layout (library-owned buffers):
-    //   rec      T[n_envs][16], one 16-word record per env written by the dynamics launch (AoS: one 128-byte line in
-    //            f64): 0..5 sin/cos of the post-step attitude (sphi cphi sth cth spsi cpsi), 6..8 post-step position
-    //            relative to the goal, 9 (r0+r1)+(r2+r3), 10 r4+r5, 11 r7 (reward terms that need no radar, already
-    //            combined in numpy's summation order), 12 log_precision(delta_d), 13 delta_d, 14 done-condition bits
-    //            0..2 as a number, 15 NaN poison word (0 for a finite pose).  The record of a LISTED env, as the ray launch
-    //            reads it, holds everything that launch needs besides the obstacle rows: words 6..8 are the post-step
-    //            position itself and word 14 the running return before this step (REC_POS, REC_EPR)
+    //   rec      T[n_envs][16], the 16-word record of an env, computed in registers by the dynamics launch (AoS: one
+    //            128-byte line in f64): 0..5 sin/cos of the post-step attitude (sphi cphi sth cth spsi cpsi), 6..8
+    //            post-step position relative to the goal, 9 (r0+r1)+(r2+r3), 10 r4+r5, 11 r7 (reward terms that need no
+    //            radar, already combined in numpy's summation order), 12 log_precision(delta_d), 13 delta_d, 14
+    //            done-condition bits 0..2 as a number, 15 NaN poison word (0 for a finite pose).  It is stored only for
+    //            the LISTED envs, in the form the ray launch reads: everything that launch needs besides the obstacle
+    //            rows, with words 6..8 the post-step position itself and word 14 the running return before this step
+    //            (REC_POS, REC_EPR)
     //   obsf     float4[n_obsf][n_envs]: float copy of the obstacles RELATIVE TO THE GOAL for the cull (written by every
     //            reset and by dockauv_refresh_obstacles): capsule k -> slots 2k (bot - goal, radius), 2k+1 (unit axis
     //            (top - bot) / L, L); sphere s -> slot 2 n_caps + s (centre - goal, radius)
@@ -78,12 +79,12 @@ struct KParams {
     T *rec;
     float4 *obsf;
     T *obsd;
-    int32_t n_obsf, cull_exact;      // cull_exact: coordinates too large for the float cull -> decide everything in T
+    int32_t n_obsf, cull_exact;      // cull_exact: coordinates too large for the float cull -> decide everything in T (the step's copy then has n_obsf = 0: no float record is staged)
     int32_t tpe_rays;                // the thread-per-env ray launch covers this radar (2x2 pooling, <= 64 pooled cells)
     unsigned long long *view_list;
     uint32_t *ended_list;
     unsigned int *view_count;
-    int32_t counters_zeroed_at_end;  // 1: the last CTA of the episode-end launch saves and zeroes the list counters (steps for which pipe_fuses_cull holds); 0: the dynamics launch zeroes them at its start
+    int32_t counters_zeroed_at_end;  // 1: the last CTA of the episode-end launch saves and zeroes the list counters (steps with obstacles, pipe_has_obstacles); 0: block 0 of the dynamics launch zeroes them at its start
     int32_t sm_count;
     int32_t sparse_minv;             // M_inv has only the z_G pattern (diagonal + [0,4] [4,0] [1,3] [3,1]) filled in
     T *delta_d_out;

@@ -10,7 +10,7 @@ namespace dockauv {
 // One step of k's env range.  *n_launches receives how many kernels it enqueued (valid when it returns cudaSuccess).
 // marks (nullable): kMaxStepLaunches + 1 events; when given, the multi-launch layouts record one before their first
 // launch and one after each launch, *n_marks receives how many were recorded (0 for single-launch layouts)
-constexpr int kMaxStepLaunches = 6;
+constexpr int kMaxStepLaunches = 3;
 template <typename T>
 cudaError_t launch_step(const KParams<T> &k, int vehicle, int layout, cudaStream_t st, int *n_launches,
                         cudaEvent_t *marks = nullptr, int *n_marks = nullptr);
@@ -18,23 +18,16 @@ cudaError_t launch_step(const KParams<T> &k, int vehicle, int layout, cudaStream
 template <typename T>
 cudaError_t launch_reset(const KParams<T> &k, const uint8_t *mask_dev, cudaStream_t st);
 
-#ifndef DOCKAUV_FUSE_MAX_OBSF
-#define DOCKAUV_FUSE_MAX_OBSF 20    // pipeline layout: the cull + finish code runs inside the dynamics launch when an env has at most this many float4 obstacle records: 80 KB of shared memory per 256-thread CTA, two CTAs per SM stay resident
-#endif
-// whether the dynamics launch of the pipeline layout takes the cull + finish code in
-template <typename T>
-inline bool pipe_fuses_cull(const KParams<T> &k) {
-    return k.n_caps + k.n_sph > 0 && !k.cull_exact && k.n_obsf > 0 && k.n_obsf <= DOCKAUV_FUSE_MAX_OBSF;
-}
-
 // Work-list counters (KParams::view_count): one block of kCounterWords words per concurrently stepped env range; the
 // range that starts at env b uses block b / kCounterEnvs.  Words 0..kListCounters-1 are the live counters (view lists of
-// class 1, 2, 3, ended list); steps with the cull code fused into the dynamics launch keep their values at the end of
-// the most recent step in kCounterLast.. (dockauv_last_list_counts), and kCounterTicket is the ticket of the episode-end
-// launch, whose last CTA saves and zeroes the live counters.
+// class 1, 2, 3, ended list).  Steps with obstacles (pipe_has_obstacles) keep their values at the end of the most recent
+// step in kCounterLast.. (dockauv_last_list_counts), and kCounterTicket is the ticket of the episode-end launch, whose last
+// CTA saves and zeroes the live counters; obstacle-free steps have them zeroed by block 0 of the dynamics launch.
 constexpr int kCounterWords = 16, kCounterEnvs = 128;
 constexpr int kListCounters = 4, kCounterLast = 4, kCounterTicket = 8;
 inline int64_t counter_block(int64_t env_begin) { return kCounterWords * (env_begin / kCounterEnvs); }
+template <typename T>
+inline bool pipe_has_obstacles(const KParams<T> &k) { return k.n_caps + k.n_sph > 0; }
 
 // The library-owned buffers of the pipeline layout for n envs, as byte offsets into one allocation (every piece 256-byte
 // aligned): per-env records T[n][16], float obstacle records float4[n_obsf][n], obstacle rows T[n][n_obst][8], three view

@@ -4,16 +4,15 @@
 //      + cull        obs[0:16], done conditions 0..2, the reward terms that need no radar -- a 16-word record per env
 //      + finish      (post-step attitude sines / cosines, position relative to the goal, the reward terms already combined
 //                   in numpy's summation order, delta_d, condition bits) that stays in REGISTERS for the second half of the
-//                   thread (FINISH): the walk over the env's obstacles in FLOAT (float4 records relative to the goal,
-//                   written at reset, waiting in shared memory since the start of the thread; cull_pair_rec): body
-//                   collision (re-decided in T when within 2 mm of the threshold) and the range / field-of-view culls.
+//                   thread: the walk over the env's obstacles in FLOAT (float4 records relative to the goal, written at
+//                   reset, waiting in shared memory since the start of the thread; cull_pair_rec): body collision
+//                   (re-decided in T when within 2 mm of the threshold) and the range / field-of-view culls.
 //                   Envs with something in view (24 % on the C4 workload) are appended to a compact list and their record
 //                   goes to KParams::rec.  Done flag, condition bits and counters are final here for EVERY env (coalesced
 //                   stores); an env with nothing in view is finished completely -- all ray cells read max_dist, r_oa = 0:
 //                   reward, running return, statistics -- and goes on a second list if its episode ended.
-//                   (Obstacle-free scenarios: the same code with no obstacle to walk over finishes every env.  More float
-//                   records than fit in shared memory, or coordinates too large for them: the cull + finish code runs as a
-//                   launch of its own, cull_finish_kernel, on records read back from KParams::rec.)
+//                   (Obstacle-free scenarios: the same code with no obstacle to walk over finishes every env.  Coordinates
+//                   too large for float records: the same walk decides everything in T from the obstacle rows.)
 //   2. rays+finish  rays_thread_kernel: persistent grid.  The listed envs with one or two obstacles in view with LANES =
 //                   ENVS (tiles of 128), the others by one warp each (lanes = rays, next entry in flight while the current
 //                   one is cast; radar_env, dockauv_rays.cuh) on the first CTAs of the same launch; then the reward with its
@@ -37,9 +36,6 @@ namespace dockauv {
 #define DOCKAUV_MINB_A 2            // its min-CTAs hint: (256, 2) = 128 registers, 16 warps per SM
 #endif
 constexpr int kDynThreads = DOCKAUV_DYN_THREADS;
-#ifndef DOCKAUV_MINB_CULL
-#define DOCKAUV_MINB_CULL 4
-#endif
 #ifndef DOCKAUV_MINB_TPE
 #define DOCKAUV_MINB_TPE 4          // thread-per-env ray launch: (128, 4) = 128 registers
 #endif
@@ -151,19 +147,21 @@ __device__ __forceinline__ T step_reward(const KParams<T> &p, T A, T B, T r7, T 
 }
 
 // ------------------------------------------------------------------------------------------------------- 1. dynamics
-// CUR: the ocean current is evaluated (scenario with a current, injected current or noise); SPM: sparse M_inv / C / G;
-// FINISH: the cull + finish code (section 2) runs in this launch, on the record while it is still in registers (scenarios
-// without obstacles too: every ray reads max_dist and nothing can collide, so every env is finished here).
+// CUR: the ocean current is evaluated (scenario with a current, injected current or noise); SPM: sparse M_inv / C / G.
+// The cull + finish code (section 2) runs in this launch, on the record while it is still in registers (scenarios without
+// obstacles too: every ray reads max_dist and nothing can collide, so every env is finished here).
 
 // shared memory of one dynamics CTA: park[kParkWords][kDynThreads] words of T that are only needed after the integration
-// (position, goal; FINISH: running return, step counter), filled by cp.async into the thread's own slots -- no register
-// during the integration and no memory round trip after it
+// (position, goal, running return, step counter), filled by cp.async into the thread's own slots -- no register during
+// the integration and no memory round trip after it
 constexpr int kParkWords = 8;
 
-// one env of the dynamics launch: the env's record is left in w[kRecWords] and its post-step position in pos[3].
-//   stage(): the caller's own cp.async copies for this env (issued after the plain loads)
-template <typename T, int VEH, int NU, bool CUR, bool SPM, typename STAGE>
-__device__ __forceinline__ void dynamics_env(const KParams<T> &p, const int64_t i, T *dyn_park, T w[kRecWords], T pos[3], STAGE stage) {
+// one env of the dynamics launch: the env's record is left in w[kRecWords] and its post-step position in pos[3]; its
+// running return, step counter (park rows 6, 7) and float obstacle records (s_obs, [slot][kDynThreads]) are copied into
+// shared memory for the cull + finish code (the cp.async wait after the integration covers them)
+template <typename T, int VEH, int NU, bool CUR, bool SPM>
+__device__ __forceinline__ void dynamics_env(const KParams<T> &p, const int64_t i, T *dyn_park, const float4 *s_obs,
+                                             T w[kRecWords], T pos[3]) {
     const int64_t N = p.n_envs;
     // ---- what the integration starts from goes first: plain loads; the asynchronous copies of everything that is needed
     //      later queue up behind them (issued ahead of the loads, the 21 copies of a thread delayed its first use of a loaded
@@ -180,8 +178,11 @@ __device__ __forceinline__ void dynamics_env(const KParams<T> &p, const int64_t 
         for (int c = 0; c < 3; c++) cp_async_word<T>(sa + c * kPlane, p.state + (int64_t)c * N + i);
 #pragma unroll
         for (int c = 0; c < 3; c++) cp_async_word<T>(sa + (3 + c) * kPlane, p.goal + (int64_t)c * N + i);
+        cp_async_word<T>(sa + 6 * kPlane, p.ep_return + i);
+        cp_async_word<int32_t>(sa + 7 * kPlane, p.t_steps + i);
+        const unsigned so = (unsigned)__cvta_generic_to_shared(s_obs);
+        for (int sl = 0; sl < p.n_obsf; sl++) cp_async_16(so + (unsigned)(sl * kDynThreads * 16), p.obsf + (int64_t)sl * N + i);
     }
-    stage();
     T tr0[6];
     Mth<T>::sincos_(y[0], &tr0[0], &tr0[1]);
     Mth<T>::sincos_(y[1], &tr0[2], &tr0[3]);
@@ -236,25 +237,17 @@ __device__ __forceinline__ void dynamics_env(const KParams<T> &p, const int64_t 
 }
 
 // ------------------------------------------------------------------------------------------------------- 2. cull + finish
-// One env through the float culls and everything that can be finished without rays; called by EVERY thread of a CTA of
-// CTA threads (the list appends are warp-collective; `active` = the thread has an env).
-//   trig / prel      sin / cos of the post-step attitude, position relative to the goal (record words 0..8)
-//   fetch(slot)      float obstacle record `slot` of this env (KParams::obsf layout), from wherever the caller keeps it
-//   late()           CullLate: the record words 9..15, running return and step counter -- asked for AFTER the obstacle loop,
-//                    so that a caller that has them in memory does not hold them in registers through the loop
-//   pos_of(q)        post-step position (only for pairs within 2 mm of the collision threshold)
+// One env through the float culls and everything that can be finished without rays; called by EVERY thread of a dynamics
+// CTA (the list appends are warp-collective; `active` = the thread has an env).
+//   w        the env's record (dynamics_env)
+//   pos      post-step position (only for pairs within 2 mm of the collision threshold, and the exact culls)
+//   s_obs    the env's float obstacle records in shared memory, [slot][kDynThreads] (KParams::obsf layout)
+//   park     the thread's first park slot (running return in row 6, step counter in row 7), read after the obstacle loop
 // Returns whether the env is on a view list (its record must then be in KParams::rec for the ray launch, with REC_POS
 // and REC_EPR filled in).
 template <typename T>
-struct CullLate {
-    T A, B, r7, lp_d, delta_d, cond012, poison, ep_return;
-    int32_t t_steps;
-};
-
-template <typename T, int CTA, typename FETCH, typename LATE, typename POS>
 __device__ __forceinline__ bool cull_finish_env(const KParams<T> &p, const int64_t i, const int64_t i0, const bool active,
-                                                const T trig[6], const T prel_T[3], FETCH fetch, LATE late, POS pos_of) {
-    const int64_t N = p.n_envs;
+                                                const T w[kRecWords], const T pos[3], const float4 *s_obs, const T *park) {
     const int lane = threadIdx.x & 31;
     WarpStats bs;
     bool listed = false, ended = false;      // ended: episode over and nothing in view -> on the list of the episode-end launch
@@ -263,22 +256,23 @@ __device__ __forceinline__ bool cull_finish_env(const KParams<T> &p, const int64
     uint32_t cond = 0;
     if (active) {
         const int n_caps = p.n_caps, n_sph = p.n_sph, n_obst = n_caps + n_sph;
+        const T *trig = w + REC_TRIG;
         if (n_obst > 0 && !p.cull_exact) {
             // ---- float culls + collision pre-test (cull_pair_rec)
             float Rf[9], prel[3];
             rzyx<float>((float)trig[0], (float)trig[1], (float)trig[2], (float)trig[3], (float)trig[4], (float)trig[5], Rf);
 #pragma unroll
-            for (int c = 0; c < 3; c++) prel[c] = (float)prel_T[c];
+            for (int c = 0; c < 3; c++) prel[c] = (float)w[REC_PREL + c];
             // the next obstacle's record is requested before the current one is evaluated
-            float4 q0 = fetch(0), q1 = n_caps > 0 ? fetch(1) : make_float4(0.f, 0.f, 0.f, 0.f);
+            float4 q0 = s_obs[0], q1 = n_caps > 0 ? s_obs[kDynThreads] : make_float4(0.f, 0.f, 0.f, 0.f);
             int slot = n_caps > 0 ? 2 : 1;
 #pragma unroll 1
             for (int k = 0; k < n_obst; k++) {
                 const bool is_cap = k < n_caps;
                 const float4 c0 = q0, c1 = q1;
                 if (k + 1 < n_obst) {
-                    q0 = fetch(slot);
-                    if (k + 1 < n_caps) q1 = fetch(slot + 1);
+                    q0 = s_obs[slot * kDynThreads];
+                    if (k + 1 < n_caps) q1 = s_obs[(slot + 1) * kDynThreads];
                     slot += (k + 1 < n_caps) ? 2 : 1;
                 }
                 int hit3;
@@ -286,8 +280,7 @@ __device__ __forceinline__ bool cull_finish_env(const KParams<T> &p, const int64
                 cull_pair_rec<T>(p, prel, Rf, c0, c1, is_cap, hit3, view);
                 bool hit = hit3 == 1;
                 if (hit3 == 2) {      // within 2 mm of the collision threshold (or NaN): decided in T like the other layouts
-                    T pos[3], ob[kObstRowWords];
-                    pos_of(pos);
+                    T ob[kObstRowWords];
                     load_obstacle_row<T>(obstacle_row<T>(p, i, k), ob);
                     hit = obstacle_body_hit<T>(p, pos, ob, is_cap);
                 }
@@ -296,9 +289,8 @@ __device__ __forceinline__ bool cull_finish_env(const KParams<T> &p, const int64
             }
         } else if (n_obst > 0) {
             // ---- coordinates too large for float records: everything in T (obstacle_pair)
-            T Rm[9], pos[3];
+            T Rm[9];
             rzyx<T>(trig[0], trig[1], trig[2], trig[3], trig[4], trig[5], Rm);
-            pos_of(pos);
 #pragma unroll 1
             for (int k = 0; k < n_obst; k++) {
                 const bool is_cap = k < n_caps;
@@ -310,38 +302,38 @@ __device__ __forceinline__ bool cull_finish_env(const KParams<T> &p, const int64
                 info |= hit ? (1u << 16) : 0u;
             }
         }
-        const CullLate<T> L = late();
+        const T ep_return = park[6 * kDynThreads];
+        const int32_t t_steps = reinterpret_cast<const int32_t *>(park + 7 * kDynThreads)[0];
         // a non-finite pose goes through the warp-per-env ray path, which reproduces the reference's treatment of it
         // (radar_env; without obstacles every ray reads max_dist whatever the pose, docking3d.py:441)
-        poison_free = L.poison == T(0);
+        poison_free = w[REC_POISON] == T(0);
         listed = (info & 0xffffu) != 0u || (n_obst > 0 && !poison_free);
         // ---- everything that does not depend on the rays is final for EVERY env: done, condition bits, counters.
         //      Stores of all lanes of the warp -> full sectors (a listed env only lacks its obstacle-avoidance term: its
         //      reward word is provisional here and rewritten by the ray launch together with the running return)
-        const int32_t t_steps = L.t_steps;
-        cond = done_conditions<T>(p, (uint32_t)L.cond012, t_steps, (info >> 16) != 0u);
+        cond = done_conditions<T>(p, (uint32_t)w[REC_COND], t_steps, (info >> 16) != 0u);
         const bool done = cond != 0;
         const int32_t t_new = t_steps + 1;
         const T r_oa = p.sum_beta_oa / p.sum_beta_oa - T(1);      // docking3d.py:792 with every ray at max_dist: exactly 0
-        const T reward = step_reward<T>(p, L.A, L.B, L.r7, L.lp_d, r_oa, cond);
+        const T reward = step_reward<T>(p, w[REC_A], w[REC_B], w[REC_R7], w[REC_LPD], r_oa, cond);
         p.reward[i] = reward;
         p.done[i] = done ? 1 : 0;
         if (p.cond_bits) p.cond_bits[i] = (uint8_t)cond;
-        if (p.delta_d_out) p.delta_d_out[i] = L.delta_d;
+        if (p.delta_d_out) p.delta_d_out[i] = w[REC_DD];
         if (done && p.ep_len_out) p.ep_len_out[i] = t_new;
         if (listed) {
             p.t_steps[i] = t_new;        // the ray launch reads it back (and zeroes it if it re-initialises the env)
         } else {
             // ---- nothing in view: pooled cells all ones, r_oa = 0
             store_clear_cells<T>(p, i);
-            const T ep_ret = L.ep_return + reward;
+            const T ep_ret = ep_return + reward;
             if (done) {
                 if (p.ep_return_out) p.ep_return_out[i] = ep_ret;
                 bs.done = true;
                 bs.cond = cond;
                 bs.length = t_new;
                 bs.ep_return = (double)ep_ret;
-                bs.delta_d = (double)L.delta_d;
+                bs.delta_d = (double)w[REC_DD];
                 bs.nan = reward != reward;      // episodes that ended on a NaN reward
                 ended = true;
             }
@@ -376,135 +368,37 @@ __device__ __forceinline__ bool cull_finish_env(const KParams<T> &p, const int64
         else if (cls == 3) p.view_list[2 * p.n_envs + b3 + __popc(m3 & below)] = entry;
         if (ended) p.ended_list[b4 + __popc(m4 & below)] = (uint32_t)(i - p.env_begin);
     }
-    bs.flush_direct(p.stats, threadIdx.x == 0 ? (int)min((int64_t)CTA, p.env_end - i0) : 0);
+    bs.flush_direct(p.stats, threadIdx.x == 0 ? (int)min((int64_t)kDynThreads, p.env_end - i0) : 0);
     return listed;
 }
 
-// ---- the dynamics launch (with the cull + finish code in it when FINISH)
-// FINISH: the env's running return, step counter and float obstacle records travel global -> shared by cp.async at the
-// very start (records: [slot][thread], dynamic shared memory: 16 n_obsf bytes per thread) and wait there through the
-// integration; the record never leaves the registers unless the env ends up on a view list.  Against the separate cull
-// launch this saves the record's round trip through HBM (128 B written for every env, 128 B read back) and every memory
-// wait of the obstacle loop.
-template <typename T, int VEH, int NU, bool CUR, bool SPM, bool FINISH>
+// ---- the dynamics launch with the cull + finish code in it
+// The env's running return, step counter and float obstacle records travel global -> shared by cp.async at the very start
+// (records: [slot][thread], dynamic shared memory: 16 n_obsf bytes per thread) and wait there through the integration;
+// the record never leaves the registers unless the env ends up on a view list.  Against a cull launch of its own this
+// saves the record's round trip through HBM (128 B written for every env, 128 B read back) and every memory wait of the
+// obstacle loop.
+template <typename T, int VEH, int NU, bool CUR, bool SPM>
 __global__ void __launch_bounds__(kDynThreads, DOCKAUV_MINB_A) dynamics_kernel(const __grid_constant__ KParams<T> p) {
-    extern __shared__ __align__(16) unsigned char dyn_smem[];      // FINISH: float4 [n_obsf][kDynThreads]
+    extern __shared__ __align__(16) unsigned char dyn_smem[];      // float4 [n_obsf][kDynThreads]
     __shared__ __align__(8) T dyn_park[kParkWords * kDynThreads];
     const int64_t i0 = p.env_begin + (int64_t)blockIdx.x * kDynThreads;
     const int64_t i = i0 + threadIdx.x;
     const bool active = i < p.env_end;
     prefetch_dynamics_inputs<T, NU>(p, i, threadIdx.x & 31, true);
     T w[kRecWords], pos[3];
-    // a launch after this one appends to the lists: this launch empties them, unless the episode-end launch does.
-    // Without obstacles this launch appends to them itself: block 0 zeroes the counters long before any other block has
-    // finished its integration, which CUDA does not guarantee to be ordered (DESIGN.md section 8)
-    if (!(FINISH && p.counters_zeroed_at_end) && blockIdx.x == 0 && threadIdx.x < kListCounters) p.view_count[threadIdx.x] = 0u;
-    if (!FINISH) {
-        if (!active) return;
-        dynamics_env<T, VEH, NU, CUR, SPM>(p, i, dyn_park, w, pos, []() {});
-        RecIO<T>::store(p.rec + i * kRecWords, w);
-        return;
-    }
+    // steps with obstacles: the episode-end launch empties the lists.  Without obstacles this launch is the only one that
+    // appends to them: block 0 zeroes the counters long before any other block has finished its integration, which CUDA
+    // does not guarantee to be ordered (DESIGN.md section 8)
+    if (!p.counters_zeroed_at_end && blockIdx.x == 0 && threadIdx.x < kListCounters) p.view_count[threadIdx.x] = 0u;
     const float4 *s_obs = reinterpret_cast<const float4 *>(dyn_smem) + threadIdx.x;
-    if (active) {
-        dynamics_env<T, VEH, NU, CUR, SPM>(p, i, dyn_park, w, pos, [&]() {
-            const unsigned sp = (unsigned)__cvta_generic_to_shared(dyn_park + threadIdx.x);
-            constexpr unsigned kPlane = kDynThreads * (unsigned)sizeof(T);
-            cp_async_word<T>(sp + 6 * kPlane, p.ep_return + i);
-            cp_async_word<int32_t>(sp + 7 * kPlane, p.t_steps + i);
-            const unsigned sa = (unsigned)__cvta_generic_to_shared(s_obs);
-            for (int sl = 0; sl < p.n_obsf; sl++)
-                asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa + (unsigned)(sl * kDynThreads * 16)),
-                             "l"(p.obsf + (int64_t)sl * p.n_envs + i) : "memory");
-        });      // (the cp.async wait after the integration covers the records)
-    }
-    const bool listed = cull_finish_env<T, kDynThreads>(
-        p, i, i0, active, w + REC_TRIG, w + REC_PREL, [&](int sl) { return s_obs[sl * kDynThreads]; },
-        [&]() {
-            CullLate<T> L;
-            L.A = w[REC_A]; L.B = w[REC_B]; L.r7 = w[REC_R7]; L.lp_d = w[REC_LPD]; L.delta_d = w[REC_DD];
-            L.cond012 = w[REC_COND]; L.poison = w[REC_POISON];
-            L.ep_return = dyn_park[6 * kDynThreads + threadIdx.x];
-            L.t_steps = reinterpret_cast<const int32_t *>(dyn_park + 7 * kDynThreads + threadIdx.x)[0];
-            return L;
-        },
-        [&](T q[3]) { q[0] = pos[0]; q[1] = pos[1]; q[2] = pos[2]; });
+    if (active) dynamics_env<T, VEH, NU, CUR, SPM>(p, i, dyn_park, s_obs, w, pos);
+    const bool listed = cull_finish_env<T>(p, i, i0, active, w, pos, s_obs, dyn_park + threadIdx.x);
     if (listed) {      // the ray launch reads it
 #pragma unroll
         for (int c = 0; c < 3; c++) w[REC_POS + c] = pos[c];
         w[REC_EPR] = dyn_park[6 * kDynThreads + threadIdx.x];
         RecIO<T>::store(p.rec + i * kRecWords, w);
-    }
-}
-
-// ---- the cull + finish launch on its own (records from KParams::rec; used when the dynamics launch cannot take it in)
-constexpr int kCullThreads = 256;
-
-template <typename T>
-__global__ void __launch_bounds__(kCullThreads, DOCKAUV_MINB_CULL) cull_finish_kernel(const __grid_constant__ KParams<T> p) {
-    // the words needed only after the obstacle loop (reward terms, condition / poison words, running return, step counter)
-    // travel global -> shared by cp.async into the thread's own slots, [slot][thread]: no register, no wait up front.  As
-    // plain loads these values were spilled to the stack under the 64-register cap, the spill stores waited for the loads
-    // (13 % of this launch's stall samples) and the reloads after the loop for lines that had left L1 again (another 15 %)
-    __shared__ __align__(16) unsigned char cull_park[4 * kCullThreads * 16];
-    const int64_t N = p.n_envs;
-    const int64_t i0 = p.env_begin + (int64_t)blockIdx.x * kCullThreads;
-    const int64_t i = i0 + threadIdx.x;
-    const bool active = i < p.env_end;
-    const T *rec = p.rec + i * kRecWords;
-    T w[10];
-#pragma unroll
-    for (int c = 0; c < 10; c++) w[c] = T(0);
-    if (active) {
-        if (!p.cull_exact)
-            for (int sl = 0; sl < p.n_obsf; sl++) asm volatile("prefetch.global.L2 [%0];" ::"l"(p.obsf + (int64_t)sl * N + i));
-        RecIO<T>::template load<0, 5>(rec, w);       // trig, prel, A
-        const unsigned sa = (unsigned)__cvta_generic_to_shared(cull_park) + (unsigned)threadIdx.x * 16u;
-        constexpr unsigned kPlane = kCullThreads * 16u;
-        if (sizeof(T) == 8) {
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa), "l"(rec + 10) : "memory");              // B, r7
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa + kPlane), "l"(rec + 12) : "memory");     // lp_d, delta_d
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa + 2 * kPlane), "l"(rec + 14) : "memory"); // cond, poison
-            asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(sa + 3 * kPlane), "l"(p.ep_return + i) : "memory");
-        } else {
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa), "l"(rec + 8) : "memory");               // prel_z, A, B, r7
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa + kPlane), "l"(rec + 12) : "memory");     // lp_d, delta_d, cond, poison
-            asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(sa + 3 * kPlane), "l"(p.ep_return + i) : "memory");
-        }
-        asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(sa + 3 * kPlane + 8u), "l"(p.t_steps + i) : "memory");
-    }
-    const T A = w[REC_A];
-    const float4 *ob = p.obsf + i;
-    const bool listed = cull_finish_env<T, kCullThreads>(
-        p, i, i0, active, w + REC_TRIG, w + REC_PREL, [&](int sl) { return ob[(int64_t)sl * N]; },
-        [&]() {
-            CullLate<T> L;
-            cp_async_wait_all();      // this thread's own slots: no barrier
-            const unsigned char *sp = cull_park + threadIdx.x * 16;
-            constexpr int kPlane = kCullThreads * 16;
-            if (sizeof(T) == 8) {
-                const double2 a = *reinterpret_cast<const double2 *>(sp), b = *reinterpret_cast<const double2 *>(sp + kPlane);
-                const double2 c = *reinterpret_cast<const double2 *>(sp + 2 * kPlane);
-                L.B = (T)a.x; L.r7 = (T)a.y; L.lp_d = (T)b.x; L.delta_d = (T)b.y; L.cond012 = (T)c.x; L.poison = (T)c.y;
-                L.ep_return = (T)*reinterpret_cast<const double *>(sp + 3 * kPlane);
-            } else {
-                const float4 a = *reinterpret_cast<const float4 *>(sp), b = *reinterpret_cast<const float4 *>(sp + kPlane);
-                L.B = (T)a.z; L.r7 = (T)a.w; L.lp_d = (T)b.x; L.delta_d = (T)b.y; L.cond012 = (T)b.z; L.poison = (T)b.w;
-                L.ep_return = (T)*reinterpret_cast<const float *>(sp + 3 * kPlane);
-            }
-            L.t_steps = *reinterpret_cast<const int32_t *>(sp + 3 * kPlane + 8);
-            L.A = A;
-            return L;
-        },
-        [&](T q[3]) {
-#pragma unroll
-            for (int c = 0; c < 3; c++) q[c] = p.state[(int64_t)c * N + i];
-        });
-    if (listed) {      // the record in the ray launch's form (the running return is still in this thread's slot)
-        T *r = p.rec + i * kRecWords;
-#pragma unroll
-        for (int c = 0; c < 3; c++) r[REC_POS + c] = p.state[(int64_t)c * N + i];
-        r[REC_EPR] = *reinterpret_cast<const T *>(cull_park + 3 * kCullThreads * 16 + threadIdx.x * 16);
     }
 }
 
@@ -845,10 +739,10 @@ __global__ void __launch_bounds__(kResetCta) episode_end_kernel(const __grid_con
         }
         if (p.auto_reset) reset_envs_cta<T, BANK>(p, ie, valid);
     }
-    // ---- steps whose dynamics launch appends to the lists itself (cull code fused in) cannot have that launch empty
-    //      them: the last CTA to get here saves the list counters of this step and zeroes them for the next one (every CTA
-    //      has read the ended count and its list entries by now).  Other steps skip this: the ticket's round trip is on
-    //      the critical path of small batches (65,536-env SimpleDocking3d step: 24.3 against 22.6 us)
+    // ---- steps with obstacles: the last CTA to get here saves the list counters of this step and zeroes them for the
+    //      next one (every CTA has read the ended count and its list entries by now).  Obstacle-free steps skip this and
+    //      have block 0 of the dynamics launch zero them: the ticket's round trip is on the critical path of small
+    //      batches (65,536-env SimpleDocking3d step: 24.3 against 22.6 us)
     if (!p.counters_zeroed_at_end) return;
     // (no fence: what must precede the ticket are this CTA's READS of the counter and of its list entries, and their values
     // have been consumed by now; a __threadfence() here waited for every reset store of the CTA: 37 % of this launch's samples)
@@ -881,20 +775,20 @@ static cudaError_t launch_dependent(void (*kern)(KArgs...), unsigned blocks, uns
     return cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
 }
 
-template <typename T, int VEH, int NU, bool FINISH>
+template <typename T, int VEH, int NU>
 static cudaError_t launch_dynamics(const KParams<T> &k, unsigned blocks, cudaStream_t st) {
     const bool cur = k.has_current != 0, spm = k.sparse_minv != 0;
-    const int smem = FINISH ? k.n_obsf * kDynThreads * 16 : 0;
+    const int smem = k.n_obsf * kDynThreads * 16;
     auto go = [&](auto kern) {
         const cudaError_t e = allow_dyn_smem(kern, smem, kParkWords * kDynThreads * (int)sizeof(T));
         if (e != cudaSuccess) return e;
         kern<<<blocks, kDynThreads, smem, st>>>(k);
         return cudaGetLastError();
     };
-    if (cur && spm) return go(dynamics_kernel<T, VEH, NU, true, true, FINISH>);
-    if (cur) return go(dynamics_kernel<T, VEH, NU, true, false, FINISH>);
-    if (spm) return go(dynamics_kernel<T, VEH, NU, false, true, FINISH>);
-    return go(dynamics_kernel<T, VEH, NU, false, false, FINISH>);
+    if (cur && spm) return go(dynamics_kernel<T, VEH, NU, true, true>);
+    if (cur) return go(dynamics_kernel<T, VEH, NU, true, false>);
+    if (spm) return go(dynamics_kernel<T, VEH, NU, false, true>);
+    return go(dynamics_kernel<T, VEH, NU, false, false>);
 }
 
 // the ray launch over the n envs of kc's range, RPL rays per lane
@@ -941,22 +835,13 @@ static cudaError_t launch_step_pipe(const KParams<T> &k, cudaStream_t st, int *n
         n_mark++;
     };
     mark();
-    const bool has_obstacles = k.n_caps + k.n_sph > 0;
-    const unsigned dyn_blocks = (unsigned)((n + kDynThreads - 1) / kDynThreads);
-    // the cull + finish code runs inside the dynamics launch whenever the float records of a CTA fit in shared memory, and
-    // in scenarios without obstacles, where it finishes every env (no cull, no rays)
-    const bool fuse = pipe_fuses_cull(k);
-    kc.counters_zeroed_at_end = fuse ? 1 : 0;
-    cudaError_t e = fuse || !has_obstacles ? launch_dynamics<T, VEH, NU, true>(kc, dyn_blocks, st)
-                                           : launch_dynamics<T, VEH, NU, false>(kc, dyn_blocks, st);
+    const bool has_obstacles = pipe_has_obstacles(k);
+    kc.counters_zeroed_at_end = has_obstacles ? 1 : 0;
+    if (k.cull_exact) kc.n_obsf = 0;      // the exact culls read no float record: the dynamics launch stages none
+    cudaError_t e = launch_dynamics<T, VEH, NU>(kc, (unsigned)((n + kDynThreads - 1) / kDynThreads), st);
     if (e != cudaSuccess) return e;
     mark();
     if (has_obstacles) {
-        if (!fuse) {
-            cull_finish_kernel<T><<<(unsigned)((n + kCullThreads - 1) / kCullThreads), kCullThreads, 0, st>>>(kc);
-            if ((e = cudaGetLastError()) != cudaSuccess) return e;
-            mark();
-        }
         // rays per lane: 2 covers the stock 63-ray and the 64-ray radar; 8 covers everything up to DOCKAUV_MAX_RAYS
         e = k.n_rays <= 64 ? launch_rays<T, 2>(kc, n, st) : launch_rays<T, 8>(kc, n, st);
         if (e != cudaSuccess) return e;

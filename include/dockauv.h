@@ -416,8 +416,7 @@ DOCKAUV_API int dockauv_rollout_captures(DockauvHandle *h, int64_t *n_captures);
 DOCKAUV_API int dockauv_enable_timing(DockauvHandle *h, int enabled);
 DOCKAUV_API int dockauv_last_step_ms(DockauvHandle *h, float *ms);
 /* Per-launch CUDA-event times (ms) of the most recent timed dockauv_step of a multi-launch layout, in launch order
- * (DOCKAUV_LAYOUT_PIPELINE: dynamics + cull + finish [, cull + finish when it runs as a launch of its own], rays + finish
- * (only with obstacles), episode end); *n_launches = 0
+ * (DOCKAUV_LAYOUT_PIPELINE: dynamics + cull + finish, rays + finish (only with obstacles), episode end); *n_launches = 0
  * for the single-launch layouts. */
 DOCKAUV_API int dockauv_last_step_launch_ms(DockauvHandle *h, float *ms, int capacity, int *n_launches);
 

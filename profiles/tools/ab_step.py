@@ -1,5 +1,7 @@
 """One line per library variant: device-timed step of the C4 workload at 1M envs (40 steps after a burn-in), its
-per-launch CUDA-event times, the C2 workload at 65,536 envs and SimpleDocking3d at 1M envs.
+per-launch CUDA-event times, the C2 workload at 65,536 envs and SimpleDocking3d at 1M envs; then, with their per-launch
+times too, ObstaclesDocking3d at 1M envs with the most float obstacle records a handle can have (8 capsules + 8 spheres)
+and with coordinates too large for float records (max_dist_from_goal = 2500: exact culls).
 
     DOCKAUV_LIB=.../libdockauv_<tag>.so python profiles/tools/ab_step.py [tag]
 """
@@ -34,19 +36,24 @@ cfg["radar"] = dict(RADAR_64)
 N = 1 << 20
 gen = torch.Generator(device="cuda").manual_seed(1)
 pool = [torch.rand(N, 6, device="cuda", generator=gen) * 2 - 1 for _ in range(8)]
-env = envs.ObstaclesDocking3d(cfg, num_envs=N, seed=0, n_synthetic_spheres=3)
-env.reset()
-ms_c4 = timed(env, pool, 40, 140)
-ms_c4b = timed(env, pool, 40, 0)
-env.enable_timing(True)
-per = []
-for k in range(16):
-    env.step(pool[k % 8])
-    per.append(env.last_step_ms()[1])
-env.enable_timing(False)
-per = np.array(per).mean(axis=0)
-env.close()
-out = f"{tag:14s} C4 1M {min(ms_c4, ms_c4b):.4f} ms ({N / min(ms_c4, ms_c4b) * 1e3:.3e}/s) launches " + " ".join(f"{x * 1e3:.0f}" for x in per) + " us"
+
+
+def step_and_launches(env):
+    """best of two 40-step windows after a burn-in, and the mean per-launch times of 16 timed steps"""
+    env.reset()
+    ms = min(timed(env, pool, 40, 140), timed(env, pool, 40, 0))
+    env.enable_timing(True)
+    per = []
+    for k in range(16):
+        env.step(pool[k % 8])
+        per.append(env.last_step_ms()[1])
+    env.enable_timing(False)
+    env.close()
+    return ms, " ".join(f"{x * 1e3:.0f}" for x in np.array(per).mean(axis=0))
+
+
+ms_c4, per = step_and_launches(envs.ObstaclesDocking3d(cfg, num_envs=N, seed=0, n_synthetic_spheres=3))
+out = f"{tag:14s} C4 1M {ms_c4:.4f} ms ({N / ms_c4 * 1e3:.3e}/s) launches {per} us"
 if not quick:
     env = envs.SimpleDocking3d(dict(BASE_CONFIG), num_envs=N, seed=0)
     env.reset()
@@ -59,4 +66,9 @@ if not quick:
     ms_c2 = timed(env, pool2, 400, 100)
     env.close()
     out += f" | Simple 1M {ms_s:.4f} ms | C2 65536 {ms_c2 * 1e3:.1f} us ({n2 / ms_c2 * 1e3:.3e}/s)"
+    ms_88, per = step_and_launches(envs.ObstaclesDocking3d(cfg, num_envs=N, seed=0, n_synthetic_spheres=8, n_capsules=8))
+    out += f" | 8+8 1M {ms_88:.4f} ms launches {per} us"
+    cfg_far = dict(cfg, max_dist_from_goal=2500.0)
+    ms_far, per = step_and_launches(envs.ObstaclesDocking3d(cfg_far, num_envs=N, seed=0, n_synthetic_spheres=3))
+    out += f" | 2.5km 1M {ms_far:.4f} ms launches {per} us"
 print(out, flush=True)

@@ -3,7 +3,7 @@
 bench.py quotes for `roofline.traffic` / `executed_pipe_frac` (with the hash of the kernel sources it was captured from,
 so that a stale capture is never quoted).
 
-    ncu -i gpurun_out/prof_pipe_cur.ncu-rep --page raw --csv > profiles/r02/<tag>_pipeline_ncu_raw.csv
+    ncu -i profile_out/prof_pipe_cur.ncu-rep --page raw --csv > profiles/r02/<tag>_pipeline_ncu_raw.csv
     python profiles/tools/ncu_launch_json.py profiles/r02/<tag>_pipeline_ncu_raw.csv C4 524288 [f64]
 
 The third argument is the number of envs each captured launch covered (a 1M-env step runs as two halves).
@@ -19,8 +19,7 @@ sys.path.insert(0, ROOT)
 from bench import kernel_source_hash  # noqa: E402
 
 SCALE = {"byte": 1.0, "Kbyte": 1e3, "Mbyte": 1e6, "Gbyte": 1e9, "ns": 1e-3, "us": 1.0, "ms": 1e3, "s": 1e6}
-NAMES = (("dynamics_kernel", "dynamics"), ("cull_finish_kernel", "cull_finish"), ("rays_finish_kernel", "rays_finish"),
-         ("rays_thread_kernel", "rays_finish"),
+NAMES = (("dynamics_kernel", "dynamics_cull_finish"), ("rays_finish_kernel", "rays_finish"), ("rays_thread_kernel", "rays_finish"),
          ("episode_end_kernel", "episode_end"))
 
 
@@ -41,11 +40,6 @@ def main():
         short = next((s for k, s in NAMES if k in kname), None)
         if short is None:
             continue
-        if short == "dynamics":
-            # dynamics_kernel<T, VEH, NU, CUR, SPM, FINISH>: the last template argument says whether the cull + finish code runs in it
-            args = kname[kname.index("<") + 1:kname.index(">(")].replace("(bool)", "").split(",")
-            if args[-1].strip() in ("1", "true"):
-                short = "dynamics_cull_finish"
         per[short].append({
             "us": val(r, "gpu__time_duration.sum"),
             "dram_bytes": val(r, "dram__bytes_read.sum") + val(r, "dram__bytes_write.sum"),

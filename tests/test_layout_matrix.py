@@ -9,8 +9,8 @@ from tests.golden_utils import rel_err
 
 pytestmark = pytest.mark.gpu
 
-# (8 capsule + 8 sphere slots = 24 float records per env: more than the dynamics launch takes in, so the cull + finish code
-# runs as a launch of its own; every other obstacle case runs it fused)
+# (8 capsule + 8 sphere slots = 24 float records per env, the most a handle can have: 96 KB of them in shared memory per
+# CTA of the dynamics launch)
 CASES = [("ObstaclesDocking3d", dict(n_synthetic_spheres=3)), ("ObstaclesCurrentDocking3d", dict(n_synthetic_spheres=8)),
          ("ObstaclesDocking3d", dict(n_synthetic_spheres=8, n_capsules=8)),
          ("ObstaclesNoCapDocking3d", {}), ("CapsuleCurrentDocking3d", {}), ("SimpleCurrentDocking3d", {}),
@@ -33,9 +33,13 @@ def test_all_layouts_agree_on_odd_batch(name, kw):
                                    generator=torch.Generator(device=e.device).manual_seed(3))
     gen = torch.Generator(device="cuda").manual_seed(0)
     n_done = 0
+    # a pipeline step: dynamics + cull + finish, rays + finish (with obstacles), episode end
+    step_launches = 3 if es[2].n_capsules + es[2].n_spheres > 0 else 2
     for t in range(24):
         a = torch.rand(N, es[0].n_actions, device="cuda", generator=gen) * 2 - 1
+        n0 = es[2].launch_count()
         outs = [e.step(a) for e in es]
+        assert es[2].launch_count() - n0 == step_launches, (name, t)
         o0, r0, d0, i0 = outs[0]
         n_done += int(d0.sum())
         for (o, r, d, info), l in zip(outs[1:], layouts[1:]):
@@ -69,7 +73,7 @@ def test_all_layouts_agree_on_odd_batch(name, kw):
 
 def test_exact_cull_matches_float_cull():
     """Handles whose coordinates are too large for float obstacle records (max_dist_from_goal + max_dist > 2 km) cull in
-    double in a launch of their own: same flags / observations / rewards as the thread-per-env kernel."""
+    double, in the same three launches per step: same flags / observations / rewards as the thread-per-env kernel."""
     import torch
     from gym_dockauv_b200 import envs
     from gym_dockauv_b200.config import BASE_CONFIG, RADAR_64
@@ -83,7 +87,9 @@ def test_exact_cull_matches_float_cull():
     gen = torch.Generator(device="cuda").manual_seed(4)
     for t in range(40):
         a = torch.rand(N, 6, device="cuda", generator=gen) * 2 - 1
+        n0 = es[1].launch_count()
         (o0, r0, d0, i0), (o1, r1, d1, i1) = [e.step(a) for e in es]
+        assert es[1].launch_count() - n0 == 3, t
         assert torch.equal(d0, d1) and torch.equal(i0["cond_bits"], i1["cond_bits"]) and torch.equal(o0, o1), t
         assert rel_err(r1.cpu().numpy(), r0.cpu().numpy()) < 1e-12, t
     assert rel_err(es[1].state.cpu().numpy(), es[0].state.cpu().numpy()) < 1e-12
@@ -94,9 +100,9 @@ def test_exact_cull_matches_float_cull():
 @pytest.mark.parametrize("kw", [dict(n_synthetic_spheres=3), dict(n_synthetic_spheres=8, n_capsules=8)])
 def test_list_counts_match_the_step_outputs(kw):
     """dockauv_last_list_counts after a step: the ended count is the number of done flags, the listed count the number of
-    envs with a pooled ray cell below 1 or more (listed = something in view, a superset of real hits) -- with the cull code
-    inside the dynamics launch (counters saved and zeroed by the episode-end launch) and as a launch of its own.  After a
-    rollout the counts are those of its last step: without a graph, at the capture and at a replay."""
+    envs with a pooled ray cell below 1 or more (listed = something in view, a superset of real hits; counters saved and
+    zeroed by the episode-end launch), with few and with the most float records per env.  After a rollout the counts are
+    those of its last step: without a graph, at the capture and at a replay."""
     import torch
     from gym_dockauv_b200 import envs
     from gym_dockauv_b200.config import BASE_CONFIG, RADAR_64

@@ -14,7 +14,7 @@ a field-of-view plane, the range limit or the collision threshold, so every case
   D  collision band: centre / axis distance = radius + safety_radius + delta (sphere, capsule side, end cap, foot point
      at bot / top, vehicle inside an obstacle)
   E  work lists: 8 capsules + 8 spheres with exactly k in view (k = 0..16), every slot alone, two-obstacle type mixes
-  F  record-count boundary: (capsules, spheres) = (8, 4) fused cull, (8, 5) cull launch, (0, 1), (1, 0)
+  F  float record counts: (capsules, spheres) = (8, 4), (8, 5), (0, 1), (1, 0)
   G  1985 m from the goal: max_dist_from_goal + max_dist = 2000 (float records) and 2000.5 (exact culls)
   H  non-finite pose (NaN / inf in position or velocity) with obstacles in view
 
