@@ -396,6 +396,8 @@ extern "C" int dockauv_create(const DockauvParams *p, int64_t n_envs, int device
         h->pipe = pipe_buffers(n_envs, h->esz, p->n_capsules, p->n_spheres);
         cudaError_t e2 = cudaMalloc(&h->pipe_buf, h->pipe.bytes);
         if (e2 == cudaSuccess) e2 = cudaMemset(h->pipe_buf, 0, h->pipe.bytes);
+        // list counters start all ones (any start works while the words of a block are equal): the first step wraps them
+        if (e2 == cudaSuccess) e2 = cudaMemset((char *)h->pipe_buf + h->pipe.counters, 0xff, 4 * h->pipe.n_counters);
         if (e2 != cudaSuccess) {
             dockauv_destroy(h);
             return fail(DOCKAUV_ECUDA, "device allocation of the pipeline buffers failed: %s", cudaGetErrorString(e2));
@@ -1152,6 +1154,7 @@ extern "C" int dockauv_set_taps(DockauvHandle *h, const int64_t *env_ids_host, i
     CUDA_TRY(cudaMalloc(&tp.mem, off));
     CUDA_TRY(cudaMemset(tp.mem, 0, off));
     char *m = (char *)tp.mem;
+    if (pipe) CUDA_TRY(cudaMemset(m + o_pipe + tp.pipe.counters, 0xff, 4 * tp.pipe.n_counters));      // as dockauv_create
     auto place = [&](DockauvBuffers &b, const Shadow &o) {
         b.state = m + o.state; b.u_prev = m + o.u; b.goal = m + o.goal; b.heading_goal = m + o.hg; b.current = m + o.cur;
         b.capsules = m + o.caps; b.spheres = m + o.sph; b.ep_return = m + o.epr;
@@ -1544,12 +1547,11 @@ extern "C" int dockauv_last_list_counts(DockauvHandle *h, int64_t *n_listed, int
         CUDA_TRY(cudaMemcpyAsync(host.data(), k.view_count, n_cnt * sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaStreamSynchronize(st));
         for (int64_t b : h->last_begins) {
-            // with obstacles the live counters are zero again at the end of the step, and the copies hold its values
-            const size_t w = (size_t)counter_block(b) + (pipe_has_obstacles(k) ? kCounterLast : 0);
-            if (w + kListCounters <= n_cnt) {
-                *n_listed += (int64_t)host[w] + host[w + 1] + host[w + 2];
-                *n_ended += host[w + 3];
-            }
+            const size_t w = (size_t)counter_block(b);
+            if (w + kCounterWords > n_cnt) continue;
+            auto length = [&](int c) { return (int64_t)(host[w + c] - host[w + kCounterStart + c]); };      // mod 2^32
+            *n_listed += length(0) + length(1) + length(2);
+            *n_ended += length(3);
         }
         return DOCKAUV_OK;
     });

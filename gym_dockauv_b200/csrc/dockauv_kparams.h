@@ -73,9 +73,10 @@ struct KParams {
     //   obsd     T[n_envs][n_caps + n_sph][8]: env-major bit copy of the obstacles as stored, one 8-word row each
     //            (capsule: bot, top, radius, 0; sphere: centre, radius, 0, 0, 0), written wherever obsf is; the pipeline
     //            layout reads its obstacles in T from here (a row is one 64-byte piece in f64 instead of 7 planes)
-    //   view_list / ended_list / view_count: work lists, two counters per concurrently stepped range: envs with
-    //            something in view (local env index | in-view mask << 32 | condition bits << 48) for the ray launch, envs
-    //            whose episode ended (local env index) for the episode-end launch
+    //   view_list / ended_list / view_count: work lists, one counter block per concurrently stepped range (running
+    //            counts and their values at the start and end of the step, dockauv_launch.h): envs with something in
+    //            view (local env index | in-view mask << 32 | condition bits << 48) for the ray launch, envs whose
+    //            episode ended (local env index) for the episode-end launch
     T *rec;
     float4 *obsf;
     T *obsd;
@@ -84,7 +85,6 @@ struct KParams {
     unsigned long long *view_list;
     uint32_t *ended_list;
     unsigned int *view_count;
-    int32_t counters_zeroed_at_end;  // 1: the last CTA of the episode-end launch saves and zeroes the list counters (steps with obstacles, pipe_has_obstacles); 0: block 0 of the dynamics launch zeroes them at its start
     int32_t sm_count;
     int32_t sparse_minv;             // M_inv has only the z_G pattern (diagonal + [0,4] [4,0] [1,3] [3,1]) filled in
     T *delta_d_out;

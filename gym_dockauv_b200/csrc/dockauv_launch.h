@@ -19,12 +19,17 @@ template <typename T>
 cudaError_t launch_reset(const KParams<T> &k, const uint8_t *mask_dev, cudaStream_t st);
 
 // Work-list counters (KParams::view_count): one block of kCounterWords words per concurrently stepped env range; the
-// range that starts at env b uses block b / kCounterEnvs.  Words 0..kListCounters-1 are the live counters (view lists of
-// class 1, 2, 3, ended list).  Steps with obstacles (pipe_has_obstacles) keep their values at the end of the most recent
-// step in kCounterLast.. (dockauv_last_list_counts), and kCounterTicket is the ticket of the episode-end launch, whose last
-// CTA saves and zeroes the live counters; obstacle-free steps have them zeroed by block 0 of the dynamics launch.
+// range that starts at env b uses block b / kCounterEnvs.  Per list c (view lists of class 1, 2, 3, ended list):
+//   word c                       count: running total of the appends (atomicAdd), never reset
+//   word kCounterStart + c       its value when the current / most recent step began (block 0 of the dynamics launch
+//                                copies it from the word below at the start of every step)
+//   word kCounterNextStart + c   its value when the most recent step ended (block 0 of the episode-end launch, after the
+//                                wait for the launches before it)
+// A list's length is count - start, an append's slot its ticket - next start, both in modular uint32 arithmetic (the
+// counters wrap; the buffers start all ones).  Every word is written in one launch and read by other CTAs only in later
+// ones, so no CTA depends on another of its own launch (DESIGN.md section 3).
 constexpr int kCounterWords = 16, kCounterEnvs = 128;
-constexpr int kListCounters = 4, kCounterLast = 4, kCounterTicket = 8;
+constexpr int kListCounters = 4, kCounterStart = 4, kCounterNextStart = 8;
 inline int64_t counter_block(int64_t env_begin) { return kCounterWords * (env_begin / kCounterEnvs); }
 template <typename T>
 inline bool pipe_has_obstacles(const KParams<T> &k) { return k.n_caps + k.n_sph > 0; }

@@ -354,12 +354,15 @@ __device__ __forceinline__ bool cull_finish_env(const KParams<T> &p, const int64
                                          ((unsigned long long)cond << 48);
         // the four appends of a warp (three view classes, ended list) reserve their slots with ONE atomic instruction: lane c
         // adds the warp's count to counter c, so the four round trips overlap (as four dependent atomics they were 15 % of
-        // this launch's stall samples)
+        // this launch's stall samples); the list's start, loaded beside the atomic, turns the ticket into a slot
         const unsigned m1 = __ballot_sync(0xffffffffu, cls == 1), m2 = __ballot_sync(0xffffffffu, cls == 2);
         const unsigned m3 = __ballot_sync(0xffffffffu, cls == 3), m4 = __ballot_sync(0xffffffffu, ended);
         const unsigned mine = lane == 0 ? m1 : (lane == 1 ? m2 : (lane == 2 ? m3 : (lane == 3 ? m4 : 0u)));
         unsigned base = 0;
-        if (mine) base = atomicAdd(&p.view_count[lane], (unsigned)__popc(mine));
+        if (mine) {
+            const unsigned first = p.view_count[kCounterNextStart + lane];
+            base = atomicAdd(&p.view_count[lane], (unsigned)__popc(mine)) - first;
+        }
         const unsigned b1 = __shfl_sync(0xffffffffu, base, 0), b2 = __shfl_sync(0xffffffffu, base, 1);
         const unsigned b3 = __shfl_sync(0xffffffffu, base, 2), b4 = __shfl_sync(0xffffffffu, base, 3);
         const unsigned below = (1u << lane) - 1u;
@@ -387,10 +390,9 @@ __global__ void __launch_bounds__(kDynThreads, DOCKAUV_MINB_A) dynamics_kernel(c
     const bool active = i < p.env_end;
     prefetch_dynamics_inputs<T, NU>(p, i, threadIdx.x & 31, true);
     T w[kRecWords], pos[3];
-    // steps with obstacles: the episode-end launch empties the lists.  Without obstacles this launch is the only one that
-    // appends to them: block 0 zeroes the counters long before any other block has finished its integration, which CUDA
-    // does not guarantee to be ordered (DESIGN.md section 8)
-    if (!p.counters_zeroed_at_end && blockIdx.x == 0 && threadIdx.x < kListCounters) p.view_count[threadIdx.x] = 0u;
+    // the lists of this step start where the previous step's ended (nobody reads the start words in this launch)
+    if (blockIdx.x == 0 && threadIdx.x < kListCounters)
+        p.view_count[kCounterStart + threadIdx.x] = p.view_count[kCounterNextStart + threadIdx.x];
     const float4 *s_obs = reinterpret_cast<const float4 *>(dyn_smem) + threadIdx.x;
     if (active) dynamics_env<T, VEH, NU, CUR, SPM>(p, i, dyn_park, s_obs, w, pos);
     const bool listed = cull_finish_env<T>(p, i, i0, active, w, pos, s_obs, dyn_park + threadIdx.x);
@@ -403,6 +405,14 @@ __global__ void __launch_bounds__(kDynThreads, DOCKAUV_MINB_A) dynamics_kernel(c
 }
 
 // ------------------------------------------------------------------------------------------------------- 3. rays + finish
+// one append to the ended list by the ray launch (~1 % of the listed envs): the list's start is loaded beside the atomic,
+// so the two round trips overlap (loaded once per thread, it stayed live through the ray loops: up to 3 more registers)
+template <typename T>
+__device__ __forceinline__ unsigned ended_slot(const KParams<T> &p) {
+    const unsigned first = p.view_count[kCounterNextStart + 3];
+    return atomicAdd(&p.view_count[3], 1u) - first;
+}
+
 // Shared memory of one warp of the ray launch (T words):
 //   stage[2][kStageWords]   the data of two list entries (double buffer, filled by cp.async one entry ahead):
 //                           0..15 the env's record (ray launch form), 16 + 8 k .. obstacle row k, k < 16
@@ -457,7 +467,7 @@ __device__ __forceinline__ void rays_warp_loop(const KParams<T> &p, unsigned cha
     T *s_warp = reinterpret_cast<T *>(smem_raw) + warp * L.warp_words;
     T *s_pre = s_warp + L.pre_off;
     T *s_ray = s_warp + L.ray_off;
-    const unsigned count = p.view_count[2];
+    const unsigned count = p.view_count[2] - p.view_count[kCounterStart + 2];
     const unsigned long long *list = p.view_list + 2 * p.n_envs;
     unsigned idx = w_global;
     if (idx >= count) return;
@@ -528,7 +538,7 @@ __device__ __forceinline__ void rays_warp_loop(const KParams<T> &p, unsigned cha
             else if (lane == DOCKAUV_STAT_SUM_FINAL_DELTA_D) mine = (double)s_ent[REC_DD];
             else if (lane == DOCKAUV_STAT_NAN_ENVS) mine = (reward != reward) ? 1.0 : 0.0;
             stat_acc += mine;
-            if (lane == 0) p.ended_list[atomicAdd(&p.view_count[3], 1u)] = (uint32_t)cur;
+            if (lane == 0) p.ended_list[ended_slot(p)] = (uint32_t)cur;
         }
         __syncwarp();
         cur = nxt;
@@ -659,7 +669,7 @@ __device__ __forceinline__ void rays_thread_tile(const KParams<T> &p, const T *s
             bs.delta_d = (double)wf[5];
             bs.nan = reward != reward;
             bs.flush_direct(p.stats, 0);
-            p.ended_list[atomicAdd(&p.view_count[3], 1u)] = (uint32_t)entry;
+            p.ended_list[ended_slot(p)] = (uint32_t)entry;
         }
     }
 }
@@ -678,7 +688,7 @@ __global__ void __launch_bounds__(kTpeThreads, DOCKAUV_MINB_TPE) rays_thread_ker
         return;
     }
     const unsigned bid = blockIdx.x - warp_ctas, n_ctas = gridDim.x - warp_ctas;
-    const unsigned c1 = p.view_count[0], c2 = p.view_count[1];
+    const unsigned c1 = p.view_count[0] - p.view_count[kCounterStart], c2 = p.view_count[1] - p.view_count[kCounterStart + 1];
     const unsigned t2 = (c2 + kTpeThreads - 1) / kTpeThreads, t1 = (c1 + kTpeThreads - 1) / kTpeThreads;
     if (bid >= t1 + t2) return;
     const int n_rr = p.n_rr, n_r = p.n_rays;
@@ -711,7 +721,7 @@ __global__ void __launch_bounds__(kTpeThreads, DOCKAUV_MINB_TPE) rays_thread_ker
 template <typename T, bool BANK>
 __global__ void __launch_bounds__(kResetCta) episode_end_kernel(const __grid_constant__ KParams<T> p) {
     grid_dependency_wait();
-    const unsigned n_ended = p.view_count[3];
+    const unsigned n_ended = p.view_count[3] - p.view_count[kCounterStart + 3];
     const int n_obs = p.n_obs;
     const int lane = threadIdx.x & 31, role = threadIdx.x >> 5;
     // every thread of a CTA runs the same number of trips (reset_envs_cta has a barrier)
@@ -739,24 +749,10 @@ __global__ void __launch_bounds__(kResetCta) episode_end_kernel(const __grid_con
         }
         if (p.auto_reset) reset_envs_cta<T, BANK>(p, ie, valid);
     }
-    // ---- steps with obstacles: the last CTA to get here saves the list counters of this step and zeroes them for the
-    //      next one (every CTA has read the ended count and its list entries by now).  Obstacle-free steps skip this and
-    //      have block 0 of the dynamics launch zero them: the ticket's round trip is on the critical path of small
-    //      batches (65,536-env SimpleDocking3d step: 24.3 against 22.6 us)
-    if (!p.counters_zeroed_at_end) return;
-    // (no fence: what must precede the ticket are this CTA's READS of the counter and of its list entries, and their values
-    // have been consumed by now; a __threadfence() here waited for every reset store of the CTA: 37 % of this launch's samples)
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        if (atomicAdd(&p.view_count[kCounterTicket], 1u) == gridDim.x - 1) {
-#pragma unroll
-            for (int c = 0; c < kListCounters; c++) {
-                p.view_count[kCounterLast + c] = p.view_count[c];
-                p.view_count[c] = 0u;
-            }
-            p.view_count[kCounterTicket] = 0u;
-        }
-    }
+    // every append of this step has completed (the wait above): the next step's lists start here (no CTA of this launch
+    // reads these words)
+    if (blockIdx.x == 0 && threadIdx.x < kListCounters)
+        p.view_count[kCounterNextStart + threadIdx.x] = p.view_count[threadIdx.x];
 }
 
 // ------------------------------------------------------------------------------------------------------- launcher
@@ -835,13 +831,11 @@ static cudaError_t launch_step_pipe(const KParams<T> &k, cudaStream_t st, int *n
         n_mark++;
     };
     mark();
-    const bool has_obstacles = pipe_has_obstacles(k);
-    kc.counters_zeroed_at_end = has_obstacles ? 1 : 0;
     if (k.cull_exact) kc.n_obsf = 0;      // the exact culls read no float record: the dynamics launch stages none
     cudaError_t e = launch_dynamics<T, VEH, NU>(kc, (unsigned)((n + kDynThreads - 1) / kDynThreads), st);
     if (e != cudaSuccess) return e;
     mark();
-    if (has_obstacles) {
+    if (pipe_has_obstacles(k)) {
         // rays per lane: 2 covers the stock 63-ray and the 64-ray radar; 8 covers everything up to DOCKAUV_MAX_RAYS
         e = k.n_rays <= 64 ? launch_rays<T, 2>(kc, n, st) : launch_rays<T, 8>(kc, n, st);
         if (e != cudaSuccess) return e;

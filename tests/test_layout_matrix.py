@@ -97,37 +97,61 @@ def test_exact_cull_matches_float_cull():
         e.close()
 
 
-@pytest.mark.parametrize("kw", [dict(n_synthetic_spheres=3), dict(n_synthetic_spheres=8, n_capsules=8)])
+@pytest.mark.parametrize("kw", [dict(n_synthetic_spheres=3), dict(n_synthetic_spheres=8, n_capsules=8),
+                                dict(scenario="SimpleDocking3d")])
 def test_list_counts_match_the_step_outputs(kw):
     """dockauv_last_list_counts after a step: the ended count is the number of done flags, the listed count the number of
-    envs with a pooled ray cell below 1 or more (listed = something in view, a superset of real hits; counters saved and
-    zeroed by the episode-end launch), with few and with the most float records per env.  After a rollout the counts are
-    those of its last step: without a graph, at the capture and at a replay."""
+    envs with a pooled ray cell below 1 or more (listed = something in view, a superset of real hits; none without
+    obstacles), with few and with the most float records per env and without obstacles.  A count is the difference of a
+    running counter and its value when the step began; the counters start all ones, so every run crosses the 2^32 wrap.
+    After a rollout the counts are those of its last step: without a graph, at the capture and at a replay.
+    2^18 envs are stepped in two parts, except in steps with timing enabled (the whole batch as one range, on the first
+    part's counter block): those alternate with the others, and every step's outputs equal a never-timed twin's."""
     import torch
     from gym_dockauv_b200 import envs
     from gym_dockauv_b200.config import BASE_CONFIG, RADAR_64
     cfg = dict(BASE_CONFIG)
     cfg["radar"] = dict(RADAR_64)
+    kw = dict(kw)
+    make = envs.SCENARIOS[kw.pop("scenario", "ObstaclesDocking3d")]
     N = 40000                      # one launch group; also stepped in two parts below
     T = 4
 
     def check(n, obs, done, where):
         n_listed, n_ended = env.last_list_counts()
         assert n_ended == int(done.sum()), where
+        if env.n_capsules + env.n_spheres == 0:
+            assert n_listed == 0, (where, n_listed)
         # observation rows of finished envs are zeroed; among the others a cell below 1 needs an obstacle in view
         hit = int(((obs[:, 16:] < 1.0).any(1) & ~done.bool()).sum())
         assert hit <= n_listed <= n, (where, hit, n_listed)
 
+    def bits(x):
+        return x.view(torch.uint8)
+
     for n in (N, 1 << 18):
-        env = envs.ObstaclesDocking3d(cfg, num_envs=n, seed=2, **kw)
-        env.reset()
-        env.t_steps += 990          # episodes end inside the run
+        mixed = n == 1 << 18
+        env = make(cfg, num_envs=n, seed=2, **kw)
+        twin = make(cfg, num_envs=n, seed=2, **kw) if mixed else None
+        for e in (env, twin) if mixed else (env,):
+            e.reset()
+            e.t_steps += 990        # episodes end inside the run
         gen = torch.Generator(device="cuda").manual_seed(1)
         for t in range(14):
-            obs, _, done, info = env.step(torch.rand(n, 6, device="cuda", generator=gen) * 2 - 1)
+            a = torch.rand(n, env.n_actions, device="cuda", generator=gen) * 2 - 1
+            if mixed:
+                env.enable_timing(t % 2 == 1)
+            obs, rew, done, info = env.step(a)
             check(n, obs, done, (n, t))
+            if mixed:
+                obs2, rew2, done2, info2 = twin.step(a)
+                assert torch.equal(bits(obs), bits(obs2)) and torch.equal(done, done2), (n, t)
+                assert torch.equal(info["cond_bits"], info2["cond_bits"]) and torch.equal(bits(rew), bits(rew2)), (n, t)
         assert env.get_stats()["episodes"] > 0
-        acts = torch.empty(T, n, 6, device="cuda")
+        if mixed:
+            env.enable_timing(False)
+            twin.close()
+        acts = torch.empty(T, n, env.n_actions, device="cuda")
         obs = torch.zeros(T, n, env.n_observations, device="cuda")
         rew = torch.zeros(T, n, dtype=env.dtype, device="cuda")
         done = torch.zeros(T, n, dtype=torch.uint8, device="cuda")
