@@ -513,10 +513,55 @@ __device__ __forceinline__ void capsule_pre(const T pos[3], const T bot[3], cons
     q.r = r;
 }
 
+// sphere centre to vehicle: oc = pos - c, d2 = |oc|^2
+template <typename T>
+__device__ __forceinline__ void sphere_offset(const T pos[3], const T c[3], T oc[3], T &d2) {
+    d2 = T(0);
+#pragma unroll
+    for (int k = 0; k < 3; k++) {
+        oc[k] = pos[k] - c[k];
+        d2 += oc[k] * oc[k];
+    }
+}
+
+// The record the ray tests read -- capsule: ba[3] oa[3] baba baoa c c2a c2b, sphere: oc[3] c
+template <typename T>
+__device__ __forceinline__ void capsule_ray_record(const CapPre<T> &q, T *w) {
+    w[0] = q.ba[0]; w[1] = q.ba[1]; w[2] = q.ba[2];
+    w[3] = q.oa[0]; w[4] = q.oa[1]; w[5] = q.oa[2];
+    w[6] = q.baba; w[7] = q.baoa; w[8] = q.c; w[9] = q.c2a; w[10] = q.c2b;
+}
+
+template <typename T>
+__device__ __forceinline__ void sphere_ray_record(const T oc[3], T d2, T rad, T *w) {
+    w[0] = oc[0]; w[1] = oc[1]; w[2] = oc[2]; w[3] = d2 - rad * rad;
+}
+
+// a length from its square: 0 stays 0, NaN stays NaN
+template <typename T>
+__device__ __forceinline__ T length_from_sq(T d2) {
+    return d2 > T(0) ? Mth<T>::sqrt_pos(d2) : d2;
+}
+
+// Distance from the vehicle to the capsule's axis segment: dist_line_point (shape.py:393-417) with one reciprocal instead
+// of three divisions and hypot.  inv_n (out): 1 / |top - bot|
+template <typename T>
+__device__ __forceinline__ T capsule_axis_dist(const CapPre<T> &q, T &inv_n) {
+    inv_n = Mth<T>::rsqrt_pos(q.baba);
+    const T sp = -q.baoa * inv_n;                                                         // (bot - pos) . d
+    const T tp = (q.oc2[0] * q.ba[0] + q.oc2[1] * q.ba[1] + q.oc2[2] * q.ba[2]) * inv_n;  // (pos - top) . d
+    T hh = sp;
+    if (tp > hh || tp != tp) hh = tp;
+    if (T(0) > hh) hh = T(0);
+    T cr[3];
+    cross3(q.oa, q.ba, cr);
+    const T perp2 = (cr[0] * cr[0] + cr[1] * cr[1] + cr[2] * cr[2]) * (inv_n * inv_n);
+    return length_from_sq(hh * hh + perp2);
+}
+
 // Ray-independent work for one (env, obstacle) pair, shared by every radar layout:
-//   * the record the ray tests read -- capsule: ba[3] oa[3] baba baoa c c2a c2b, sphere: oc[3] c (written if REC);
-//   * the body-collision test (shape.py:182-210 with the safety radius of auvsim.py:43): dist_line_point
-//     (shape.py:393-417) with one reciprocal instead of three divisions and hypot;
+//   * the ray-test record (written if REC);
+//   * the body-collision test (shape.py:182-210 with the safety radius of auvsim.py:43);
 //   * two exact radar culls.  A culled obstacle can only yield "no positive distance" or a distance beyond max_dist,
 //     both of which end as max_dist (sensor.py:117):
 //       - range: nearest surface point farther than max_dist;
@@ -538,22 +583,9 @@ __device__ __forceinline__ void obstacle_pair(const KParams<T> &p, const T pos[3
         rad = ob[6];
         CapPre<T> q;
         capsule_pre<T>(pos, bot, top, rad, q);
-        if (REC) {
-            w[0] = q.ba[0]; w[1] = q.ba[1]; w[2] = q.ba[2];
-            w[3] = q.oa[0]; w[4] = q.oa[1]; w[5] = q.oa[2];
-            w[6] = q.baba; w[7] = q.baoa; w[8] = q.c; w[9] = q.c2a; w[10] = q.c2b;
-        }
-        const T inv_n = Mth<T>::rsqrt_pos(q.baba);
-        const T sp = -q.baoa * inv_n;                                                         // (bot - pos) . d
-        const T tp = (q.oc2[0] * q.ba[0] + q.oc2[1] * q.ba[1] + q.oc2[2] * q.ba[2]) * inv_n;  // (pos - top) . d
-        T hh = sp;
-        if (tp > hh || tp != tp) hh = tp;
-        if (T(0) > hh) hh = T(0);
-        T cr[3];
-        cross3(q.oa, q.ba, cr);
-        const T perp2 = (cr[0] * cr[0] + cr[1] * cr[1] + cr[2] * cr[2]) * (inv_n * inv_n);
-        const T dd = hh * hh + perp2;
-        dist = dd > T(0) ? Mth<T>::sqrt_pos(dd) : dd;        // 0 stays 0, NaN stays NaN
+        if (REC) capsule_ray_record<T>(q, w);
+        T inv_n;
+        dist = capsule_axis_dist<T>(q, inv_n);
         const T Rr = (cull + rad) * T(1.000001);
         const T oaoa = q.c2a + rad * rad;
         const T D = q.baoa * q.baoa - q.baba * (oaoa - Rr * Rr);
@@ -569,17 +601,11 @@ __device__ __forceinline__ void obstacle_pair(const KParams<T> &p, const T pos[3
             q1[c] = s_hi * q.ba[c] - q.oa[c];
         }
     } else {
-        T oc[3], d2 = T(0);
-#pragma unroll
-        for (int c = 0; c < 3; c++) {
-            oc[c] = pos[c] - ob[c];
-            d2 += oc[c] * oc[c];
-        }
+        T oc[3], d2;
+        sphere_offset<T>(pos, ob, oc, d2);
         rad = ob[3];
-        if (REC) {
-            w[0] = oc[0]; w[1] = oc[1]; w[2] = oc[2]; w[3] = d2 - rad * rad;
-        }
-        dist = d2 > T(0) ? Mth<T>::sqrt_pos(d2) : d2;
+        if (REC) sphere_ray_record<T>(oc, d2, rad, w);
+        dist = length_from_sq(d2);
 #pragma unroll
         for (int c = 0; c < 3; c++) q0[c] = q1[c] = -oc[c];
     }
@@ -607,31 +633,24 @@ __device__ __forceinline__ void obstacle_pair(const KParams<T> &p, const T pos[3
     in_view = !outside;
 }
 
-// Just the ray-test record of obstacle_pair (same expressions, same bits): what the ray launch needs once the cull
-// launch has decided collision and visibility.
+// Just the ray-test record of obstacle_pair: what the ray launch needs once the cull code has decided collision and
+// visibility.
 template <typename T>
 __device__ __forceinline__ void obstacle_ray_record(const T pos[3], const T ob[7], bool is_cap, T *w) {
     if (is_cap) {
         const T bot[3] = {ob[0], ob[1], ob[2]}, top[3] = {ob[3], ob[4], ob[5]};
         CapPre<T> q;
         capsule_pre<T>(pos, bot, top, ob[6], q);
-        w[0] = q.ba[0]; w[1] = q.ba[1]; w[2] = q.ba[2];
-        w[3] = q.oa[0]; w[4] = q.oa[1]; w[5] = q.oa[2];
-        w[6] = q.baba; w[7] = q.baoa; w[8] = q.c; w[9] = q.c2a; w[10] = q.c2b;
+        capsule_ray_record<T>(q, w);
     } else {
-        T oc[3], d2 = T(0);
-#pragma unroll
-        for (int c = 0; c < 3; c++) {
-            oc[c] = pos[c] - ob[c];
-            d2 += oc[c] * oc[c];
-        }
-        const T rad = ob[3];
-        w[0] = oc[0]; w[1] = oc[1]; w[2] = oc[2]; w[3] = d2 - rad * rad;
+        T oc[3], d2;
+        sphere_offset<T>(pos, ob, oc, d2);
+        sphere_ray_record<T>(oc, d2, ob[3], w);
     }
 }
 
-// Just the body-collision decision of obstacle_pair (same expressions, same bits): used by the cull code for the
-// pairs its float pre-test leaves undecided.
+// Just the body-collision decision of obstacle_pair: used by the cull code for the pairs its float pre-test leaves
+// undecided.
 template <typename T>
 __device__ __forceinline__ bool obstacle_body_hit(const KParams<T> &p, const T pos[3], const T ob[7], bool is_cap) {
     T rad, dist;
@@ -640,26 +659,13 @@ __device__ __forceinline__ bool obstacle_body_hit(const KParams<T> &p, const T p
         rad = ob[6];
         CapPre<T> q;
         capsule_pre<T>(pos, bot, top, rad, q);
-        const T inv_n = Mth<T>::rsqrt_pos(q.baba);
-        const T sp = -q.baoa * inv_n;
-        const T tp = (q.oc2[0] * q.ba[0] + q.oc2[1] * q.ba[1] + q.oc2[2] * q.ba[2]) * inv_n;
-        T hh = sp;
-        if (tp > hh || tp != tp) hh = tp;
-        if (T(0) > hh) hh = T(0);
-        T cr[3];
-        cross3(q.oa, q.ba, cr);
-        const T perp2 = (cr[0] * cr[0] + cr[1] * cr[1] + cr[2] * cr[2]) * (inv_n * inv_n);
-        const T dd = hh * hh + perp2;
-        dist = dd > T(0) ? Mth<T>::sqrt_pos(dd) : dd;
+        T inv_n;
+        dist = capsule_axis_dist<T>(q, inv_n);
     } else {
-        T d2 = T(0);
-#pragma unroll
-        for (int c = 0; c < 3; c++) {
-            const T oc = pos[c] - ob[c];
-            d2 += oc * oc;
-        }
+        T oc[3], d2;
+        sphere_offset<T>(pos, ob, oc, d2);
         rad = ob[3];
-        dist = d2 > T(0) ? Mth<T>::sqrt_pos(d2) : d2;
+        dist = length_from_sq(d2);
     }
     return dist <= rad + p.safety_radius;
 }

@@ -51,40 +51,53 @@ __device__ __forceinline__ void store_obstacle_row(T *row, const T o[kObstRowWor
     }
 }
 
-// Obstacle rows (KParams::obsd) and float obstacle records of env i for the cull code (KParams::obsf, see
-// cull_pair_rec), from the obstacles and the goal as they are stored (T).  Float records: capsule k -> slots 2k, 2k+1;
-// sphere s -> slot 2 n_caps + s.  The pipeline layout allocates both or neither.
-template <typename T>
-__device__ __forceinline__ void store_capsule_record(const KParams<T> &p, int64_t i, int k, const T cap[7], const T goal[3]) {
+// Obstacle k of env i (numbered as obstacle_row) as stored (T): a capsule bot[3] top[3] r (NW = 7) or a sphere
+// centre[3] r (NW = 4).  The library keeps two copies of it, written here from the obstacle and the goal: the obstacle
+// row (KParams::obsd) and the float record(s) for the cull code (KParams::obsf, see cull_pair_rec): capsule k -> slots
+// 2k, 2k+1; sphere s = k - n_caps -> slot 2 n_caps + s.  The pipeline layout allocates both or neither.
+template <typename T, int NW>
+__device__ __forceinline__ void store_obstacle_copies(const KParams<T> &p, int64_t i, int k, const T (&ob)[NW],
+                                                      const T goal[3]) {
+    static_assert(NW == 7 || NW == 4, "capsule: 7 words, sphere: 4");
+    constexpr bool is_cap = NW == 7;
     if (p.obsf == nullptr) return;
+    const T *o = ob;       // a pointer: o[4..6] below are only read for a capsule
     {
-        const T row[kObstRowWords] = {cap[0], cap[1], cap[2], cap[3], cap[4], cap[5], cap[6], T(0)};
+        const T row[kObstRowWords] = {o[0], o[1], o[2], o[3], is_cap ? o[4] : T(0), is_cap ? o[5] : T(0),
+                                      is_cap ? o[6] : T(0), T(0)};
         store_obstacle_row<T>(obstacle_row<T>(p, i, k), row);
     }
-    const double ob[7] = {(double)cap[0], (double)cap[1], (double)cap[2], (double)cap[3], (double)cap[4], (double)cap[5], (double)cap[6]};
+    const double obd[7] = {(double)o[0], (double)o[1], (double)o[2], (double)o[3], is_cap ? (double)o[4] : 0.0,
+                           is_cap ? (double)o[5] : 0.0, is_cap ? (double)o[6] : 0.0};
     const double g[3] = {(double)goal[0], (double)goal[1], (double)goal[2]};
     float4 q0, q1;
-    obstacle_record_f32(ob, g, true, q0, q1);
-    p.obsf[(int64_t)(2 * k) * p.n_envs + i] = q0;
-    p.obsf[(int64_t)(2 * k + 1) * p.n_envs + i] = q1;
-}
-
-template <typename T>
-__device__ __forceinline__ void store_sphere_record(const KParams<T> &p, int64_t i, int s, const T sph[4], const T goal[3]) {
-    if (p.obsf == nullptr) return;
-    {
-        const T row[kObstRowWords] = {sph[0], sph[1], sph[2], sph[3], T(0), T(0), T(0), T(0)};
-        store_obstacle_row<T>(obstacle_row<T>(p, i, p.n_caps + s), row);
+    obstacle_record_f32(obd, g, is_cap, q0, q1);
+    if (is_cap) {
+        p.obsf[(int64_t)(2 * k) * p.n_envs + i] = q0;
+        p.obsf[(int64_t)(2 * k + 1) * p.n_envs + i] = q1;
+    } else {
+        const int s = k - p.n_caps;
+        p.obsf[(int64_t)(2 * p.n_caps + s) * p.n_envs + i] = q0;
     }
-    const double ob[7] = {(double)sph[0], (double)sph[1], (double)sph[2], (double)sph[3], 0.0, 0.0, 0.0};
-    const double g[3] = {(double)goal[0], (double)goal[1], (double)goal[2]};
-    float4 q0, q1;
-    obstacle_record_f32(ob, g, false, q0, q1);
-    p.obsf[(int64_t)(2 * p.n_caps + s) * p.n_envs + i] = q0;
 }
 
-// Rebuilds the obstacle rows and float obstacle records of env i from the bound buffers (after the caller wrote obstacles or goals itself:
-// dockauv_refresh_obstacles).
+// Obstacle k of env i, in T or as drawn in double, rounded to T into the caller's planes (capsule k: capsules[k*7+j],
+// sphere s = k - n_caps: spheres[s*4+j]) and into the library's copies
+template <typename T, typename S, int NW>
+__device__ __forceinline__ void store_obstacle(const KParams<T> &p, int64_t i, int k, const S (&ob)[NW], const T goal[3]) {
+    const int64_t N = p.n_envs;
+    T *plane = NW == 7 ? p.capsules + (int64_t)(k * 7) * N : p.spheres + (int64_t)((k - p.n_caps) * 4) * N;
+    T o[NW];
+#pragma unroll
+    for (int j = 0; j < NW; j++) {
+        o[j] = (T)ob[j];
+        plane[(int64_t)j * N + i] = o[j];
+    }
+    store_obstacle_copies<T>(p, i, k, o, goal);
+}
+
+// Rebuilds the library's obstacle copies of env i from the bound buffers (after the caller wrote obstacles or goals
+// itself: dockauv_refresh_obstacles).
 template <typename T>
 __global__ void refresh_obstacles_kernel(const __grid_constant__ KParams<T> p) {
     const int64_t N = p.n_envs;
@@ -95,13 +108,13 @@ __global__ void refresh_obstacles_kernel(const __grid_constant__ KParams<T> p) {
         T cap[7];
 #pragma unroll
         for (int j = 0; j < 7; j++) cap[j] = p.capsules[(int64_t)(k * 7 + j) * N + i];
-        store_capsule_record<T>(p, i, k, cap, goal);
+        store_obstacle_copies<T>(p, i, k, cap, goal);
     }
     for (int s = 0; s < p.n_sph; s++) {
         T sph[4];
 #pragma unroll
         for (int j = 0; j < 4; j++) sph[j] = p.spheres[(int64_t)(s * 4 + j) * N + i];
-        store_sphere_record<T>(p, i, s, sph, goal);
+        store_obstacle_copies<T>(p, i, p.n_caps + s, sph, goal);
     }
 }
 
@@ -147,25 +160,6 @@ __device__ __forceinline__ void reset_env_role(const KParams<T> &p, int64_t i, i
         goal[2] = (u89[0] - 0.5) * 4.0;
     }
     const T goal_t[3] = {(T)goal[0], (T)goal[1], (T)goal[2]};
-    // obstacle rows (T) + their float records for the cull code
-    auto put_capsule = [&](int k, const double cap[7]) {
-        T c[7];
-#pragma unroll
-        for (int j = 0; j < 7; j++) {
-            c[j] = (T)cap[j];
-            p.capsules[(int64_t)(k * 7 + j) * N + i] = c[j];
-        }
-        store_capsule_record<T>(p, i, k, c, goal_t);
-    };
-    auto put_sphere = [&](int k, const double sph[4]) {
-        T c[4];
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            c[j] = (T)sph[j];
-            p.spheres[(int64_t)(k * 4 + j) * N + i] = c[j];
-        }
-        store_sphere_record<T>(p, i, k, c, goal_t);
-    };
     if (role == 0) {
         double u01[2], u23[2], u45[2];
         U2(0, u01);
@@ -205,16 +199,16 @@ __device__ __forceinline__ void reset_env_role(const KParams<T> &p, int64_t i, i
             sincos(theta, &s, &c);
             const double x = c * 6, y = s * 6;
             const double cap[7] = {x, y, half, x, y, -half, 1.0};
-            put_capsule(first_pillar + k, cap);
+            store_obstacle<T>(p, i, first_pillar + k, cap, goal_t);
         }
     } else if (role == 5) {
         if (has_dock) {
             const double cap[7] = {0, 0, 2.0, 0, 0, -2.0, 1.0};              // bot = 2*position - top, shape.py:105-108
-            put_capsule(0, cap);
+            store_obstacle<T>(p, i, 0, cap, goal_t);
         }
         for (int kc = first_pillar + n_pillars; kc < p.n_caps; kc++) {         // unused slots: far away, zero radius
             const double cap[7] = {1e6, 1e6, 1e6, 1e6, 1e6, 1e6 + 1.0, 0.0};
-            put_capsule(kc, cap);
+            store_obstacle<T>(p, i, kc, cap, goal_t);
         }
         double cur[5] = {0, 0, 0, 0, 0};
         if (scn == DOCKAUV_SCN_SIMPLE_CURRENT || scn == DOCKAUV_SCN_CAPSULE_CURRENT || scn == DOCKAUV_SCN_OBSTACLES_CURRENT) {
@@ -237,10 +231,10 @@ __device__ __forceinline__ void reset_env_role(const KParams<T> &p, int64_t i, i
                 double q = sqrt(1 - z * z), s, c;
                 sincos(az, &s, &c);
                 const double sph[4] = {rr * q * c, rr * q * s, rr * z, 1.0};
-                put_sphere(ks, sph);
+                store_obstacle<T>(p, i, p.n_caps + ks, sph, goal_t);
             } else {
                 const double sph[4] = {1e6, 1e6, 1e6, 0.0};
-                put_sphere(ks, sph);
+                store_obstacle<T>(p, i, p.n_caps + ks, sph, goal_t);
             }
         }
     }
@@ -344,16 +338,11 @@ __device__ __forceinline__ void bank_reset_role(const KParams<T> &p, int64_t i, 
             if (s < p.n_caps) {
                 T cap[7];
                 load_bank_span<T, 7>(row, kBankObst + 7 * s, cap);
-#pragma unroll
-                for (int j = 0; j < 7; j++) p.capsules[(int64_t)(s * 7 + j) * N + i] = cap[j];
-                store_capsule_record<T>(p, i, s, cap, goal);
+                store_obstacle<T>(p, i, s, cap, goal);
             } else {
-                const int k = s - p.n_caps;
                 T sph[4];
-                load_bank_span<T, 4>(row, kBankObst + 7 * p.n_caps + 4 * k, sph);
-#pragma unroll
-                for (int j = 0; j < 4; j++) p.spheres[(int64_t)(k * 4 + j) * N + i] = sph[j];
-                store_sphere_record<T>(p, i, k, sph, goal);
+                load_bank_span<T, 4>(row, kBankObst + 7 * p.n_caps + 4 * (s - p.n_caps), sph);
+                store_obstacle<T>(p, i, s, sph, goal);
             }
         }
     }
