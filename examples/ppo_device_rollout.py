@@ -3,9 +3,12 @@
 ``train()`` (gym_dockauv/train.py:21-82: ``MODEL('MlpPolicy', env).learn(...)``) without a host round trip per step:
 
     python examples/ppo_device_rollout.py [--envs 16384] [--steps 64] [--iters 20] [--record-envs K --record-dir DIR]
+                                          [--fused]
 
 * rollouts: ``DeviceRolloutBuffer.collect`` -- the step kernels write observation / reward / done of step t straight
-  into row t of the buffer;
+  into row t of the buffer; with ``--fused``, ``DeviceRolloutBuffer.collect_fused``: the same networks evaluated by the
+  library's policy kernel between the steps of one captured rollout (the graph is captured once and replayed every
+  iteration: the update rewrites the parameters in place);
 * advantages: ``dockauv_gae`` (one kernel over the stacked rows);
 * the policy / value networks and the clipped-surrogate update are plain PyTorch (they are not part of the step path);
 * ``--record-envs K``: the episodes of K envs spread over the batch are recorded on the device while the run trains
@@ -26,6 +29,7 @@ import torch.nn as nn  # noqa: E402
 from gym_dockauv_b200 import envs  # noqa: E402
 from gym_dockauv_b200.config import TRAIN_CONFIG  # noqa: E402
 from gym_dockauv_b200.episode_export import TrainingRecorder  # noqa: E402
+from gym_dockauv_b200.policy import FusedActorCritic  # noqa: E402
 from gym_dockauv_b200.rollout import DeviceRolloutBuffer  # noqa: E402
 
 
@@ -54,6 +58,7 @@ def main():
     ap.add_argument("--scenario", default="ObstaclesDocking3d")
     ap.add_argument("--record-envs", type=int, default=0, help="record the episodes of this many envs (at most 1024)")
     ap.add_argument("--record-dir", default="episode_storage")
+    ap.add_argument("--fused", action="store_true", help="collect with the policy kernel (DeviceRolloutBuffer.collect_fused)")
     args = ap.parse_args()
     env = envs.SCENARIOS[args.scenario](TRAIN_CONFIG, num_envs=args.envs, seed=0)
     buf = DeviceRolloutBuffer(env, args.steps, gamma=0.99, gae_lambda=0.95)
@@ -64,12 +69,17 @@ def main():
         rec = TrainingRecorder(env, ids, args.record_dir, title="ppo", capacity=max(args.steps, 64))
     net = ActorCritic(env.n_observations, env.n_actions).to(env.device)
     opt = torch.optim.Adam(net.parameters(), lr=3e-4)
+    fused = FusedActorCritic([net.pi[0], net.pi[2], net.pi[4]], [net.v[0], net.v[2], net.v[4]], net.log_std) \
+        if args.fused else None
     for it in range(args.iters):
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        last_obs = buf.collect(net.act)
-        with torch.no_grad():
-            buf.compute_returns_and_advantage(net.v(last_obs).squeeze(-1))
+        if fused is not None:
+            buf.compute_returns_and_advantage(buf.collect_fused(fused))
+        else:
+            last_obs = buf.collect(net.act)
+            with torch.no_grad():
+                buf.compute_returns_and_advantage(net.v(last_obs).squeeze(-1))
         torch.cuda.synchronize()
         t_collect = time.perf_counter() - t0
         info = buf.episode_infos()
@@ -92,8 +102,9 @@ def main():
         n_ep = info["l"].numel()
         mean_r = float(info["r"].mean()) if n_ep else float("nan")
         mean_l = float(info["l"].float().mean()) if n_ep else float("nan")
+        captures = f"  graph captures {env.rollout_policy_captures()} " if fused is not None else ""
         print(f"iter {it:3d}  episodes {n_ep:7d}  mean return {mean_r:10.2f}  mean length {mean_l:7.1f}  "
-              f"collect {args.envs * args.steps / t_collect:.3g} env-steps/s (policy included)", flush=True)
+              f"collect {args.envs * args.steps / t_collect:.3g} env-steps/s (policy included){captures}", flush=True)
     env.close()
 
 

@@ -3,8 +3,9 @@ or was built against another ABI this module raises, and so does every env const
 import ctypes as C
 import os
 
-from .params import (ABI_VERSION, DockauvBuffers, DockauvDebugOut, DockauvParams, DockauvReplayRing,
-                     DockauvReplaySample, DockauvRolloutOut, DockauvScenarioBank, DockauvStepOut, DockauvTapBuffers)
+from .params import (ABI_VERSION, DockauvBuffers, DockauvDebugOut, DockauvParams, DockauvPolicy, DockauvPolicyOut,
+                     DockauvReplayRing, DockauvReplaySample, DockauvRolloutOut, DockauvScenarioBank, DockauvStepOut,
+                     DockauvTapBuffers)
 
 LIB_PATH = os.environ.get("DOCKAUV_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_lib",
                                                         "libdockauv_b200.so")   # DOCKAUV_LIB: tuning builds only
@@ -27,6 +28,8 @@ SYMBOLS = {
     "dockauv_step_graph_captures": (_i, [_vp, C.POINTER(_i64)]),
     "dockauv_step_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _i, C.POINTER(DockauvStepOut)]),
     "dockauv_rollout": (_i, [_vp, _vp, _i, _i, C.POINTER(DockauvRolloutOut), _i, _i, _vp]),
+    "dockauv_rollout_policy": (_i, [_vp, C.POINTER(DockauvPolicy), _vp, _i, C.POINTER(DockauvRolloutOut),
+                                    C.POINTER(DockauvPolicyOut), _i, _i, _vp]),
     "dockauv_set_taps": (_i, [_vp, C.POINTER(_i64), _i, _i, C.POINTER(DockauvTapBuffers)]),
     "dockauv_set_scenario_bank": (_i, [_vp, C.POINTER(DockauvScenarioBank), _vp]),
     "dockauv_gae": (_i, [_vp, _i, _vp, _vp, _vp, _i, _i64, C.c_float, C.c_float, _vp, _vp, _vp]),
@@ -40,6 +43,7 @@ SYMBOLS = {
     "dockauv_launch_count": (_i, [_vp, C.POINTER(_i64)]),
     "dockauv_last_list_counts": (_i, [_vp, C.POINTER(_i64), C.POINTER(_i64), _vp]),
     "dockauv_rollout_captures": (_i, [_vp, C.POINTER(_i64)]),
+    "dockauv_rollout_policy_captures": (_i, [_vp, C.POINTER(_i64)]),
     "dockauv_enable_timing": (_i, [_vp, _i]),
     "dockauv_last_step_ms": (_i, [_vp, C.POINTER(C.c_float)]),
     "dockauv_last_step_launch_ms": (_i, [_vp, C.POINTER(C.c_float), _i, C.POINTER(_i)]),

@@ -19,6 +19,7 @@
 
 #include "dockauv_device.cuh"
 #include "dockauv_launch.h"
+#include "dockauv_policy.cuh"
 
 using namespace dockauv;
 
@@ -153,6 +154,17 @@ struct DockauvHandle {
         uint64_t seed;
     };
     GraphCache<RolloutKey> rg{1};
+    // closed-loop rollout graphs (dockauv_rollout_policy): a trainer alternates a training and an evaluation rollout
+    struct PolicyKey {
+        DockauvPolicy pol;
+        const float *obs0;
+        DockauvRolloutOut out;
+        DockauvPolicyOut pout;
+        int64_t n_steps, auto_reset;
+        uint64_t seed;
+    };
+    GraphCache<PolicyKey> pg{4};
+    float *pol_actions = nullptr;  // f32[N][n_u]: the policy's clipped actions, read by the step (allocated on first use)
     // step graph cache: the launch sequence of ONE dockauv_step (launches of both halves, fork / join events) captured per
     // set of pointers and replayed; trainers alternate between a handful of action / output tensors
     struct StepKey {
@@ -199,6 +211,7 @@ static int pooled_dim(int n, int b) { return (n + b - 1) / b; }
 static void drop_graphs(DockauvHandle *h) {      // captured launch sequences hold the old pointers / seed
     h->rg.clear();
     h->sg.clear();
+    h->pg.clear();
 }
 
 // f(k) with the handle's KParams in its precision: the one place that chooses between kd and kf
@@ -442,6 +455,7 @@ extern "C" int dockauv_destroy(DockauvHandle *h) {
     if (h->tap.dst) cudaStreamDestroy(h->tap.dst);
     if (h->tap.ev_dbg) cudaEventDestroy(h->tap.ev_dbg);
     if (h->bank_check) cudaFree(h->bank_check);
+    if (h->pol_actions) cudaFree(h->pol_actions);
     drop_graphs(h);
     delete h;
     return DOCKAUV_OK;
@@ -1013,24 +1027,26 @@ extern "C" int dockauv_step_host(DockauvHandle *h, const void *actions_host, int
 }
 
 // ------------------------------------------------------------------------------------------- stacked rollout
+// row t of every output of a stacked rollout
+static DockauvStepOut rollout_step_out(const DockauvHandle *h, const DockauvRolloutOut &o, int t) {
+    const size_t N = (size_t)h->n_envs, esz = h->esz, orow = (size_t)h->n_obs * N;
+    DockauvStepOut so;
+    so.obs = o.obs + orow * t;
+    so.reward = (char *)o.reward + esz * N * t;
+    so.done = o.done + N * t;
+    so.cond_bits = o.cond_bits ? o.cond_bits + N * t : nullptr;
+    so.terminal_obs = o.terminal_obs ? o.terminal_obs + orow * t : nullptr;
+    so.ep_return_out = o.ep_return_out ? (char *)o.ep_return_out + esz * N * t : nullptr;
+    so.ep_len_out = o.ep_len_out ? o.ep_len_out + N * t : nullptr;
+    so.delta_d_out = o.delta_d_out ? (char *)o.delta_d_out + esz * N * t : nullptr;
+    return so;
+}
+
 static int rollout_issue(DockauvHandle *h, const void *actions, int action_dtype, int n_steps,
                          const DockauvRolloutOut &o, int auto_reset, cudaStream_t st) {
     const int64_t N = h->n_envs;
-    const size_t esz = h->esz;
     const size_t arow = (action_dtype == DOCKAUV_ACT_F32 ? 4 : 8) * (size_t)h->params.n_u * (size_t)N;
-    const size_t orow = (size_t)h->n_obs * (size_t)N;
-    auto out_of_step = [&](int t) {
-        DockauvStepOut so;
-        so.obs = o.obs + orow * t;
-        so.reward = (char *)o.reward + esz * (size_t)N * t;
-        so.done = o.done + (size_t)N * t;
-        so.cond_bits = o.cond_bits ? o.cond_bits + (size_t)N * t : nullptr;
-        so.terminal_obs = o.terminal_obs ? o.terminal_obs + orow * t : nullptr;
-        so.ep_return_out = o.ep_return_out ? (char *)o.ep_return_out + esz * (size_t)N * t : nullptr;
-        so.ep_len_out = o.ep_len_out ? o.ep_len_out + (size_t)N * t : nullptr;
-        so.delta_d_out = o.delta_d_out ? (char *)o.delta_d_out + esz * (size_t)N * t : nullptr;
-        return so;
-    };
+    auto out_of_step = [&](int t) { return rollout_step_out(h, o, t); };
     if (h->tap.n > 0) {
         // the taps need one pre-step snapshot per step, so every step is forked and joined on its own (the halves of a
         // batch stepped in parts cannot run their T steps as one chain each)
@@ -1077,6 +1093,160 @@ extern "C" int dockauv_rollout(DockauvHandle *h, const void *actions_dev, int ac
     key.seed = h->params.seed;
     return graph_call(h, h->rg, key, "rollout", st, [&](cudaStream_t cs) {
         return rollout_issue(h, actions_dev, action_dtype, n_steps, *out, auto_reset, cs);
+    });
+}
+
+// ------------------------------------------------------------------------------------------- closed-loop rollout
+template <int H, int NU>
+static cudaError_t launch_policy_hu(const PolicyLaunch &p, size_t smem, cudaStream_t st) {
+    auto kernel = policy_kernel<H, NU>;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    int dev = 0, sms = 0, per_sm = 0;
+    if (e == cudaSuccess) e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    // one thread per env; the CTA shrinks (down to one warp) until the range fills every SM with at least one CTA, so a
+    // small batch is spread over the whole GPU; persistent CTAs beyond that (each stages the weights once)
+    const int64_t n = p.env_end - p.env_begin;
+    int threads = 256;
+    while (threads > 32 && (n + threads - 1) / threads < sms) threads /= 2;
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem);
+    if (e != cudaSuccess) return e;
+    const int64_t blocks = std::min<int64_t>((n + threads - 1) / threads, (int64_t)std::max(per_sm, 1) * sms);
+    kernel<<<(unsigned)blocks, threads, smem, st>>>(p);
+    return cudaGetLastError();
+}
+
+template <int H>
+static cudaError_t launch_policy_h(const PolicyLaunch &p, int n_u, size_t smem, cudaStream_t st) {
+    switch (n_u) {
+        case 3: return launch_policy_hu<H, 3>(p, smem, st);     // LAUV
+        case 6: return launch_policy_hu<H, 6>(p, smem, st);     // BlueROV2 joystick
+        case 8: return launch_policy_hu<H, 8>(p, smem, st);     // BlueROV2 direct
+        default: return cudaErrorInvalidValue;
+    }
+}
+
+// One policy evaluation over envs [b, e): the observations `obs` ([N][n_obs]) -> actions, values, log-probs of one
+// rollout row (value_only: values only) and the clipped actions the next step reads.
+static int policy_range(DockauvHandle *h, const DockauvPolicy &pol, const float *obs, float *actions, float *values,
+                        float *log_probs, bool value_only, int64_t b, int64_t e, cudaStream_t st) {
+    PolicyLaunch p;
+    memset(&p, 0, sizeof(p));
+    for (int k = 0; k < 3; k++) {
+        p.pi_w[k] = pol.pi_w[k];
+        p.pi_b[k] = pol.pi_b[k];
+        p.vf_w[k] = pol.vf_w[k];
+        p.vf_b[k] = pol.vf_b[k];
+    }
+    p.log_std = pol.log_std;
+    p.obs = obs;
+    p.actions = actions;
+    p.act_clipped = h->pol_actions;
+    p.values = values;
+    p.log_probs = log_probs;
+    const int n_u = h->params.n_u;
+    for (int k = 0; k < n_u; k++) {      // the float32 bounds of action_space (envs.py), as np.clip sees them
+        p.u_lo[k] = (float)h->params.u_lo[k];
+        p.u_hi[k] = (float)h->params.u_hi[k];
+    }
+    p.seed = h->params.seed;
+    p.env_id0 = h->params.env_id0;
+    p.t_steps = h->bound_bufs.t_steps;
+    p.episode = h->bound_bufs.episode;
+    p.env_begin = b;
+    p.env_end = e;
+    p.n_obs = h->n_obs;
+    p.deterministic = pol.deterministic != 0;
+    p.value_only = value_only ? 1 : 0;
+    const size_t smem = policy_smem_bytes(h->n_obs, pol.hidden, n_u);
+    cudaError_t err = cudaErrorInvalidValue;
+    switch (pol.hidden) {
+        case 32: err = launch_policy_h<32>(p, n_u, smem, st); break;
+        case 64: err = launch_policy_h<64>(p, n_u, smem, st); break;
+        case 96: err = launch_policy_h<96>(p, n_u, smem, st); break;
+        case 128: err = launch_policy_h<128>(p, n_u, smem, st); break;
+    }
+    if (err != cudaSuccess) return fail(DOCKAUV_ECUDA, "policy kernel launch failed: %s", cudaGetErrorString(err));
+    h->launches += 1;
+    return DOCKAUV_OK;
+}
+
+static int rollout_policy_issue(DockauvHandle *h, const DockauvPolicy &pol, const float *obs0, int n_steps,
+                                const DockauvRolloutOut &o, const DockauvPolicyOut &po, int auto_reset, cudaStream_t st) {
+    const size_t N = (size_t)h->n_envs, arow = (size_t)h->params.n_u * N;
+    auto obs_of_step = [&](int t) { return t == 0 ? obs0 : o.obs + (size_t)h->n_obs * N * (t - 1); };
+    auto policy = [&](int t, int64_t b, int64_t e, cudaStream_t s) {
+        return policy_range(h, pol, obs_of_step(t), po.actions + arow * t, po.values + N * t, po.log_probs + N * t, false,
+                            b, e, s);
+    };
+    auto bootstrap = [&](int64_t b, int64_t e, cudaStream_t s) {
+        if (!po.last_values) return DOCKAUV_OK;
+        return policy_range(h, pol, obs_of_step(n_steps), nullptr, po.last_values, nullptr, true, b, e, s);
+    };
+    if (h->tap.n > 0) {
+        // as in rollout_issue: the taps need one pre-step snapshot per step, so every step is forked and joined on its own
+        for (int t = 0; t < n_steps; t++) {
+            const DockauvStepOut so = rollout_step_out(h, o, t);
+            int rc = policy(t, 0, h->n_envs, st);
+            if (rc == DOCKAUV_OK)
+                rc = step_call(h, h->pol_actions, DOCKAUV_ACT_F32, nullptr, &so, nullptr, auto_reset, st, false);
+            if (rc != DOCKAUV_OK) return rc;
+        }
+        return bootstrap(0, h->n_envs, st);
+    }
+    // envs never interact: each part of a batch stepped in parts runs its T (policy, step) pairs as one chain
+    return over_ranges(h, false, st, [&](int64_t b, int64_t e, cudaStream_t s) {
+        for (int t = 0; t < n_steps; t++) {
+            const DockauvStepOut so = rollout_step_out(h, o, t);
+            int rc = policy(t, b, e, s);
+            if (rc == DOCKAUV_OK)
+                rc = step_range(h, h->pol_actions, DOCKAUV_ACT_F32, nullptr, &so, nullptr, auto_reset, b, e, s);
+            if (rc != DOCKAUV_OK) return rc;
+        }
+        return bootstrap(b, e, s);
+    });
+}
+
+extern "C" int dockauv_rollout_policy(DockauvHandle *h, const DockauvPolicy *pol, const float *obs0_dev, int n_steps,
+                                      const DockauvRolloutOut *out, const DockauvPolicyOut *pout, int auto_reset,
+                                      int use_graph, void *stream) {
+    // what needs no handle first
+    if (!pol || !obs0_dev || !out || !pout) return fail(DOCKAUV_EINVAL, "null argument (policy, obs0, out and pout are required)");
+    for (int k = 0; k < 3; k++)
+        if (!pol->pi_w[k] || !pol->pi_b[k] || !pol->vf_w[k] || !pol->vf_b[k])
+            return fail(DOCKAUV_EINVAL, "policy layer %d: a weight or bias pointer is null", k);
+    if (!pol->log_std) return fail(DOCKAUV_EINVAL, "policy log_std is null");
+    if (pol->hidden < 32 || pol->hidden > 128 || pol->hidden % 32 != 0)
+        return fail(DOCKAUV_EINVAL, "policy hidden width must be a multiple of 32 in 32..128, got %d", pol->hidden);
+    if (n_steps <= 0) return fail(DOCKAUV_EINVAL, "n_steps must be positive");
+    if (!out->obs || !out->reward || !out->done) return fail(DOCKAUV_EINVAL, "obs, reward and done outputs are required");
+    if (!pout->actions || !pout->values || !pout->log_probs)
+        return fail(DOCKAUV_EINVAL, "policy outputs actions, values and log_probs are required");
+    if (!h) return fail(DOCKAUV_EINVAL, "null handle");
+    if (!h->bound) return fail(DOCKAUV_ESTATE, "dockauv_bind must be called before dockauv_rollout_policy");
+    const size_t smem = policy_smem_bytes(h->n_obs, pol->hidden, h->params.n_u);
+    if (smem > kPolicyMaxSmem)
+        return fail(DOCKAUV_EINVAL, "policy weights need %zu bytes of shared memory (n_obs %d, hidden %d, n_u %d); one CTA "
+                                    "holds at most %zu", smem, h->n_obs, pol->hidden, h->params.n_u, kPolicyMaxSmem);
+    if (check_rows(h, out->obs, out->terminal_obs) != DOCKAUV_OK) return DOCKAUV_EINVAL;
+    DeviceGuard guard(h->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    // the step's action buffer: allocated before any capture, its pointer is baked into every graph
+    if (!h->pol_actions) CUDA_TRY(cudaMalloc((void **)&h->pol_actions, sizeof(float) * h->params.n_u * (size_t)h->n_envs));
+    if (out->ep_len_out)
+        CUDA_TRY(cudaMemsetAsync(out->ep_len_out, 0, sizeof(int32_t) * (size_t)h->n_envs * (size_t)n_steps, st));
+    if (!use_graph) return rollout_policy_issue(h, *pol, obs0_dev, n_steps, *out, *pout, auto_reset, st);
+    DockauvHandle::PolicyKey key;
+    memset(&key, 0, sizeof(key));
+    key.pol = *pol;
+    key.obs0 = obs0_dev;
+    key.out = *out;
+    key.pout = *pout;
+    key.n_steps = n_steps;
+    key.auto_reset = auto_reset;
+    key.seed = h->params.seed;
+    return graph_call(h, h->pg, key, "policy rollout", st, [&](cudaStream_t cs) {
+        return rollout_policy_issue(h, *pol, obs0_dev, n_steps, *out, *pout, auto_reset, cs);
     });
 }
 
@@ -1560,6 +1730,12 @@ extern "C" int dockauv_last_list_counts(DockauvHandle *h, int64_t *n_listed, int
 extern "C" int dockauv_rollout_captures(DockauvHandle *h, int64_t *n) {
     if (!h || !n) return fail(DOCKAUV_EINVAL, "null argument");
     *n = h->rg.captures;
+    return DOCKAUV_OK;
+}
+
+extern "C" int dockauv_rollout_policy_captures(DockauvHandle *h, int64_t *n) {
+    if (!h || !n) return fail(DOCKAUV_EINVAL, "null argument");
+    *n = h->pg.captures;
     return DOCKAUV_OK;
 }
 

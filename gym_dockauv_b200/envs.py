@@ -23,8 +23,8 @@ import torch
 from . import _capi
 from .config import BASE_CONFIG, REGISTRATION_DICT
 from .params import (ACT_F32, ACT_F64, F32, F64, MAX_TAPS, N_STATS, SCENARIO_IDS, STAT_NAMES, TAP_FIELDS, DockauvBuffers,
-                     DockauvDebugOut, DockauvRolloutOut, DockauvScenarioBank, DockauvStepOut, DockauvTapBuffers,
-                     pack_params)
+                     DockauvDebugOut, DockauvPolicyOut, DockauvRolloutOut, DockauvScenarioBank, DockauvStepOut,
+                     DockauvTapBuffers, pack_params)
 
 DONE_NAMES = ("Done-Goal_reached", "Done-out_pos", "Done-out_att", "Done-max_t", "Done-collision")
 
@@ -270,6 +270,36 @@ class BaseDocking3d:
                                               int(bool(use_graph)), self._stream()))
         self.t_total_steps += T
 
+    def rollout_policy(self, policy, obs0, obs, reward, done, actions, values, log_probs, last_values=None,
+                       cond_bits=None, terminal_obs=None, ep_return_out=None, ep_len_out=None, use_graph=True,
+                       delta_d_out=None):
+        """T steps of a closed loop in ONE library call (dockauv_rollout_policy): ``policy`` (a ``FusedActorCritic``)
+        picks each step's actions on the device from ``obs0`` [N, n_obs] for step 0 and row t - 1 of ``obs`` after that.
+        Row t of ``actions`` f32 [T, N, n_u] (raw samples, before clipping to ``action_space``), ``values`` and
+        ``log_probs`` f32 [T, N] receive the policy's outputs, rows of ``obs`` / ``reward`` / ``done`` (and the optional
+        outputs) the step's, as in ``rollout``; ``last_values`` f32 [N] (optional) receives V(row T - 1 of ``obs``).
+        With ``use_graph`` the launch sequence is captured once per set of tensors and replayed; parameters updated in
+        place are read by the replay."""
+        policy.check_env(self)
+        T, N = int(obs.shape[0]), self.num_envs
+        checks = [(obs0, (N, self.n_observations), torch.float32), (obs, (T, N, self.n_observations), torch.float32),
+                  (reward, (T, N), self.dtype), (done, (T, N), torch.uint8),
+                  (actions, (T, N, self.n_actions), torch.float32), (values, (T, N), torch.float32),
+                  (log_probs, (T, N), torch.float32)]
+        if last_values is not None:
+            checks.append((last_values, (N,), torch.float32))
+        for t, shape, dt in checks:
+            if tuple(t.shape) != shape or t.dtype != dt or not t.is_contiguous() or t.device != self.device:
+                raise ValueError(f"tensor must be contiguous {dt} {shape} on {self.device}")
+        self._check_rows(obs, terminal_obs)
+        out = DockauvRolloutOut(*[_ptr(t) for t in (obs, reward, done, cond_bits, terminal_obs, ep_return_out,
+                                                    ep_len_out, delta_d_out)])
+        pout = DockauvPolicyOut(*[_ptr(t) for t in (actions, values, log_probs, last_values)])
+        _capi.check(self._lib.dockauv_rollout_policy(self._handle, C.byref(policy.struct), _ptr(obs0), T, C.byref(out),
+                                                     C.byref(pout), int(self.auto_reset), int(bool(use_graph)),
+                                                     self._stream()))
+        self.t_total_steps += T
+
     def gae(self, rewards, values, last_values, dones, gamma, gae_lambda, advantages, returns):
         """Generalised advantage estimation over a stacked rollout on the device (dockauv_gae): ``rewards`` [T, N]
         in the env dtype or float32, ``values`` f32 [T, N], ``last_values`` f32 [N], ``dones`` uint8 [T, N];
@@ -511,6 +541,12 @@ class BaseDocking3d:
         """How many times ``rollout(use_graph=True)`` had to capture its launch sequence (replays do not)."""
         n = C.c_int64()
         _capi.check(self._lib.dockauv_rollout_captures(self._handle, C.byref(n)))
+        return n.value
+
+    def rollout_policy_captures(self):
+        """How many times ``rollout_policy(use_graph=True)`` had to capture its launch sequence (replays do not)."""
+        n = C.c_int64()
+        _capi.check(self._lib.dockauv_rollout_policy_captures(self._handle, C.byref(n)))
         return n.value
 
     # ------------------------------------------------------------------ conveniences mirroring the reference's info dict

@@ -94,6 +94,25 @@ class DockauvScenarioBank(C.Structure):
                 ("row_stride", C.c_int64)]
 
 
+class DockauvPolicy(C.Structure):
+    _fields_ = [("pi_w", C.c_void_p * 3), ("pi_b", C.c_void_p * 3), ("vf_w", C.c_void_p * 3), ("vf_b", C.c_void_p * 3),
+                ("log_std", C.c_void_p), ("hidden", C.c_int32), ("deterministic", C.c_int32)]
+
+
+class DockauvPolicyOut(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in ("actions", "values", "log_probs", "last_values")]
+
+
+# dockauv_rollout_policy: shared memory one CTA may hold (sm_100), and what both nets' f32 weights take there
+# (gym_dockauv_b200/csrc/dockauv_policy.cuh: every piece padded to a multiple of 4 floats)
+POLICY_MAX_SMEM = 232448
+
+
+def policy_smem_bytes(n_obs, hidden, n_u):
+    net = lambda n_out: n_obs * hidden + 2 * hidden + hidden * hidden + n_out * hidden + (n_out + 3) // 4 * 4  # noqa: E731
+    return 4 * (net(n_u) + net(1) + (n_u + 3) // 4 * 4)
+
+
 def skew(a):
     """S(a) b = a x b (utils/geomutils.py:106-128)."""
     return np.array([[0.0, -a[2], a[1]], [a[2], 0.0, -a[0]], [-a[1], a[0], 0.0]])

@@ -41,6 +41,7 @@ class DeviceRolloutBuffer:
         self.log_probs = z(T, N)
         self.advantages = z(T, N)
         self.returns = z(T, N)
+        self.last_values = z(N)                          # collect_fused: V(last_obs), the GAE bootstrap
         self.cond_bits = z(T, N, dtype=torch.uint8)
         self.ep_return = z(T, N, dtype=env.dtype)
         self.ep_length = z(T, N, dtype=torch.int32)
@@ -105,6 +106,18 @@ class DeviceRolloutBuffer:
         self._starts[1:].copy_(self.dones)
         self.full = True
         return self.last_obs
+
+    def collect_fused(self, policy, use_graph=True):
+        """Closed-loop rollout with the actor-critic evaluated on the device (``env.rollout_policy``): one library call
+        fills the rows ``collect`` fills (actions as sampled, before clipping; values; log-probs) and ``last_values``.
+        ``policy``: a ``FusedActorCritic``.  Returns ``last_values`` (the value of ``last_obs``)."""
+        self._carry_over()
+        self.env.rollout_policy(policy, self._obs[0], self._obs[1:], self.rewards, self.dones, self.actions, self.values,
+                                self.log_probs, last_values=self.last_values, cond_bits=self.cond_bits,
+                                ep_return_out=self.ep_return, ep_len_out=self.ep_length, use_graph=use_graph)
+        self._starts[1:].copy_(self.dones)
+        self.full = True
+        return self.last_values
 
     # ------------------------------------------------------------------ consumption
     def compute_returns_and_advantage(self, last_values):

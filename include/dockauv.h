@@ -20,6 +20,8 @@
  *   dockauv_rollout                    the step loop of the caller: model.learn() -> collect_rollouts of SB3's
  *                                      on-policy algorithms (train.py:64-71) and predict()'s while-loop
  *                                      (train.py:107-118), for action sequences that are known up front
+ *   dockauv_rollout_policy             the same loops with SB3's MlpPolicy choosing the actions on the device
+ *                                      (OnPolicyAlgorithm.collect_rollouts, predict(deterministic=True))
  *   dockauv_gae                        RolloutBuffer.compute_returns_and_advantage of the PPO caller
  *                                      (stable-baselines3 1.5.0, requirements.txt; selected at train.py:64)
  *   dockauv_replay_sample              ReplayBuffer.sample of the SAC caller (MODEL = SAC at train.py:64)
@@ -299,6 +301,43 @@ DOCKAUV_API int dockauv_step_host(DockauvHandle *h, const void *actions_host, in
 DOCKAUV_API int dockauv_rollout(DockauvHandle *h, const void *actions_dev, int action_dtype, int n_steps,
                     const DockauvRolloutOut *out, int auto_reset, int use_graph, void *stream);
 
+/* Closed-loop rollout: stable-baselines3's default MlpPolicy (separate pi and vf nets n_obs -> H -> H with Tanh,
+ * action_net H -> n_u, value_net H -> 1, state-independent log_std, diagonal Gaussian) picks each step's actions on the
+ * device.  H is a multiple of 32 in 32..128, and both nets' f32 weights must fit one CTA's shared memory (227 KB;
+ * n_obs 36, H 64: 53 KB); DOCKAUV_EINVAL otherwise. */
+typedef struct DockauvPolicy {        /* caller-owned f32 device tensors, nn.Linear layout: weight [out][in], bias [out] */
+    const float *pi_w[3], *pi_b[3];   /* n_obs->H, H->H, H->n_u */
+    const float *vf_w[3], *vf_b[3];   /* n_obs->H, H->H, H->1 */
+    const float *log_std;             /* [n_u] */
+    int32_t hidden, deterministic;
+} DockauvPolicy;
+typedef struct DockauvPolicyOut {     /* f32, device */
+    float *actions;                   /* [T][N][n_u] raw samples (SB3 RolloutBuffer.actions) */
+    float *values, *log_probs;        /* [T][N] */
+    float *last_values;               /* [N], nullable: V(observation after step T-1), the GAE bootstrap */
+} DockauvPolicyOut;
+
+/* T steps of collect_rollouts (or, with deterministic != 0, of predict()'s loop) in one call.  Step t's policy reads
+ * obs0_dev ([N][n_obs], f32) for t = 0 and row t-1 of out->obs otherwise, and writes, per env:
+ *   actions   a = mu + sigma eps (deterministic: a = mu), as SB3's RolloutBuffer stores it
+ *   values    V(obs)
+ *   log_probs sum_k (-eps_k^2 / 2 - log sigma_k - log(2 pi) / 2)  (deterministic: eps = 0)
+ * and the step reads a clipped to the action space [u_lo, u_hi] (np.clip in collect_rollouts) as float32 actions, from a
+ * library-owned [N][n_u] buffer.  eps comes from the handle's Philox4x32-10 key at counter (global id lo, global id hi,
+ * episode, 0xC0000000 | (t_steps mod 2^29) << 1 | j), j = 0, 1, with the env's episode and t_steps before the step;
+ * Box-Muller on the 32-bit words (w >> 8) gives four normals per block (eps_{4j..4j+3}; DESIGN.md section 5.4).  So the
+ * actions depend on (seed, global id, episode, t) only: they do not change with sharding, and a reset with the same seed
+ * reproduces the rollout bit for bit.  With last_values set, one more policy evaluation writes V(row T-1 of out->obs).
+ * Everything else is as in dockauv_rollout (ep_len_out zero-filled first, row alignment checked, taps recorded).  The
+ * arguments are checked on the host first (the checks that need no handle before the null-handle check).
+ * Graphs (use_graph != 0): one CUDA graph per (policy pointers, hidden, deterministic, obs0, outputs, T, auto_reset,
+ * seed), a few cached per handle, so a training rollout and a deterministic evaluation rollout alternate without
+ * re-capture.  Weights rewritten in place (optimizer.step()) are read by the next replay; re-allocated parameters (e.g.
+ * .to()) are new pointers and are captured anew. */
+DOCKAUV_API int dockauv_rollout_policy(DockauvHandle *h, const DockauvPolicy *pol, const float *obs0_dev, int n_steps,
+                                       const DockauvRolloutOut *out, const DockauvPolicyOut *pout, int auto_reset,
+                                       int use_graph, void *stream);
+
 /* Record the envs env_ids_host[0..n_taps) (local indices, distinct, < n_envs, n_taps <= DOCKAUV_MAX_TAPS) on every
  * following dockauv_step / dockauv_rollout into the ring `bufs` (capacity slots); n_taps = 0 removes the taps (capacity
  * and bufs are then ignored).  Zeroes *bufs->count and drops the cached step and rollout graphs.
@@ -413,6 +452,8 @@ DOCKAUV_API int dockauv_launch_count(DockauvHandle *h, int64_t *n_launches);
 DOCKAUV_API int dockauv_last_list_counts(DockauvHandle *h, int64_t *n_listed, int64_t *n_ended, void *stream);
 /* how many times dockauv_rollout(use_graph) had to capture its launch sequence (a replay with the same pointers does not) */
 DOCKAUV_API int dockauv_rollout_captures(DockauvHandle *h, int64_t *n_captures);
+/* the same for dockauv_rollout_policy(use_graph) */
+DOCKAUV_API int dockauv_rollout_policy_captures(DockauvHandle *h, int64_t *n_captures);
 DOCKAUV_API int dockauv_enable_timing(DockauvHandle *h, int enabled);
 DOCKAUV_API int dockauv_last_step_ms(DockauvHandle *h, float *ms);
 /* Per-launch CUDA-event times (ms) of the most recent timed dockauv_step of a multi-launch layout, in launch order
