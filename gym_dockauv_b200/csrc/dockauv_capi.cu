@@ -146,24 +146,19 @@ struct DockauvHandle {
     float *st_obs = nullptr;
     void *st_reward = nullptr;
     uint8_t *st_done = nullptr, *st_cond = nullptr;
-    // rollout graph cache: one captured launch sequence, re-captured when the key changes
+    // a rollout's arguments (rollout_issue), which are also the key of its graph
     struct RolloutKey {
-        const void *actions;
+        DockauvPolicy pol;             // zero for an open-loop rollout
+        const void *input;             // open loop: the actions [T][N][n_u]; closed loop: obs0 [N][n_obs]
         DockauvRolloutOut out;
+        DockauvPolicyOut pout;         // zero for an open-loop rollout
         int64_t n_steps, action_dtype, auto_reset;
         uint64_t seed;
     };
+    // open-loop rollout graphs (dockauv_rollout): one captured launch sequence, re-captured when the key changes
     GraphCache<RolloutKey> rg{1};
     // closed-loop rollout graphs (dockauv_rollout_policy): a trainer alternates a training and an evaluation rollout
-    struct PolicyKey {
-        DockauvPolicy pol;
-        const float *obs0;
-        DockauvRolloutOut out;
-        DockauvPolicyOut pout;
-        int64_t n_steps, auto_reset;
-        uint64_t seed;
-    };
-    GraphCache<PolicyKey> pg{4};
+    GraphCache<RolloutKey> pg{4};
     float *pol_actions = nullptr;  // f32[N][n_u]: the policy's clipped actions, read by the step (allocated on first use)
     // step graph cache: the launch sequence of ONE dockauv_step (launches of both halves, fork / join events) captured per
     // set of pointers and replayed; trainers alternate between a handful of action / output tensors
@@ -1026,77 +1021,7 @@ extern "C" int dockauv_step_host(DockauvHandle *h, const void *actions_host, int
     return DOCKAUV_OK;
 }
 
-// ------------------------------------------------------------------------------------------- stacked rollout
-// row t of every output of a stacked rollout
-static DockauvStepOut rollout_step_out(const DockauvHandle *h, const DockauvRolloutOut &o, int t) {
-    const size_t N = (size_t)h->n_envs, esz = h->esz, orow = (size_t)h->n_obs * N;
-    DockauvStepOut so;
-    so.obs = o.obs + orow * t;
-    so.reward = (char *)o.reward + esz * N * t;
-    so.done = o.done + N * t;
-    so.cond_bits = o.cond_bits ? o.cond_bits + N * t : nullptr;
-    so.terminal_obs = o.terminal_obs ? o.terminal_obs + orow * t : nullptr;
-    so.ep_return_out = o.ep_return_out ? (char *)o.ep_return_out + esz * N * t : nullptr;
-    so.ep_len_out = o.ep_len_out ? o.ep_len_out + N * t : nullptr;
-    so.delta_d_out = o.delta_d_out ? (char *)o.delta_d_out + esz * N * t : nullptr;
-    return so;
-}
-
-static int rollout_issue(DockauvHandle *h, const void *actions, int action_dtype, int n_steps,
-                         const DockauvRolloutOut &o, int auto_reset, cudaStream_t st) {
-    const int64_t N = h->n_envs;
-    const size_t arow = (action_dtype == DOCKAUV_ACT_F32 ? 4 : 8) * (size_t)h->params.n_u * (size_t)N;
-    auto out_of_step = [&](int t) { return rollout_step_out(h, o, t); };
-    if (h->tap.n > 0) {
-        // the taps need one pre-step snapshot per step, so every step is forked and joined on its own (the halves of a
-        // batch stepped in parts cannot run their T steps as one chain each)
-        for (int t = 0; t < n_steps; t++) {
-            const DockauvStepOut so = out_of_step(t);
-            int rc = step_call(h, (const char *)actions + arow * t, action_dtype, nullptr, &so, nullptr, auto_reset, st, false);
-            if (rc != DOCKAUV_OK) return rc;
-        }
-        return DOCKAUV_OK;
-    }
-    // without taps, envs never interact and the actions are all known: each part of a batch stepped in parts runs its T
-    // steps as ONE chain on its own stream, forked from / joined to the caller's stream once per rollout instead of once
-    // per step
-    return over_ranges(h, false, st, [&](int64_t b, int64_t e, cudaStream_t s) {
-        for (int t = 0; t < n_steps; t++) {
-            const DockauvStepOut so = out_of_step(t);
-            const int rc = step_range(h, (const char *)actions + arow * t, action_dtype, nullptr, &so, nullptr, auto_reset, b, e, s);
-            if (rc != DOCKAUV_OK) return rc;
-        }
-        return DOCKAUV_OK;
-    });
-}
-
-extern "C" int dockauv_rollout(DockauvHandle *h, const void *actions_dev, int action_dtype, int n_steps,
-                               const DockauvRolloutOut *out, int auto_reset, int use_graph, void *stream) {
-    if (!h || !actions_dev || !out) return fail(DOCKAUV_EINVAL, "null argument");
-    if (!h->bound) return fail(DOCKAUV_ESTATE, "dockauv_bind must be called before dockauv_rollout");
-    if (!out->obs || !out->reward || !out->done) return fail(DOCKAUV_EINVAL, "obs, reward and done outputs are required");
-    if (action_dtype != DOCKAUV_ACT_F32 && action_dtype != DOCKAUV_ACT_F64) return fail(DOCKAUV_EINVAL, "bad action dtype");
-    if (n_steps <= 0) return fail(DOCKAUV_EINVAL, "n_steps must be positive");
-    if (check_rows(h, out->obs, out->terminal_obs) != DOCKAUV_OK) return DOCKAUV_EINVAL;
-    DeviceGuard guard(h->device);
-    cudaStream_t st = (cudaStream_t)stream;
-    if (out->ep_len_out)
-        CUDA_TRY(cudaMemsetAsync(out->ep_len_out, 0, sizeof(int32_t) * (size_t)h->n_envs * (size_t)n_steps, st));
-    if (!use_graph) return rollout_issue(h, actions_dev, action_dtype, n_steps, *out, auto_reset, st);
-    DockauvHandle::RolloutKey key;
-    memset(&key, 0, sizeof(key));
-    key.actions = actions_dev;
-    key.out = *out;
-    key.n_steps = n_steps;
-    key.action_dtype = action_dtype;
-    key.auto_reset = auto_reset;
-    key.seed = h->params.seed;
-    return graph_call(h, h->rg, key, "rollout", st, [&](cudaStream_t cs) {
-        return rollout_issue(h, actions_dev, action_dtype, n_steps, *out, auto_reset, cs);
-    });
-}
-
-// ------------------------------------------------------------------------------------------- closed-loop rollout
+// ------------------------------------------------------------------------------------------- policy launch
 template <int H, int NU>
 static cudaError_t launch_policy_hu(const PolicyLaunch &p, size_t smem, cudaStream_t st) {
     auto kernel = policy_kernel<H, NU>;
@@ -1171,40 +1096,107 @@ static int policy_range(DockauvHandle *h, const DockauvPolicy &pol, const float 
     return DOCKAUV_OK;
 }
 
-static int rollout_policy_issue(DockauvHandle *h, const DockauvPolicy &pol, const float *obs0, int n_steps,
-                                const DockauvRolloutOut &o, const DockauvPolicyOut &po, int auto_reset, cudaStream_t st) {
-    const size_t N = (size_t)h->n_envs, arow = (size_t)h->params.n_u * N;
-    auto obs_of_step = [&](int t) { return t == 0 ? obs0 : o.obs + (size_t)h->n_obs * N * (t - 1); };
+// ------------------------------------------------------------------------------------------- stacked rollout
+// row t of every output of a stacked rollout
+static DockauvStepOut rollout_step_out(const DockauvHandle *h, const DockauvRolloutOut &o, int t) {
+    const size_t N = (size_t)h->n_envs, esz = h->esz, orow = (size_t)h->n_obs * N;
+    DockauvStepOut so;
+    so.obs = o.obs + orow * t;
+    so.reward = (char *)o.reward + esz * N * t;
+    so.done = o.done + N * t;
+    so.cond_bits = o.cond_bits ? o.cond_bits + N * t : nullptr;
+    so.terminal_obs = o.terminal_obs ? o.terminal_obs + orow * t : nullptr;
+    so.ep_return_out = o.ep_return_out ? (char *)o.ep_return_out + esz * N * t : nullptr;
+    so.ep_len_out = o.ep_len_out ? o.ep_len_out + N * t : nullptr;
+    so.delta_d_out = o.delta_d_out ? (char *)o.delta_d_out + esz * N * t : nullptr;
+    return so;
+}
+
+// The launches of one rollout.  Open loop (pol null): step t reads row t of r.input, the caller's actions.  Closed loop:
+// before step t a policy launch reads r.input (obs0) for t = 0 and row t - 1 of r.out.obs after that, and writes the
+// clipped actions that the step reads from h->pol_actions (r.action_dtype is DOCKAUV_ACT_F32); with r.pout.last_values
+// set, one more launch after the last step writes V(row T - 1 of r.out.obs).
+static int rollout_issue(DockauvHandle *h, const DockauvPolicy *pol, const DockauvHandle::RolloutKey &r, cudaStream_t st) {
+    const size_t N = (size_t)h->n_envs, n_u = (size_t)h->params.n_u;
+    const int n_steps = (int)r.n_steps, action_dtype = (int)r.action_dtype, auto_reset = (int)r.auto_reset;
+    const DockauvRolloutOut &o = r.out;
+    const DockauvPolicyOut &po = r.pout;
+    const size_t arow = (action_dtype == DOCKAUV_ACT_F32 ? 4 : 8) * n_u * N;
+    auto actions_of_step = [&](int t) { return pol ? (const void *)h->pol_actions : (const char *)r.input + arow * t; };
+    auto obs_of_step = [&](int t) { return t == 0 ? (const float *)r.input : o.obs + (size_t)h->n_obs * N * (t - 1); };
     auto policy = [&](int t, int64_t b, int64_t e, cudaStream_t s) {
-        return policy_range(h, pol, obs_of_step(t), po.actions + arow * t, po.values + N * t, po.log_probs + N * t, false,
-                            b, e, s);
+        if (!pol) return DOCKAUV_OK;
+        return policy_range(h, *pol, obs_of_step(t), po.actions + n_u * N * t, po.values + N * t, po.log_probs + N * t,
+                            false, b, e, s);
     };
     auto bootstrap = [&](int64_t b, int64_t e, cudaStream_t s) {
-        if (!po.last_values) return DOCKAUV_OK;
-        return policy_range(h, pol, obs_of_step(n_steps), nullptr, po.last_values, nullptr, true, b, e, s);
+        if (!pol || !po.last_values) return DOCKAUV_OK;
+        return policy_range(h, *pol, obs_of_step(n_steps), nullptr, po.last_values, nullptr, true, b, e, s);
     };
     if (h->tap.n > 0) {
-        // as in rollout_issue: the taps need one pre-step snapshot per step, so every step is forked and joined on its own
+        // the taps need one pre-step snapshot per step, so every step is forked and joined on its own (the parts of a
+        // batch stepped in parts cannot run their T steps as one chain each), and the policy covers the whole batch
         for (int t = 0; t < n_steps; t++) {
             const DockauvStepOut so = rollout_step_out(h, o, t);
             int rc = policy(t, 0, h->n_envs, st);
             if (rc == DOCKAUV_OK)
-                rc = step_call(h, h->pol_actions, DOCKAUV_ACT_F32, nullptr, &so, nullptr, auto_reset, st, false);
+                rc = step_call(h, actions_of_step(t), action_dtype, nullptr, &so, nullptr, auto_reset, st, false);
             if (rc != DOCKAUV_OK) return rc;
         }
         return bootstrap(0, h->n_envs, st);
     }
-    // envs never interact: each part of a batch stepped in parts runs its T (policy, step) pairs as one chain
+    // without taps, envs never interact: each part of a batch stepped in parts runs its T (policy, step) pairs as ONE
+    // chain on its own stream, forked from / joined to the caller's stream once per rollout instead of once per step
     return over_ranges(h, false, st, [&](int64_t b, int64_t e, cudaStream_t s) {
         for (int t = 0; t < n_steps; t++) {
             const DockauvStepOut so = rollout_step_out(h, o, t);
             int rc = policy(t, b, e, s);
             if (rc == DOCKAUV_OK)
-                rc = step_range(h, h->pol_actions, DOCKAUV_ACT_F32, nullptr, &so, nullptr, auto_reset, b, e, s);
+                rc = step_range(h, actions_of_step(t), action_dtype, nullptr, &so, nullptr, auto_reset, b, e, s);
             if (rc != DOCKAUV_OK) return rc;
         }
         return bootstrap(b, e, s);
     });
+}
+
+// Both rollout entry points after their own argument checks: ep_len_out zero-filled, then the launches issued directly
+// or (use_graph) replayed from the graph cached under the rollout's key, open loop in h->rg, closed loop in h->pg.
+static int rollout_run(DockauvHandle *h, const DockauvPolicy *pol, const void *input, int action_dtype, int n_steps,
+                       const DockauvRolloutOut &out, const DockauvPolicyOut *pout, int auto_reset, int use_graph,
+                       void *stream) {
+    if (check_rows(h, out.obs, out.terminal_obs) != DOCKAUV_OK) return DOCKAUV_EINVAL;
+    DeviceGuard guard(h->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    // the closed loop's action buffer: allocated before any capture, its pointer is baked into every graph
+    if (pol && !h->pol_actions)
+        CUDA_TRY(cudaMalloc((void **)&h->pol_actions, sizeof(float) * h->params.n_u * (size_t)h->n_envs));
+    if (out.ep_len_out)
+        CUDA_TRY(cudaMemsetAsync(out.ep_len_out, 0, sizeof(int32_t) * (size_t)h->n_envs * (size_t)n_steps, st));
+    DockauvHandle::RolloutKey key;
+    memset(&key, 0, sizeof(key));
+    if (pol) {
+        key.pol = *pol;
+        key.pout = *pout;
+    }
+    key.input = input;
+    key.out = out;
+    key.n_steps = n_steps;
+    key.action_dtype = action_dtype;
+    key.auto_reset = auto_reset;
+    key.seed = h->params.seed;
+    auto issue = [&](cudaStream_t s) { return rollout_issue(h, pol, key, s); };
+    if (!use_graph) return issue(st);
+    return graph_call(h, pol ? h->pg : h->rg, key, pol ? "policy rollout" : "rollout", st, issue);
+}
+
+extern "C" int dockauv_rollout(DockauvHandle *h, const void *actions_dev, int action_dtype, int n_steps,
+                               const DockauvRolloutOut *out, int auto_reset, int use_graph, void *stream) {
+    if (!h || !actions_dev || !out) return fail(DOCKAUV_EINVAL, "null argument");
+    if (!h->bound) return fail(DOCKAUV_ESTATE, "dockauv_bind must be called before dockauv_rollout");
+    if (!out->obs || !out->reward || !out->done) return fail(DOCKAUV_EINVAL, "obs, reward and done outputs are required");
+    if (action_dtype != DOCKAUV_ACT_F32 && action_dtype != DOCKAUV_ACT_F64) return fail(DOCKAUV_EINVAL, "bad action dtype");
+    if (n_steps <= 0) return fail(DOCKAUV_EINVAL, "n_steps must be positive");
+    return rollout_run(h, nullptr, actions_dev, action_dtype, n_steps, *out, nullptr, auto_reset, use_graph, stream);
 }
 
 extern "C" int dockauv_rollout_policy(DockauvHandle *h, const DockauvPolicy *pol, const float *obs0_dev, int n_steps,
@@ -1228,26 +1220,7 @@ extern "C" int dockauv_rollout_policy(DockauvHandle *h, const DockauvPolicy *pol
     if (smem > kPolicyMaxSmem)
         return fail(DOCKAUV_EINVAL, "policy weights need %zu bytes of shared memory (n_obs %d, hidden %d, n_u %d); one CTA "
                                     "holds at most %zu", smem, h->n_obs, pol->hidden, h->params.n_u, kPolicyMaxSmem);
-    if (check_rows(h, out->obs, out->terminal_obs) != DOCKAUV_OK) return DOCKAUV_EINVAL;
-    DeviceGuard guard(h->device);
-    cudaStream_t st = (cudaStream_t)stream;
-    // the step's action buffer: allocated before any capture, its pointer is baked into every graph
-    if (!h->pol_actions) CUDA_TRY(cudaMalloc((void **)&h->pol_actions, sizeof(float) * h->params.n_u * (size_t)h->n_envs));
-    if (out->ep_len_out)
-        CUDA_TRY(cudaMemsetAsync(out->ep_len_out, 0, sizeof(int32_t) * (size_t)h->n_envs * (size_t)n_steps, st));
-    if (!use_graph) return rollout_policy_issue(h, *pol, obs0_dev, n_steps, *out, *pout, auto_reset, st);
-    DockauvHandle::PolicyKey key;
-    memset(&key, 0, sizeof(key));
-    key.pol = *pol;
-    key.obs0 = obs0_dev;
-    key.out = *out;
-    key.pout = *pout;
-    key.n_steps = n_steps;
-    key.auto_reset = auto_reset;
-    key.seed = h->params.seed;
-    return graph_call(h, h->pg, key, "policy rollout", st, [&](cudaStream_t cs) {
-        return rollout_policy_issue(h, *pol, obs0_dev, n_steps, *out, *pout, auto_reset, cs);
-    });
+    return rollout_run(h, pol, obs0_dev, DOCKAUV_ACT_F32, n_steps, *out, pout, auto_reset, use_graph, stream);
 }
 
 // ------------------------------------------------------------------------------------------- episode taps: setup

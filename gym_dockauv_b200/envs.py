@@ -192,16 +192,7 @@ class BaseDocking3d:
         """One env.step() for every env.  ``actions``: [N, n_u] CUDA tensor, float32 or float64 (the dtype selects
         the reference's dtype-dependent arithmetic, see include/dockauv.h).  Returns (obs, reward, done, info);
         all tensors are views of buffers that the next step overwrites."""
-        if actions.device != self.device:
-            raise ValueError(f"actions live on {actions.device}, env on {self.device}; use step_host for host arrays")
-        if actions.shape != (self.num_envs, self.n_actions):
-            raise ValueError(f"actions must have shape {(self.num_envs, self.n_actions)}, got {tuple(actions.shape)}")
-        if actions.dtype == torch.float32:
-            adt = ACT_F32
-        elif actions.dtype == torch.float64:
-            adt = ACT_F64
-        else:
-            raise TypeError("actions must be float32 or float64")
+        adt = self._action_dtype(actions, (self.num_envs, self.n_actions))
         actions = actions.contiguous()
         if noise is not None:
             noise = noise.to(device=self.device, dtype=self.dtype).contiguous()
@@ -224,6 +215,12 @@ class BaseDocking3d:
             return ACT_F64
         raise TypeError("actions must be float32 or float64")
 
+    def _check_tensors(self, *checks):
+        """Every (tensor, shape, dtype): that shape and dtype, contiguous, on the env's device."""
+        for t, shape, dt in checks:
+            if tuple(t.shape) != shape or t.dtype != dt or not t.is_contiguous() or t.device != self.device:
+                raise ValueError(f"tensor must be contiguous {dt} {shape} on {self.device}")
+
     def _check_rows(self, *rows):
         """Observation rows are written with 128-bit stores when n_obs is a multiple of 4 (include/dockauv.h)."""
         if self.n_observations % 4 == 0:
@@ -237,10 +234,8 @@ class BaseDocking3d:
         writes the observation / reward / done of this step straight into them, nothing is copied afterwards.
         ``obs`` f32 [N, n_obs], ``reward`` env dtype [N], ``done`` uint8 [N]; all contiguous, on the env's device."""
         adt = self._action_dtype(actions, (self.num_envs, self.n_actions))
-        for t, shape, dt in ((obs, (self.num_envs, self.n_observations), torch.float32),
-                             (reward, (self.num_envs,), self.dtype), (done, (self.num_envs,), torch.uint8)):
-            if tuple(t.shape) != shape or t.dtype != dt or not t.is_contiguous() or t.device != self.device:
-                raise ValueError(f"output tensor must be contiguous {dt} {shape} on {self.device}")
+        self._check_tensors((obs, (self.num_envs, self.n_observations), torch.float32),
+                            (reward, (self.num_envs,), self.dtype), (done, (self.num_envs,), torch.uint8))
         self._check_rows(obs, terminal_obs)
         out = DockauvStepOut(*[_ptr(t) for t in (obs, reward, done, cond_bits, terminal_obs, ep_return_out,
                                                  ep_len_out, delta_d_out)])
@@ -255,17 +250,11 @@ class BaseDocking3d:
         replayed logs) in ONE library call: row t of ``obs`` [T, N, n_obs] / ``reward`` [T, N] / ``done`` [T, N]
         receives the outputs of step t.  With ``use_graph`` the launch sequence is captured into a CUDA graph the
         first time and replayed afterwards (same tensors -> same graph)."""
-        T = int(actions.shape[0])
-        adt = self._action_dtype(actions, (T, self.num_envs, self.n_actions))
-        for t, shape, dt in ((obs, (T, self.num_envs, self.n_observations), torch.float32),
-                             (reward, (T, self.num_envs), self.dtype), (done, (T, self.num_envs), torch.uint8)):
-            if tuple(t.shape) != shape or t.dtype != dt or not t.is_contiguous() or t.device != self.device:
-                raise ValueError(f"output tensor must be contiguous {dt} {shape} on {self.device}")
-        if not actions.is_contiguous():
-            raise ValueError("actions must be contiguous")
-        self._check_rows(obs, terminal_obs)
-        out = DockauvRolloutOut(*[_ptr(t) for t in (obs, reward, done, cond_bits, terminal_obs, ep_return_out,
-                                                    ep_len_out, delta_d_out)])
+        T, N = int(actions.shape[0]), self.num_envs
+        adt = self._action_dtype(actions, (T, N, self.n_actions))
+        self._check_tensors((obs, (T, N, self.n_observations), torch.float32), (reward, (T, N), self.dtype),
+                            (done, (T, N), torch.uint8), (actions, (T, N, self.n_actions), actions.dtype))
+        out = self._rollout_out(obs, reward, done, cond_bits, terminal_obs, ep_return_out, ep_len_out, delta_d_out)
         _capi.check(self._lib.dockauv_rollout(self._handle, _ptr(actions), adt, T, C.byref(out), int(self.auto_reset),
                                               int(bool(use_graph)), self._stream()))
         self.t_total_steps += T
@@ -288,17 +277,19 @@ class BaseDocking3d:
                   (log_probs, (T, N), torch.float32)]
         if last_values is not None:
             checks.append((last_values, (N,), torch.float32))
-        for t, shape, dt in checks:
-            if tuple(t.shape) != shape or t.dtype != dt or not t.is_contiguous() or t.device != self.device:
-                raise ValueError(f"tensor must be contiguous {dt} {shape} on {self.device}")
-        self._check_rows(obs, terminal_obs)
-        out = DockauvRolloutOut(*[_ptr(t) for t in (obs, reward, done, cond_bits, terminal_obs, ep_return_out,
-                                                    ep_len_out, delta_d_out)])
+        self._check_tensors(*checks)
+        out = self._rollout_out(obs, reward, done, cond_bits, terminal_obs, ep_return_out, ep_len_out, delta_d_out)
         pout = DockauvPolicyOut(*[_ptr(t) for t in (actions, values, log_probs, last_values)])
         _capi.check(self._lib.dockauv_rollout_policy(self._handle, C.byref(policy.struct), _ptr(obs0), T, C.byref(out),
                                                      C.byref(pout), int(self.auto_reset), int(bool(use_graph)),
                                                      self._stream()))
         self.t_total_steps += T
+
+    def _rollout_out(self, obs, reward, done, cond_bits, terminal_obs, ep_return_out, ep_len_out, delta_d_out):
+        """The stacked outputs of ``rollout`` and ``rollout_policy`` as the library's struct."""
+        self._check_rows(obs, terminal_obs)
+        return DockauvRolloutOut(*[_ptr(t) for t in (obs, reward, done, cond_bits, terminal_obs, ep_return_out,
+                                                     ep_len_out, delta_d_out)])
 
     def gae(self, rewards, values, last_values, dones, gamma, gae_lambda, advantages, returns):
         """Generalised advantage estimation over a stacked rollout on the device (dockauv_gae): ``rewards`` [T, N]
@@ -308,13 +299,9 @@ class BaseDocking3d:
         prec = F64 if rewards.dtype == torch.float64 else F32
         if rewards.dtype not in (torch.float64, torch.float32):
             raise TypeError("rewards must be float64 or float32")
-        for t, shape, dt in ((values, (T, N), torch.float32), (last_values, (N,), torch.float32),
-                             (dones, (T, N), torch.uint8), (advantages, (T, N), torch.float32),
-                             (returns, (T, N), torch.float32)):
-            if tuple(t.shape) != shape or t.dtype != dt or not t.is_contiguous() or t.device != self.device:
-                raise ValueError(f"tensor must be contiguous {dt} {shape} on {self.device}")
-        if not rewards.is_contiguous():
-            raise ValueError("rewards must be contiguous")
+        self._check_tensors((values, (T, N), torch.float32), (last_values, (N,), torch.float32),
+                            (dones, (T, N), torch.uint8), (advantages, (T, N), torch.float32),
+                            (returns, (T, N), torch.float32), (rewards, (T, N), rewards.dtype))
         with torch.cuda.device(self.device):
             _capi.check(self._lib.dockauv_gae(_ptr(rewards), prec, _ptr(values), _ptr(last_values), _ptr(dones), T, N,
                                               float(gamma), float(gae_lambda), _ptr(advantages), _ptr(returns),

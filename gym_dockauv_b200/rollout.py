@@ -74,6 +74,10 @@ class DeviceRolloutBuffer:
             self._starts[0].copy_(self._starts[self.n_steps])
         self.ep_length.zero_()
 
+    def _finish(self):
+        self._starts[1:].copy_(self.dones)       # observation t + 1 starts an episode when step t ended one
+        self.full = True
+
     # ------------------------------------------------------------------ collection
     def collect(self, policy):
         """Closed-loop rollout: ``policy(obs) -> (actions, values, log_probs)`` (device tensors; actions [N, n_u]
@@ -89,8 +93,7 @@ class DeviceRolloutBuffer:
             env.step_into(a if a.dtype in (torch.float32, torch.float64) else self.actions[t], self._obs[t + 1],
                           self.rewards[t], self.dones[t], cond_bits=self.cond_bits[t],
                           ep_return_out=self.ep_return[t], ep_len_out=self.ep_length[t])
-        self._starts[1:].copy_(self.dones)
-        self.full = True
+        self._finish()
         return self.last_obs
 
     def collect_open_loop(self, actions=None, generator=None, use_graph=True):
@@ -103,8 +106,7 @@ class DeviceRolloutBuffer:
             self.actions.copy_(actions)
         self.env.rollout(self.actions, self._obs[1:], self.rewards, self.dones, cond_bits=self.cond_bits,
                          ep_return_out=self.ep_return, ep_len_out=self.ep_length, use_graph=use_graph)
-        self._starts[1:].copy_(self.dones)
-        self.full = True
+        self._finish()
         return self.last_obs
 
     def collect_fused(self, policy, use_graph=True):
@@ -115,8 +117,7 @@ class DeviceRolloutBuffer:
         self.env.rollout_policy(policy, self._obs[0], self._obs[1:], self.rewards, self.dones, self.actions, self.values,
                                 self.log_probs, last_values=self.last_values, cond_bits=self.cond_bits,
                                 ep_return_out=self.ep_return, ep_len_out=self.ep_length, use_graph=use_graph)
-        self._starts[1:].copy_(self.dones)
-        self.full = True
+        self._finish()
         return self.last_values
 
     # ------------------------------------------------------------------ consumption
