@@ -3,10 +3,12 @@
 ``MODEL = SAC`` (gym_dockauv/train.py:64: ``MODEL('MlpPolicy', env).learn(...)``) without a host round trip per step:
 
     python examples/sac_device_replay.py [--envs 16384] [--slots 16] [--steps 32] [--batch 8192] [--gradient-steps 32]
-                                         [--iters 20] [--scenario ObstaclesDocking3d]
+                                         [--iters 20] [--scenario ObstaclesDocking3d] [--fused]
 
 * collection: ``DeviceReplayBuffer.collect`` -- the step kernels write observation, reward, done flag and terminal
-  observation of every step straight into the replay ring;
+  observation of every step straight into the replay ring; with ``--fused``, ``DeviceReplayBuffer.collect_fused`` --
+  the same actor evaluated by the library's tensor-core kernel between the steps of one captured launch chain (bf16
+  operands, f32 accumulation);
 * minibatches: ``DeviceReplayBuffer.sample`` -- one kernel (``dockauv_replay_sample``) draws the batch and gathers its
   rows, with SB3's ``ReplayBufferSamples`` fields;
 * the networks and the update are plain PyTorch with SB3 SAC's defaults: tanh-squashed Gaussian actor, twin Q critics,
@@ -30,6 +32,7 @@ import torch.nn.functional as F  # noqa: E402
 
 from gym_dockauv_b200 import envs  # noqa: E402
 from gym_dockauv_b200.config import TRAIN_CONFIG  # noqa: E402
+from gym_dockauv_b200.policy import FusedSquashedActor  # noqa: E402
 from gym_dockauv_b200.replay import DeviceReplayBuffer  # noqa: E402
 
 
@@ -76,6 +79,7 @@ def main():
     ap.add_argument("--gradient-steps", type=int, default=32)
     ap.add_argument("--iters", type=int, default=20)
     ap.add_argument("--scenario", default="ObstaclesDocking3d")
+    ap.add_argument("--fused", action="store_true", help="collect with the actor evaluated on the device (collect_fused)")
     args = ap.parse_args()
     env = envs.SCENARIOS[args.scenario](TRAIN_CONFIG, num_envs=args.envs, seed=0)
     buf = DeviceReplayBuffer(env, args.slots, seed=0)
@@ -88,11 +92,18 @@ def main():
     opt_critic = torch.optim.Adam(critic.parameters(), lr=3e-4)
     opt_alpha = torch.optim.Adam([log_alpha], lr=3e-4)
     gamma, tau, target_entropy = 0.99, 0.005, -float(n_u)
+    if args.fused:      # the head's row slices are views of the live parameters: Adam's in-place updates are seen
+        net = actor.net
+        w, b = net[4].weight, net[4].bias
+        fused = FusedSquashedActor([net[0], net[2]], w[:n_u], b[:n_u], w[n_u:], b[n_u:])
     for it in range(args.iters):
         env.clear_stats()
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        buf.collect(actor.act, args.steps)
+        if args.fused:
+            buf.collect_fused(fused, args.steps)
+        else:
+            buf.collect(actor.act, args.steps)
         torch.cuda.synchronize()
         t1 = time.perf_counter()
         for _ in range(args.gradient_steps):

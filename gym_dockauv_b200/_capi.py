@@ -4,8 +4,8 @@ import ctypes as C
 import os
 
 from .params import (ABI_VERSION, DockauvBuffers, DockauvDebugOut, DockauvParams, DockauvPolicy, DockauvPolicyOut,
-                     DockauvReplayRing, DockauvReplaySample, DockauvRolloutOut, DockauvScenarioBank, DockauvStepOut,
-                     DockauvTapBuffers)
+                     DockauvReplayRing, DockauvReplaySample, DockauvRolloutOut, DockauvScenarioBank,
+                     DockauvSquashedActor, DockauvStepOut, DockauvTapBuffers)
 
 LIB_PATH = os.environ.get("DOCKAUV_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_lib",
                                                         "libdockauv_b200.so")   # DOCKAUV_LIB: tuning builds only
@@ -35,6 +35,8 @@ SYMBOLS = {
     "dockauv_gae": (_i, [_vp, _i, _vp, _vp, _vp, _i, _i64, C.c_float, C.c_float, _vp, _vp, _vp]),
     "dockauv_replay_sample": (_i, [C.POINTER(DockauvReplayRing), _i, _i, _i64, _i, _i, _i64, _i64, _i64, C.c_uint64,
                                    C.c_uint64, C.POINTER(DockauvReplaySample), _vp]),
+    "dockauv_replay_collect": (_i, [_vp, C.POINTER(DockauvSquashedActor), C.POINTER(DockauvReplayRing), _i, _i, _i, _i,
+                                    _i, _vp]),
     "dockauv_stats_ptr": (_i, [_vp, C.POINTER(_vp)]),
     "dockauv_fold_stats": (_i, [_vp, _vp]),
     "dockauv_get_stats": (_i, [_vp, C.POINTER(C.c_double), _vp]),
@@ -44,6 +46,7 @@ SYMBOLS = {
     "dockauv_last_list_counts": (_i, [_vp, C.POINTER(_i64), C.POINTER(_i64), _vp]),
     "dockauv_rollout_captures": (_i, [_vp, C.POINTER(_i64)]),
     "dockauv_rollout_policy_captures": (_i, [_vp, C.POINTER(_i64)]),
+    "dockauv_replay_collect_captures": (_i, [_vp, C.POINTER(_i64)]),
     "dockauv_enable_timing": (_i, [_vp, _i]),
     "dockauv_last_step_ms": (_i, [_vp, C.POINTER(C.c_float)]),
     "dockauv_last_step_launch_ms": (_i, [_vp, C.POINTER(C.c_float), _i, C.POINTER(_i)]),

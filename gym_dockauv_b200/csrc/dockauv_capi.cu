@@ -20,6 +20,7 @@
 #include "dockauv_device.cuh"
 #include "dockauv_launch.h"
 #include "dockauv_policy.cuh"
+#include "dockauv_sac_actor.cuh"
 
 using namespace dockauv;
 
@@ -152,6 +153,9 @@ struct DockauvHandle {
         const void *input;             // open loop: the actions [T][N][n_u]; closed loop: obs0 [N][n_obs]
         DockauvRolloutOut out;
         DockauvPolicyOut pout;         // zero for an open-loop rollout
+        DockauvSquashedActor act;      // ring collection only (dockauv_replay_collect), else zero
+        DockauvReplayRing ring;        // ring collection only: the ring the steps write into
+        int64_t n_slots, start_slot;   // ring collection only: S and s0
         int64_t n_steps, action_dtype, auto_reset;
         uint64_t seed;
     };
@@ -159,6 +163,8 @@ struct DockauvHandle {
     GraphCache<RolloutKey> rg{1};
     // closed-loop rollout graphs (dockauv_rollout_policy): a trainer alternates a training and an evaluation rollout
     GraphCache<RolloutKey> pg{4};
+    // ring collection graphs (dockauv_replay_collect): a training collection, an evaluation and a few start slots
+    GraphCache<RolloutKey> cg{4};
     float *pol_actions = nullptr;  // f32[N][n_u]: the policy's clipped actions, read by the step (allocated on first use)
     // step graph cache: the launch sequence of ONE dockauv_step (launches of both halves, fork / join events) captured per
     // set of pointers and replayed; trainers alternate between a handful of action / output tensors
@@ -207,6 +213,7 @@ static void drop_graphs(DockauvHandle *h) {      // captured launch sequences ho
     h->rg.clear();
     h->sg.clear();
     h->pg.clear();
+    h->cg.clear();
 }
 
 // f(k) with the handle's KParams in its precision: the one place that chooses between kd and kf
@@ -1096,6 +1103,72 @@ static int policy_range(DockauvHandle *h, const DockauvPolicy &pol, const float 
     return DOCKAUV_OK;
 }
 
+// ------------------------------------------------------------------------------------------- SAC actor launch
+template <int H, int NU>
+static cudaError_t launch_sac_actor_hu(const SacActorLaunch &p, size_t smem, cudaStream_t st) {
+    auto kernel = sac_actor_kernel<H, NU>;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    int dev = 0, sms = 0, per_sm = 0;
+    if (e == cudaSuccess) e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    // a warp per 16-env tile, tiles dealt to the CTAs round robin: a small batch is spread over every SM, persistent
+    // CTAs beyond that.  The CTA keeps all its warps even when some get no tile: staging the weights (each CTA reads
+    // and converts all of them once) is what a small batch waits for, and it goes as fast as the CTA has threads.
+    const int64_t tiles = (p.env_end - p.env_begin + 15) / 16;
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, 32 * kSacWarps, smem);
+    if (e != cudaSuccess) return e;
+    const int64_t blocks = std::min<int64_t>(tiles, (int64_t)std::max(per_sm, 1) * sms);
+    kernel<<<(unsigned)blocks, 32 * kSacWarps, smem, st>>>(p);
+    return cudaGetLastError();
+}
+
+template <int H>
+static cudaError_t launch_sac_actor_h(const SacActorLaunch &p, int n_u, size_t smem, cudaStream_t st) {
+    switch (n_u) {
+        case 3: return launch_sac_actor_hu<H, 3>(p, smem, st);     // LAUV
+        case 6: return launch_sac_actor_hu<H, 6>(p, smem, st);     // BlueROV2 joystick
+        case 8: return launch_sac_actor_hu<H, 8>(p, smem, st);     // BlueROV2 direct
+        default: return cudaErrorInvalidValue;
+    }
+}
+
+// One actor evaluation over envs [b, e): the observations `obs` ([N][n_obs]) -> the squashed actions ([N][n_u]) the
+// next step reads
+static int actor_range(DockauvHandle *h, const DockauvSquashedActor &act, const float *obs, float *actions, int64_t b,
+                       int64_t e, cudaStream_t st) {
+    SacActorLaunch p;
+    memset(&p, 0, sizeof(p));
+    p.w0 = act.w[0];
+    p.b0 = act.b[0];
+    p.w1 = act.w[1];
+    p.b1 = act.b[1];
+    p.mu_w = act.mu_w;
+    p.mu_b = act.mu_b;
+    p.log_std_w = act.log_std_w;
+    p.log_std_b = act.log_std_b;
+    p.obs = obs;
+    p.actions = actions;
+    p.t_steps = h->bound_bufs.t_steps;
+    p.episode = h->bound_bufs.episode;
+    p.seed = h->params.seed;
+    p.env_id0 = h->params.env_id0;
+    p.env_begin = b;
+    p.env_end = e;
+    p.n_obs = h->n_obs;
+    p.deterministic = act.deterministic != 0;
+    const int n_u = h->params.n_u;
+    const size_t smem = sac_actor_smem_bytes(h->n_obs, act.hidden, n_u);
+    cudaError_t err = cudaErrorInvalidValue;
+    switch (act.hidden) {
+        case 64: err = launch_sac_actor_h<64>(p, n_u, smem, st); break;
+        case 128: err = launch_sac_actor_h<128>(p, n_u, smem, st); break;
+        case 256: err = launch_sac_actor_h<256>(p, n_u, smem, st); break;
+    }
+    if (err != cudaSuccess) return fail(DOCKAUV_ECUDA, "SAC actor kernel launch failed: %s", cudaGetErrorString(err));
+    h->launches += 1;
+    return DOCKAUV_OK;
+}
+
 // ------------------------------------------------------------------------------------------- stacked rollout
 // row t of every output of a stacked rollout
 static DockauvStepOut rollout_step_out(const DockauvHandle *h, const DockauvRolloutOut &o, int t) {
@@ -1112,19 +1185,40 @@ static DockauvStepOut rollout_step_out(const DockauvHandle *h, const DockauvRoll
     return so;
 }
 
-// The launches of one rollout.  Open loop (pol null): step t reads row t of r.input, the caller's actions.  Closed loop:
-// before step t a policy launch reads r.input (obs0) for t = 0 and row t - 1 of r.out.obs after that, and writes the
-// clipped actions that the step reads from h->pol_actions (r.action_dtype is DOCKAUV_ACT_F32); with r.pout.last_values
-// set, one more launch after the last step writes V(row T - 1 of r.out.obs).
-static int rollout_issue(DockauvHandle *h, const DockauvPolicy *pol, const DockauvHandle::RolloutKey &r, cudaStream_t st) {
+// ring slot t of the replay ring as the outputs of one step: obs of slot t + 1, reward, done and terminal_obs of slot t
+static DockauvStepOut ring_step_out(const DockauvHandle *h, const DockauvReplayRing &ring, int S, int slot) {
+    const size_t N = (size_t)h->n_envs, orow = (size_t)h->n_obs * N;
+    DockauvStepOut so;
+    memset(&so, 0, sizeof(so));
+    so.obs = (float *)ring.obs + orow * ((slot + 1) % S);
+    so.reward = (char *)ring.reward + h->esz * N * slot;
+    so.done = (uint8_t *)ring.done + N * slot;
+    so.terminal_obs = (float *)ring.terminal_obs + orow * slot;
+    return so;
+}
+
+// The launches of one rollout.  Open loop (pol and act null): step t reads row t of r.input, the caller's actions.
+// Closed loop: before step t a policy launch reads r.input (obs0) for t = 0 and row t - 1 of r.out.obs after that, and
+// writes the clipped actions that the step reads from h->pol_actions (r.action_dtype is DOCKAUV_ACT_F32); with
+// r.pout.last_values set, one more launch after the last step writes V(row T - 1 of r.out.obs).  Ring collection (act):
+// with slot = (s0 + t) % S, before step t an actor launch reads obs[slot] of r.ring and writes actions[slot], which the
+// step reads as float32; the step writes obs[slot + 1] and reward, done, terminal_obs of the slot (ring_step_out).
+static int rollout_issue(DockauvHandle *h, const DockauvPolicy *pol, const DockauvSquashedActor *act,
+                         const DockauvHandle::RolloutKey &r, cudaStream_t st) {
     const size_t N = (size_t)h->n_envs, n_u = (size_t)h->params.n_u;
     const int n_steps = (int)r.n_steps, action_dtype = (int)r.action_dtype, auto_reset = (int)r.auto_reset;
     const DockauvRolloutOut &o = r.out;
     const DockauvPolicyOut &po = r.pout;
     const size_t arow = (action_dtype == DOCKAUV_ACT_F32 ? 4 : 8) * n_u * N;
-    auto actions_of_step = [&](int t) { return pol ? (const void *)h->pol_actions : (const char *)r.input + arow * t; };
+    auto slot = [&](int t) { return (int)((r.start_slot + t) % r.n_slots); };
+    auto ring_actions = [&](int t) { return (float *)r.ring.actions + n_u * N * slot(t); };
+    auto actions_of_step = [&](int t) {
+        return act ? (const void *)ring_actions(t) : pol ? (const void *)h->pol_actions : (const char *)r.input + arow * t;
+    };
     auto obs_of_step = [&](int t) { return t == 0 ? (const float *)r.input : o.obs + (size_t)h->n_obs * N * (t - 1); };
+    auto step_out = [&](int t) { return act ? ring_step_out(h, r.ring, (int)r.n_slots, slot(t)) : rollout_step_out(h, o, t); };
     auto policy = [&](int t, int64_t b, int64_t e, cudaStream_t s) {
+        if (act) return actor_range(h, *act, r.ring.obs + (size_t)h->n_obs * N * slot(t), ring_actions(t), b, e, s);
         if (!pol) return DOCKAUV_OK;
         return policy_range(h, *pol, obs_of_step(t), po.actions + n_u * N * t, po.values + N * t, po.log_probs + N * t,
                             false, b, e, s);
@@ -1137,7 +1231,7 @@ static int rollout_issue(DockauvHandle *h, const DockauvPolicy *pol, const Docka
         // the taps need one pre-step snapshot per step, so every step is forked and joined on its own (the parts of a
         // batch stepped in parts cannot run their T steps as one chain each), and the policy covers the whole batch
         for (int t = 0; t < n_steps; t++) {
-            const DockauvStepOut so = rollout_step_out(h, o, t);
+            const DockauvStepOut so = step_out(t);
             int rc = policy(t, 0, h->n_envs, st);
             if (rc == DOCKAUV_OK)
                 rc = step_call(h, actions_of_step(t), action_dtype, nullptr, &so, nullptr, auto_reset, st, false);
@@ -1149,7 +1243,7 @@ static int rollout_issue(DockauvHandle *h, const DockauvPolicy *pol, const Docka
     // chain on its own stream, forked from / joined to the caller's stream once per rollout instead of once per step
     return over_ranges(h, false, st, [&](int64_t b, int64_t e, cudaStream_t s) {
         for (int t = 0; t < n_steps; t++) {
-            const DockauvStepOut so = rollout_step_out(h, o, t);
+            const DockauvStepOut so = step_out(t);
             int rc = policy(t, b, e, s);
             if (rc == DOCKAUV_OK)
                 rc = step_range(h, actions_of_step(t), action_dtype, nullptr, &so, nullptr, auto_reset, b, e, s);
@@ -1159,12 +1253,15 @@ static int rollout_issue(DockauvHandle *h, const DockauvPolicy *pol, const Docka
     });
 }
 
-// Both rollout entry points after their own argument checks: ep_len_out zero-filled, then the launches issued directly
-// or (use_graph) replayed from the graph cached under the rollout's key, open loop in h->rg, closed loop in h->pg.
-static int rollout_run(DockauvHandle *h, const DockauvPolicy *pol, const void *input, int action_dtype, int n_steps,
-                       const DockauvRolloutOut &out, const DockauvPolicyOut *pout, int auto_reset, int use_graph,
-                       void *stream) {
-    if (check_rows(h, out.obs, out.terminal_obs) != DOCKAUV_OK) return DOCKAUV_EINVAL;
+// The rollout entry points after their own argument checks: ep_len_out zero-filled, then the launches issued directly
+// or (use_graph) replayed from the graph cached under the rollout's key, open loop in h->rg, closed loop in h->pg, ring
+// collection (act and ring set, out zero) in h->cg.
+static int rollout_run(DockauvHandle *h, const DockauvPolicy *pol, const DockauvSquashedActor *act,
+                       const DockauvReplayRing *ring, int n_slots, int start_slot, const void *input, int action_dtype,
+                       int n_steps, const DockauvRolloutOut &out, const DockauvPolicyOut *pout, int auto_reset,
+                       int use_graph, void *stream) {
+    if (check_rows(h, ring ? ring->obs : out.obs, ring ? ring->terminal_obs : out.terminal_obs) != DOCKAUV_OK)
+        return DOCKAUV_EINVAL;
     DeviceGuard guard(h->device);
     cudaStream_t st = (cudaStream_t)stream;
     // the closed loop's action buffer: allocated before any capture, its pointer is baked into every graph
@@ -1178,15 +1275,22 @@ static int rollout_run(DockauvHandle *h, const DockauvPolicy *pol, const void *i
         key.pol = *pol;
         key.pout = *pout;
     }
+    if (act) {
+        key.act = *act;
+        key.ring = *ring;
+        key.n_slots = n_slots;
+        key.start_slot = start_slot;
+    }
     key.input = input;
     key.out = out;
     key.n_steps = n_steps;
     key.action_dtype = action_dtype;
     key.auto_reset = auto_reset;
     key.seed = h->params.seed;
-    auto issue = [&](cudaStream_t s) { return rollout_issue(h, pol, key, s); };
+    auto issue = [&](cudaStream_t s) { return rollout_issue(h, pol, act, key, s); };
     if (!use_graph) return issue(st);
-    return graph_call(h, pol ? h->pg : h->rg, key, pol ? "policy rollout" : "rollout", st, issue);
+    return graph_call(h, act ? h->cg : pol ? h->pg : h->rg, key,
+                      act ? "ring collection" : pol ? "policy rollout" : "rollout", st, issue);
 }
 
 extern "C" int dockauv_rollout(DockauvHandle *h, const void *actions_dev, int action_dtype, int n_steps,
@@ -1196,7 +1300,8 @@ extern "C" int dockauv_rollout(DockauvHandle *h, const void *actions_dev, int ac
     if (!out->obs || !out->reward || !out->done) return fail(DOCKAUV_EINVAL, "obs, reward and done outputs are required");
     if (action_dtype != DOCKAUV_ACT_F32 && action_dtype != DOCKAUV_ACT_F64) return fail(DOCKAUV_EINVAL, "bad action dtype");
     if (n_steps <= 0) return fail(DOCKAUV_EINVAL, "n_steps must be positive");
-    return rollout_run(h, nullptr, actions_dev, action_dtype, n_steps, *out, nullptr, auto_reset, use_graph, stream);
+    return rollout_run(h, nullptr, nullptr, nullptr, 0, 0, actions_dev, action_dtype, n_steps, *out, nullptr, auto_reset,
+                       use_graph, stream);
 }
 
 extern "C" int dockauv_rollout_policy(DockauvHandle *h, const DockauvPolicy *pol, const float *obs0_dev, int n_steps,
@@ -1220,7 +1325,38 @@ extern "C" int dockauv_rollout_policy(DockauvHandle *h, const DockauvPolicy *pol
     if (smem > kPolicyMaxSmem)
         return fail(DOCKAUV_EINVAL, "policy weights need %zu bytes of shared memory (n_obs %d, hidden %d, n_u %d); one CTA "
                                     "holds at most %zu", smem, h->n_obs, pol->hidden, h->params.n_u, kPolicyMaxSmem);
-    return rollout_run(h, pol, obs0_dev, DOCKAUV_ACT_F32, n_steps, *out, pout, auto_reset, use_graph, stream);
+    return rollout_run(h, pol, nullptr, nullptr, 0, 0, obs0_dev, DOCKAUV_ACT_F32, n_steps, *out, pout, auto_reset,
+                       use_graph, stream);
+}
+
+extern "C" int dockauv_replay_collect(DockauvHandle *h, const DockauvSquashedActor *actor, const DockauvReplayRing *ring,
+                                      int n_slots, int start_slot, int n_steps, int auto_reset, int use_graph,
+                                      void *stream) {
+    // what needs no handle first
+    if (!actor || !ring) return fail(DOCKAUV_EINVAL, "null argument (actor and ring are required)");
+    for (int k = 0; k < 2; k++)
+        if (!actor->w[k] || !actor->b[k])
+            return fail(DOCKAUV_EINVAL, "actor latent_pi layer %d: a weight or bias pointer is null", k);
+    if (!actor->mu_w || !actor->mu_b) return fail(DOCKAUV_EINVAL, "actor mu: a weight or bias pointer is null");
+    if (!actor->log_std_w || !actor->log_std_b) return fail(DOCKAUV_EINVAL, "actor log_std: a weight or bias pointer is null");
+    if (!ring->obs || !ring->terminal_obs || !ring->actions || !ring->reward || !ring->done)
+        return fail(DOCKAUV_EINVAL, "a ring buffer is null (ring obs, terminal_obs, actions, reward, done are required)");
+    if (actor->hidden != 64 && actor->hidden != 128 && actor->hidden != 256)
+        return fail(DOCKAUV_EINVAL, "actor hidden width must be 64, 128 or 256, got %d", actor->hidden);
+    if (n_steps <= 0) return fail(DOCKAUV_EINVAL, "n_steps must be positive");
+    if (n_slots < 2 || n_slots > 64) return fail(DOCKAUV_EINVAL, "n_slots must be in 2..64, got %d", n_slots);
+    if (start_slot < 0 || start_slot >= n_slots)
+        return fail(DOCKAUV_EINVAL, "start_slot must be in 0..n_slots - 1 = %d, got %d", n_slots - 1, start_slot);
+    if (!h) return fail(DOCKAUV_EINVAL, "null handle");
+    if (!h->bound) return fail(DOCKAUV_ESTATE, "dockauv_bind must be called before dockauv_replay_collect");
+    const size_t smem = sac_actor_smem_bytes(h->n_obs, actor->hidden, h->params.n_u);
+    if (smem > kPolicyMaxSmem)
+        return fail(DOCKAUV_EINVAL, "actor weights need %zu bytes of shared memory (n_obs %d, hidden %d, n_u %d); one CTA "
+                                    "holds at most %zu", smem, h->n_obs, actor->hidden, h->params.n_u, kPolicyMaxSmem);
+    DockauvRolloutOut none;
+    memset(&none, 0, sizeof(none));
+    return rollout_run(h, nullptr, actor, ring, n_slots, start_slot, nullptr, DOCKAUV_ACT_F32, n_steps, none, nullptr,
+                       auto_reset, use_graph, stream);
 }
 
 // ------------------------------------------------------------------------------------------- episode taps: setup
@@ -1709,6 +1845,12 @@ extern "C" int dockauv_rollout_captures(DockauvHandle *h, int64_t *n) {
 extern "C" int dockauv_rollout_policy_captures(DockauvHandle *h, int64_t *n) {
     if (!h || !n) return fail(DOCKAUV_EINVAL, "null argument");
     *n = h->pg.captures;
+    return DOCKAUV_OK;
+}
+
+extern "C" int dockauv_replay_collect_captures(DockauvHandle *h, int64_t *n) {
+    if (!h || !n) return fail(DOCKAUV_EINVAL, "null argument");
+    *n = h->cg.captures;
     return DOCKAUV_OK;
 }
 

@@ -113,6 +113,22 @@ def policy_smem_bytes(n_obs, hidden, n_u):
     return 4 * (net(n_u) + net(1) + (n_u + 3) // 4 * 4)
 
 
+class DockauvSquashedActor(C.Structure):
+    _fields_ = [("w", C.c_void_p * 2), ("b", C.c_void_p * 2), ("mu_w", C.c_void_p), ("mu_b", C.c_void_p),
+                ("log_std_w", C.c_void_p), ("log_std_b", C.c_void_p), ("hidden", C.c_int32), ("deterministic", C.c_int32)]
+
+
+# dockauv_replay_collect: what the SAC actor's bf16 weights, f32 biases and the per-warp epilogue tiles of its 8 warps
+# take in shared memory (gym_dockauv_b200/csrc/dockauv_sac_actor.cuh: layer 0's columns padded to a multiple of 16,
+# every bf16 row by 8 more; the two heads one 16-row block); n_u <= 8 does not change it
+SAC_ACTOR_HIDDEN = (64, 128, 256)
+
+
+def sac_actor_smem_bytes(n_obs, hidden, n_u):
+    H, k0p = hidden, (n_obs + 15) // 16 * 16
+    return 2 * (H * (k0p + 8) + H * (H + 8) + 16 * (H + 8)) + 4 * (2 * H + 16) + 4 * 8 * 16 * 16
+
+
 def skew(a):
     """S(a) b = a x b (utils/geomutils.py:106-128)."""
     return np.array([[0.0, -a[2], a[1]], [a[2], 0.0, -a[0]], [-a[1], a[0], 0.0]])

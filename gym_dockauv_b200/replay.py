@@ -7,6 +7,8 @@ go through host arrays, so this buffer keeps everything in HBM:
 
 * ``collect`` lets the step kernels write observation, reward, done flag and terminal observation of step t straight
   into the ring slots (``env.step_into``); no observation is copied after the kernel;
+* ``collect_fused`` does the same with SAC's actor evaluated on the device (``policy.FusedSquashedActor``): the
+  actor and step launches of all steps are one library call (``dockauv_replay_collect``), replayed as a CUDA graph;
 * ``sample`` is one kernel (``dockauv_replay_sample``) that draws the minibatch and gathers its rows, next observations
   at episode ends included, into float32 tensors with the field names of SB3's ``ReplayBufferSamples``.
 
@@ -101,6 +103,30 @@ class DeviceReplayBuffer:
             env.step_into(self.actions[s], self.obs[s1], self.rewards[s], self.dones[s], terminal_obs=self.terminal_obs[s])
             self.t += 1
         return self.obs[self.t % S]
+
+    def collect_fused(self, actor, n_steps, use_graph=True):
+        """``collect`` with a ``FusedSquashedActor`` evaluated on the device before each step: ONE library call on the
+        env's current stream for all ``n_steps`` steps.  Step t's actor reads the observation of its slot and writes the
+        actions into it (float32, unclipped, unscaled, as ``collect`` stores them), and the step reads them from there.
+        With ``use_graph`` the launch sequence is captured once per (actor, start slot, ``n_steps``) and replayed: with
+        ``n_steps`` a multiple of ``n_slots`` every call replays the same graph.  Returns the observation the next step
+        acts on."""
+        env, S, T = self.env, self.n_slots, int(n_steps)
+        actor.check_env(env)
+        if T <= 0:
+            raise ValueError(f"n_steps must be positive, got {n_steps}")
+        _capi.check(self._lib.dockauv_replay_collect(env._handle, C.byref(actor.struct), C.byref(self._ring), S,
+                                                     self.t % S, T, int(env.auto_reset), int(bool(use_graph)),
+                                                     env._stream()))
+        self.t += T
+        env.t_total_steps += T
+        return self.obs[self.t % S]
+
+    def collect_captures(self):
+        """How many times ``collect_fused(use_graph=True)`` had to capture its launch sequence (replays do not)."""
+        n = C.c_int64()
+        _capi.check(self._lib.dockauv_replay_collect_captures(self.env._handle, C.byref(n)))
+        return n.value
 
     def sample(self, batch_size, return_index=False):
         """``batch_size`` transitions drawn uniformly over the valid (transition, env) pairs, as float32 device tensors

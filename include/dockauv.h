@@ -25,6 +25,8 @@
  *   dockauv_gae                        RolloutBuffer.compute_returns_and_advantage of the PPO caller
  *                                      (stable-baselines3 1.5.0, requirements.txt; selected at train.py:64)
  *   dockauv_replay_sample              ReplayBuffer.sample of the SAC caller (MODEL = SAC at train.py:64)
+ *   dockauv_replay_collect             OffPolicyAlgorithm.collect_rollouts of the SAC caller: SAC's actor picks the
+ *                                      actions on the device and the steps fill the replay ring
  *   DockauvDebugOut (state_dot, ...)   EpisodeDataStorage.update          utils/datastorage.py:268-288
  *   dockauv_set_taps                   the same, during training: every step of a few chosen envs recorded on
  *                                      the device (interval_datastorage, config.py; datastorage.py:268-288)
@@ -428,6 +430,42 @@ DOCKAUV_API int dockauv_replay_sample(const DockauvReplayRing *ring, int reward_
                                       int n_obs, int n_u, int64_t t_first, int64_t n_valid, int64_t batch,
                                       uint64_t seed, uint64_t draw, const DockauvReplaySample *out, void *stream);
 
+/* Off-policy collection on the device: stable-baselines3 1.5.0's SAC Actor (SAC's MlpPolicy, default H = 256) picks
+ * each step's actions, and the steps write straight into a replay ring.
+ *   latent_pi = Linear(n_obs, H), ReLU, Linear(H, H), ReLU;  mu = Linear(H, n_u);  log_std = Linear(H, n_u) clamped to
+ *   [-20, 2];  a = tanh(mu + exp(log_std) eps), or a = tanh(mu) with deterministic != 0 (predict(deterministic=True)).
+ * eps is the noise of dockauv_rollout_policy: Philox4x32-10 at (global id lo, global id hi, episode,
+ * 0xC0000000 | (t_steps mod 2^29) << 1 | j) with the env's counters before the step, so the actions depend on (seed,
+ * global id, episode, t) only.  H is 64, 128 or 256.  The actor runs on the tensor cores with bf16 operands: the
+ * observation, every weight matrix and each hidden activation after bias and ReLU are rounded to bf16 (round to nearest
+ * even); products are accumulated in f32; biases, the clamp, exp, the noise and tanh are f32.  The SAC update recomputes
+ * log-probabilities and Q-values from the stored (observation, action) pairs, so only the stored action, which is
+ * exactly what the step read, has to be exact.  The bf16 weights must fit one CTA's shared memory (227 KB; n_obs 36,
+ * H 256: 178 KB); DOCKAUV_EINVAL otherwise. */
+typedef struct DockauvSquashedActor {   /* caller-owned f32 device tensors, nn.Linear layout */
+    const float *w[2], *b[2];           /* latent_pi: n_obs->H, H->H, ReLU after each */
+    const float *mu_w, *mu_b;           /* H->n_u */
+    const float *log_std_w, *log_std_b; /* H->n_u, clamped to [-20, 2] */
+    int32_t hidden, deterministic;
+} DockauvSquashedActor;
+
+/* n_steps steps of SB3's OffPolicyAlgorithm.collect_rollouts in one call, writing THROUGH `ring` (its pointers are
+ * const only because dockauv_replay_sample reads them).  With S = n_slots (2..64) and s0 = start_slot (0..S-1), step t
+ * (0 <= t < n_steps):
+ *   the actor reads obs[(s0 + t) % S] and writes actions[(s0 + t) % S] (f32, unclipped and unscaled);
+ *   the step reads those actions as float32 and writes obs[(s0 + t + 1) % S], and reward, done and terminal_obs of slot
+ *   (s0 + t) % S;
+ * so the ring ends up as n_steps dockauv_step calls with the same actions would leave it.  reward is real[S][N] in the
+ * handle's precision.  The arguments that need no handle are checked first, then the bind state and the shared-memory
+ * limit, then the alignment of the ring's observation arrays.  Taps are recorded as in dockauv_rollout.
+ * Graphs (use_graph != 0): one CUDA graph per (actor pointers, hidden, deterministic, ring, S, s0, n_steps, auto_reset,
+ * seed), four cached per handle; with n_steps a multiple of S every call replays the same graph.  Weights rewritten in
+ * place (optimizer.step()) are read by the next replay.  The steps run inside this launch chain and use none of the step
+ * graphs of dockauv_step. */
+DOCKAUV_API int dockauv_replay_collect(DockauvHandle *h, const DockauvSquashedActor *actor, const DockauvReplayRing *ring,
+                                       int n_slots, int start_slot, int n_steps, int auto_reset, int use_graph,
+                                       void *stream);
+
 /* Episode statistics accumulated on the device since the last clear (DOCKAUV_STAT_*).  stats_dev points at
  * double[DOCKAUV_N_STATS] on the device: it is the send buffer of the per-rollout NCCL all-reduce.  The kernels
  * accumulate into DOCKAUV_STAT_COPIES replicas of the vector (same-address atomics of 10^4 warps per step would
@@ -454,6 +492,8 @@ DOCKAUV_API int dockauv_last_list_counts(DockauvHandle *h, int64_t *n_listed, in
 DOCKAUV_API int dockauv_rollout_captures(DockauvHandle *h, int64_t *n_captures);
 /* the same for dockauv_rollout_policy(use_graph) */
 DOCKAUV_API int dockauv_rollout_policy_captures(DockauvHandle *h, int64_t *n_captures);
+/* the same for dockauv_replay_collect(use_graph) */
+DOCKAUV_API int dockauv_replay_collect_captures(DockauvHandle *h, int64_t *n_captures);
 DOCKAUV_API int dockauv_enable_timing(DockauvHandle *h, int enabled);
 DOCKAUV_API int dockauv_last_step_ms(DockauvHandle *h, float *ms);
 /* Per-launch CUDA-event times (ms) of the most recent timed dockauv_step of a multi-launch layout, in launch order
